@@ -3,7 +3,7 @@
 evaluations per second of RANSAC essential-matrix estimation (+ cheirality vote and
 triangulation of the inliers), BASELINE.json configs[2]: 100k correspondences x 64k hypotheses.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload ...] [--dump-outputs DIR]
 
 One "step" = one complete estimate on a synthetic two-view scene (40 % outliers): device
 sampler -> eight-point fit of every hypothesis -> scoring -> selection -> inlier mask of the
@@ -99,7 +99,52 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-fp32-variant", action="store_true")
     ap.add_argument("--no-pipeline", action="store_true", help="config4: one context instead of the two-context pipeline")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="native arm: write the results of the last timed step as DIR/<name>.npy (float64; rank 0's on "
+                         "several GPUs); the inputs depend only on the arguments, so two builds compare output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the native arm")
+    return args
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(directory, arrays):
+    """Save each array as directory/<name>.npy in float64 (integers up to 2^53 stay exact).  Every value must be
+    finite: placeholders such as the NaN of an untriangulated point are left out by the caller, not written."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes + 128 for a in arrays.values())  # + the .npy header
+    if total > DUMP_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte limit")
+    bad = [k for k, a in arrays.items() if not np.isfinite(a).all()]
+    if bad:
+        raise SystemExit(f"--dump-outputs: non-finite values in {bad}")
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), a)
+
+
+def two_view_outputs(res):
+    """One estimate's results, from Engine.two_view's tuple (one GPU) or two_view_sharded's dict (several GPUs): the
+    winner, the four poses of its decomposition with their cheirality votes, the inlier list, the cheirality pass bits
+    of every inlier (bit b: passes pose b) and the points triangulated for the inliers that pass the voted pose (the
+    library returns NaN rows for the others)."""
+    if isinstance(res, tuple):
+        best, _, _, poses, num, idx, ok, X = res
+        res = dict(err=best.err, index=best.index, count=best.count_extra, E=best.E, num_invalid=best.num_invalid,
+                   poses=poses, num_inliers=num, inlier_idx=idx, pass_bits=ok, points=X)
+    p = res["poses"]
+    ok = res["pass_bits"]
+    passing = ((ok >> p.best) & 1).astype(bool) if p.best >= 0 else np.zeros(len(ok), dtype=bool)
+    return {"E": np.reshape(res["E"], (3, 3)), "best_err": res["err"], "best_index": res["index"],
+            "count_extra": res["count"], "num_invalid": res["num_invalid"], "num_inliers": res["num_inliers"],
+            "pose_R": np.reshape(p.R, (4, 3, 3)), "pose_t": np.reshape(p.t, (4, 3)), "pose_sv": p.sv,
+            "pose_counts": p.counts, "pose_best": p.best, "inlier_idx": res["inlier_idx"], "pass_bits": res["pass_bits"],
+            "points": res["points"][passing]}
 
 
 # ----------------------------------------------------------------------------------------------
@@ -588,17 +633,17 @@ def main():
     def step_resident(seed):
         if world == 1:  # one GPU: no merge step, so selection -> mask -> pose vote -> triangulation is one C call
             eng.sample_device(seed, h_rank)
-            best, _, _, poses, num, idx, ok, X = eng.two_view(THR, MIN_EXTRA, AGG, "min_error", 50.0, want_mask=False,
-                                                              want_sed=False)
+            res = eng.two_view(THR, MIN_EXTRA, AGG, "min_error", 50.0, want_mask=False, want_sed=False)
+            best, num = res[0], res[4]
             if best.index < 0:
                 raise RuntimeError("no model found")
-            return {"index": int(best.index)}, num
+            return {"index": int(best.index)}, num, res
         # several GPUs: records all-gathered device-to-device (the one collective), merged by a kernel, tail enqueued
         # behind it - the host synchronises once per estimate
         r = distributed.two_view_sharded(THR, MIN_EXTRA, AGG, h_rank, seed, engine=eng, rank=rank, world=world, native=True)
         if r["owner"] < 0:
             raise RuntimeError("no model found")
-        return r, r["num_inliers"]
+        return r, r["num_inliers"], r
 
     def step_e2e(seed):
         if world == 1:
@@ -628,7 +673,7 @@ def main():
     for s in range(args.steps):
         flush_l2()
         ev[s][0].record(stream)
-        _, num_inl = step_resident(s)
+        _, num_inl, last = step_resident(s)
         ev[s][1].record(stream)
     barrier()
     clocks.mark_end()
@@ -702,7 +747,7 @@ def main():
             for s in range(args.steps):
                 flush_l2()
                 ev3[s][0].record(stream)
-                r32, _ = step_resident(s)
+                r32, _, _ = step_resident(s)
                 ev3[s][1].record(stream)
                 t, _ = eng.get_timing()
                 sc += t.get("score", 0.0)
@@ -800,6 +845,8 @@ def main():
         if not args.no_cpu_baseline and world == 1:
             line["cpu_baseline"] = cpu_baseline_subprocess(args, args.workload)
         line.update(extras)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, two_view_outputs(last))
         emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -883,6 +930,9 @@ def bench_pairs(args, eng, world, rank, barrier, flush_l2, torch, dist):
             "clocks": clk,
             "gpu_launches": l1 - l0,
         }
+        if args.dump_outputs:
+            found = out["best_index"] >= 0  # a pair without a model has no E and an infinite error (best_index -1)
+            dump_outputs(args.dump_outputs, dict(out, E=out["E"][found], best_err=out["best_err"][found]))
         emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -956,6 +1006,8 @@ def bench_config1(args, eng, world, rank, barrier, flush_l2, torch, dist):
                                     "sample": f"the UNMODIFIED reference on this exact workload: {t['seconds']:.1f} s per estimate, "
                                               "recorded in the build container by tools/time_true_reference.py (the reference "
                                               "cannot travel to the GPU box)"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"E": e, "inlier_pairs": np.reshape([[a.x, a.y, b.x, b.y] for a, b in pairs], (-1, 4))})
         emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -972,11 +1024,11 @@ def bench_frontend(args, eng, world, rank, barrier, flush_l2, torch, dist):
     stream = torch.cuda.current_stream()
 
     def step():
-        c1, _, _ = eng.harris_corners(img1, 600, 2, 0.04)
-        c2, _, _ = eng.harris_corners(img2, 600, 2, 0.04)
+        c1, s1, _ = eng.harris_corners(img1, 600, 2, 0.04)
+        c2, s2, _ = eng.harris_corners(img2, 600, 2, 0.04)
         bb, bs, keep, _ = eng.match_brute_force(img1, img2, c1, c2, kind="ncc", window=9, ratio_test=True, crosscheck=True,
                                                 ratio_threshold=0.7)
-        return c1, c2, bb, keep
+        return c1, s1, c2, s2, bb, bs, keep
 
     clocks = ClockSampler(int(os.environ.get("LOCAL_RANK", "0")))
     clocks.start()
@@ -990,7 +1042,7 @@ def bench_frontend(args, eng, world, rank, barrier, flush_l2, torch, dist):
     for _ in range(args.steps):
         flush_l2()
         ev0.record(stream)
-        c1, c2, bb, keep = step()
+        c1, s1, c2, s2, bb, bs, keep = step()
         ev1.record(stream)
         ev1.synchronize()
         ms += ev0.elapsed_time(ev1)
@@ -1030,6 +1082,10 @@ def bench_frontend(args, eng, world, rank, barrier, flush_l2, torch, dist):
                                     "sample": f"vectorised-numpy Harris on both images ({t_h:.2f} s) + {rows} of {len(o1)} rows "
                                               f"of the per-pair NCC loop, extrapolated ({t_m:.1f} s)"}
             line["parity"] = bool(np.array_equal(o1, c1) and np.array_equal(o2, c2))
+        if args.dump_outputs:
+            kept = np.flatnonzero(keep)  # (a, b, score) of every kept match, as the matcher's list of Match
+            dump_outputs(args.dump_outputs, {"corners_a": c1, "corner_scores_a": s1, "corners_b": c2, "corner_scores_b": s2,
+                                             "matches": np.stack([kept, bb[kept], bs[kept]], 1)})
         emit(line)
     if world > 1:
         dist.destroy_process_group()

@@ -3,8 +3,8 @@
 The reference (Bazs/structure_from_motion) is pure Python.  It lives at ``/root/reference`` in the
 build container; ``baseline/install_reference.py`` pip-installs it, unmodified, into the git-ignored
 ``baseline/_ref/`` so that a copy travels to the GPU box.  This loader is used (a) by
-``tests/golden/make_golden.py`` to generate the committed golden vectors, (b) by tests (skipped when
-the reference is absent) that pin ``oracle/restatement.py`` against the real thing and (c) by
+``tests/golden/make_golden.py`` to generate the committed golden vectors, which pin
+``oracle/restatement.py`` and ``oracle/front_end.py`` against the real thing, and (b) by
 ``bench.py``'s CPU legs, which time the reference itself beside the GPU.
 
 Four shims are needed because of dependency drift (SURVEY.md §8(c)); none of them

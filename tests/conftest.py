@@ -10,7 +10,6 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a B200 (run with -m gpu on the GPU box)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
 
 
 def _have_gpu() -> bool:
@@ -24,14 +23,9 @@ def _have_gpu() -> bool:
 
 def pytest_collection_modifyitems(config, items):
     gpu = _have_gpu()
-    from oracle import reference_shims
-
-    ref = reference_shims.reference_available()
     for item in items:
         if "gpu" in item.keywords and not gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "reference" in item.keywords and not ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))
 
 
 @pytest.fixture(scope="session")

@@ -239,6 +239,7 @@ def main():
     dump("line_ransac_known_answer.json", dict(points=allp, model=list(model), inliers=np.array(inl),
                                                state_after=list(random.getstate()[1])))
     front_end_golden()
+    reference_outputs_golden()
 
 
 def synthetic_image_pair(seed, h=72, w=96):
@@ -327,10 +328,62 @@ def harris_golden():
     dump("harris_known_answer.json", out)
 
 
+def reference_outputs_golden():
+    """What tests/test_oracle.py::test_restatement_matches_live_reference and
+    tests/test_front_end_oracle.py::test_front_end_matches_live_reference compare against: the reference's
+    estimate_essential_mat_with_ransac for every aggregation, its pose and triangulation of the winner's inliers, and
+    its matcher and Harris detector on small crops of the front-end fixtures."""
+    import functools
+
+    K, x1, x2, *_ = make_scene(150, 0.3, seed=2)
+    fa = [F(x=float(p[0]), y=float(p[1])) for p in x1]
+    fb = [F(x=float(p[0]), y=float(p[1])) for p in x2]
+    ms = [M(a_index=i, b_index=i) for i in range(150)]
+    runs = []
+    for method in ("sum", "square", "mean", "rms"):
+        random.seed(9)
+        e, pairs = ref.epipolar_ransac.estimate_essential_mat_with_ransac(
+            K, fa, fb, ms, 1.5e-6, min_num_extra_inliers=4,
+            error_aggregation_method=ref.ransac.ErrorAggregationMethod(method), max_iterations=40)
+        runs.append(dict(method=method, E=e, pairs=[[a.x, a.y, b.x, b.y] for a, b in pairs],
+                         rng_state_after=list(random.getstate()[1])))
+    ia, ib = [a for a, _ in pairs], [b for _, b in pairs]
+    R, t, mask = ref.eight_point.recover_r_t_from_e(e.copy(), K, ia, ib)
+    X = ref.triangulation.triangulate_points(ia, ib, K, ref.transforms.Transform3D.from_rmat_t(R, t))
+    dump("ransac_methods_known_answer.json", dict(
+        K=K, pts_a=x1, pts_b=x2, seed=9, threshold=1.5e-6, min_extra=4, max_iterations=40, runs=runs,
+        R=R, t=t, mask=np.asarray(mask), X=X))
+
+    with open(os.path.join(OUT, "matching_known_answer.json")) as f:
+        m = json.load(f)
+    img_a, img_b = np.array(m["image_a"], dtype=np.uint8), np.array(m["image_b"], dtype=np.uint8)
+    feats_a, feats_b = np.array(m["feats_a"])[:12], np.array(m["feats_b"])[:11]
+    fa = [F(x=float(x), y=float(y)) for x, y in feats_a]
+    fb = [F(x=float(x), y=float(y)) for x, y in feats_b]
+    VS = ref.matching.ValidationStrategy
+    cases = []
+    for kind, fn, w in [("ncc", ref.ncc.calculate_ncc, 5), ("ssd", ref.ssd.calculate_ssd, 3)]:
+        score = functools.partial(fn, img_a, img_b, window_size=w)
+        matches = []
+        for strategies in [None, VS.RATIO_TEST, {VS.RATIO_TEST, VS.CROSSCHECK}]:
+            got = ref.matching.match_brute_force(fa, fb, score, validation_strategies=strategies, ratio_test_threshold=0.8)
+            names = [] if strategies is None else sorted(x.name for x in (strategies if isinstance(strategies, set) else {strategies}))
+            matches.append(dict(strategies=names, matches=[[x.a_index, x.b_index, x.match_score] for x in got]))
+        cases.append(dict(kind=kind, window=w, scores=[[score(a, b) for b in fb] for a in fa], matching=matches))
+    with open(os.path.join(OUT, "harris_known_answer.json")) as f:
+        img = np.array(json.load(f)["image"], dtype=np.uint8)[:24, :30]
+    corners = ref.harris.detect_harris_corners(img, num_corners=15)
+    dump("front_end_known_answer.json", dict(
+        num_features=[12, 11], ratio=0.8, cases=cases, harris=dict(rows=24, cols=30, num_corners=15,
+                                                                    corners=[[float(c.x), float(c.y)] for c in corners])))
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "front_end":
         front_end_golden()
     elif len(sys.argv) > 1 and sys.argv[1] == "harris":
         harris_golden()
+    elif len(sys.argv) > 1 and sys.argv[1] == "reference_outputs":
+        reference_outputs_golden()
     else:
         main()

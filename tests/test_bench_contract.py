@@ -42,3 +42,38 @@ def test_native_arm_line():
     assert d["gpu_launches"] >= 2 * 6 and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["kind"] == "port"
     assert {"sm_mhz", "sm_max_mhz", "reasons"} <= set(d["clocks"])
     assert "workload" in d["config"] and "config3" in d["config"]["workload"]
+
+
+def test_argument_errors():
+    for flags in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *flags], capture_output=True, text=True,
+                             timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and not out.stdout and "error" in out.stderr, flags
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_last_timed_step(engine, tmp_path):
+    """--dump-outputs writes the results of the last timed step: config 2's scene with the device sampler seeded by
+    the step index, so with --steps 3 the estimate of seed 2."""
+    import numpy as np
+
+    from structure_from_motion_b200.scenes import make_scene
+
+    d = _run("--workload", "config2", "--steps", "3", "--warmup", "1", "--no-cpu-baseline", "--no-e2e",
+             "--no-fp32-variant", "--dump-outputs", str(tmp_path / "out"))
+    assert d["steps"] == 3
+    got = {p.stem: np.load(p) for p in (tmp_path / "out").glob("*.npy")}
+    assert all(a.dtype == np.float64 and np.isfinite(a).all() for a in got.values())
+    assert sum(p.stat().st_size for p in (tmp_path / "out").iterdir()) <= 64 * 10 ** 6
+    K, x1, x2, *_ = make_scene(10_000, 0.4, seed=0)
+    engine.upload_pairs(x1, x2, K)
+    engine.sample_device(2, 16_384)
+    best, _, _, poses, num, idx, ok, X = engine.two_view(1.5e-6, 10, "rms", "min_error", 50.0, want_mask=False,
+                                                         want_sed=False)
+    assert got["best_index"] == best.index and got["best_err"] == best.err and got["count_extra"] == best.count_extra
+    assert np.array_equal(got["E"].reshape(9), np.array(best.E)) and got["num_inliers"] == num
+    assert np.array_equal(got["inlier_idx"], idx) and np.array_equal(got["pass_bits"], ok)
+    passing = ((ok >> poses.best) & 1).astype(bool)  # the library's rows for the other inliers are NaN
+    assert passing.any() and np.isnan(X[~passing]).all() and np.array_equal(got["points"], X[passing])
+    assert got["pose_best"] == poses.best and got["pose_counts"].tolist() == list(poses.counts)
+    assert np.array_equal(got["pose_R"].reshape(4, 9), np.array(poses.R))

@@ -1,7 +1,5 @@
 """The front-end oracle (oracle/front_end.py: brute-force matcher, NCC/SSD, Harris, cross-correlation) pinned
-against golden vectors generated from the unmodified reference (tests/golden/make_golden.py) and — in the build
-container only — live against /root/reference.  No GPU needed."""
-import functools
+against golden vectors generated from the unmodified reference (tests/golden/make_golden.py).  No GPU needed."""
 import json
 import os
 
@@ -134,29 +132,21 @@ def test_cross_correlate_matches_reference(harris_golden):
         fe.cross_correlate(img[:2, :2], np.ones((3, 3)))
 
 
-@pytest.mark.reference
 def test_front_end_matches_live_reference(matching_golden, harris_golden):
-    from oracle import reference_shims
-
-    ref = reference_shims.load()
+    """Score matrices, matches and Harris corners on crops of the fixtures against what the unmodified reference
+    returned for them (front_end_known_answer.json, tests/golden/make_golden.py)."""
     d = matching_golden
-    F = ref.feature.Feature
-    fa = [F(x=float(x), y=float(y)) for x, y in d["feats_a"][:12]]
-    fb = [F(x=float(x), y=float(y)) for x, y in d["feats_b"][:11]]
-    VS = ref.matching.ValidationStrategy
-    for kind, fn, w in [("ncc", ref.ncc.calculate_ncc, 5), ("ssd", ref.ssd.calculate_ssd, 3)]:
-        score = functools.partial(fn, d["image_a"], d["image_b"], window_size=w)
-        S = fe.score_matrix(d["image_a"], d["image_b"], d["feats_a"][:12], d["feats_b"][:11], kind, w)
-        assert np.array_equal(S, np.array([[score(a, b) for b in fb] for a in fa]))
-        for strategies in [None, VS.RATIO_TEST, {VS.RATIO_TEST, VS.CROSSCHECK}]:
-            m = ref.matching.match_brute_force(fa, fb, score, validation_strategies=strategies, ratio_test_threshold=0.8)
-            s = set() if strategies is None else (strategies if isinstance(strategies, set) else {strategies})
-            got = fe.match_from_scores(S, VS.RATIO_TEST in s, VS.CROSSCHECK in s, 0.8)
-            assert [(x.a_index, x.b_index, x.match_score) for x in m] == got
-    img = harris_golden["image"][:24, :30]
-    corners = ref.harris.detect_harris_corners(img, num_corners=15)
-    xy, _, _ = fe.harris_corners(img, 15)
-    assert sorted((float(c.x), float(c.y)) for c in corners) == sorted(map(tuple, xy))
+    g = load("front_end_known_answer.json")
+    na, nb = g["num_features"]
+    for case in g["cases"]:
+        S = fe.score_matrix(d["image_a"], d["image_b"], d["feats_a"][:na], d["feats_b"][:nb], case["kind"], case["window"])
+        assert np.array_equal(S, np.array(case["scores"]))
+        for m in case["matching"]:
+            got = fe.match_from_scores(S, "RATIO_TEST" in m["strategies"], "CROSSCHECK" in m["strategies"], g["ratio"])
+            assert [[a, b, s] for a, b, s in got] == m["matches"], (case["kind"], m["strategies"])
+    h = g["harris"]
+    xy, _, _ = fe.harris_corners(harris_golden["image"][:h["rows"], :h["cols"]], h["num_corners"])
+    assert sorted(map(tuple, h["corners"])) == sorted(map(tuple, xy))
 
 
 # ---- property-based checks (the reference's own suite uses hypothesis for its geometry tests) ----

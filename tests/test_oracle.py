@@ -1,6 +1,5 @@
 """The oracle pinned: oracle/restatement.py and oracle/sed_exact.c against the golden vectors
-generated from the unmodified reference (tests/golden/make_golden.py), and — in the build
-container only — live against /root/reference."""
+generated from the unmodified reference (tests/golden/make_golden.py)."""
 import json
 import os
 import random
@@ -128,33 +127,22 @@ def test_c_scorer_batch_matches_restatement():
         np.testing.assert_allclose(s2[h], (sed[samp | extra] ** 2).sum(), rtol=1e-13)
 
 
-@pytest.mark.reference
 def test_restatement_matches_live_reference():
-    """Build container only: the unmodified reference, run here, against the restatement."""
-    from oracle import reference_shims
-
-    ref = reference_shims.load()
-    F, M = ref.feature.Feature, ref.matching.Match
-    K, x1, x2, *_ = make_scene(150, 0.3, seed=2)
-    fa = [F(x=float(p[0]), y=float(p[1])) for p in x1]
-    fb = [F(x=float(p[0]), y=float(p[1])) for p in x2]
-    ms = [M(a_index=i, b_index=i) for i in range(150)]
-    for method in ("sum", "square", "mean", "rms"):
-        random.seed(9)
-        e, pairs = ref.epipolar_ransac.estimate_essential_mat_with_ransac(
-            K, fa, fb, ms, 1.5e-6, min_num_extra_inliers=4,
-            error_aggregation_method=ref.ransac.ErrorAggregationMethod(method), max_iterations=40)
-        st = random.getstate()
-        random.seed(9)
-        r = o.ransac_essential(K, x1[:, 0], x1[:, 1], x2[:, 0], x2[:, 1], 1.5e-6, 4, method, 40, exact_sed=True)
-        assert random.getstate() == st
-        assert np.array_equal(e, r["E"])
-        assert [(p[0].x, p[1].x) for p in pairs] == [(x1[i, 0], x2[i, 0]) for i in r["inlier_indices"]]
-    inl = r["inlier_indices"]
-    R, t, mask = ref.eight_point.recover_r_t_from_e(e.copy(), K, [fa[i] for i in inl], [fb[i] for i in inl])
-    R2, t2, mask2, _ = o.recover_r_t_from_e(e.copy(), K, x1[inl, 0], x1[inl, 1], x2[inl, 0], x2[inl, 1])
-    assert np.array_equal(R, R2) and np.array_equal(t, t2) and np.array_equal(mask, mask2)
-    X = ref.triangulation.triangulate_points([fa[i] for i in inl], [fb[i] for i in inl], K,
-                                             ref.transforms.Transform3D.from_rmat_t(R, t))
-    X2 = o.triangulate_points(x1[inl, 0], x1[inl, 1], x2[inl, 0], x2[inl, 1], K, o.tmat(R, t))
-    assert np.array_equal(X, X2)
+    """The restatement against what the unmodified reference returned on the same 150 correspondences
+    (tests/golden/make_golden.py): E, the inlier pairs in order and the global RNG state after the run for every
+    aggregation, then the pose vote and triangulation of the last winner's inliers, all bit for bit."""
+    d = load("ransac_methods_known_answer.json")
+    K, x1, x2 = np.array(d["K"]), np.array(d["pts_a"]), np.array(d["pts_b"])
+    for run in d["runs"]:
+        random.seed(d["seed"])
+        r = o.ransac_essential(K, x1[:, 0], x1[:, 1], x2[:, 0], x2[:, 1], d["threshold"], d["min_extra"], run["method"],
+                               d["max_iterations"], exact_sed=True)
+        assert list(random.getstate()[1]) == run["rng_state_after"]
+        assert np.array_equal(r["E"], np.array(run["E"]))
+        inl = r["inlier_indices"]
+        assert np.concatenate([x1[inl], x2[inl]], 1).tolist() == run["pairs"]
+    R, t, mask, _ = o.recover_r_t_from_e(r["E"].copy(), K, x1[inl, 0], x1[inl, 1], x2[inl, 0], x2[inl, 1])
+    assert np.array_equal(R, np.array(d["R"])) and np.array_equal(t, np.array(d["t"]))
+    assert np.array_equal(mask, np.array(d["mask"]))
+    X = o.triangulate_points(x1[inl, 0], x1[inl, 1], x2[inl, 0], x2[inl, 1], K, o.tmat(R, t))
+    assert np.array_equal(X, np.array(d["X"]))
