@@ -175,6 +175,27 @@ int sfm_inlier_mask(sfm_ctx *ctx, double threshold, uint8_t *mask, double *sed);
 int sfm_ransac_essential(sfm_ctx *ctx, double threshold, double min_extra, int aggregation,
                          int selection, sfm_best *best, uint8_t *mask, double *sed);
 
+/* ---- homography (planar scenes, rotation-only pairs) ----------------------------------
+ * H (row-major, H[8] == 1) maps image-A pixels to image-B pixels.  Upload the correspondences with K = I (pixel
+ * coordinates), then a sample table or the device sampler: each row's columns 0-3 are the minimal sample.  The error
+ * is the symmetric transfer error in px^2 (|x_b - pi(H x_a)|^2 + |x_a - pi(adj(H) x_b)|^2); a correspondence is an
+ * inlier iff the division-free test F Q + G P <= thr P Q holds with p2 != 0 and q2 != 0 (csrc/sfm_homography.cuh
+ * pins the evaluation order).  A sample with three collinear points in either image, or an H[2,2] that is 0 or not
+ * finite, is invalid: it is never a candidate and is counted in sfm_best.num_invalid / first_invalid. */
+/* The exact 4-point solve for every row of the current table or device draw.  H_out: double[h][9] (zeros for an
+ * invalid sample) or NULL; valid_out: uint8[h] or NULL. */
+int sfm_fit_homography(sfm_ctx *ctx, double *H_out, uint8_t *valid_out);
+/* RANSAC homography in one call: fit -> score -> select (fit_with_ransac with 4-point samples: samples never counted,
+ * always in the error; the aggregation and selection rules of sfm_score) -> mask of the winner.  Needs n >= 8
+ * correspondences (the sampler draws 8 distinct indices per row).  best->E carries H, best->sample[4..7] = -1.
+ * Optional (NULL = not wanted): mask uint8[n] / err double[n] = decision / transfer error under the winner;
+ * count_extra_h int32[h] (-1 = invalid), err_h double[h] (+inf = not a candidate).  sfm_near_ties works afterwards. */
+int sfm_ransac_homography(sfm_ctx *ctx, double threshold, double min_extra, int aggregation, int selection,
+                          sfm_best *best, uint8_t *mask, double *err, int32_t *count_extra_h, double *err_h);
+/* Decision and transfer error of every correspondence under H (double[9], row-major), or under the winner of the
+ * last sfm_ransac_homography when H is NULL.  mask uint8[n], err double[n]; either may be NULL. */
+int sfm_homography_mask(sfm_ctx *ctx, const double *H, double threshold, uint8_t *mask, double *err);
+
 /* ---- pose + triangulation ------------------------------------------------------------ */
 typedef struct sfm_poses {
     double R[4][9];      /* (R1,t) (R1,-t) (R2,t) (R2,-t)  — eight_point.py:210-212 order */

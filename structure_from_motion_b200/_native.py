@@ -71,6 +71,9 @@ _SIGNATURES = {
     "sfm_get_rescored": (C.c_int, [_P, C.POINTER(C.c_int64)]),
     "sfm_inlier_mask": (C.c_int, [_P, C.c_double, _P, _P]),
     "sfm_ransac_essential": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.POINTER(Best), _P, _P]),
+    "sfm_fit_homography": (C.c_int, [_P, _P, _P]),
+    "sfm_ransac_homography": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.POINTER(Best), _P, _P, _P, _P]),
+    "sfm_homography_mask": (C.c_int, [_P, _P, C.c_double, _P, _P]),
     "sfm_decompose_essential": (C.c_int, [_P, _P, C.POINTER(Poses)]),
     "sfm_recover_pose": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_int64, C.c_int64, C.c_double, C.POINTER(Poses), _P]),
     "sfm_recover_pose_pixels": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int64, C.c_int64, C.c_double,
@@ -349,6 +352,38 @@ class Engine:
                                                SELECT[selection], C.byref(b), _ptr(mask), _ptr(sed)),
                  "sfm_ransac_essential")
         return b, mask, sed
+
+    # -- homography --------------------------------------------------------------------------
+    def fit_homography(self):
+        """The 4-point solve for every row of the current table / device draw -> (H [h,3,3], valid bool[h])."""
+        h = self.h_count
+        H = np.empty((h, 3, 3), dtype=np.float64)
+        valid = np.empty(h, dtype=np.uint8)
+        self._ck(self.lib.sfm_fit_homography(self.h, _ptr(H), _ptr(valid)), "sfm_fit_homography")
+        return H, valid.astype(bool)
+
+    def ransac_homography(self, threshold, min_extra=0.0, aggregation="rms", selection="min_error",
+                          want_mask=True, want_arrays=False):
+        """fit -> score -> select -> mask in one call.  Returns (best, mask uint8[n], err[n], count_extra[h], err[h]);
+        the per-hypothesis arrays are None unless want_arrays."""
+        b = Best()
+        mask = np.empty(self.n, dtype=np.uint8) if want_mask else None
+        err = np.empty(self.n, dtype=np.float64) if want_mask else None
+        cnt = np.empty(self.h_count, dtype=np.int32) if want_arrays else None
+        err_h = np.empty(self.h_count, dtype=np.float64) if want_arrays else None
+        self._ck(self.lib.sfm_ransac_homography(self.h, float(threshold), float(min_extra), AGG[aggregation],
+                                                SELECT[selection], C.byref(b), _ptr(mask), _ptr(err), _ptr(cnt),
+                                                _ptr(err_h)), "sfm_ransac_homography")
+        return b, mask, err, cnt, err_h
+
+    def homography_mask(self, H, threshold):
+        """(decision bool[n], transfer error [n]) under H (3x3), or under the last estimate's winner when H is None."""
+        Ha = None if H is None else _f64(H).reshape(9)
+        mask = np.empty(self.n, dtype=np.uint8)
+        err = np.empty(self.n, dtype=np.float64)
+        self._ck(self.lib.sfm_homography_mask(self.h, _ptr(Ha), float(threshold), _ptr(mask), _ptr(err)),
+                 "sfm_homography_mask")
+        return mask.astype(bool), err
 
     # -- pose / triangulation ---------------------------------------------------------------
     def decompose_essential(self, E):

@@ -16,6 +16,7 @@
 #include "sfm_fit.cuh"
 #include "sfm_linalg.cuh"
 #include "sfm_score.cuh"
+#include "sfm_homography.cuh"
 #include "sfm_pose.cuh"
 #include "sfm_tail.cuh"
 #include "sfm_misc.cuh"
@@ -101,6 +102,8 @@ struct sfm_ctx {
     long long first_len = 0;  // batched: correspondences of the first pair (what the AUTO pilot samples)
     long long raw_stride = 1;
     bool batched = false, has_pts = false, has_table = false, has_models = false, has_score = false;
+    bool models_h = false;       // the current models are homographies (sfm_fit_homography), not essential matrices
+    int hscore_occ = 0;          // resident blocks per SM of k_score_homography (queried once)
     bool table_pending = false;  // sfm_sample_device was called: the table is drawn by the fit kernel (or on demand)
     unsigned long long smp_seed = 0, smp_stream = 0;
     long long smp_offset = 0;
@@ -565,6 +568,7 @@ static int fit_launch(sfm_ctx* c, bool want_eig) {
     if (int r = check_launch(c, "k_fit")) return r;
     c->toc(T_FIT);
     c->has_models = true;
+    c->models_h = false;
     c->has_score = false;
     return 0;
 }
@@ -607,18 +611,71 @@ int sfm_set_models(sfm_ctx* c, const double* E, const uint8_t* valid, int64_t h)
     CU(cudaStreamSynchronize(c->stream));
     c->h = h;
     c->has_models = true;
+    c->models_h = false;
     c->has_score = false;
     c->acc_clean = false;
     return 0;
 }
 
 // ---- score + select ---------------------------------------------------------------------
+// K3 of a scoring call (essential matrices or homographies): finalise, rescore, select into the selection record
+static int finalise_launch(sfm_ctx* c, int kind, double thr, double min_extra, int agg, int mode, bool use_table,
+                           long long idx_offset, int sums, int e2, int force_rescore, unsigned long long* acc_dev) {
+    const long long h = c->h, P = c->npairs;
+    const size_t H = (size_t)h * P;
+    const int fblocks = (int)((h + 255) / 256);
+    c->tic(T_SELECT);
+    FinalArgs f;
+    f.pts = c->pts.as<Corr>();
+    f.offsets = c->batched ? c->offsets.as<long long>() : nullptr;
+    f.E = c->E.as<double>();
+    f.valid = c->valid.as<uint8_t>();
+    f.table = use_table ? c->table.as<int32_t>() : nullptr;
+    f.h = h;
+    f.n = c->n;
+    f.idx_offset = idx_offset;
+    f.htotal = (long long)H;
+    f.acc = acc_dev;
+    f.inv_scale1 = ldexp(1.0, e2 - kFixedBits);
+    f.sums = sums;
+    f.inv_scale2 = ldexp(1.0, 2 * e2 - kFixedBits);
+    f.thr = thr;
+    f.min_extra = min_extra;
+    f.agg = agg;
+    f.mode = mode;
+    f.count_extra = c->count_extra.as<int32_t>();
+    f.S1 = c->S1.as<double>();
+    f.S2 = c->S2.as<double>();
+    f.err = c->err.as<double>();
+    f.block_out = c->blocks.as<Best>();
+    if (int r = c->blockinv.reserve((size_t)fblocks * P * 16)) return r;
+    f.block_inv = c->blockinv.as<long long>();
+    if (int r = c->record.reserve((size_t)P * sizeof(SelectRecord))) return r;
+    f.force_rescore = force_rescore;
+    f.rescored = reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(acc_dev + H * kAccWords) + 8);
+    f.tickets = reinterpret_cast<unsigned*>(reinterpret_cast<char*>(acc_dev + H * kAccWords) + 64);
+    c->rescored_dev = f.rescored;
+    f.out = c->best.as<Best>();
+    f.invalid_out = c->invalid.as<long long>();
+    f.record = c->record.as<SelectRecord>();
+    f.fitflag = c->fitflag.as<unsigned>();
+    if (kind == MODEL_H) CU(chain_launch(c, k_finalise<MODEL_H>, dim3((unsigned)fblocks, (unsigned)P), dim3(256), 0, f));
+    else CU(chain_launch(c, k_finalise<MODEL_E>, dim3((unsigned)fblocks, (unsigned)P), dim3(256), 0, f));
+    if (int r = check_launch(c, "k_finalise")) return r;
+    c->toc(T_SELECT);
+    c->has_score = true;
+    c->last_idx_offset = idx_offset;
+    c->winner_set = false;
+    return 0;
+}
+
 static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int mode, bool use_table,
                         long long idx_offset, long long max_len, bool both_sums = false) {
     // K2 accumulates only the sum the aggregation needs (ransac.py:96-108) unless the caller wants both
     int sums = both_sums ? (SUM_S1 | SUM_S2) : ((agg == AGG_SUM || agg == AGG_MEAN) ? SUM_S1 : SUM_S2);
     if (mode == SELECT_MSAC) sums |= SUM_S1;  // the MSAC cost is built from the sum of the inlier distances
     if (!c->has_pts || !c->has_models) return fail(SFM_ERR_STATE, "score needs correspondences and fitted models");
+    if (c->models_h) return fail(SFM_ERR_STATE, "the models are homographies: score them with sfm_ransac_homography");
     if (use_table && !c->has_table) return fail(SFM_ERR_STATE, "sample rule requested but no table is loaded");
     if (use_table)
         if (int r = ensure_table(c)) return r;
@@ -801,48 +858,7 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
         c->toc(T_SCORE);
     }
 
-    c->tic(T_SELECT);
-    FinalArgs f;
-    f.pts = c->pts.as<Corr>();
-    f.offsets = c->batched ? c->offsets.as<long long>() : nullptr;
-    f.E = c->E.as<double>();
-    f.valid = c->valid.as<uint8_t>();
-    f.table = use_table ? c->table.as<int32_t>() : nullptr;
-    f.h = h;
-    f.n = c->n;
-    f.idx_offset = idx_offset;
-    f.htotal = (long long)H;
-    f.acc = acc_dev;
-    f.inv_scale1 = ldexp(1.0, e2 - kFixedBits);
-    f.sums = sums;
-    f.inv_scale2 = ldexp(1.0, 2 * e2 - kFixedBits);
-    f.thr = thr;
-    f.min_extra = min_extra;
-    f.agg = agg;
-    f.mode = mode;
-    f.count_extra = c->count_extra.as<int32_t>();
-    f.S1 = c->S1.as<double>();
-    f.S2 = c->S2.as<double>();
-    f.err = c->err.as<double>();
-    f.block_out = c->blocks.as<Best>();
-    if (int r = c->blockinv.reserve((size_t)fblocks * P * 16)) return r;
-    f.block_inv = c->blockinv.as<long long>();
-    if (int r = c->record.reserve((size_t)P * sizeof(SelectRecord))) return r;
-    f.force_rescore = force_rescore;
-    f.rescored = reinterpret_cast<unsigned long long*>(reinterpret_cast<char*>(acc_dev + H * kAccWords) + 8);
-    f.tickets = reinterpret_cast<unsigned*>(reinterpret_cast<char*>(acc_dev + H * kAccWords) + 64);
-    c->rescored_dev = f.rescored;
-    f.out = c->best.as<Best>();
-    f.invalid_out = c->invalid.as<long long>();
-    f.record = c->record.as<SelectRecord>();
-    f.fitflag = c->fitflag.as<unsigned>();
-    CU(chain_launch(c, k_finalise, dim3((unsigned)fblocks, (unsigned)P), dim3(256), 0, f));
-    if (int r = check_launch(c, "k_finalise")) return r;
-    c->toc(T_SELECT);
-    c->has_score = true;
-    c->last_idx_offset = idx_offset;
-    c->winner_set = false;
-    return 0;
+    return finalise_launch(c, MODEL_E, thr, min_extra, agg, mode, use_table, idx_offset, sums, e2, force_rescore, acc_dev);
 }
 
 int sfm_score(sfm_ctx* c, double thr, double min_extra, int agg, int mode, int use_table, int64_t idx_offset,
@@ -963,6 +979,7 @@ int sfm_inlier_mask(sfm_ctx* c, double thr, uint8_t* mask, double* sed) {
     if (int r = use(c)) return r;
     if (!c->has_pts || c->batched) return fail(SFM_ERR_STATE, "no single-pair correspondences loaded");
     if (!c->winner_set) return fail(SFM_ERR_STATE, "no winner: call sfm_get_best or sfm_set_winner first");
+    if (c->models_h && c->winner_local >= 0) return fail(SFM_ERR_STATE, "the winner is a homography: use sfm_homography_mask");
     if (int r = mask_launch(c, thr, nullptr)) return r;
     if (mask) CU(cudaMemcpyAsync(mask, c->mask.p, (size_t)c->n, cudaMemcpyDeviceToHost, c->stream));
     if (sed) CU(cudaMemcpyAsync(sed, c->sed.p, (size_t)c->n * 8, cudaMemcpyDeviceToHost, c->stream));
@@ -983,6 +1000,162 @@ int sfm_ransac_essential(sfm_ctx* c, double thr, double min_extra, int agg, int 
         if (sed) CU(cudaMemcpyAsync(sed, c->sed.p, (size_t)c->n * 8, cudaMemcpyDeviceToHost, c->stream));
     }
     return fetch_best(c, best);
+}
+
+// ---- homography (sfm_homography.cuh) -------------------------------------------------------
+static int fit_h_launch(sfm_ctx* c) {
+    if (!c->has_pts || !c->has_table) return fail(SFM_ERR_STATE, "fit needs correspondences and a sample table");
+    if (c->batched) return fail(SFM_ERR_STATE, "homography estimation is a single-pair call");
+    const long long h = c->h;
+    if (int r = c->E.reserve((size_t)h * 72)) return r;
+    if (int r = c->valid.reserve((size_t)h)) return r;
+    const size_t acc_tail = 64 + 4;  // work counter | rescore counter | K3 ticket, cleared with the planes
+    if (int r = c->acc.reserve((size_t)h * kAccWords * 8 + acc_tail)) return r;
+    c->tic(T_FIT);
+    CU(chain_launch(c, k_fit_homography, dim3((unsigned)((h + kFitHThreads - 1) / kFitHThreads)), dim3(kFitHThreads), 0,
+                    c->pts.as<Corr>(), c->table.as<int32_t>(), h, c->E.as<double>(), c->valid.as<uint8_t>(),
+                    c->acc.as<unsigned long long>(), kAccWords, (int)((acc_tail + 7) / 8), c->table_pending ? 1 : 0,
+                    c->smp_seed, c->smp_stream, c->smp_offset, c->n));
+    if (int r = check_launch(c, "k_fit_homography")) return r;
+    c->toc(T_FIT);
+    c->table_pending = false;
+    c->acc_clean = true;
+    c->acc_planes_for = (size_t)h;
+    c->has_models = true;
+    c->models_h = true;
+    c->has_score = false;
+    return 0;
+}
+
+static int score_h_launch(sfm_ctx* c, double thr, double min_extra, int agg, int mode) {
+    if (agg < 0 || agg > 3) return fail(SFM_ERR_ARG, "bad aggregation %d", agg);
+    if (mode < 0 || mode > 2) return fail(SFM_ERR_ARG, "bad selection %d", mode);
+    int sums = (agg == AGG_SUM || agg == AGG_MEAN) ? SUM_S1 : SUM_S2;
+    if (mode == SELECT_MSAC) sums |= SUM_S1;
+    // the same threshold ranges as the E path: below 0, NaN and above 1e100 the scorer is skipped and K3 rescores
+    const bool skip_k2 = !(thr >= 0.0) || thr > 1e100;
+    const int force_rescore = (thr > 1e100) ? 1 : 0;
+    const long long h = c->h, n = c->n;
+    // an inlier's value F/P + G/Q can exceed thr by a few ulps (the decision is division-free): the fixed-point scale
+    // leaves room for that, value < thr (1 + 2^-20) < 2^e2
+    int e2 = 0;
+    if (thr > 0.0 && !skip_k2) (void)frexp(thr * (1.0 + 0x1p-20), &e2);
+    if (e2 < -400) e2 = -400;
+    if (int r = c->count_extra.reserve((size_t)h * 4)) return r;
+    if (int r = c->S1.reserve((size_t)h * 8)) return r;
+    if (int r = c->S2.reserve((size_t)h * 8)) return r;
+    if (int r = c->err.reserve((size_t)h * 8)) return r;
+    const int fblocks = (int)((h + 255) / 256);
+    if (int r = c->blocks.reserve((size_t)fblocks * sizeof(Best))) return r;
+    if (int r = c->best.reserve(sizeof(Best))) return r;
+    if (int r = c->invalid.reserve(16)) return r;
+    const size_t acc_tail = 64 + 4;
+    if (int r = c->acc.reserve((size_t)h * kAccWords * 8 + acc_tail)) return r;
+    unsigned long long* acc = c->acc.as<unsigned long long>();
+    const size_t smem = kHScoreWarps * sizeof(HScoreWarpSmem);
+    if (!c->hscore_occ) {
+        int o = 0;
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, k_score_homography<kHScoreHpt>, kHScoreThreads, smem));
+        c->hscore_occ = o > 0 ? o : 1;
+    }
+    // persistent warps over (correspondence split, group of 32 * HPT hypotheses) items; an item holds at most
+    // kMaxItemPoints correspondences so that a lane's 32-bit chunk words cannot overflow
+    const long long grid_blocks = (long long)c->sm_count * c->hscore_occ;
+    const long long hblocks = (h + 32ll * kHScoreHpt - 1) / (32ll * kHScoreHpt);
+    const long long tiles = (n + kHTile - 1) / kHTile;
+    long long nsplit = (grid_blocks * kHScoreWarps * 32 + hblocks - 1) / hblocks;
+    const long long max_split = tiles / 2 > 0 ? tiles / 2 : 1;
+    if (nsplit > max_split) nsplit = max_split;
+    const long long min_split = (n + kMaxItemPoints - 1) / kMaxItemPoints;
+    if (nsplit < min_split) nsplit = min_split;
+    const long long chunk = ((tiles + nsplit - 1) / nsplit) * kHTile;
+    nsplit = (n + chunk - 1) / chunk;
+    HScoreArgs a;
+    a.pts = c->pts.as<Corr>();
+    a.H = c->E.as<double>();
+    a.n = n;
+    a.h = h;
+    a.thr = thr;
+    a.scale1 = ldexp(1.0, 63 - e2);
+    a.scale2 = ldexp(1.0, 63 - 2 * e2);
+    a.sums = sums;
+    a.chunk = chunk;
+    a.hblocks = (int)hblocks;
+    a.nsplit = (int)nsplit;
+    a.total_items = hblocks * nsplit;
+    a.work_counter = reinterpret_cast<unsigned*>(acc + (size_t)h * kAccWords);
+    a.acc = acc;
+    c->tic(T_SCORE);
+    // the fit kernel leaves the accumulators cleared; a second score of the same models clears here
+    if (!(c->acc_clean && c->acc_planes_for == (size_t)h))
+        CU(cudaMemsetAsync(c->acc.p, 0, (size_t)h * kAccWords * 8 + acc_tail, c->stream));
+    c->acc_clean = false;
+    if (!skip_k2) {
+        const long long want = (a.total_items + kHScoreWarps - 1) / kHScoreWarps;
+        CU(chain_launch(c, k_score_homography<kHScoreHpt>, dim3((unsigned)(grid_blocks < want ? grid_blocks : want)),
+                        dim3(kHScoreThreads), smem, a));
+        if (int r = check_launch(c, "k_score_homography")) return r;
+    }
+    c->toc(T_SCORE);
+    return finalise_launch(c, MODEL_H, thr, min_extra, agg, mode, true, 0, sums, e2, force_rescore, acc);
+}
+
+static int hmask_launch(sfm_ctx* c, double thr, const double* H_dev, const Best* best_dev) {
+    if (int r = c->mask.reserve((size_t)c->n)) return r;
+    if (int r = c->sed.reserve((size_t)c->n * 8)) return r;
+    c->tic(T_MASK);
+    CU(chain_launch(c, k_homography_mask, dim3((unsigned)((c->n + 255) / 256)), dim3(256), 0, c->pts.as<Corr>(), c->n,
+                    H_dev, best_dev, thr, c->mask.as<uint8_t>(), c->sed.as<double>()));
+    if (int r = check_launch(c, "k_homography_mask")) return r;
+    c->toc(T_MASK);
+    return 0;
+}
+
+int sfm_fit_homography(sfm_ctx* c, double* H_out, uint8_t* valid_out) {
+    if (int r = use(c)) return r;
+    if (int r = fit_h_launch(c)) return r;
+    if (H_out) CU(cudaMemcpyAsync(H_out, c->E.p, (size_t)c->h * 72, cudaMemcpyDeviceToHost, c->stream));
+    if (valid_out) CU(cudaMemcpyAsync(valid_out, c->valid.p, (size_t)c->h, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int sfm_ransac_homography(sfm_ctx* c, double thr, double min_extra, int agg, int mode, sfm_best* best, uint8_t* mask,
+                          double* err, int32_t* count_extra_h, double* err_h) {
+    if (int r = use(c)) return r;
+    if (!best) return fail(SFM_ERR_ARG, "best is null");
+    if (c->batched) return fail(SFM_ERR_STATE, "single-pair call on a batched context");
+    if (c->has_pts && c->n < 8) return fail(SFM_ERR_ARG, "need at least 8 correspondences, got %lld", c->n);
+    if (int r = fit_h_launch(c)) return r;
+    if (int r = score_h_launch(c, thr, min_extra, agg, mode)) return r;
+    if (mask || err) {
+        if (int r = hmask_launch(c, thr, c->E.as<double>(), c->best.as<Best>())) return r;
+        if (mask) CU(cudaMemcpyAsync(mask, c->mask.p, (size_t)c->n, cudaMemcpyDeviceToHost, c->stream));
+        if (err) CU(cudaMemcpyAsync(err, c->sed.p, (size_t)c->n * 8, cudaMemcpyDeviceToHost, c->stream));
+    }
+    if (count_extra_h) CU(cudaMemcpyAsync(count_extra_h, c->count_extra.p, (size_t)c->h * 4, cudaMemcpyDeviceToHost, c->stream));
+    if (err_h) CU(cudaMemcpyAsync(err_h, c->err.p, (size_t)c->h * 8, cudaMemcpyDeviceToHost, c->stream));
+    return fetch_best(c, best);
+}
+
+int sfm_homography_mask(sfm_ctx* c, const double* H, double thr, uint8_t* mask, double* err) {
+    if (int r = use(c)) return r;
+    if (!c->has_pts || c->batched) return fail(SFM_ERR_STATE, "no single-pair correspondences loaded");
+    const double* H_dev;
+    if (H) {
+        if (int r = c->winnerE.reserve(72)) return r;
+        CU(cudaMemcpyAsync(c->winnerE.p, H, 72, cudaMemcpyHostToDevice, c->stream));
+        H_dev = c->winnerE.as<double>();
+    } else {
+        if (!c->models_h || !c->winner_set || c->winner_local < 0)
+            return fail(SFM_ERR_STATE, "no homography winner: pass H or run sfm_ransac_homography first");
+        H_dev = c->E.as<double>() + 9 * c->winner_local;
+    }
+    if (int r = hmask_launch(c, thr, H_dev, nullptr)) return r;
+    if (mask) CU(cudaMemcpyAsync(mask, c->mask.p, (size_t)c->n, cudaMemcpyDeviceToHost, c->stream));
+    if (err) CU(cudaMemcpyAsync(err, c->sed.p, (size_t)c->n * 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
 }
 
 // ---- pose + triangulation ---------------------------------------------------------------

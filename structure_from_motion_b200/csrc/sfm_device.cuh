@@ -100,6 +100,64 @@ __device__ __forceinline__ double sed_full_decision(const double (&e)[9], double
 }
 
 // ------------------------------------------------------------------------------------
+// Homography transfer error (sfm_homography.cuh; oracle: oracle_transfer_exact in oracle/transfer_exact.c)
+// ------------------------------------------------------------------------------------
+// adj(H) maps image-B points back to image A without a division.  Pinned order: every model consumer (fit, scorer,
+// K3, mask) recomputes it from H with these nine fma's, so all of them see the same bits.
+__device__ __forceinline__ void homography_adj(const double (&h)[9], double (&a)[9]) {
+    a[0] = __fma_rn(h[4], h[8], -__dmul_rn(h[5], h[7]));
+    a[1] = __fma_rn(h[2], h[7], -__dmul_rn(h[1], h[8]));
+    a[2] = __fma_rn(h[1], h[5], -__dmul_rn(h[2], h[4]));
+    a[3] = __fma_rn(h[5], h[6], -__dmul_rn(h[3], h[8]));
+    a[4] = __fma_rn(h[0], h[8], -__dmul_rn(h[2], h[6]));
+    a[5] = __fma_rn(h[2], h[3], -__dmul_rn(h[0], h[5]));
+    a[6] = __fma_rn(h[3], h[7], -__dmul_rn(h[4], h[6]));
+    a[7] = __fma_rn(h[1], h[6], -__dmul_rn(h[0], h[7]));
+    a[8] = __fma_rn(h[0], h[4], -__dmul_rn(h[1], h[3]));
+}
+
+// The four squared terms of the symmetric transfer error of one correspondence (pixel coordinates):
+// p = H (xa, ya, 1), q = adj(H) (xb, yb, 1), F = (p0 - xb p2)^2 + (p1 - yb p2)^2, G = (q0 - xa q2)^2 + (q1 - ya q2)^2,
+// P = p2^2, Q = q2^2.  22 FP64 issue slots.
+struct TransferTerms {
+    double F, G, P, Q;
+    bool finite_w;  // p2 != 0 && q2 != 0 (tested on the bit patterns: integer pipe, same truth table)
+};
+__device__ __forceinline__ TransferTerms transfer_terms(const double (&h)[9], const double (&a)[9], double xa, double ya,
+                                                        double xb, double yb) {
+    const double p0 = __fma_rn(h[0], xa, __fma_rn(h[1], ya, h[2]));
+    const double p1 = __fma_rn(h[3], xa, __fma_rn(h[4], ya, h[5]));
+    const double p2 = __fma_rn(h[6], xa, __fma_rn(h[7], ya, h[8]));
+    const double q0 = __fma_rn(a[0], xb, __fma_rn(a[1], yb, a[2]));
+    const double q1 = __fma_rn(a[3], xb, __fma_rn(a[4], yb, a[5]));
+    const double q2 = __fma_rn(a[6], xb, __fma_rn(a[7], yb, a[8]));
+    const double u = __fma_rn(-xb, p2, p0), v = __fma_rn(-yb, p2, p1);
+    const double s = __fma_rn(-xa, q2, q0), t = __fma_rn(-ya, q2, q1);
+    TransferTerms r;
+    r.F = __fma_rn(u, u, __dmul_rn(v, v));
+    r.G = __fma_rn(s, s, __dmul_rn(t, t));
+    r.P = __dmul_rn(p2, p2);
+    r.Q = __dmul_rn(q2, q2);
+    r.finite_w = ((__double_as_longlong(p2) << 1) != 0) && ((__double_as_longlong(q2) << 1) != 0);
+    return r;
+}
+// inlier decision, division-free: F Q + G P <= (thr P) Q  (+4 slots: 26 in all, plus the compare)
+__device__ __forceinline__ bool transfer_inlier(const TransferTerms& r, double thr) {
+    return r.finite_w && (__fma_rn(r.F, r.Q, __dmul_rn(r.G, r.P)) <= __dmul_rn(__dmul_rn(thr, r.P), r.Q));
+}
+// the error in px^2: F / P + G / Q
+__device__ __forceinline__ double transfer_value(const TransferTerms& r) {
+    return __dadd_rn(__ddiv_rn(r.F, r.P), __ddiv_rn(r.G, r.Q));
+}
+// decision and value together (K3's sample rule and rescore, the mask kernel)
+__device__ __forceinline__ bool transfer_exact(const double (&h)[9], const double (&a)[9], double xa, double ya, double xb,
+                                               double yb, double thr, double& value) {
+    const TransferTerms r = transfer_terms(h, a, xa, ya, xb, yb);
+    value = transfer_value(r);
+    return transfer_inlier(r, thr);
+}
+
+// ------------------------------------------------------------------------------------
 // Philox4x32-10 (Salmon et al., SC'11) — counter-based generator for the device sampler
 // ------------------------------------------------------------------------------------
 __host__ __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2,

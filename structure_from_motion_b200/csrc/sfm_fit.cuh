@@ -180,26 +180,11 @@ __device__ __forceinline__ void finish_fit(double (&F)[9], double s1, double c1x
 // ------------------------------------------------------------------------------------
 enum { FIT_INVALID = 0, FIT_VALID = 1, FIT_AMBIGUOUS = 2 };
 
-__device__ __forceinline__ int eight_point_fit_qr(const Corr (&c)[8], double (&E)[9]) {
-    double s1, c1x, c1y, s2, c2x, c2y;
-    double M[9][8];  // M[i][k] = y_k[i]: column k is the design row of correspondence k
-    {
-        double xa[8], ya[8], xb[8], yb[8], nxa[8], nya[8], nxb[8], nyb[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            xa[i] = c[i].xa; ya[i] = c[i].ya; xb[i] = c[i].xb; yb[i] = c[i].yb;
-        }
-        hartley(xa, ya, nxa, nya, s1, c1x, c1y);
-        hartley(xb, yb, nxb, nyb, s2, c2x, c2y);
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {  // eight_point.py:376-393
-            M[0][k] = __dmul_rn(nxb[k], nxa[k]); M[1][k] = __dmul_rn(nxb[k], nya[k]); M[2][k] = nxb[k];
-            M[3][k] = __dmul_rn(nyb[k], nxa[k]); M[4][k] = __dmul_rn(nyb[k], nya[k]); M[5][k] = nyb[k];
-            M[6][k] = nxa[k]; M[7][k] = nya[k]; M[8][k] = 1.0;
-        }
-    }
-    double beta[8], rdiag[8];
-    bool rank_ok = true;
+// Householder QR of a 9x8 matrix in registers (M[i][k]: column k is one design row), shared by the eight-point fit
+// and the homography DLT (whose A^T has the same shape: two rows per correspondence, four correspondences).  On
+// return column k holds the reflector v_k on and below the diagonal (H_k = I - beta_k v_k v_k^T), R's strictly upper
+// part is above it and its diagonal is rdiag; rank_ok is cleared when a column is exactly zero.
+__device__ __forceinline__ void householder_qr_9x8(double (&M)[9][8], double (&beta)[8], double (&rdiag)[8], bool& rank_ok) {
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
         // reflector for x = M[k..8][k]:  v = x - alpha e_1, alpha = -sign(x_0) |x|, H = I - beta v v^T
@@ -225,6 +210,44 @@ __device__ __forceinline__ int eight_point_fit_qr(const Corr (&c)[8], double (&E
             for (int i = k; i < 9; ++i) M[i][j] = fma(-w, M[i][k], M[i][j]);
         }
     }
+}
+
+// null vector z = H_1 ... H_8 e_9 of the factored matrix
+__device__ __forceinline__ void householder_null_vector(const double (&M)[9][8], const double (&beta)[8], double (&z)[9]) {
+#pragma unroll
+    for (int i = 0; i < 9; ++i) z[i] = (i == 8) ? 1.0 : 0.0;
+#pragma unroll
+    for (int k = 7; k >= 0; --k) {
+        double w = 0.0;
+#pragma unroll
+        for (int i = k; i < 9; ++i) w = fma(M[i][k], z[i], w);
+        w *= beta[k];
+#pragma unroll
+        for (int i = k; i < 9; ++i) z[i] = fma(-w, M[i][k], z[i]);
+    }
+}
+
+__device__ __forceinline__ int eight_point_fit_qr(const Corr (&c)[8], double (&E)[9]) {
+    double s1, c1x, c1y, s2, c2x, c2y;
+    double M[9][8];  // M[i][k] = y_k[i]: column k is the design row of correspondence k
+    {
+        double xa[8], ya[8], xb[8], yb[8], nxa[8], nya[8], nxb[8], nyb[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            xa[i] = c[i].xa; ya[i] = c[i].ya; xb[i] = c[i].xb; yb[i] = c[i].yb;
+        }
+        hartley(xa, ya, nxa, nya, s1, c1x, c1y);
+        hartley(xb, yb, nxb, nyb, s2, c2x, c2y);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {  // eight_point.py:376-393
+            M[0][k] = __dmul_rn(nxb[k], nxa[k]); M[1][k] = __dmul_rn(nxb[k], nya[k]); M[2][k] = nxb[k];
+            M[3][k] = __dmul_rn(nyb[k], nxa[k]); M[4][k] = __dmul_rn(nyb[k], nya[k]); M[5][k] = nyb[k];
+            M[6][k] = nxa[k]; M[7][k] = nya[k]; M[8][k] = 1.0;
+        }
+    }
+    double beta[8], rdiag[8];
+    bool rank_ok = true;
+    householder_qr_9x8(M, beta, rdiag, rank_ok);
     // sigma_min(R)^2 bounds; R = rdiag on the diagonal, M[i][j] (i < j) above it
     double min_r2 = rdiag[0] * rdiag[0];
 #pragma unroll
@@ -255,17 +278,7 @@ __device__ __forceinline__ int eight_point_fit_qr(const Corr (&c)[8], double (&E
     }
     // null vector z = H_1 ... H_8 e_9
     double z[9];
-#pragma unroll
-    for (int i = 0; i < 9; ++i) z[i] = (i == 8) ? 1.0 : 0.0;
-#pragma unroll
-    for (int k = 7; k >= 0; --k) {
-        double w = 0.0;
-#pragma unroll
-        for (int i = k; i < 9; ++i) w = fma(M[i][k], z[i], w);
-        w *= beta[k];
-#pragma unroll
-        for (int i = k; i < 9; ++i) z[i] = fma(-w, M[i][k], z[i]);
-    }
+    householder_null_vector(M, beta, z);
     finish_fit(z, s1, c1x, c1y, s2, c2x, c2y, E);  // v_min.reshape((3,3)) (:424-425)
     return status;
 }

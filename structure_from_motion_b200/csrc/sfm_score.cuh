@@ -823,20 +823,51 @@ struct FinalArgs {
     unsigned* fitflag;             // K1's ambiguous-sample counter: reset here for the next fit (may be null)
 };
 
+// The model K3 selects among: the essential matrix (8-point samples, SED in K-normalised coordinates) or the homography
+// (4-point samples, symmetric transfer error in pixels; sfm_homography.cuh).  The kind fixes the sample size and the
+// exact scorer of the sample rule and of the rescore; the selection rule itself is the same.
+enum { MODEL_E = 0, MODEL_H = 1 };
+template <int KIND> struct ExactModel;
+template <> struct ExactModel<MODEL_E> {
+    static constexpr int kSample = 8;
+    double e[9];
+    __device__ __forceinline__ void load(const double* m) {
+#pragma unroll
+        for (int k = 0; k < 9; ++k) e[k] = m[k];
+    }
+    __device__ __forceinline__ bool eval(const Corr& c, double thr, double& v) const {
+        v = sed_exact(e, c.xa, c.ya, c.xb, c.yb);
+        return v <= thr;  // ransac.py:73
+    }
+};
+template <> struct ExactModel<MODEL_H> {
+    static constexpr int kSample = 4;
+    double h[9], adj[9];
+    __device__ __forceinline__ void load(const double* m) {
+#pragma unroll
+        for (int k = 0; k < 9; ++k) h[k] = m[k];
+        homography_adj(h, adj);
+    }
+    __device__ __forceinline__ bool eval(const Corr& c, double thr, double& v) const {
+        return transfer_exact(h, adj, c.xa, c.ya, c.xb, c.yb, thr, v);
+    }
+};
+
 // the sample rule + aggregation + candidate test of one hypothesis (ransac.py:63-64, 70-76, 96-108), given the count and
 // the sums over ALL correspondences with sed <= thr
+template <int KIND>
 __device__ __forceinline__ bool finalise_one(const FinalArgs& a, const Corr* pts, long long i, long long npts, bool valid,
                                              long long cnt, double s1, double s2, double& err_out, long long& cnt_out,
                                              double& s1_out, double& s2_out) {
+    constexpr int KS = ExactModel<KIND>::kSample;
     const double msac = __dadd_rn(s1, __dmul_rn(a.thr, (double)(npts - cnt)));  // K2 saw every correspondence
     if (a.table && valid) {
-        double e[9];
-#pragma unroll
-        for (int k = 0; k < 9; ++k) e[k] = a.E[9 * i + k];
-        for (int k = 0; k < 8; ++k) {
+        ExactModel<KIND> m;
+        m.load(a.E + 9 * i);
+        for (int k = 0; k < KS; ++k) {
             const Corr c = pts[a.table[8 * i + k]];
-            const double sv = sed_exact(e, c.xa, c.ya, c.xb, c.yb);
-            if (sv <= a.thr) {
+            double sv;
+            if (m.eval(c, a.thr, sv)) {
                 cnt -= 1;  // was counted by K2, but samples are not "extra" inliers
             } else {
                 s1 = __dadd_rn(s1, sv);  // not counted by K2, but always part of the error
@@ -844,7 +875,7 @@ __device__ __forceinline__ bool finalise_one(const FinalArgs& a, const Corr* pts
             }
         }
     }
-    const double n = (double)((a.table ? 8 : 0) + cnt);
+    const double n = (double)((a.table ? KS : 0) + cnt);
     double err;
     switch (a.agg) {
         case AGG_SUM: err = s1; break;
@@ -863,6 +894,7 @@ __device__ __forceinline__ bool finalise_one(const FinalArgs& a, const Corr* pts
 // block: exact scorer over all correspondences, double-double sums in a fixed order (strided partials, fixed tree), so
 // the result is still independent of scheduling, sharding and scoring variant.  Block arg-min, then the last block of
 // the pair to finish (ticket) reduces the per-block results into the selection record.
+template <int KIND>
 __global__ void __launch_bounds__(256) k_finalise(const FinalArgs a) {
     chain_enter();
     __shared__ Best sm[32];
@@ -890,7 +922,10 @@ __global__ void __launch_bounds__(256) k_finalise(const FinalArgs a) {
         const unsigned __int128 v2 = (a.sums & SUM_S2) ? fixed_value(a.acc + (1 + kChunks) * a.htotal + i, a.htotal) : 0;
         // truncation loses < 1 unit per term: the sum is good to 2^-53 relative iff V >= cnt * 2^53
         const unsigned __int128 need = (unsigned __int128)(unsigned long long)cnt << 53;
-        const bool coarse = cnt > 0 && (((a.sums & SUM_S1) && v1 < need) || ((a.sums & SUM_S2) && v2 < need));
+        bool coarse = cnt > 0 && (((a.sums & SUM_S1) && v1 < need) || ((a.sums & SUM_S2) && v2 < need));
+        // a 4-point fit reproduces its own samples to rounding level, so nearly every homography has a coarse sum (its
+        // samples and little else): those that cannot be candidates (count_extra <= cnt < min_extra) are not rescored
+        if constexpr (KIND == MODEL_H) coarse = coarse && !((double)cnt < a.min_extra);
         if (valid && (a.force_rescore || coarse)) {
             s_list[atomicAdd(&s_nlist, 1)] = tid;
         } else {
@@ -898,7 +933,7 @@ __global__ void __launch_bounds__(256) k_finalise(const FinalArgs a) {
             const double s2 = (a.sums & SUM_S2) ? u128_to_double(v2) * a.inv_scale2 : qnan;
             double err, s1o, s2o;
             long long c2;
-            const bool cand = finalise_one(a, pts, i, npts, valid, cnt, s1, s2, err, c2, s1o, s2o);
+            const bool cand = finalise_one<KIND>(a, pts, i, npts, valid, cnt, s1, s2, err, c2, s1o, s2o);
             a.count_extra[i] = valid ? (int32_t)c2 : -1;
             a.S1[i] = s1o;
             a.S2[i] = s2o;
@@ -912,15 +947,14 @@ __global__ void __launch_bounds__(256) k_finalise(const FinalArgs a) {
     for (int q = 0; q < nlist; ++q) {
         const int owner = s_list[q];
         const long long hi_ = (long long)blockIdx.y * a.h + blockIdx.x * (long long)blockDim.x + owner;
-        double e[9];
-#pragma unroll
-        for (int k = 0; k < 9; ++k) e[k] = a.E[9 * hi_ + k];
+        ExactModel<KIND> m;
+        m.load(a.E + 9 * hi_);
         dd p1{0.0, 0.0}, p2{0.0, 0.0};
         long long pc = 0;
         for (long long j = tid; j < npts; j += 256) {
             const Corr c = pts[j];
-            const double sv = sed_exact(e, c.xa, c.ya, c.xb, c.yb);
-            if (sv <= a.thr) {  // ransac.py:73
+            double sv;
+            if (m.eval(c, a.thr, sv)) {
                 pc += 1;
                 dd_add(p1, sv);
                 dd_add(p2, __dmul_rn(sv, sv));
@@ -945,7 +979,7 @@ __global__ void __launch_bounds__(256) k_finalise(const FinalArgs a) {
             for (int w = 1; w < 8; ++w) { dd_merge(t1, s_dd[0][w]); dd_merge(t2, s_dd[1][w]); c += s_cnt[w]; }
             double err, s1o, s2o;
             long long c2;
-            const bool cand = finalise_one(a, pts, hi_, npts, true, c, (a.sums & SUM_S1) ? t1.hi : qnan,
+            const bool cand = finalise_one<KIND>(a, pts, hi_, npts, true, c, (a.sums & SUM_S1) ? t1.hi : qnan,
                                            (a.sums & SUM_S2) ? t2.hi : qnan, err, c2, s1o, s2o);
             a.count_extra[hi_] = (int32_t)c2;
             a.S1[hi_] = s1o;
@@ -1012,7 +1046,8 @@ __global__ void __launch_bounds__(256) k_finalise(const FinalArgs a) {
         r.first_invalid = s_ninv ? s_first2 : -1;
         const long long w = (long long)blockIdx.y * a.h + (g.idx >= 0 ? g.idx - a.idx_offset : 0);
         for (int k = 0; k < 9; ++k) r.E[k] = g.idx >= 0 ? a.E[9 * w + k] : 0.0;
-        for (int k = 0; k < 8; ++k) r.sample[k] = (a.table && g.idx >= 0) ? a.table[8 * w + k] : -1;
+        for (int k = 0; k < 8; ++k)
+            r.sample[k] = (a.table && g.idx >= 0 && k < ExactModel<KIND>::kSample) ? a.table[8 * w + k] : -1;
     }
 }
 

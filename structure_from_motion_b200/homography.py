@@ -1,0 +1,186 @@
+"""RANSAC homography estimation on arrays (numpy in, numpy out) — the model for planar scenes and rotation-only pairs,
+where the essential matrix is not determined by the data (coplanar points) or vanishes (t = 0).
+
+H maps image-A pixels to image-B pixels (x_b ~ H x_a) and is returned divided by H[2,2].  The error is the symmetric
+transfer error in px^2, ``|x_b - pi(H x_a)|^2 + |x_a - pi(adj(H) x_b)|^2``, and a correspondence is an inlier iff the
+division-free form of ``error <= threshold`` holds (csrc/sfm_homography.cuh pins the evaluation order).  The RANSAC
+loop is the reference's ``fit_with_ransac(data, 4, ...)`` (lib/ransac/ransac.py:19-93): 4-point samples, never counted
+as extra inliers and always part of the error, the same aggregation methods, defaults and strict-< selection as
+``two_view.ransac_essential_arrays``.  A sample with three collinear points (in either image) is skipped and counted
+in ``num_invalid`` / ``first_invalid``.  Everything numeric runs in libsfm_b200.so; there is no CPU fallback.
+"""
+from __future__ import annotations
+
+import dataclasses
+import random
+from typing import Optional
+
+import numpy as np
+
+from . import _native
+from .two_view import _agg_name, _get_state_words, _reference_error, _resolve_near_ties, _set_state_words
+
+_SAMPLE = 4  # points per minimal sample
+
+
+@dataclasses.dataclass
+class HomographyResult:
+    H: np.ndarray                 # (3,3), H[2,2] == 1, image A -> image B
+    best_index: int               # winning iteration (global hypothesis index)
+    error: float                  # aggregated error of the winner
+    count_extra: int              # inliers beyond the 4 samples
+    inlier_indices: np.ndarray    # int64; samples, then the rest in that iteration's permutation order (reference
+                                  # sampler) or ascending (table / device sampler)
+    mask: np.ndarray              # bool[n]: inlier decision under the winner
+    err: np.ndarray               # float64[n]: transfer error under the winner (px^2)
+    sample: np.ndarray            # int32[4] the winner's minimal sample
+    num_invalid: int              # degenerate samples (skipped)
+    first_invalid: int            # earliest such iteration, -1 if none
+
+
+def ransac_homography_arrays(
+    pts_a,
+    pts_b,
+    threshold: float,
+    min_num_extra_inliers=None,
+    error_aggregation_method=None,
+    max_iterations: Optional[int] = None,
+    *,
+    sampler: str = "reference",
+    seed: int = 0,
+    hyp_offset: int = 0,
+    selection: str = "min_error",
+    engine: Optional[_native.Engine] = None,
+    table: Optional[np.ndarray] = None,
+) -> HomographyResult:
+    """RANSAC homography from [n,2] arrays of matched pixel coordinates (n >= 8).
+
+    sampler: "reference" — ``random.shuffle`` of the data list per iteration on the process-global state, sample =
+             the first 4 entries; the state advances exactly as ``fit_with_ransac(data, 4, ...)`` would advance it;
+             "device" — Philox sampler on the GPU (``seed``, ``hyp_offset`` for split runs); "table" — the given int
+             table, [H,4] or [H,8] (columns 0-3 are the sample).
+    threshold: on the symmetric transfer error in px^2.  Defaults: 100 iterations, RMS, 0 extra inliers.
+    """
+    if max_iterations is None:
+        max_iterations = 100  # ransac.py:48-49
+    if min_num_extra_inliers is None:
+        min_num_extra_inliers = 0  # ransac.py:52-53
+    agg = _agg_name(error_aggregation_method)
+    pts_a = np.ascontiguousarray(pts_a, dtype=np.float64).reshape(-1, 2)
+    pts_b = np.ascontiguousarray(pts_b, dtype=np.float64).reshape(-1, 2)
+    if pts_a.shape != pts_b.shape:
+        raise ValueError("pts_a and pts_b must have the same shape")
+    n = pts_a.shape[0]
+    H = int(max_iterations)
+
+    def no_model():
+        return ValueError(f"No model could be found with at least {min_num_extra_inliers + _SAMPLE} inliers.")
+
+    if sampler not in ("reference", "device", "table"):
+        raise ValueError(f"unknown sampler {sampler!r}")
+    if H <= 0 and sampler != "table":
+        raise no_model()  # ransac.py:88-91 (loop never ran)
+    if n < 8:
+        raise ValueError(f"RANSAC homography needs at least 8 correspondences, got {n}")
+    eng = engine or _native.get_engine()
+
+    if sampler == "reference":
+        version, words, gauss = _get_state_words()
+        ref_sampler = _native.ReferenceSampler(words, n, H)  # columns 0-3 = perm[:4], the shuffle is size-independent
+        table, words = ref_sampler.table, ref_sampler.final_state
+    elif sampler == "table":
+        table = np.ascontiguousarray(table, dtype=np.int32)
+        if table.ndim != 2 or table.shape[1] not in (_SAMPLE, 8) or table.shape[0] == 0:
+            raise ValueError(f"expected a [H,4] or [H,8] sample table, got shape {table.shape}")
+        if table.shape[1] == _SAMPLE:
+            table = np.ascontiguousarray(np.concatenate([table, table], axis=1))  # columns 4-7 are never read
+        H = table.shape[0]
+
+    eng.upload_pairs(pts_a, pts_b, np.eye(3))  # K = I: the records hold pixel coordinates
+    if sampler == "device":
+        eng.sample_device(seed, H, hyp_offset=hyp_offset)
+    else:
+        eng.set_table(table)
+    best, mask, err, _, _ = eng.ransac_homography(threshold, float(min_num_extra_inliers), agg, selection)
+    if sampler == "reference":
+        _set_state_words(version, words, gauss)  # no exception aborts the loop: every shuffle happened
+    if best.index < 0:
+        raise no_model()
+
+    def rows(t):
+        return np.asarray(table[t][:_SAMPLE], dtype=np.int64)
+
+    def order_after(t):
+        if sampler == "reference":
+            return ref_sampler.after(t)[1][_SAMPLE:].astype(np.int64)
+        keep = np.ones(n, dtype=bool)
+        keep[table[t][:_SAMPLE]] = False
+        return np.nonzero(keep)[0]
+
+    def score(t):
+        H_t, _ = eng.get_models(t, 1)
+        return eng.homography_mask(H_t[0], threshold)
+
+    if sampler != "device" and selection == "min_error":
+        # near-ties are settled in the reference's list order and summation (SURVEY.md H1), as on the E path
+        ties, total = eng.near_ties(1e-12, 64)
+        if 1 < total <= 64:
+            t, e = _resolve_near_ties(eng, ties, threshold, agg, rows, order_after, score)
+            if t is not None and t != int(best.index):
+                H_t, _ = eng.get_models(t, 1)
+                best.index = t
+                best.E[:] = tuple(H_t.reshape(9))
+                m2, err = score(t)
+                mask = m2
+                best.count_extra = int(m2.sum() - m2[rows(t)].sum())
+                best.err = e
+
+    mask = np.asarray(mask).astype(bool)
+    local = int(best.index)
+    sample = np.array(best.sample[:_SAMPLE], dtype=np.int32)
+    if sampler != "device":
+        sample = np.asarray(table[local][:_SAMPLE], dtype=np.int32)
+    is_sample = np.zeros(n, dtype=bool)
+    is_sample[sample] = True
+    if sampler == "reference":
+        rest = order_after(local)  # the permutation of the winning iteration, replayed from the nearest snapshot
+        extra = rest[mask[rest]]
+    else:
+        extra = np.nonzero(mask & ~is_sample)[0]
+    return HomographyResult(
+        H=np.array(best.E, dtype=np.float64).reshape(3, 3),
+        best_index=local + (hyp_offset if sampler == "device" else 0),
+        error=float(best.err),
+        count_extra=int(best.count_extra),
+        inlier_indices=np.concatenate([sample.astype(np.int64), extra]),
+        mask=mask,
+        err=err,
+        sample=sample,
+        num_invalid=int(best.num_invalid),
+        first_invalid=int(best.first_invalid),
+    )
+
+
+def fit_homography_arrays(pts_a, pts_b, engine: Optional[_native.Engine] = None) -> np.ndarray:
+    """The exact homography through 4 correspondences ([4,2] pixel arrays), H[2,2] == 1.  Raises ValueError when three
+    of the points are collinear in either image (no unique solution)."""
+    pts_a = np.ascontiguousarray(pts_a, dtype=np.float64).reshape(-1, 2)
+    pts_b = np.ascontiguousarray(pts_b, dtype=np.float64).reshape(-1, 2)
+    if pts_a.shape[0] != _SAMPLE or pts_b.shape[0] != _SAMPLE:
+        raise ValueError("Exactly four matches are needed")
+    eng = engine or _native.get_engine()
+    eng.upload_pairs(pts_a, pts_b, np.eye(3))
+    eng.set_table(np.array([[0, 1, 2, 3, 0, 1, 2, 3]], dtype=np.int32))
+    H, valid = eng.fit_homography()
+    if not valid[0]:
+        raise ValueError("Degenerate sample: three of the four points are collinear")
+    return H[0]
+
+
+def transfer_error_arrays(H, pts_a, pts_b, threshold: float = np.inf, engine: Optional[_native.Engine] = None):
+    """(inlier decision bool[n], symmetric transfer error float64[n] in px^2) of every correspondence under H."""
+    pts_a = np.ascontiguousarray(pts_a, dtype=np.float64).reshape(-1, 2)
+    pts_b = np.ascontiguousarray(pts_b, dtype=np.float64).reshape(-1, 2)
+    eng = engine or _native.get_engine()
+    eng.upload_pairs(pts_a, pts_b, np.eye(3))
+    return eng.homography_mask(np.asarray(H, dtype=np.float64).reshape(3, 3), threshold)

@@ -84,3 +84,35 @@ def make_image_pair(seed: int = 0, h: int = 480, w: int = 640, f: float = 520.0,
     img1 = tex + rng.normal(0, noise, (h, w))
     to_u8 = lambda a: np.clip(np.round(a), 0, 255).astype(np.uint8)  # noqa: E731
     return to_u8(img1), to_u8(img2), K, R, t
+
+
+def make_planar_scene(n: int, outlier_frac: float, seed: int, noise_px: float = 0.5, rotation_only: bool = False,
+                      f: float = 800.0, w: int = 1280, h: int = 960):
+    """Return (K, x1[n,2], x2[n,2], H_true, outlier_idx) in pixel coordinates for points on one plane.
+
+    The cameras are those of ``make_scene`` (cam1 = [I|0], cam2 = [R|t]; t = 0 when ``rotation_only``).  The points lie
+    on the plane n^T X = d with n = unit(0.15, -0.1, 1), d = 6, tilted against both image planes and in front of both
+    cameras; H_true = K (R + t n^T / d) K^-1 maps image-1 pixels to image-2 pixels (the construction of
+    ``make_image_pair``), divided by its [2,2] entry.  Noise and outliers as in ``make_scene``."""
+    rng = np.random.default_rng(seed)
+    K = np.array([[f, 0.0, w / 2], [0.0, f, h / 2], [0.0, 0.0, 1.0]])
+    nrm = np.array([0.15, -0.1, 1.0])
+    nrm /= np.linalg.norm(nrm)
+    d = 6.0
+    R = euler_xyz_intrinsic(2.0, -8.0, 1.0)
+    t = np.zeros(3) if rotation_only else np.array([-1.0, 0.05, 0.1])
+    # rays through uniform image-1 pixels, cut with the plane
+    u = np.column_stack([rng.uniform(0, w, n), rng.uniform(0, h, n), np.ones(n)])
+    rays = (np.linalg.inv(K) @ u.T).T
+    X = rays * (d / (rays @ nrm))[:, None]
+    x1 = u[:, :2].copy()
+    X2 = (R @ X.T).T + t
+    x2 = (K @ X2.T).T
+    x2 = x2[:, :2] / x2[:, 2:]
+    x1 += rng.normal(0, noise_px, x1.shape)
+    x2 += rng.normal(0, noise_px, x2.shape)
+    n_out = int(round(outlier_frac * n))
+    idx = rng.choice(n, n_out, replace=False)
+    x2[idx] = np.column_stack([rng.uniform(0, w, n_out), rng.uniform(0, h, n_out)])
+    H_true = K @ (R + np.outer(t, nrm) / d) @ np.linalg.inv(K)
+    return K, np.ascontiguousarray(x1), np.ascontiguousarray(x2), H_true / H_true[2, 2], idx

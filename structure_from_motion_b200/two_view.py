@@ -53,18 +53,25 @@ def _reference_error(errors, agg: str) -> float:
     return np.sqrt(np.mean(np.square(errors))).item()
 
 
-def _resolve_near_ties(eng, ties, threshold, agg, rows, order_after):
+def _resolve_near_ties(eng, ties, threshold, agg, rows, order_after, score=None):
     """SURVEY.md H1.  The GPU selects on exactly rounded sums; the reference keeps ``model_error < best_model_error``
     (ransac.py:83) on errors summed in list order.  For the hypotheses whose errors agree to 1e-12 the list-order error
     is recomputed here from the device's exact per-correspondence scores and the strict ``<`` is replayed in iteration
-    order.  rows(t) -> the 8 sample indices of hypothesis t; order_after(t) -> the correspondences that follow the
-    samples in that iteration's list (the permutation tail for the reference sampler).  Returns the local index."""
+    order.  rows(t) -> the sample indices of hypothesis t; order_after(t) -> the correspondences that follow the
+    samples in that iteration's list (the permutation tail for the reference sampler); score(t) -> (inlier decision
+    bool[n], per-correspondence error [n]) under hypothesis t, by default the SED of ``eng``'s essential matrix t
+    against ``threshold``.  Returns the local index."""
+    if score is None:
+        def score(t):
+            eng.set_winner(t)
+            _, sed = eng.inlier_mask(threshold)
+            return sed <= threshold, sed
+
     best_t, best_err = None, float("inf")
     for t in ties:  # ascending = iteration order
-        eng.set_winner(int(t))
-        _, sed = eng.inlier_mask(threshold)
+        inl, sed = score(int(t))
         rest = order_after(int(t))
-        errs = [float(v) for v in sed[rows(int(t))]] + [float(v) for v in sed[rest][sed[rest] <= threshold]]
+        errs = [float(v) for v in sed[rows(int(t))]] + [float(v) for v in sed[rest][inl[rest]]]
         e = _reference_error(errs, agg)
         if e < best_err:
             best_t, best_err = int(t), e
