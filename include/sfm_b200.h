@@ -227,7 +227,8 @@ int sfm_triangulate(sfm_ctx *ctx, const double *P1, const double *P2, const doub
  * winner -> decomposition -> cheirality vote -> triangulation of the passing inliers with
  * P1 = K[I|0], P2 = K[R|t], all on the device.  inlier_idx int64[cap] receives the indices
  * (ascending) of the winner's inliers, pass uint8[cap] the vote result per inlier, X
- * double[cap][3] the points (NaN rows where pass == 0). */
+ * double[cap][3] the points (NaN rows where pass == 0).  SFM_ERR_STATE when the winner is a homography
+ * (sfm_homography_pose_and_triangulate decomposes those). */
 int sfm_pose_and_triangulate(sfm_ctx *ctx, double threshold, double distance_threshold,
                              sfm_poses *poses, int64_t cap, int64_t *num_inliers,
                              int64_t *inlier_idx, uint8_t *pass, double *X);
@@ -245,6 +246,42 @@ int sfm_two_view_async(sfm_ctx *ctx, double threshold, double min_extra, int agg
                        double distance_threshold, uint8_t *mask, double *sed);
 int sfm_two_view_fetch(sfm_ctx *ctx, sfm_best *best, sfm_poses *poses, int64_t cap, int64_t *num_inliers,
                        int64_t *inlier_idx, uint8_t *pass, double *X);
+
+/* ---- pose + triangulation from a homography (planar scenes, rotation-only pairs) ------------
+ * Hn = K^-1 H K (one K for both images), divided by its middle singular value and negated when det(Hn) < 0 (both
+ * camera centres on the same side of the plane).  Candidates: the SVD construction of Ma, Soatto, Kosecka & Sastry,
+ * "An Invitation to 3-D Vision", Alg. 5.2, in the order (R+, T+, N+), (R+, -T+, -N+), (R-, T-, N-), (R-, -T-, -N-);
+ * t = T / |T|, n = N, d = 1 / |T|.  The order of the four depends on eigenvector signs: compare candidate sets.
+ * Rotation-only (sv[0] - sv[2] < rotation_tolerance, 1e-2 ~ 0.6 degrees of plane-induced parallax): all four slots hold
+ * the rotation nearest to Hn with t = 0, n = NaN, d = inf; no vote, best = -1. */
+typedef struct sfm_hposes {
+    double R[4][9];
+    double t[4][3];      /* unit; 0 when rotation_only                                    */
+    double n[4][3];      /* plane n^T X = d in camera-1 coordinates, units of the baseline */
+    double d[4];
+    double sv[3];        /* singular values of K^-1 H K scaled so that sv[1] == 1          */
+    int64_t counts[4];   /* cheirality votes: every passing inlier counts                  */
+    int32_t best;        /* voted candidate (first maximum); -1 no vote (rotation only); -2 no model */
+    int32_t rotation_only;
+} sfm_hposes;
+/* The decomposition of one homography H (double[9], pixel coordinates) with K (double[9]). */
+int sfm_decompose_homography(sfm_ctx *ctx, const double *H, const double *K, double rotation_tolerance,
+                             sfm_hposes *out);
+/* The tail of the current homography winner (sfm_ransac_homography / sfm_set_winner on homography models): the
+ * winner's inliers (decision under H plus its 4 sample points) -> decomposition -> cheirality vote (the test of
+ * sfm_pose_and_triangulate on K-normalised coordinates, P1 = [I|0], P2 = [R|t]) -> DLT of the inliers passing the
+ * voted candidate in pixel coordinates (P1 = K[I|0], P2 = K[R|t]).  inlier_idx, pass, X and cap as in
+ * sfm_pose_and_triangulate; a rotation-only pair has no passing inlier and NaN points. */
+int sfm_homography_pose_and_triangulate(sfm_ctx *ctx, const double *K, double threshold, double distance_threshold,
+                                        double rotation_tolerance, sfm_hposes *poses, int64_t cap,
+                                        int64_t *num_inliers, int64_t *inlier_idx, uint8_t *pass, double *X);
+/* sfm_ransac_homography + sfm_homography_pose_and_triangulate in one call: the winner never leaves the device between
+ * selection and the tail, the host synchronises once for the fixed-size results.  mask / err (optional) are those of
+ * sfm_ransac_homography. */
+int sfm_two_view_homography(sfm_ctx *ctx, const double *K, double threshold, double min_extra, int aggregation,
+                            int selection, double distance_threshold, double rotation_tolerance, sfm_best *best,
+                            sfm_hposes *poses, int64_t cap, int64_t *num_inliers, int64_t *inlier_idx, uint8_t *pass,
+                            double *X, uint8_t *mask, double *err);
 
 /* ---- batched image pairs (pair-sharded workloads) ------------------------------------ */
 /* P independent pairs; pair p owns correspondences [offsets[p], offsets[p+1]) of the

@@ -38,6 +38,12 @@ class Poses(C.Structure):
                 ("counts", C.c_int64 * 4), ("best", C.c_int32), ("reserved", C.c_int32)]
 
 
+class HPoses(C.Structure):
+    _fields_ = [("R", (C.c_double * 9) * 4), ("t", (C.c_double * 3) * 4), ("n", (C.c_double * 3) * 4),
+                ("d", C.c_double * 4), ("sv", C.c_double * 3), ("counts", C.c_int64 * 4), ("best", C.c_int32),
+                ("rotation_only", C.c_int32)]
+
+
 _P = C.c_void_p
 _SIGNATURES = {
     "sfm_version": (C.c_int, []),
@@ -85,6 +91,12 @@ _SIGNATURES = {
                                C.c_int64, C.POINTER(C.c_int64), _P, _P, _P, _P, _P]),
     "sfm_two_view_async": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.c_double, _P, _P]),
     "sfm_two_view_fetch": (C.c_int, [_P, C.POINTER(Best), C.POINTER(Poses), C.c_int64, C.POINTER(C.c_int64), _P, _P, _P]),
+    "sfm_decompose_homography": (C.c_int, [_P, _P, _P, C.c_double, C.POINTER(HPoses)]),
+    "sfm_homography_pose_and_triangulate": (C.c_int, [_P, _P, C.c_double, C.c_double, C.c_double, C.POINTER(HPoses),
+                                                      C.c_int64, C.POINTER(C.c_int64), _P, _P, _P]),
+    "sfm_two_view_homography": (C.c_int, [_P, _P, C.c_double, C.c_double, C.c_int, C.c_int, C.c_double, C.c_double,
+                                          C.POINTER(Best), C.POINTER(HPoses), C.c_int64, C.POINTER(C.c_int64), _P, _P,
+                                          _P, _P, _P]),
     "sfm_score_async": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.POINTER(_P)]),
     "sfm_sharded_tail": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_double, C.c_double]),
     "sfm_sharded_fetch": (C.c_int, [_P, C.POINTER(Best), C.POINTER(C.c_int32), C.POINTER(Poses), C.c_int64,
@@ -384,6 +396,50 @@ class Engine:
         self._ck(self.lib.sfm_homography_mask(self.h, _ptr(Ha), float(threshold), _ptr(mask), _ptr(err)),
                  "sfm_homography_mask")
         return mask.astype(bool), err
+
+    def decompose_homography(self, H, K, rotation_tolerance=1e-2):
+        """The four (R, t, n, d) candidates of H (3x3, pixels) with K -> HPoses (sfm_hposes)."""
+        Ha, Ka = _f64(H).reshape(9), _f64(K).reshape(9)
+        p = HPoses()
+        self._ck(self.lib.sfm_decompose_homography(self.h, _ptr(Ha), _ptr(Ka), float(rotation_tolerance), C.byref(p)),
+                 "sfm_decompose_homography")
+        return p
+
+    def homography_pose_and_triangulate(self, K, threshold, distance_threshold=50.0, rotation_tolerance=1e-2, cap=None):
+        """Tail of the current homography winner -> (HPoses, num_inliers, inlier_idx, pass_bits, X)."""
+        cap = self.n if cap is None else int(cap)
+        Ka = _f64(K).reshape(9)
+        p = HPoses()
+        num = C.c_int64(0)
+        idx = np.empty(cap, dtype=np.int64)
+        ok = np.empty(cap, dtype=np.uint8)
+        X = np.empty((cap, 3), dtype=np.float64)
+        self._ck(self.lib.sfm_homography_pose_and_triangulate(self.h, _ptr(Ka), float(threshold), float(distance_threshold),
+                                                              float(rotation_tolerance), C.byref(p), cap, C.byref(num),
+                                                              _ptr(idx), _ptr(ok), _ptr(X)),
+                 "sfm_homography_pose_and_triangulate")
+        m = min(int(num.value), cap)
+        return p, int(num.value), idx[:m], ok[:m], X[:m]
+
+    def two_view_homography(self, K, threshold, min_extra=0.0, aggregation="rms", selection="min_error",
+                            distance_threshold=50.0, rotation_tolerance=1e-2, cap=None):
+        """ransac_homography + homography_pose_and_triangulate in one C call (one synchronisation for the fixed-size
+        results).  Returns (best, mask, err, HPoses, num_inliers, inlier_idx, pass_bits, X)."""
+        cap = self.n if cap is None else int(cap)
+        Ka = _f64(K).reshape(9)
+        b, p = Best(), HPoses()
+        num = C.c_int64(0)
+        idx = np.empty(cap, dtype=np.int64)
+        ok = np.empty(cap, dtype=np.uint8)
+        X = np.empty((cap, 3), dtype=np.float64)
+        mask = np.empty(self.n, dtype=np.uint8)
+        err = np.empty(self.n, dtype=np.float64)
+        self._ck(self.lib.sfm_two_view_homography(self.h, _ptr(Ka), float(threshold), float(min_extra), AGG[aggregation],
+                                                  SELECT[selection], float(distance_threshold), float(rotation_tolerance),
+                                                  C.byref(b), C.byref(p), cap, C.byref(num), _ptr(idx), _ptr(ok), _ptr(X),
+                                                  _ptr(mask), _ptr(err)), "sfm_two_view_homography")
+        m = min(int(num.value), cap)
+        return b, mask, err, p, int(num.value), idx[:m], ok[:m], X[:m]
 
     # -- pose / triangulation ---------------------------------------------------------------
     def decompose_essential(self, E):

@@ -98,6 +98,7 @@ struct sfm_ctx {
     Buf m_img, m_feat, m_W, m_ss, m_ok, m_S, m_out;
     Buf h_img, h_gx, h_gy, h_corner, h_alive, h_key, h_idx, h_small, h_xy;
     Buf mask, sed, poses, pass, X, idx, scan, tmp, tailstate, num, winrec, bout;
+    Buf planes, hK;  // the homography tail's HPlane and the K it was called with (the upload's K stays in Ks)
     long long n = 0, h = 0, npairs = 1;
     long long first_len = 0;  // batched: correspondences of the first pair (what the AUTO pilot samples)
     long long raw_stride = 1;
@@ -110,6 +111,7 @@ struct sfm_ctx {
     bool acc_clean = false;  // K2's accumulators (+ tail words) are zero: the fit kernel cleared them
     size_t acc_planes_for = 0;  // hypotheses (all pairs) the cleared accumulators were laid out for
     double Kstage[9] = {0};
+    double hstage[18] = {0};  // H and K of sfm_decompose_homography, K of the homography tail, staged for async copies
     const void* occ_fn[4] = {nullptr, nullptr, nullptr, nullptr};  // scoring kernels whose launch configuration is cached
     int occ_blocks[4] = {0, 0, 0, 0};
     int occ_next = 0;
@@ -291,6 +293,7 @@ int sfm_destroy(sfm_ctx* c) {
     Buf* bufs[] = {&c->raw, &c->pts, &c->offsets, &c->Ks, &c->table, &c->E, &c->valid, &c->eig, &c->acc,
                    &c->count_extra, &c->S1, &c->S2, &c->err, &c->blocks, &c->best,
                    &c->invalid, &c->winnerE, &c->record, &c->merged, &c->rows, &c->blockinv, &c->mask, &c->sed, &c->poses, &c->pass, &c->X, &c->idx,
+                   &c->planes, &c->hK,
                    &c->scan, &c->tmp, &c->gathered, &c->tailstate, &c->num, &c->winrec, &c->bout, &c->spts, &c->bounds, &c->fitflag,
                    &c->m_img, &c->m_feat, &c->m_W, &c->m_ss, &c->m_ok, &c->m_S, &c->m_out,
                    &c->h_img, &c->h_gx, &c->h_gy, &c->h_corner, &c->h_alive, &c->h_key, &c->h_idx, &c->h_small, &c->h_xy};
@@ -1279,8 +1282,10 @@ int sfm_triangulate(sfm_ctx* c, const double* P1, const double* P2, const double
 // The tail of apps/sfm.py:133-186 for the winner described by rec_dev (one SelectRecord per pair on the device):
 // T1 inlier mask + ordered compaction + decomposition, T2 4-pose cheirality + vote, T3 triangulation of the passing
 // inliers - three launches, nothing synchronised (see sfm_tail.cuh).  max_len = the longest pair.
+// kind = MODEL_H: the winner is a homography of a single pair; hpose_stage_k has put the caller's K in c->hK.
 static int pose_tail_launch(sfm_ctx* c, double thr, double dist_thr, const SelectRecord* rec_dev, long long max_len,
-                            uint8_t* mask_host = nullptr, double* sed_host = nullptr) {
+                            uint8_t* mask_host = nullptr, double* sed_host = nullptr, int kind = MODEL_E,
+                            double rot_tol = 0.0) {
     const long long n = c->n, P = c->npairs;
     if (max_len < 1) max_len = 1;
     const int nblk = (int)((max_len + kTailPerBlock - 1) / kTailPerBlock);
@@ -1316,8 +1321,16 @@ static int pose_tail_launch(sfm_ctx* c, double thr, double dist_thr, const Selec
     a.stride = c->raw_stride;
     a.Ks = c->Ks.as<double>();
     a.X = c->X.as<double>();
+    a.planes = nullptr;
+    a.rot_tol = rot_tol;
+    if (kind == MODEL_H) {
+        if (int r = c->planes.reserve(sizeof(HPlane))) return r;
+        a.planes = c->planes.as<HPlane>();
+        a.Ks = c->hK.as<double>();
+    }
     c->tic(T_MASK);
-    CU(chain_launch(c, k_tail_mask, dim3((unsigned)nblk, (unsigned)P), dim3(kTailBlock), 0, a));
+    if (kind == MODEL_H) CU(chain_launch(c, k_tail_mask<MODEL_H>, dim3((unsigned)nblk, (unsigned)P), dim3(kTailBlock), 0, a));
+    else CU(chain_launch(c, k_tail_mask<MODEL_E>, dim3((unsigned)nblk, (unsigned)P), dim3(kTailBlock), 0, a));
     if (int r = check_launch(c, "k_tail_mask")) return r;
     c->toc(T_MASK);
     // the caller's mask is "sed <= thr" (the forced sample points live in the compacted list only)
@@ -1327,7 +1340,9 @@ static int pose_tail_launch(sfm_ctx* c, double thr, double dist_thr, const Selec
     // grids sized for the machine (grid-stride inside): the number of inliers is only known on the device
     const long long cap_blocks = P >= 64 ? 8 : 2ll * c->sm_count;
     const long long g2 = (4 * max_len + 127) / 128, g3 = (max_len + 127) / 128;
-    CU(chain_launch(c, k_tail_cheirality, dim3((unsigned)(g2 < cap_blocks ? g2 : cap_blocks), (unsigned)P), dim3(128), 0, a));
+    const dim3 grid2((unsigned)(g2 < cap_blocks ? g2 : cap_blocks), (unsigned)P);
+    if (kind == MODEL_H) CU(chain_launch(c, k_tail_cheirality<MODEL_H>, grid2, dim3(128), 0, a));
+    else CU(chain_launch(c, k_tail_cheirality<MODEL_E>, grid2, dim3(128), 0, a));
     if (int r = check_launch(c, "k_tail_cheirality")) return r;
     c->toc(T_POSE);
     c->tic(T_TRI);
@@ -1356,7 +1371,7 @@ static int host_winner_record(sfm_ctx* c, const SelectRecord** out) {
 constexpr long long kSpecInliers = 2048;
 
 static int pose_tail_fetch(sfm_ctx* c, sfm_poses* poses, int64_t cap, int64_t* num_inliers, int64_t* inlier_idx,
-                           uint8_t* pass, double* X, sfm_best* best /* may be null */) {
+                           uint8_t* pass, double* X, sfm_best* best /* may be null */, HPlane* planes = nullptr) {
     const long long* cnt_dev = c->num.as<long long>();
     const long long spec = c->n < kSpecInliers ? c->n : kSpecInliers;
     const size_t o_idx = 64 + ((sizeof(SelectRecord) + 63) / 64) * 64, o_pass = o_idx + (size_t)spec * 8,
@@ -1366,6 +1381,7 @@ static int pose_tail_fetch(sfm_ctx* c, sfm_poses* poses, int64_t cap, int64_t* n
     CU(cudaMemcpyAsync(hp, cnt_dev, 8, cudaMemcpyDeviceToHost, c->stream));
     if (best) CU(cudaMemcpyAsync(hp + 64, c->record.p, sizeof(SelectRecord), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(poses, c->poses.p, sizeof(PoseSet), cudaMemcpyDeviceToHost, c->stream));
+    if (planes) CU(cudaMemcpyAsync(planes, c->planes.p, sizeof(HPlane), cudaMemcpyDeviceToHost, c->stream));
     if (spec > 0) {
         if (inlier_idx) CU(cudaMemcpyAsync(hp + o_idx, c->idx.p, (size_t)spec * 8, cudaMemcpyDeviceToHost, c->stream));
         if (pass) CU(cudaMemcpyAsync(hp + o_pass, c->pass.p, (size_t)spec, cudaMemcpyDeviceToHost, c->stream));
@@ -1413,10 +1429,110 @@ int sfm_pose_and_triangulate(sfm_ctx* c, double thr, double dist_thr, sfm_poses*
     if (!poses || !num_inliers) return fail(SFM_ERR_ARG, "null argument");
     if (!c->has_pts || c->batched) return fail(SFM_ERR_STATE, "no single-pair correspondences loaded");
     if (!c->winner_set) return fail(SFM_ERR_STATE, "no winner: run sfm_ransac_essential / sfm_get_best first");
+    if (c->models_h && c->winner_local >= 0)
+        return fail(SFM_ERR_STATE, "the winner is a homography: use sfm_homography_pose_and_triangulate");
     const SelectRecord* rec = nullptr;
     if (int r = host_winner_record(c, &rec)) return r;
     if (int r = pose_tail_launch(c, thr, dist_thr, rec, c->n)) return r;
     return pose_tail_fetch(c, poses, cap, num_inliers, inlier_idx, pass, X, nullptr);
+}
+
+// ---- homography pose (sfm_hpose.cuh) -------------------------------------------------------
+static void pack_hposes(const PoseSet& p, const HPlane& pl, sfm_hposes* out) {
+    memcpy(out->R, p.R, sizeof out->R);
+    memcpy(out->t, p.t, sizeof out->t);
+    memcpy(out->n, pl.n, sizeof out->n);
+    memcpy(out->d, pl.d, sizeof out->d);
+    memcpy(out->sv, p.sv, sizeof out->sv);
+    memcpy(out->counts, p.counts, sizeof out->counts);
+    out->best = p.best;
+    out->rotation_only = pl.rotation_only;
+}
+
+static int hpose_args(const double* K, double rot_tol) {
+    if (!K) return fail(SFM_ERR_ARG, "null camera matrix");
+    for (int i = 0; i < 9; ++i)
+        if (!std::isfinite(K[i])) return fail(SFM_ERR_ARG, "the camera matrix is not finite");
+    const double det = K[0] * (K[4] * K[8] - K[5] * K[7]) - K[1] * (K[3] * K[8] - K[5] * K[6]) +
+                       K[2] * (K[3] * K[7] - K[4] * K[6]);
+    if (det == 0.0 || K[0] == 0.0 || K[4] == 0.0) return fail(SFM_ERR_ARG, "the camera matrix is singular");
+    if (std::isnan(rot_tol)) return fail(SFM_ERR_ARG, "rotation_tolerance is NaN");
+    return 0;
+}
+
+// the caller's K to the device (staged in the context: the async copy must not read caller memory later)
+static int hpose_stage_k(sfm_ctx* c, const double* K) {
+    if (int r = c->hK.reserve(72)) return r;
+    memcpy(c->hstage + 9, K, 72);
+    CU(cudaMemcpyAsync(c->hK.p, c->hstage + 9, 72, cudaMemcpyHostToDevice, c->stream));
+    return 0;
+}
+
+int sfm_decompose_homography(sfm_ctx* c, const double* H, const double* K, double rotation_tolerance, sfm_hposes* out) {
+    if (int r = use(c)) return r;
+    if (!H || !out) return fail(SFM_ERR_ARG, "null argument");
+    if (int r = hpose_args(K, rotation_tolerance)) return r;
+    if (int r = c->tmp.reserve(144)) return r;
+    if (int r = c->poses.reserve(sizeof(PoseSet))) return r;
+    if (int r = c->planes.reserve(sizeof(HPlane))) return r;
+    memcpy(c->hstage, H, 72);
+    memcpy(c->hstage + 9, K, 72);
+    CU(cudaMemcpyAsync(c->tmp.p, c->hstage, 144, cudaMemcpyHostToDevice, c->stream));
+    k_decompose_homography<<<1, 32, 0, c->stream>>>(c->tmp.as<double>(), c->tmp.as<double>() + 9, rotation_tolerance,
+                                                    c->poses.as<PoseSet>(), c->planes.as<HPlane>());
+    if (int r = check_launch(c, "k_decompose_homography")) return r;
+    PoseSet p;
+    HPlane pl;
+    CU(cudaMemcpyAsync(&p, c->poses.p, sizeof p, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(&pl, c->planes.p, sizeof pl, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    pack_hposes(p, pl, out);
+    return 0;
+}
+
+int sfm_homography_pose_and_triangulate(sfm_ctx* c, const double* K, double thr, double dist_thr, double rotation_tolerance,
+                                        sfm_hposes* poses, int64_t cap, int64_t* num_inliers, int64_t* inlier_idx,
+                                        uint8_t* pass, double* X) {
+    if (int r = use(c)) return r;
+    if (!poses || !num_inliers) return fail(SFM_ERR_ARG, "null argument");
+    if (int r = hpose_args(K, rotation_tolerance)) return r;
+    if (!c->has_pts || c->batched) return fail(SFM_ERR_STATE, "no single-pair correspondences loaded");
+    if (!c->models_h || !c->winner_set || c->winner_local < 0)
+        return fail(SFM_ERR_STATE, "no homography winner: run sfm_ransac_homography or sfm_set_winner first");
+    const SelectRecord* rec = nullptr;
+    if (int r = host_winner_record(c, &rec)) return r;
+    if (int r = hpose_stage_k(c, K)) return r;
+    if (int r = pose_tail_launch(c, thr, dist_thr, rec, c->n, nullptr, nullptr, MODEL_H, rotation_tolerance)) return r;
+    PoseSet p;
+    HPlane pl;
+    if (int r = pose_tail_fetch(c, reinterpret_cast<sfm_poses*>(&p), cap, num_inliers, inlier_idx, pass, X, nullptr, &pl))
+        return r;
+    pack_hposes(p, pl, poses);
+    return 0;
+}
+
+int sfm_two_view_homography(sfm_ctx* c, const double* K, double thr, double min_extra, int agg, int mode, double dist_thr,
+                            double rotation_tolerance, sfm_best* best, sfm_hposes* poses, int64_t cap, int64_t* num_inliers,
+                            int64_t* inlier_idx, uint8_t* pass, double* X, uint8_t* mask, double* err) {
+    if (int r = use(c)) return r;
+    if (!best || !poses || !num_inliers) return fail(SFM_ERR_ARG, "null argument");
+    if (int r = hpose_args(K, rotation_tolerance)) return r;
+    if (c->batched) return fail(SFM_ERR_STATE, "single-pair call on a batched context");
+    if (c->has_pts && c->n < 8) return fail(SFM_ERR_ARG, "need at least 8 correspondences, got %lld", c->n);
+    // K goes first: no copy between the selection and the tail, which is chained right behind it; the winner stays on
+    // the device and the host synchronises once, at the fetch
+    if (int r = hpose_stage_k(c, K)) return r;
+    if (int r = fit_h_launch(c)) return r;
+    if (int r = score_h_launch(c, thr, min_extra, agg, mode)) return r;
+    // T1's mask / err are those of sfm_homography_mask for the winner
+    if (int r = pose_tail_launch(c, thr, dist_thr, c->record.as<SelectRecord>(), c->n, mask, err, MODEL_H, rotation_tolerance))
+        return r;
+    PoseSet p;
+    HPlane pl;
+    if (int r = pose_tail_fetch(c, reinterpret_cast<sfm_poses*>(&p), cap, num_inliers, inlier_idx, pass, X, best, &pl))
+        return r;
+    pack_hposes(p, pl, poses);
+    return 0;
 }
 
 int sfm_two_view_async(sfm_ctx* c, double thr, double min_extra, int agg, int mode, double dist_thr, uint8_t* mask,

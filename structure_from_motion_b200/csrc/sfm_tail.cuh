@@ -7,8 +7,15 @@
 //   T3 k_tail_triangulate DLT in pixel coordinates of the inliers passing the voted pose (triangulation.py:9-62)
 // The winner (model, sample row, index) is read from a SelectRecord on the device: K3's for the fused single-GPU call
 // and the batch, the merged one of a hypothesis-sharded run, or one built from a host-chosen winner.
+//
+// T1 and T2 take the model kind as a template parameter.  MODEL_E: sed_exact, the 8 sample points, decompose_essential,
+// K-normalised records, and the vote with the reference's index-0 rule.  MODEL_H (single pair): the pinned transfer
+// decision of k_homography_mask, the 4 sample points, decompose_homography (sfm_hpose.cuh) of K^-1 H K with the
+// caller's K in Ks, records in pixel coordinates (T2 normalises them with k_normalise's IEEE operations), every passing
+// inlier counts, and T2 does nothing but clear the pass bits when the pair is rotation-only.  T3 serves both.
 #pragma once
 #include "sfm_device.cuh"
+#include "sfm_hpose.cuh"
 #include "sfm_pose.cuh"
 #include "sfm_score.cuh"
 
@@ -38,6 +45,9 @@ struct TailArgs {
     long long stride;
     const double* Ks;            // [P][9]
     double* X;                   // [n_total][3] at compact positions
+    // MODEL_H only
+    HPlane* planes;              // [P] normals, distances, rotation flag beside poses
+    double rot_tol;              // rotation-only below this s1 - s3
 };
 
 // Build a record for a winner chosen by the host (sfm_set_winner / sfm_get_best): E from device memory, row from the
@@ -57,6 +67,7 @@ __device__ __forceinline__ unsigned long long ld_volatile_u64(const unsigned lon
     return v;
 }
 
+template <int KIND>
 __global__ void __launch_bounds__(kTailBlock) k_tail_mask(const TailArgs a) {
     chain_enter();
     __shared__ unsigned s_bid;
@@ -77,6 +88,9 @@ __global__ void __launch_bounds__(kTailBlock) k_tail_mask(const TailArgs a) {
     for (int k = 0; k < 9; ++k) e[k] = rec.E[k];
 #pragma unroll
     for (int k = 0; k < 8; ++k) row[k] = rec.sample[k];
+    constexpr int kSample = KIND == MODEL_H ? 4 : 8;  // points of a minimal sample
+    double adj[9];
+    if constexpr (KIND == MODEL_H) homography_adj(e, adj);
     const long long base = (long long)bid * kTailPerBlock;
     bool f[4];
     unsigned b[4];
@@ -86,13 +100,20 @@ __global__ void __launch_bounds__(kTailBlock) k_tail_mask(const TailArgs a) {
         f[k] = false;
         if (i < plen) {
             const Corr c = a.pts[pbase + i];
-            const double sv = have ? sed_exact(e, c.xa, c.ya, c.xb, c.yb) : __longlong_as_double(0x7ff8000000000000LL);
-            const bool in = have && (sv <= a.thr);  // ransac.py:73
+            double sv;
+            bool in;
+            if constexpr (KIND == MODEL_E) {
+                sv = have ? sed_exact(e, c.xa, c.ya, c.xb, c.yb) : __longlong_as_double(0x7ff8000000000000LL);
+                in = have && (sv <= a.thr);  // ransac.py:73
+            } else {  // k_homography_mask's decision and value
+                sv = __longlong_as_double(0x7ff8000000000000LL);
+                in = have && transfer_exact(e, adj, c.xa, c.ya, c.xb, c.yb, a.thr, sv);
+            }
             if (a.sed) a.sed[pbase + i] = sv;
             if (a.mask) a.mask[pbase + i] = in ? 1 : 0;
             bool smp = false;  // ransac.py:76: the sample points belong to the model's inliers whatever their score
 #pragma unroll
-            for (int q = 0; q < 8; ++q) smp |= ((long long)row[q] == i);
+            for (int q = 0; q < kSample; ++q) smp |= ((long long)row[q] == i);
             f[k] = in || (have && smp);
         }
         b[k] = __ballot_sync(0xffffffffu, f[k]);
@@ -148,12 +169,22 @@ __global__ void __launch_bounds__(kTailBlock) k_tail_mask(const TailArgs a) {
     }
     // the decomposition of the winner rides along (one thread of the first block, after it has published)
     if (bid == 0 && tid == 32) {
-        if (have) decompose_essential(e, a.poses[pair]);
-        else {
-            PoseSet& p = a.poses[pair];
-            for (int q = 0; q < 4; ++q) p.counts[q] = 0;
-            p.best = -2;
-            p.pad = 0;
+        if constexpr (KIND == MODEL_E) {
+            if (have) decompose_essential(e, a.poses[pair]);
+            else {
+                PoseSet& p = a.poses[pair];
+                for (int q = 0; q < 4; ++q) p.counts[q] = 0;
+                p.best = -2;
+                p.pad = 0;
+            }
+        } else {
+            if (have) {
+                double hn[9];
+                homography_normalise_k(e, a.Ks + 9 * (long long)pair, hn);
+                decompose_homography(hn, a.rot_tol, a.poses[pair], a.planes[pair]);
+            } else {
+                homography_no_model(a.poses[pair], a.planes[pair]);
+            }
         }
     }
 }
@@ -192,6 +223,7 @@ constexpr long long kTailSmallTri = 512;  // up to this many inliers the block t
 
 // Grid-stride: the grid is sized for the machine, not for the (unknown to the host) number of inliers - a config-3
 // winner has ~100 inliers, and 3 000 blocks that only find that out cost 30 us.
+template <int KIND>
 __global__ void __launch_bounds__(128) k_tail_cheirality(const TailArgs a) {
     chain_enter();
     __shared__ int s_cnt[4];
@@ -200,6 +232,16 @@ __global__ void __launch_bounds__(128) k_tail_cheirality(const TailArgs a) {
     const long long pbase = a.offsets ? a.offsets[pair] : 0;
     const long long m = a.num[pair];
     PoseSet* poses = a.poses + pair;
+    double fx = 1.0, fy = 1.0, cx = 0.0, cy = 0.0;
+    if constexpr (KIND == MODEL_H) {
+        if (a.planes[pair].rotation_only) {  // no vote: nothing passes, best stays -1 and T3 writes NaN points
+            for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < m; i += (long long)gridDim.x * blockDim.x)
+                a.pass[pbase + i] = 0;
+            return;
+        }
+        const double* K = a.Ks + 9 * (long long)pair;
+        fx = K[0]; fy = K[4]; cx = K[2]; cy = K[5];
+    }
     if (threadIdx.x < 4) s_cnt[threadIdx.x] = 0;
     __syncthreads();
     const int r0 = a.rec[pair].sample[0];
@@ -210,7 +252,13 @@ __global__ void __launch_bounds__(128) k_tail_cheirality(const TailArgs a) {
         bool ok = false, counts = false;
         if (i < m) {
             const long long gi = a.idx[pbase + i];
-            const Corr c = a.pts[pbase + gi];
+            Corr c = a.pts[pbase + gi];
+            if constexpr (KIND == MODEL_H) {  // pixel records: k_normalise's operations (eight_point.py:127-133)
+                c.xa = __ddiv_rn(__dsub_rn(c.xa, cx), fx);
+                c.ya = __ddiv_rn(__dsub_rn(c.ya, cy), fy);
+                c.xb = __ddiv_rn(__dsub_rn(c.xb, cx), fx);
+                c.yb = __ddiv_rn(__dsub_rn(c.yb, cy), fy);
+            }
             const double P1[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};  // Transform3D.identity() (:473)
             double P2[12];
 #pragma unroll
@@ -228,7 +276,8 @@ __global__ void __launch_bounds__(128) k_tail_cheirality(const TailArgs a) {
             // np.count_nonzero of the passing INDICES (:228-230): list position 0 never counts.  The list is the RANSAC
             // inlier list (apps/sfm.py:118-133), whose position 0 is the winner's first sample (ransac.py:76); without
             // a sample row it is the first correspondence.
-            counts = ok && !(r0 >= 0 ? (gi == (long long)r0) : (i == 0));
+            if constexpr (KIND == MODEL_E) counts = ok && !(r0 >= 0 ? (gi == (long long)r0) : (i == 0));
+            else counts = ok;  // a homography's vote counts every passing inlier
         }
         const unsigned lane = threadIdx.x & 31u;
         const unsigned okb = __ballot_sync(0xffffffffu, ok);

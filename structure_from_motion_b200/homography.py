@@ -8,6 +8,12 @@ loop is the reference's ``fit_with_ransac(data, 4, ...)`` (lib/ransac/ransac.py:
 as extra inliers and always part of the error, the same aggregation methods, defaults and strict-< selection as
 ``two_view.ransac_essential_arrays``.  A sample with three collinear points (in either image) is skipped and counted
 in ``num_invalid`` / ``first_invalid``.  Everything numeric runs in libsfm_b200.so; there is no CPU fallback.
+
+``two_view_homography_arrays`` continues from the winner to a camera pose and 3-D points, as ``two_view_arrays`` does
+from E: the decomposition of K^-1 H K into four (R, t, n, d) candidates (csrc/sfm_hpose.cuh), the cheirality vote of
+the winner's inliers and the triangulation of the inliers that pass the voted candidate.  t is a unit vector, the plane
+is n^T X = d in camera-1 coordinates in units of the baseline.  A rotation-only pair (sigma_1 - sigma_3 of the
+normalised homography below ``rotation_tolerance``) gets R, t = 0, no vote and no points.
 """
 from __future__ import annotations
 
@@ -18,6 +24,7 @@ from typing import Optional
 import numpy as np
 
 from . import _native
+from .errors import EightPointCalculationError
 from .two_view import _agg_name, _get_state_words, _reference_error, _resolve_near_ties, _set_state_words
 
 _SAMPLE = 4  # points per minimal sample
@@ -184,3 +191,115 @@ def transfer_error_arrays(H, pts_a, pts_b, threshold: float = np.inf, engine: Op
     eng = engine or _native.get_engine()
     eng.upload_pairs(pts_a, pts_b, np.eye(3))
     return eng.homography_mask(np.asarray(H, dtype=np.float64).reshape(3, 3), threshold)
+
+
+@dataclasses.dataclass
+class HomographyDecomposition:
+    candidates: list              # [(R, t, n, d)]: four, or one (R, 0, NaN, inf) when rotation_only
+    singular_values: np.ndarray   # of K^-1 H K, scaled so that the middle one is 1
+    rotation_only: bool
+
+
+def _candidates(p) -> list:
+    R = np.array(p.R, dtype=np.float64).reshape(4, 3, 3)
+    t = np.array(p.t, dtype=np.float64).reshape(4, 3)
+    n = np.array(p.n, dtype=np.float64).reshape(4, 3)
+    d = np.array(p.d, dtype=np.float64)
+    return [(R[i], t[i], n[i], float(d[i])) for i in range(1 if p.rotation_only else 4)]
+
+
+def decompose_homography_arrays(H, camera_matrix, rotation_tolerance: float = 1e-2,
+                                engine: Optional[_native.Engine] = None) -> HomographyDecomposition:
+    """Relative pose and plane candidates of a homography H (3x3, image-A pixels -> image-B pixels) for cameras with
+    intrinsics ``camera_matrix``.  The order of the four candidates depends on eigenvector signs; compare them as a
+    set."""
+    eng = engine or _native.get_engine()
+    p = eng.decompose_homography(H, camera_matrix, rotation_tolerance)
+    return HomographyDecomposition(candidates=_candidates(p), singular_values=np.array(p.sv, dtype=np.float64),
+                                   rotation_only=bool(p.rotation_only))
+
+
+@dataclasses.dataclass
+class HomographyTwoViewResult:
+    ransac: HomographyResult
+    R: np.ndarray                 # (3,3) voted rotation (the nearest rotation to K^-1 H K when rotation_only)
+    t: np.ndarray                 # (3,) unit translation; 0 when rotation_only
+    n: np.ndarray                 # (3,) plane normal, camera-1 frame; NaN when rotation_only
+    d: float                      # plane distance in units of the baseline; inf when rotation_only
+    rotation_only: bool
+    candidates: list              # [(R, t, n, d)] as decompose_homography_arrays returns them
+    counts: np.ndarray            # cheirality votes per candidate (zeros when rotation_only)
+    inlier_indices: np.ndarray    # ascending indices of the winner's inliers (samples included)
+    passing: np.ndarray           # bool per inlier: passes the voted candidate (all False when rotation_only)
+    points: np.ndarray            # [m,3] triangulated points (NaN where not passing)
+
+
+def two_view_homography_arrays(
+    camera_matrix,
+    pts_a,
+    pts_b,
+    threshold: float,
+    min_num_extra_inliers=None,
+    error_aggregation_method=None,
+    max_iterations: Optional[int] = None,
+    distance_threshold=None,
+    *,
+    rotation_tolerance: float = 1e-2,
+    sampler: str = "reference",
+    seed: int = 0,
+    selection: str = "min_error",
+    engine: Optional[_native.Engine] = None,
+    table: Optional[np.ndarray] = None,
+) -> HomographyTwoViewResult:
+    """RANSAC homography -> pose and plane candidates -> cheirality vote -> triangulation, for [n,2] pixel arrays.
+
+    The RANSAC part (``ransac``) is ``ransac_homography_arrays`` on the same arguments, random state included.  Every
+    inlier of the winner is triangulated under each candidate (K-normalised coordinates, P1 = [I|0], P2 = [R|t]); it
+    passes when both depths are >= -1e-8 and |X| <= ``distance_threshold`` (default 50), every passing inlier counts,
+    and the first maximum wins.  The passing inliers are triangulated in pixel coordinates (P1 = K[I|0], P2 = K[R|t]).
+    Raises EightPointCalculationError when no inlier passes any candidate.  With ``sampler="device"`` the estimate and
+    the tail are one library call."""
+    if distance_threshold is None:
+        distance_threshold = 50.0
+    K = np.asarray(camera_matrix, dtype=np.float64)
+    if K.shape != (3, 3):
+        raise ValueError(f"Camera intrinsic matrix is not 3x3, actual shape: {K.shape}")
+    eng = engine or _native.get_engine()
+    pa = np.ascontiguousarray(pts_a, dtype=np.float64).reshape(-1, 2)
+    pb = np.ascontiguousarray(pts_b, dtype=np.float64).reshape(-1, 2)
+    iterations = 100 if max_iterations is None else int(max_iterations)
+    if sampler == "device" and pa.shape == pb.shape and pa.shape[0] >= 8 and iterations > 0:
+        # nothing on the host depends on the winner (no near-tie replay): estimate and tail in one call
+        min_extra = 0 if min_num_extra_inliers is None else min_num_extra_inliers
+        eng.upload_pairs(pa, pb, np.eye(3))  # K = I: the records hold pixel coordinates
+        eng.sample_device(seed, iterations)
+        best, mask, err, p, _, idx, ok, X = eng.two_view_homography(
+            K, threshold, float(min_extra), _agg_name(error_aggregation_method), selection, distance_threshold,
+            rotation_tolerance)
+        if best.index < 0:
+            raise ValueError(f"No model could be found with at least {min_extra + _SAMPLE} inliers.")
+        sample = np.array(best.sample[:_SAMPLE], dtype=np.int32)
+        extra = idx[~np.isin(idx, sample)]  # the tail's list = decision | samples, ascending
+        res = HomographyResult(H=np.array(best.E, dtype=np.float64).reshape(3, 3), best_index=int(best.index),
+                               error=float(best.err), count_extra=int(best.count_extra),
+                               inlier_indices=np.concatenate([sample.astype(np.int64), extra]), mask=mask.astype(bool),
+                               err=err, sample=sample, num_invalid=int(best.num_invalid),
+                               first_invalid=int(best.first_invalid))
+    else:
+        res = ransac_homography_arrays(pa, pb, threshold, min_num_extra_inliers, error_aggregation_method, max_iterations,
+                                       sampler=sampler, seed=seed, selection=selection, engine=eng, table=table)
+        eng.set_winner(res.best_index)  # the host's winner (a near-tie replay may have moved it)
+        p, _, idx, ok, X = eng.homography_pose_and_triangulate(K, threshold, distance_threshold, rotation_tolerance)
+    cands = _candidates(p)
+    counts = np.array(p.counts, dtype=np.int64)
+    if p.rotation_only:
+        R, t, n, d = cands[0]
+        passing = np.zeros(len(idx), dtype=bool)
+    else:
+        if 0 == np.count_nonzero(counts):
+            raise EightPointCalculationError("None of the transformations pass the cheirality check.")
+        R, t, n, d = cands[int(p.best)]
+        passing = ((ok >> int(p.best)) & 1).astype(bool)
+    return HomographyTwoViewResult(ransac=res, R=R.copy(), t=t.copy(), n=n.copy(), d=d,
+                                   rotation_only=bool(p.rotation_only), candidates=cands, counts=counts,
+                                   inlier_indices=idx, passing=passing, points=X)

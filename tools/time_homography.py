@@ -10,7 +10,11 @@ Prints one JSON line: evaluations/s of the scorer and of the whole estimate, the
 implied by the 27 counted FP64 slots per evaluation (against sfm_measure_fp64_peak), the stage times, and the GPU's
 name, power limit and maximum SM clock read in the same run.
 
-    python tools/time_homography.py [--steps 20] [--warmup 3] [--out FILE]
+--tail times the fused call sfm_two_view_homography instead: the same estimate followed by the pose tail (T1 inlier
+mask + compaction + decomposition of K^-1 H K, T2 cheirality vote, T3 triangulation) and the copies of the mask, the
+errors and the per-inlier results to the host.  The stage times "mask", "pose" and "triangulate" are T1, T2 and T3.
+
+    python tools/time_homography.py [--steps 20] [--warmup 3] [--tail] [--out FILE]
 """
 from __future__ import annotations
 
@@ -40,6 +44,7 @@ def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--tail", action="store_true", help="time estimate + pose tail (sfm_two_view_homography)")
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
     args = ap.parse_args()
 
@@ -57,13 +62,19 @@ def main() -> None:
     eng.set_stream(stream.cuda_stream)  # the flush, the events and the engine in one stream order
     flush_buf = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")  # > 126 MB of L2
 
-    _, x1, x2, H_true, _ = make_planar_scene(N, OUTLIERS, seed=0)
+    K, x1, x2, H_true, _ = make_planar_scene(N, OUTLIERS, seed=0)
     eng.upload_pairs(x1, x2, np.eye(3))
     peak_dfma = eng.measure_fp64_peak()
 
+    tail = {}
+
     def step(seed):
         eng.sample_device(seed, H)
-        best, *_ = eng.ransac_homography(THR, MIN_EXTRA, "rms", "min_error", want_mask=True)
+        if args.tail:
+            best, _, _, p, num, *_ = eng.two_view_homography(K, THR, MIN_EXTRA, "rms", "min_error")
+            tail.update(num_inliers=num, counts=list(p.counts), best=int(p.best), rotation_only=int(p.rotation_only))
+        else:
+            best, *_ = eng.ransac_homography(THR, MIN_EXTRA, "rms", "min_error", want_mask=True)
         if best.index < 0:
             raise RuntimeError("no model found")
         return best
@@ -97,7 +108,7 @@ def main() -> None:
     score_rate = evals / (stage["score"] * 1e-3)
     floor_rate = peak_dfma / SLOTS
     rec = {
-        "what": "homography RANSAC, planar scene",
+        "what": "homography RANSAC + pose tail, planar scene" if args.tail else "homography RANSAC, planar scene",
         "n": N, "h": H, "outlier_frac": OUTLIERS, "threshold_px2": THR, "min_extra": MIN_EXTRA, "sampler": "device",
         "steps": args.steps, "l2": "flushed before every step",
         "k_score_homography_ms": round(stage["score"], 4),
@@ -109,6 +120,7 @@ def main() -> None:
         "pipe_floor_evals_per_s": floor_rate,
         "share_of_pipe_floor": score_rate / floor_rate,
         "stage_ms": {k: round(v, 4) for k, v in stage.items()},
+        **({"tail_ms": round(stage["mask"] + stage["pose"] + stage["triangulate"], 4), "tail": tail} if args.tail else {}),
         "winner": {"index": int(best.index), "count_extra": int(best.count_extra), "error": float(best.err),
                    "rel_dev_from_true_H": float(np.max(np.abs(H_est - H_true)) / np.max(np.abs(H_true)))},
         "gpu": gpu_info(torch.cuda.current_device()),
