@@ -433,55 +433,62 @@ static int normalise_from(sfm_ctx* c, const double* xa, const double* ya, const 
     return check_launch(c, "k_normalise");
 }
 
-static int stage_raw(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
-                     int64_t stride, int64_t n, const double** dxa, const double** dya, const double** dxb,
-                     const double** dyb) {
-    if (int r = c->raw.reserve((size_t)n * 4 * sizeof(double))) return r;
-    double* d = c->raw.as<double>();
+// Host coordinates to the device buffer d (room for 4 n doubles) in the caller's layout: four arrays (stride 1) or two
+// interleaved [n][2] arrays (stride 2).  s[] = the device addresses of xa, ya, xb, yb.
+static int stage_coords(sfm_ctx* c, double* d, const double* xa, const double* ya, const double* xb, const double* yb,
+                        int64_t stride, int64_t n, const double* s[4]) {
     if (stride == 1) {
         const double* src[4] = {xa, ya, xb, yb};
         for (int k = 0; k < 4; ++k)
             CU(cudaMemcpyAsync(d + (size_t)k * n, src[k], (size_t)n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-        *dxa = d; *dya = d + n; *dxb = d + 2 * n; *dyb = d + 3 * n;
+        s[0] = d; s[1] = d + n; s[2] = d + 2 * n; s[3] = d + 3 * n;
     } else if (stride == 2 && ya == xa + 1 && yb == xb + 1) {
         CU(cudaMemcpyAsync(d, xa, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, c->stream));
         CU(cudaMemcpyAsync(d + 2 * n, xb, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-        *dxa = d; *dya = d + 1; *dxb = d + 2 * n; *dyb = d + 2 * n + 1;
+        s[0] = d; s[1] = d + 1; s[2] = d + 2 * n; s[3] = d + 2 * n + 1;
     } else {
         return fail(SFM_ERR_ARG, "unsupported layout: stride must be 1 (four arrays) or 2 (two interleaved [n][2] arrays)");
     }
+    return 0;
+}
+
+// the uploaded pixel coordinates, kept on the device for the triangulation tail
+static int stage_raw(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
+                     int64_t stride, int64_t n, const double* s[4]) {
+    if (int r = c->raw.reserve((size_t)n * 4 * sizeof(double))) return r;
+    if (int r = stage_coords(c, c->raw.as<double>(), xa, ya, xb, yb, stride, n, s)) return r;
     c->raw_stride = stride;
     return 0;
 }
 
+// One pair's correspondences from host memory (stride 1 or 2) or from device memory (any stride, packed to stride 1).
 static int upload_pairs_impl(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
-                             int64_t stride, int64_t n, const double* K, bool sync);
-
-int sfm_upload_pairs(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
-                     int64_t stride, int64_t n, const double* K) {
-    return upload_pairs_impl(c, xa, ya, xb, yb, stride, n, K, true);
-}
-
-int sfm_upload_pairs_async(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
-                           int64_t stride, int64_t n, const double* K) {
-    return upload_pairs_impl(c, xa, ya, xb, yb, stride, n, K, false);
-}
-
-static int upload_pairs_impl(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
-                             int64_t stride, int64_t n, const double* K, bool sync) {
+                             int64_t stride, int64_t n, const double* K, bool on_device, bool sync) {
     if (int r = use(c)) return r;
     if (!xa || !ya || !xb || !yb || !K) return fail(SFM_ERR_ARG, "null argument");
     if (n <= 0 || (uint64_t)n >= kMaxPoints) return fail(SFM_ERR_ARG, "need 0 < n < 2^25 correspondences, got %lld", (long long)n);
     c->tic(T_UPLOAD);
     c->batched = false;
     c->npairs = 1;
-    const double *dxa, *dya, *dxb, *dyb;
-    if (int r = stage_raw(c, xa, ya, xb, yb, stride, n, &dxa, &dya, &dxb, &dyb)) return r;
+    const double* s[4];
+    if (on_device) {
+        if (int r = c->raw.reserve((size_t)n * 4 * sizeof(double))) return r;
+        double* d = c->raw.as<double>();
+        const double* src[4] = {xa, ya, xb, yb};
+        for (int k = 0; k < 4; ++k) {
+            CU(cudaMemcpy2DAsync(d + (size_t)k * n, sizeof(double), src[k], (size_t)stride * sizeof(double),
+                                 sizeof(double), (size_t)n, cudaMemcpyDeviceToDevice, c->stream));
+            s[k] = d + (size_t)k * n;
+        }
+        c->raw_stride = stride = 1;
+    } else if (int r = stage_raw(c, xa, ya, xb, yb, stride, n, s)) {
+        return r;
+    }
     if (int r = c->Ks.reserve(9 * sizeof(double))) return r;
     memcpy(c->Khost, K, sizeof c->Khost);
     CU(cudaMemcpyAsync(c->Ks.p, c->Khost, 9 * sizeof(double), cudaMemcpyHostToDevice, c->stream));  // context-owned copy of K
     c->n = n;
-    if (int r = normalise_from(c, dxa, dya, dxb, dyb, stride, n, n)) return r;
+    if (int r = normalise_from(c, s[0], s[1], s[2], s[3], stride, n, n)) return r;
     c->toc(T_UPLOAD);
     // the coordinate copies read caller memory: finish before returning unless the caller took that on (_async)
     if (sync) CU(cudaStreamSynchronize(c->stream));
@@ -492,34 +499,19 @@ static int upload_pairs_impl(sfm_ctx* c, const double* xa, const double* ya, con
     return 0;
 }
 
+int sfm_upload_pairs(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
+                     int64_t stride, int64_t n, const double* K) {
+    return upload_pairs_impl(c, xa, ya, xb, yb, stride, n, K, false, true);
+}
+
+int sfm_upload_pairs_async(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
+                           int64_t stride, int64_t n, const double* K) {
+    return upload_pairs_impl(c, xa, ya, xb, yb, stride, n, K, false, false);
+}
+
 int sfm_upload_pairs_d(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
                        int64_t stride, int64_t n, const double* K) {
-    if (int r = use(c)) return r;
-    if (!xa || !ya || !xb || !yb || !K) return fail(SFM_ERR_ARG, "null argument");
-    if (n <= 0 || (uint64_t)n >= kMaxPoints) return fail(SFM_ERR_ARG, "need 0 < n < 2^25 correspondences, got %lld", (long long)n);
-    c->tic(T_UPLOAD);
-    c->batched = false;
-    c->npairs = 1;
-    if (int r = c->Ks.reserve(9 * sizeof(double))) return r;
-    memcpy(c->Khost, K, sizeof c->Khost);
-    CU(cudaMemcpyAsync(c->Ks.p, K, 9 * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-    c->n = n;
-    // keep a device copy of the pixel coordinates for the triangulation tail
-    if (int r = c->raw.reserve((size_t)n * 4 * sizeof(double))) return r;
-    double* d = c->raw.as<double>();
-    const double* src[4] = {xa, ya, xb, yb};
-    for (int k = 0; k < 4; ++k)
-        CU(cudaMemcpy2DAsync(d + (size_t)k * n, sizeof(double), src[k], (size_t)stride * sizeof(double),
-                             sizeof(double), (size_t)n, cudaMemcpyDeviceToDevice, c->stream));
-    c->raw_stride = 1;
-    if (int r = normalise_from(c, d, d + n, d + 2 * n, d + 3 * n, 1, n, n)) return r;
-    c->toc(T_UPLOAD);
-    CU(cudaStreamSynchronize(c->stream));
-    c->has_pts = true;
-    c->has_table = c->has_models = c->has_score = false;
-    c->table_pending = false;
-    c->winner_set = false;
-    return 0;
+    return upload_pairs_impl(c, xa, ya, xb, yb, stride, n, K, true, true);
 }
 
 int sfm_get_normalised(sfm_ctx* c, double* out, int64_t n) {
@@ -531,6 +523,10 @@ int sfm_get_normalised(sfm_ctx* c, double* out, int64_t n) {
 }
 
 // ---- fit ----------------------------------------------------------------------------------
+// K2's accumulator buffer is [kAccWords][H] planes followed by this tail, cleared with them: +0 work counter,
+// +8 rescore counter, +16 pilot totals, +24 pilot ticket, +32 mode, +64 K3 tickets [P]
+static size_t acc_tail_bytes(long long P) { return 64 + (size_t)P * 4; }
+
 static int fit_launch(sfm_ctx* c, bool want_eig) {
     if (!c->has_pts || !c->has_table) return fail(SFM_ERR_STATE, "fit needs correspondences and a sample table");
     const size_t H = (size_t)c->h * c->npairs;
@@ -540,8 +536,8 @@ static int fit_launch(sfm_ctx* c, bool want_eig) {
         if (int r = c->eig.reserve(H * 9 * sizeof(double))) return r;
     if (int r = reserve_zeroed(c, c->fitflag, 16)) return r;  // K3 resets it after use
     if (int r = c->rows.reserve(H * sizeof(ModelRow))) return r;
-    // K2's accumulators are cleared by the fit itself: layout [kAccWords][H] | work counter, rescore counter, tickets
-    const size_t acc_tail = 64 + (size_t)c->npairs * 4;
+    // K2's accumulators are cleared by the fit itself
+    const size_t acc_tail = acc_tail_bytes(c->npairs);
     if (int r = c->acc.reserve(H * kAccWords * 8 + acc_tail)) return r;
     if (want_eig)
         if (int r = ensure_table(c)) return r;  // the Jacobi kernel reads the table
@@ -621,6 +617,48 @@ int sfm_set_models(sfm_ctx* c, const double* E, const uint8_t* valid, int64_t h)
 }
 
 // ---- score + select ---------------------------------------------------------------------
+// K3's outputs for h hypotheses in each of P pairs.  Reserved before a scoring chain's first launch: a cudaMalloc
+// between chained launches would break the chain.
+static int reserve_selection(sfm_ctx* c, long long h, long long P) {
+    const size_t H = (size_t)h * P;
+    const int fblocks = (int)((h + 255) / 256);
+    if (int r = c->count_extra.reserve(H * 4)) return r;
+    if (int r = c->S1.reserve(H * 8)) return r;
+    if (int r = c->S2.reserve(H * 8)) return r;
+    if (int r = c->err.reserve(H * 8)) return r;
+    if (int r = c->blocks.reserve((size_t)fblocks * P * sizeof(Best))) return r;
+    if (int r = c->best.reserve((size_t)P * sizeof(Best))) return r;
+    if (int r = c->invalid.reserve((size_t)P * 16)) return r;
+    return 0;
+}
+
+// Work items of a persistent scoring launch: every (hypothesis block, pair) is split along the correspondences into
+// nsplit chunks of `chunk` (a multiple of the tile), aiming at target_items items in all, keeping >= min_tiles tiles per
+// item, and at most kMaxItemPoints correspondences per item so that 32-bit chunk sums cannot overflow.
+struct ItemSplit { long long chunk, nsplit; };
+static ItemSplit split_items(long long target_items, long long hyp_items, long long max_len, long long tile) {
+    const long long tiles = (max_len + tile - 1) / tile;
+    long long nsplit = (target_items + hyp_items - 1) / hyp_items;
+    constexpr int min_tiles = 2;  // 8 -> 2: mid-size pairs (config 2) get enough items to balance the warps (+6 %)
+    const long long max_split = tiles / min_tiles > 0 ? tiles / min_tiles : 1;
+    if (nsplit > max_split) nsplit = max_split;
+    const long long min_split = (max_len + kMaxItemPoints - 1) / kMaxItemPoints;
+    if (nsplit < min_split) nsplit = min_split;
+    if (nsplit < 1) nsplit = 1;
+    const long long chunk = ((tiles + nsplit - 1) / nsplit) * tile;
+    nsplit = (max_len + chunk - 1) / chunk;
+    if (nsplit < 1) nsplit = 1;
+    return {chunk, nsplit};
+}
+
+// The fit kernels leave the accumulators cleared; a second score of the same models (or of uploaded models) clears here.
+static int clear_acc(sfm_ctx* c, size_t H, long long P) {
+    if (!(c->acc_clean && c->acc_planes_for == H))
+        CU(cudaMemsetAsync(c->acc.p, 0, H * kAccWords * 8 + acc_tail_bytes(P), c->stream));
+    c->acc_clean = false;
+    return 0;
+}
+
 // K3 of a scoring call (essential matrices or homographies): finalise, rescore, select into the selection record
 static int finalise_launch(sfm_ctx* c, int kind, double thr, double min_extra, int agg, int mode, bool use_table,
                            long long idx_offset, int sums, int e2, int force_rescore, unsigned long long* acc_dev) {
@@ -694,14 +732,7 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
     const int G = (c->variant == SFM_SCORE_SCREEN32 && thr > 1e6) ? 16 : c->group;
     const long long hblocks = (h + 32ll * hpt - 1) / (32ll * hpt);  // groups of 32*hpt hypotheses (one per warp item)
     const size_t H = (size_t)h * P;
-    if (int r = c->count_extra.reserve(H * 4)) return r;
-    if (int r = c->S1.reserve(H * 8)) return r;
-    if (int r = c->S2.reserve(H * 8)) return r;
-    if (int r = c->err.reserve(H * 8)) return r;
-    const int fblocks = (int)((h + 255) / 256);
-    if (int r = c->blocks.reserve((size_t)fblocks * P * sizeof(Best))) return r;
-    if (int r = c->best.reserve((size_t)P * sizeof(Best))) return r;
-    if (int r = c->invalid.reserve((size_t)P * 16)) return r;
+    if (int r = reserve_selection(c, h, P)) return r;
     int e2 = 0;
     if (thr > 0.0 && !skip_k2) (void)frexp(thr, &e2);  // thr = m * 2^e2, m in [0.5, 1)  =>  thr < 2^e2
     if (e2 < -400) e2 = -400;
@@ -764,23 +795,11 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
         if (fn_full)
             if (int r = occupancy(fn_full, smem_two, &occ_full)) return r;
         const long long grid_blocks = (long long)c->sm_count * occ;
-        const long long tiles = (max_len + kTile - 1) / kTile;
         constexpr int items_per_warp = 32;  // 12 -> 32 shortens the end-of-launch tail (+1 % on config 3)
-        const long long target_items = grid_blocks * kScoreWarps * items_per_warp;
-        long long nsplit = (target_items + hblocks * P - 1) / (hblocks * P);
-        constexpr int min_tiles = 2;  // 8 -> 2: mid-size pairs (config 2) get enough items to balance the warps (+6 %)
-        const long long max_split = tiles / min_tiles > 0 ? tiles / min_tiles : 1;  // keep >= min_tiles x 64 correspondences per item
-        if (nsplit > max_split) nsplit = max_split;
-        const long long min_split = (max_len + kMaxItemPoints - 1) / kMaxItemPoints;  // 32-bit chunk sums cannot overflow
-        if (nsplit < min_split) nsplit = min_split;
-        if (nsplit < 1) nsplit = 1;
-        const long long chunk = ((tiles + nsplit - 1) / nsplit) * kTile;
-        nsplit = (max_len + chunk - 1) / chunk;
-        if (nsplit < 1) nsplit = 1;
+        const ItemSplit sp = split_items(grid_blocks * kScoreWarps * items_per_warp, hblocks * P, max_len, kTile);
+        const long long chunk = sp.chunk, nsplit = sp.nsplit;
         const long long total_items = hblocks * nsplit * P;
-        // tail of the accumulator buffer (zeroed with it): work counter | rescored counter | K3 tickets [P]
-        const size_t acc_tail = 64 + (size_t)P * 4;
-        if (int r = c->acc.reserve(H * kAccWords * 8 + acc_tail)) return r;
+        if (int r = c->acc.reserve(H * kAccWords * 8 + acc_tail_bytes(P))) return r;
         const long long npts = c->n;  // total records (all pairs)
         if (f32) { if (int r = c->spts.reserve((size_t)npts * sizeof(Corr32))) return r; }
         else if (screen) { if (int r = c->spts.reserve((size_t)npts * sizeof(Corr))) return r; }
@@ -808,15 +827,11 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
         a.htotal = (long long)H;
         a.acc = c->acc.as<unsigned long long>();
         a.work_counter = reinterpret_cast<unsigned*>(a.acc + H * kAccWords);
-        // tail words behind the planes: +0 work counter, +8 rescore counter, +16 pilot totals, +24 pilot ticket, +32 mode
-        char* tailp = reinterpret_cast<char*>(a.acc + H * kAccWords);
+        char* tailp = reinterpret_cast<char*>(a.acc + H * kAccWords);  // see acc_tail_bytes
         a.mode_flag = autov ? reinterpret_cast<const int*>(tailp + 32) : nullptr;
         acc_dev = a.acc;
         c->tic(T_SCORE);
-        // the fit kernel leaves the accumulators cleared; a second score of the same models (or uploaded models) clears here
-        if (!(c->acc_clean && c->acc_planes_for == H))
-            CU(cudaMemsetAsync(c->acc.p, 0, H * kAccWords * 8 + acc_tail, c->stream));
-        c->acc_clean = false;
+        if (int r = clear_acc(c, H, P)) return r;
         if (f32 && !skip_k2) {
             k_screen_pts32<<<(unsigned)((npts + 255) / 256), 256, 0, c->stream>>>(c->pts.as<Corr>(), npts, 1.0 / s_scale,
                                                                                   reinterpret_cast<Corr32*>(c->spts.p));
@@ -878,14 +893,9 @@ int sfm_score(sfm_ctx* c, double thr, double min_extra, int agg, int mode, int u
     return 0;
 }
 
-static int fetch_best(sfm_ctx* c, sfm_best* out) {
-    // k_select left {best, invalid counters, winning E} in one record: one copy, one synchronisation
-    if (int r = ensure_pinned(c, sizeof(SelectRecord))) return r;
-    CU(cudaMemcpyAsync(c->hpin, c->record.p, sizeof(SelectRecord), cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-    SelectRecord r;
-    memcpy(&r, c->hpin, sizeof r);
-    out->err = r.best.err;
+// a selection record as the ABI's sfm_best; without a winner (index < 0) the error reads inf
+static void unpack_best(const SelectRecord& r, sfm_best* out) {
+    out->err = r.best.idx >= 0 ? r.best.err : __builtin_inf();
     out->index = r.best.idx;
     out->count_extra = r.best.count;
     out->reserved = 0;
@@ -893,11 +903,19 @@ static int fetch_best(sfm_ctx* c, sfm_best* out) {
     out->first_invalid = r.first_invalid;
     memcpy(out->E, r.E, 72);
     memcpy(out->sample, r.sample, 32);
+}
+
+static int fetch_best(sfm_ctx* c, sfm_best* out) {
+    // k_select left {best, invalid counters, winning E} in one record: one copy, one synchronisation
+    if (int r = ensure_pinned(c, sizeof(SelectRecord))) return r;
+    CU(cudaMemcpyAsync(c->hpin, c->record.p, sizeof(SelectRecord), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    SelectRecord r;
+    memcpy(&r, c->hpin, sizeof r);
+    unpack_best(r, out);
     if (r.best.idx >= 0) {
         c->winner_local = r.best.idx - c->last_idx_offset;
         c->winner_set = true;
-    } else {
-        out->err = __builtin_inf();
     }
     return 0;
 }
@@ -1012,7 +1030,7 @@ static int fit_h_launch(sfm_ctx* c) {
     const long long h = c->h;
     if (int r = c->E.reserve((size_t)h * 72)) return r;
     if (int r = c->valid.reserve((size_t)h)) return r;
-    const size_t acc_tail = 64 + 4;  // work counter | rescore counter | K3 ticket, cleared with the planes
+    const size_t acc_tail = acc_tail_bytes(1);
     if (int r = c->acc.reserve((size_t)h * kAccWords * 8 + acc_tail)) return r;
     c->tic(T_FIT);
     CU(chain_launch(c, k_fit_homography, dim3((unsigned)((h + kFitHThreads - 1) / kFitHThreads)), dim3(kFitHThreads), 0,
@@ -1044,16 +1062,8 @@ static int score_h_launch(sfm_ctx* c, double thr, double min_extra, int agg, int
     int e2 = 0;
     if (thr > 0.0 && !skip_k2) (void)frexp(thr * (1.0 + 0x1p-20), &e2);
     if (e2 < -400) e2 = -400;
-    if (int r = c->count_extra.reserve((size_t)h * 4)) return r;
-    if (int r = c->S1.reserve((size_t)h * 8)) return r;
-    if (int r = c->S2.reserve((size_t)h * 8)) return r;
-    if (int r = c->err.reserve((size_t)h * 8)) return r;
-    const int fblocks = (int)((h + 255) / 256);
-    if (int r = c->blocks.reserve((size_t)fblocks * sizeof(Best))) return r;
-    if (int r = c->best.reserve(sizeof(Best))) return r;
-    if (int r = c->invalid.reserve(16)) return r;
-    const size_t acc_tail = 64 + 4;
-    if (int r = c->acc.reserve((size_t)h * kAccWords * 8 + acc_tail)) return r;
+    if (int r = reserve_selection(c, h, 1)) return r;
+    if (int r = c->acc.reserve((size_t)h * kAccWords * 8 + acc_tail_bytes(1))) return r;
     unsigned long long* acc = c->acc.as<unsigned long long>();
     const size_t smem = kHScoreWarps * sizeof(HScoreWarpSmem);
     if (!c->hscore_occ) {
@@ -1061,18 +1071,11 @@ static int score_h_launch(sfm_ctx* c, double thr, double min_extra, int agg, int
         CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, k_score_homography<kHScoreHpt>, kHScoreThreads, smem));
         c->hscore_occ = o > 0 ? o : 1;
     }
-    // persistent warps over (correspondence split, group of 32 * HPT hypotheses) items; an item holds at most
-    // kMaxItemPoints correspondences so that a lane's 32-bit chunk words cannot overflow
+    // persistent warps over (correspondence split, group of 32 * HPT hypotheses) items
     const long long grid_blocks = (long long)c->sm_count * c->hscore_occ;
     const long long hblocks = (h + 32ll * kHScoreHpt - 1) / (32ll * kHScoreHpt);
-    const long long tiles = (n + kHTile - 1) / kHTile;
-    long long nsplit = (grid_blocks * kHScoreWarps * 32 + hblocks - 1) / hblocks;
-    const long long max_split = tiles / 2 > 0 ? tiles / 2 : 1;
-    if (nsplit > max_split) nsplit = max_split;
-    const long long min_split = (n + kMaxItemPoints - 1) / kMaxItemPoints;
-    if (nsplit < min_split) nsplit = min_split;
-    const long long chunk = ((tiles + nsplit - 1) / nsplit) * kHTile;
-    nsplit = (n + chunk - 1) / chunk;
+    const ItemSplit sp = split_items(grid_blocks * kHScoreWarps * 32, hblocks, n, kHTile);
+    const long long chunk = sp.chunk, nsplit = sp.nsplit;
     HScoreArgs a;
     a.pts = c->pts.as<Corr>();
     a.H = c->E.as<double>();
@@ -1089,10 +1092,7 @@ static int score_h_launch(sfm_ctx* c, double thr, double min_extra, int agg, int
     a.work_counter = reinterpret_cast<unsigned*>(acc + (size_t)h * kAccWords);
     a.acc = acc;
     c->tic(T_SCORE);
-    // the fit kernel leaves the accumulators cleared; a second score of the same models clears here
-    if (!(c->acc_clean && c->acc_planes_for == (size_t)h))
-        CU(cudaMemsetAsync(c->acc.p, 0, (size_t)h * kAccWords * 8 + acc_tail, c->stream));
-    c->acc_clean = false;
+    if (int r = clear_acc(c, (size_t)h, 1)) return r;
     if (!skip_k2) {
         const long long want = (a.total_items + kHScoreWarps - 1) / kHScoreWarps;
         CU(chain_launch(c, k_score_homography<kHScoreHpt>, dim3((unsigned)(grid_blocks < want ? grid_blocks : want)),
@@ -1177,23 +1177,6 @@ int sfm_decompose_essential(sfm_ctx* c, const double* E, sfm_poses* out) {
 
 static int recover_pose_impl(sfm_ctx* c, const double* E, const double* K9, const double* xa, const double* ya,
                              const double* xb, const double* yb, int64_t stride, int64_t m, double dist_thr,
-                             sfm_poses* out, uint8_t* pass4);
-
-int sfm_recover_pose(sfm_ctx* c, const double* E, const double* xa, const double* ya, const double* xb,
-                     const double* yb, int64_t stride, int64_t m, double dist_thr, sfm_poses* out,
-                     uint8_t* pass4) {
-    return recover_pose_impl(c, E, nullptr, xa, ya, xb, yb, stride, m, dist_thr, out, pass4);
-}
-
-int sfm_recover_pose_pixels(sfm_ctx* c, const double* E, const double* K, const double* xa, const double* ya,
-                            const double* xb, const double* yb, int64_t stride, int64_t m, double dist_thr,
-                            sfm_poses* out, uint8_t* pass4) {
-    if (!K) return fail(SFM_ERR_ARG, "null camera matrix");
-    return recover_pose_impl(c, E, K, xa, ya, xb, yb, stride, m, dist_thr, out, pass4);
-}
-
-static int recover_pose_impl(sfm_ctx* c, const double* E, const double* K9, const double* xa, const double* ya,
-                             const double* xb, const double* yb, int64_t stride, int64_t m, double dist_thr,
                              sfm_poses* out, uint8_t* pass4) {
     if (int r = use(c)) return r;
     if (!E || !out) return fail(SFM_ERR_ARG, "null argument");
@@ -1216,20 +1199,9 @@ static int recover_pose_impl(sfm_ctx* c, const double* E, const double* K9, cons
         const double I[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
         memcpy(c->Kstage, K9 ? K9 : I, 72);  // staged in the context: the async copy must not read caller memory later
         CU(cudaMemcpyAsync(dK, c->Kstage, 72, cudaMemcpyHostToDevice, c->stream));
-        const double *sxa, *sya, *sxb, *syb;
-        if (stride == 1) {
-            const double* src[4] = {xa, ya, xb, yb};
-            for (int k = 0; k < 4; ++k)
-                CU(cudaMemcpyAsync(draw + (size_t)k * m, src[k], (size_t)m * 8, cudaMemcpyHostToDevice, c->stream));
-            sxa = draw; sya = draw + m; sxb = draw + 2 * m; syb = draw + 3 * m;
-        } else if (stride == 2 && ya == xa + 1 && yb == xb + 1) {
-            CU(cudaMemcpyAsync(draw, xa, (size_t)m * 16, cudaMemcpyHostToDevice, c->stream));
-            CU(cudaMemcpyAsync(draw + 2 * m, xb, (size_t)m * 16, cudaMemcpyHostToDevice, c->stream));
-            sxa = draw; sya = draw + 1; sxb = draw + 2 * m; syb = draw + 2 * m + 1;
-        } else {
-            return fail(SFM_ERR_ARG, "unsupported layout: stride must be 1 or 2");
-        }
-        k_normalise<<<dim3((unsigned)((m + 255) / 256), 1), 256, 0, c->stream>>>(sxa, sya, sxb, syb, stride, m, nullptr, dK, dpts, nullptr);
+        const double* s[4];
+        if (int r = stage_coords(c, draw, xa, ya, xb, yb, stride, m, s)) return r;
+        k_normalise<<<dim3((unsigned)((m + 255) / 256), 1), 256, 0, c->stream>>>(s[0], s[1], s[2], s[3], stride, m, nullptr, dK, dpts, nullptr);
         if (int r = check_launch(c, "k_normalise")) return r;
         k_cheirality<<<(unsigned)((4 * m + 127) / 128), 128, 0, c->stream>>>(dpts, m, nullptr, nullptr, c->poses.as<PoseSet>(),
                                                                         dist_thr, c->pass.as<uint8_t>(), nullptr);
@@ -1242,6 +1214,19 @@ static int recover_pose_impl(sfm_ctx* c, const double* E, const double* K9, cons
     if (pass4 && m > 0) CU(cudaMemcpyAsync(pass4, c->pass.p, (size_t)m, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     return 0;
+}
+
+int sfm_recover_pose(sfm_ctx* c, const double* E, const double* xa, const double* ya, const double* xb,
+                     const double* yb, int64_t stride, int64_t m, double dist_thr, sfm_poses* out,
+                     uint8_t* pass4) {
+    return recover_pose_impl(c, E, nullptr, xa, ya, xb, yb, stride, m, dist_thr, out, pass4);
+}
+
+int sfm_recover_pose_pixels(sfm_ctx* c, const double* E, const double* K, const double* xa, const double* ya,
+                            const double* xb, const double* yb, int64_t stride, int64_t m, double dist_thr,
+                            sfm_poses* out, uint8_t* pass4) {
+    if (!K) return fail(SFM_ERR_ARG, "null camera matrix");
+    return recover_pose_impl(c, E, K, xa, ya, xb, yb, stride, m, dist_thr, out, pass4);
 }
 
 int sfm_triangulate(sfm_ctx* c, const double* P1, const double* P2, const double* xa, const double* ya,
@@ -1257,20 +1242,9 @@ int sfm_triangulate(sfm_ctx* c, const double* P1, const double* P2, const double
     double* draw = dP + 24;
     CU(cudaMemcpyAsync(dP, P1, 96, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(dP + 12, P2, 96, cudaMemcpyHostToDevice, c->stream));
-    const double *sxa, *sya, *sxb, *syb;
-    if (stride == 1) {
-        const double* src[4] = {xa, ya, xb, yb};
-        for (int k = 0; k < 4; ++k)
-            CU(cudaMemcpyAsync(draw + (size_t)k * m, src[k], (size_t)m * 8, cudaMemcpyHostToDevice, c->stream));
-        sxa = draw; sya = draw + m; sxb = draw + 2 * m; syb = draw + 3 * m;
-    } else if (stride == 2 && ya == xa + 1 && yb == xb + 1) {
-        CU(cudaMemcpyAsync(draw, xa, (size_t)m * 16, cudaMemcpyHostToDevice, c->stream));
-        CU(cudaMemcpyAsync(draw + 2 * m, xb, (size_t)m * 16, cudaMemcpyHostToDevice, c->stream));
-        sxa = draw; sya = draw + 1; sxb = draw + 2 * m; syb = draw + 2 * m + 1;
-    } else {
-        return fail(SFM_ERR_ARG, "unsupported layout: stride must be 1 or 2");
-    }
-    k_triangulate<<<(unsigned)((m + 127) / 128), 128, 0, c->stream>>>(sxa, sya, sxb, syb, stride, m, nullptr, dP, dP + 12,
+    const double* s[4];
+    if (int r = stage_coords(c, draw, xa, ya, xb, yb, stride, m, s)) return r;
+    k_triangulate<<<(unsigned)((m + 127) / 128), 128, 0, c->stream>>>(s[0], s[1], s[2], s[3], stride, m, nullptr, dP, dP + 12,
                                                                       nullptr, nullptr, nullptr, 0, c->X.as<double>());
     if (int r = check_launch(c, "k_triangulate")) return r;
     c->toc(T_TRI);
@@ -1370,6 +1344,15 @@ static int host_winner_record(sfm_ctx* c, const SelectRecord** out) {
 // the per-inlier arrays ride along with the fixed-size results, so that the common case needs ONE synchronisation.
 constexpr long long kSpecInliers = 2048;
 
+// the first `take` entries of the tail's per-inlier arrays, straight from the device
+static int copy_inliers(sfm_ctx* c, long long take, int64_t* inlier_idx, uint8_t* pass, double* X) {
+    if (inlier_idx) CU(cudaMemcpyAsync(inlier_idx, c->idx.p, (size_t)take * 8, cudaMemcpyDeviceToHost, c->stream));
+    if (pass) CU(cudaMemcpyAsync(pass, c->pass.p, (size_t)take, cudaMemcpyDeviceToHost, c->stream));
+    if (X) CU(cudaMemcpyAsync(X, c->X.p, (size_t)take * 24, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
 static int pose_tail_fetch(sfm_ctx* c, sfm_poses* poses, int64_t cap, int64_t* num_inliers, int64_t* inlier_idx,
                            uint8_t* pass, double* X, sfm_best* best /* may be null */, HPlane* planes = nullptr) {
     const long long* cnt_dev = c->num.as<long long>();
@@ -1393,14 +1376,7 @@ static int pose_tail_fetch(sfm_ctx* c, sfm_poses* poses, int64_t cap, int64_t* n
     if (best) {
         SelectRecord r;
         memcpy(&r, hp + 64, sizeof r);
-        best->err = r.best.idx >= 0 ? r.best.err : __builtin_inf();
-        best->index = r.best.idx;
-        best->count_extra = r.best.count;
-        best->reserved = 0;
-        best->num_invalid = r.num_invalid;
-        best->first_invalid = r.first_invalid;
-        memcpy(best->E, r.E, 72);
-        memcpy(best->sample, r.sample, 32);
+        unpack_best(r, best);
         if (r.best.idx >= 0) {
             c->winner_local = r.best.idx - c->last_idx_offset;
             c->winner_set = true;
@@ -1415,10 +1391,7 @@ static int pose_tail_fetch(sfm_ctx* c, sfm_poses* poses, int64_t cap, int64_t* n
         if (pass) memcpy(pass, hp + o_pass, (size_t)take);
         if (X) memcpy(X, hp + o_X, (size_t)take * 24);
     } else if (take > 0) {
-        if (inlier_idx) CU(cudaMemcpyAsync(inlier_idx, c->idx.p, (size_t)take * 8, cudaMemcpyDeviceToHost, c->stream));
-        if (pass) CU(cudaMemcpyAsync(pass, c->pass.p, (size_t)take, cudaMemcpyDeviceToHost, c->stream));
-        if (X) CU(cudaMemcpyAsync(X, c->X.p, (size_t)take * 24, cudaMemcpyDeviceToHost, c->stream));
-        CU(cudaStreamSynchronize(c->stream));
+        return copy_inliers(c, take, inlier_idx, pass, X);
     }
     return 0;
 }
@@ -1447,6 +1420,17 @@ static void pack_hposes(const PoseSet& p, const HPlane& pl, sfm_hposes* out) {
     memcpy(out->counts, p.counts, sizeof out->counts);
     out->best = p.best;
     out->rotation_only = pl.rotation_only;
+}
+
+// pose_tail_fetch after a homography tail: the poses and the plane as one sfm_hposes
+static int hpose_tail_fetch(sfm_ctx* c, sfm_hposes* poses, int64_t cap, int64_t* num_inliers, int64_t* inlier_idx,
+                            uint8_t* pass, double* X, sfm_best* best /* may be null */) {
+    PoseSet p;
+    HPlane pl;
+    if (int r = pose_tail_fetch(c, reinterpret_cast<sfm_poses*>(&p), cap, num_inliers, inlier_idx, pass, X, best, &pl))
+        return r;
+    pack_hposes(p, pl, poses);
+    return 0;
 }
 
 static int hpose_args(const double* K, double rot_tol) {
@@ -1503,12 +1487,7 @@ int sfm_homography_pose_and_triangulate(sfm_ctx* c, const double* K, double thr,
     if (int r = host_winner_record(c, &rec)) return r;
     if (int r = hpose_stage_k(c, K)) return r;
     if (int r = pose_tail_launch(c, thr, dist_thr, rec, c->n, nullptr, nullptr, MODEL_H, rotation_tolerance)) return r;
-    PoseSet p;
-    HPlane pl;
-    if (int r = pose_tail_fetch(c, reinterpret_cast<sfm_poses*>(&p), cap, num_inliers, inlier_idx, pass, X, nullptr, &pl))
-        return r;
-    pack_hposes(p, pl, poses);
-    return 0;
+    return hpose_tail_fetch(c, poses, cap, num_inliers, inlier_idx, pass, X, nullptr);
 }
 
 int sfm_two_view_homography(sfm_ctx* c, const double* K, double thr, double min_extra, int agg, int mode, double dist_thr,
@@ -1527,12 +1506,7 @@ int sfm_two_view_homography(sfm_ctx* c, const double* K, double thr, double min_
     // T1's mask / err are those of sfm_homography_mask for the winner
     if (int r = pose_tail_launch(c, thr, dist_thr, c->record.as<SelectRecord>(), c->n, mask, err, MODEL_H, rotation_tolerance))
         return r;
-    PoseSet p;
-    HPlane pl;
-    if (int r = pose_tail_fetch(c, reinterpret_cast<sfm_poses*>(&p), cap, num_inliers, inlier_idx, pass, X, best, &pl))
-        return r;
-    pack_hposes(p, pl, poses);
-    return 0;
+    return hpose_tail_fetch(c, poses, cap, num_inliers, inlier_idx, pass, X, best);
 }
 
 int sfm_two_view_async(sfm_ctx* c, double thr, double min_extra, int agg, int mode, double dist_thr, uint8_t* mask,
@@ -1609,26 +1583,14 @@ int sfm_sharded_fetch(sfm_ctx* c, sfm_best* best, int32_t* owner, sfm_poses* pos
     memcpy(&r, (char*)c->hpin + 64, sizeof r);
     memcpy(&lb, (char*)c->hpin + 64 + sizeof r, sizeof lb);
     memcpy(&own, (char*)c->hpin + 64 + sizeof r + sizeof lb, sizeof own);
-    best->err = r.best.idx >= 0 ? r.best.err : __builtin_inf();
-    best->index = r.best.idx;  // GLOBAL hypothesis index
-    best->count_extra = r.best.count;
-    best->reserved = 0;
-    best->num_invalid = r.num_invalid;
-    best->first_invalid = r.first_invalid;
-    memcpy(best->E, r.E, 72);
-    memcpy(best->sample, r.sample, 32);
+    unpack_best(r, best);  // index: the GLOBAL hypothesis index
     *owner = own;
     c->winner_local = lb.idx >= 0 ? lb.idx : -1;  // -1: the model lives in winnerE
     c->winner_set = r.best.idx >= 0;
     if (r.best.idx < 0) m = 0;
     *num_inliers = m;
     const long long take = m < cap ? m : cap;
-    if (take > 0) {
-        if (inlier_idx) CU(cudaMemcpyAsync(inlier_idx, c->idx.p, (size_t)take * 8, cudaMemcpyDeviceToHost, c->stream));
-        if (pass) CU(cudaMemcpyAsync(pass, c->pass.p, (size_t)take, cudaMemcpyDeviceToHost, c->stream));
-        if (X) CU(cudaMemcpyAsync(X, c->X.p, (size_t)take * 24, cudaMemcpyDeviceToHost, c->stream));
-        CU(cudaStreamSynchronize(c->stream));
-    }
+    if (take > 0) return copy_inliers(c, take, inlier_idx, pass, X);
     return 0;
 }
 
@@ -1756,9 +1718,9 @@ static int batch_core(sfm_ctx* c, const double* xa, const double* ya, const doub
     if (int r = c->Ks.reserve((size_t)npairs * 72)) return r;
     CU(cudaMemcpyAsync(c->offsets.p, offsets, (size_t)(npairs + 1) * 8, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(c->Ks.p, Ks, (size_t)npairs * 72, cudaMemcpyHostToDevice, c->stream));
-    const double *dxa, *dya, *dxb, *dyb;
-    if (int r = stage_raw(c, xa, ya, xb, yb, stride, n, &dxa, &dya, &dxb, &dyb)) return r;
-    if (int r = normalise_from(c, dxa, dya, dxb, dyb, stride, n, max_len)) return r;
+    const double* s[4];
+    if (int r = stage_raw(c, xa, ya, xb, yb, stride, n, s)) return r;
+    if (int r = normalise_from(c, s[0], s[1], s[2], s[3], stride, n, max_len)) return r;
     c->toc(T_UPLOAD);
     c->has_pts = true;
     if (int r = sample_device(c, seed, pair_id0, 0, h)) return r;
@@ -1769,8 +1731,7 @@ static int batch_core(sfm_ctx* c, const double* xa, const double* ya, const doub
 }
 
 // per-pair winners of the last batch score -> host arrays (the selection records hold everything)
-static int batch_fetch_winners(sfm_ctx* c, int64_t npairs, double* E, int64_t* best_index, double* best_err,
-                               int32_t* count_extra, int64_t* num_invalid, size_t extra_pinned, char** extra) {
+static int batch_fetch_winners(sfm_ctx* c, int64_t npairs, size_t extra_pinned, char** extra) {
     const size_t rbytes = (size_t)npairs * sizeof(SelectRecord);
     if (int r = ensure_pinned(c, rbytes + extra_pinned + 64)) return r;
     char* hp = (char*)c->hpin;
@@ -1800,7 +1761,7 @@ int sfm_batch_ransac(sfm_ctx* c, const double* xa, const double* ya, const doubl
     long long max_len = 0;
     if (int r = batch_core(c, xa, ya, xb, yb, stride, offsets, npairs, Ks, h, seed, pair_id0, thr, min_extra, agg, mode,
                            &max_len)) return r;
-    if (int r = batch_fetch_winners(c, npairs, E, best_index, best_err, count_extra, num_invalid, 0, nullptr)) return r;
+    if (int r = batch_fetch_winners(c, npairs, 0, nullptr)) return r;
     CU(cudaStreamSynchronize(c->stream));
     batch_unpack_winners((const char*)c->hpin, npairs, E, best_index, best_err, count_extra, num_invalid);
     c->has_score = false;  // per-hypothesis single-pair getters do not apply to batches
@@ -1841,7 +1802,7 @@ int sfm_batch_two_view(sfm_ctx* c, const double* xa, const double* ya, const dou
     if (int r = check_launch(c, "k_batch_pack")) return r;
     char* extra = nullptr;
     const size_t pose_bytes = (size_t)npairs * sizeof(PoseSet);
-    if (int r = batch_fetch_winners(c, npairs, E, best_index, best_err, count_extra, num_invalid, pose_bytes, &extra)) return r;
+    if (int r = batch_fetch_winners(c, npairs, pose_bytes, &extra)) return r;
     CU(cudaMemcpyAsync(poses, c->poses.p, pose_bytes, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(inlier_offsets, d_off, (size_t)(npairs + 1) * 8, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));

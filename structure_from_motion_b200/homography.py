@@ -18,14 +18,14 @@ normalised homography below ``rotation_tolerance``) gets R, t = 0, no vote and n
 from __future__ import annotations
 
 import dataclasses
-import random
 from typing import Optional
 
 import numpy as np
 
 from . import _native
 from .errors import EightPointCalculationError
-from .two_view import _agg_name, _get_state_words, _reference_error, _resolve_near_ties, _set_state_words
+from .two_view import (_agg_name, _inlier_order, _load_samples, _replay_near_ties, _restore_random_state,
+                       _tail_inliers)
 
 _SAMPLE = 4  # points per minimal sample
 
@@ -90,12 +90,7 @@ def ransac_homography_arrays(
     if n < 8:
         raise ValueError(f"RANSAC homography needs at least 8 correspondences, got {n}")
     eng = engine or _native.get_engine()
-
-    if sampler == "reference":
-        version, words, gauss = _get_state_words()
-        ref_sampler = _native.ReferenceSampler(words, n, H)  # columns 0-3 = perm[:4], the shuffle is size-independent
-        table, words = ref_sampler.table, ref_sampler.final_state
-    elif sampler == "table":
+    if sampler == "table":
         table = np.ascontiguousarray(table, dtype=np.int32)
         if table.ndim != 2 or table.shape[1] not in (_SAMPLE, 8) or table.shape[0] == 0:
             raise ValueError(f"expected a [H,4] or [H,8] sample table, got shape {table.shape}")
@@ -104,62 +99,35 @@ def ransac_homography_arrays(
         H = table.shape[0]
 
     eng.upload_pairs(pts_a, pts_b, np.eye(3))  # K = I: the records hold pixel coordinates
-    if sampler == "device":
-        eng.sample_device(seed, H, hyp_offset=hyp_offset)
-    else:
-        eng.set_table(table)
+    # reference sampler: columns 0-3 = perm[:4], the shuffle is size-independent
+    table, ref = _load_samples(eng, sampler, n, H, table, seed, hyp_offset)
     best, mask, err, _, _ = eng.ransac_homography(threshold, float(min_num_extra_inliers), agg, selection)
-    if sampler == "reference":
-        _set_state_words(version, words, gauss)  # no exception aborts the loop: every shuffle happened
+    _restore_random_state(ref)  # no exception aborts the loop: every shuffle happened
     if best.index < 0:
         raise no_model()
-
-    def rows(t):
-        return np.asarray(table[t][:_SAMPLE], dtype=np.int64)
-
-    def order_after(t):
-        if sampler == "reference":
-            return ref_sampler.after(t)[1][_SAMPLE:].astype(np.int64)
-        keep = np.ones(n, dtype=bool)
-        keep[table[t][:_SAMPLE]] = False
-        return np.nonzero(keep)[0]
 
     def score(t):
         H_t, _ = eng.get_models(t, 1)
         return eng.homography_mask(H_t[0], threshold)
 
-    if sampler != "device" and selection == "min_error":
-        # near-ties are settled in the reference's list order and summation (SURVEY.md H1), as on the E path
-        ties, total = eng.near_ties(1e-12, 64)
-        if 1 < total <= 64:
-            t, e = _resolve_near_ties(eng, ties, threshold, agg, rows, order_after, score)
-            if t is not None and t != int(best.index):
-                H_t, _ = eng.get_models(t, 1)
-                best.index = t
-                best.E[:] = tuple(H_t.reshape(9))
-                m2, err = score(t)
-                mask = m2
-                best.count_extra = int(m2.sum() - m2[rows(t)].sum())
-                best.err = e
+    # near-ties are settled in the reference's list order and summation (SURVEY.md H1), as on the E path
+    t, e = _replay_near_ties(eng, sampler, selection, table, ref, n, _SAMPLE, threshold, agg, score) or (None, None)
+    if t is not None and t != int(best.index):
+        H_t, _ = eng.get_models(t, 1)
+        best.index = t
+        best.E[:] = tuple(H_t.reshape(9))
+        mask, err = score(t)
+        best.count_extra = int(mask.sum() - mask[table[t][:_SAMPLE]].sum())
+        best.err = e
 
     mask = np.asarray(mask).astype(bool)
-    local = int(best.index)
-    sample = np.array(best.sample[:_SAMPLE], dtype=np.int32)
-    if sampler != "device":
-        sample = np.asarray(table[local][:_SAMPLE], dtype=np.int32)
-    is_sample = np.zeros(n, dtype=bool)
-    is_sample[sample] = True
-    if sampler == "reference":
-        rest = order_after(local)  # the permutation of the winning iteration, replayed from the nearest snapshot
-        extra = rest[mask[rest]]
-    else:
-        extra = np.nonzero(mask & ~is_sample)[0]
+    sample, inliers = _inlier_order(best, sampler, table, ref, mask, _SAMPLE)
     return HomographyResult(
         H=np.array(best.E, dtype=np.float64).reshape(3, 3),
-        best_index=local + (hyp_offset if sampler == "device" else 0),
+        best_index=int(best.index) + (hyp_offset if sampler == "device" else 0),
         error=float(best.err),
         count_extra=int(best.count_extra),
-        inlier_indices=np.concatenate([sample.astype(np.int64), extra]),
+        inlier_indices=inliers,
         mask=mask,
         err=err,
         sample=sample,
@@ -278,11 +246,10 @@ def two_view_homography_arrays(
             rotation_tolerance)
         if best.index < 0:
             raise ValueError(f"No model could be found with at least {min_extra + _SAMPLE} inliers.")
-        sample = np.array(best.sample[:_SAMPLE], dtype=np.int32)
-        extra = idx[~np.isin(idx, sample)]  # the tail's list = decision | samples, ascending
+        sample, inliers = _tail_inliers(best, idx, _SAMPLE)
         res = HomographyResult(H=np.array(best.E, dtype=np.float64).reshape(3, 3), best_index=int(best.index),
                                error=float(best.err), count_extra=int(best.count_extra),
-                               inlier_indices=np.concatenate([sample.astype(np.int64), extra]), mask=mask.astype(bool),
+                               inlier_indices=inliers, mask=mask.astype(bool),
                                err=err, sample=sample, num_invalid=int(best.num_invalid),
                                first_invalid=int(best.first_invalid))
     else:

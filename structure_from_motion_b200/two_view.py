@@ -87,6 +87,80 @@ def _set_state_words(version, words, gauss):
     random.setstate((version, tuple(int(w) for w in words), gauss))
 
 
+def _load_samples(eng, sampler, n, h, table, seed, hyp_offset):
+    """The minimal samples of ``h`` hypotheses onto ``eng``, after its upload.  "reference" draws the table with
+    CPython's random.shuffle semantics from the process-global state but leaves that state alone (_restore_random_state
+    advances it once the caller knows how far the reference's loop ran); "device" draws on the GPU; "table" loads
+    ``table`` ([h,8]).  Returns (table, ref): ref = (ReferenceSampler, state version, gauss) or None."""
+    ref = None
+    if sampler == "reference":
+        version, words, gauss = _get_state_words()
+        ref = (_native.ReferenceSampler(words, n, h), version, gauss)
+        table = ref[0].table
+    if sampler == "device":
+        eng.sample_device(seed, h, hyp_offset=hyp_offset)
+    else:
+        eng.set_table(table)
+    return table, ref
+
+
+def _restore_random_state(ref, iteration=None):
+    """Leave the global random state where the reference's loop does: after every shuffle, or after the shuffle of
+    ``iteration`` when the loop stops there."""
+    if ref is not None:
+        sampler, version, gauss = ref
+        words = sampler.final_state if iteration is None else sampler.after(iteration)[0]
+        _set_state_words(version, words, gauss)
+
+
+def _replay_near_ties(eng, sampler, selection, table, ref, n, k, threshold, agg, score=None):
+    """The near-tie replay of ``_resolve_near_ties`` for a k-point sample, where the reference's list order is known:
+    the sample, then the rest of that iteration's permutation (reference sampler) or ascending (table).  Returns its
+    (local index, error), or None when it does not run: device sampler, other selections, or no 2..64 near-ties."""
+    if sampler == "device" or selection != "min_error":
+        return None
+    ties, total = eng.near_ties(1e-12, 64)
+    if not 1 < total <= 64:
+        return None
+
+    def rows(t):
+        return np.asarray(table[t][:k], dtype=np.int64)
+
+    def order_after(t):
+        if ref is not None:
+            return ref[0].after(t)[1][k:].astype(np.int64)
+        keep = np.ones(n, dtype=bool)
+        keep[table[t][:k]] = False
+        return np.nonzero(keep)[0]
+
+    return _resolve_near_ties(eng, ties, threshold, agg, rows, order_after, score)
+
+
+def _inlier_order(best, sampler, table, ref, mask, k):
+    """(sample int32[k], inlier indices int64) of the winner: the sample, then the other inliers in the reference's
+    order — the rest of the winning iteration's permutation (reference sampler) or ascending (table, device)."""
+    local = int(best.index)
+    if sampler == "device":
+        sample = np.array(best.sample[:k], dtype=np.int32)
+    else:
+        sample = np.asarray(table[local][:k], dtype=np.int32)
+    if ref is not None:
+        rest = ref[0].after(local)[1][k:].astype(np.int64)  # replayed from the nearest snapshot
+        extra = rest[mask[rest]]
+    else:
+        is_sample = np.zeros(mask.shape[0], dtype=bool)
+        is_sample[sample] = True
+        extra = np.nonzero(mask & ~is_sample)[0]
+    return sample, np.concatenate([sample.astype(np.int64), extra])
+
+
+def _tail_inliers(best, idx, k):
+    """(sample int32[k], inlier indices int64) of a winner selected on the device: the sample, then the rest of the
+    tail's compacted list (decision | sample, ascending)."""
+    sample = np.array(best.sample[:k], dtype=np.int32)
+    return sample, np.concatenate([sample.astype(np.int64), idx[~np.isin(idx, sample)]])
+
+
 def ransac_essential_arrays(
     camera_matrix,
     pts_a,
@@ -133,20 +207,12 @@ def ransac_essential_arrays(
             random.shuffle(list(range(n)))  # the reference shuffles once before the fitter raises
         raise ValueError("Eight feature pairs are expected.")  # epipolar_ransac.py:31-32
     eng = engine or _native.get_engine()
-
-    if sampler == "reference":
-        version, words, gauss = _get_state_words()
-        ref_sampler = _native.ReferenceSampler(words, n, H)
-        table, words = ref_sampler.table, ref_sampler.final_state
-    elif sampler == "table":
+    if sampler == "table":
         table = np.ascontiguousarray(table, dtype=np.int32).reshape(-1, 8)
         H = table.shape[0]
 
     eng.upload_pairs(pts_a, pts_b, camera_matrix)
-    if sampler == "device":
-        eng.sample_device(seed, H, hyp_offset=hyp_offset)
-    else:
-        eng.set_table(table)
+    table, ref = _load_samples(eng, sampler, n, H, table, seed, hyp_offset)
     if _tail is None:
         best, mask, sed = eng.ransac_essential(threshold, float(min_num_extra_inliers), agg, selection)
     else:  # two_view_arrays: selection, inlier mask, pose vote and triangulation in one C call
@@ -154,62 +220,34 @@ def ransac_essential_arrays(
                                               _tail["distance_threshold"])
         _tail["out"] = rest
 
-    if sampler == "reference":
-        if best.num_invalid > 0 and on_degenerate == "raise":
-            # the reference aborts inside iteration first_invalid: only that many shuffles happened
-            w, _ = ref_sampler.after(int(best.first_invalid))
-            _set_state_words(version, w, gauss)
-        else:
-            _set_state_words(version, words, gauss)
     if best.num_invalid > 0 and on_degenerate == "raise":
+        # the reference aborts inside iteration first_invalid: only that many shuffles happened
+        _restore_random_state(ref, int(best.first_invalid))
         raise EightPointCalculationError(EIGHT_POINT_ERROR_MESSAGE)  # eight_point.py:417-421
+    _restore_random_state(ref)
     if best.index < 0:
         raise no_model()
 
-    if sampler != "device" and selection == "min_error":
-        # H1: a definite list order exists (reference sampler: the permutation; table: samples then ascending), so
-        # near-ties are settled in the reference's own summation order
-        ties, total = eng.near_ties(1e-12, 64)
-        if total > 1 and total <= 64:
-            def rows(t):
-                return np.asarray(table[t], dtype=np.int64)
-
-            def order_after(t):
-                if sampler == "reference":
-                    return ref_sampler.after(t)[1][8:].astype(np.int64)
-                keep = np.ones(n, dtype=bool)
-                keep[table[t]] = False
-                return np.nonzero(keep)[0]
-
-            t, _ = _resolve_near_ties(eng, ties, threshold, agg, rows, order_after)
-            if t is not None and t != int(best.index):
-                E_t, _ = eng.get_models(t, 1)
-                best.index = t
-                best.E[:] = tuple(E_t.reshape(9))
-                eng.set_winner(t)
-                m2, sed = eng.inlier_mask(threshold)
-                mask = m2.astype(np.uint8)
-                best.count_extra = int(m2.sum() - m2[table[t]].sum())
-                errs = [float(v) for v in sed[rows(t)]] + [float(v) for v in sed[order_after(t)][sed[order_after(t)] <= threshold]]
-                best.err = _reference_error(errs, agg)
-                if _tail is not None:
-                    _tail["out"] = list(eng.pose_and_triangulate(threshold, _tail["distance_threshold"]))
-            else:
-                eng.set_winner(int(best.index))
+    # H1: near-ties are settled in the reference's own list order and summation
+    tie = _replay_near_ties(eng, sampler, selection, table, ref, n, 8, threshold, agg)
+    if tie is not None:
+        t, e = tie
+        if t is not None and t != int(best.index):
+            E_t, _ = eng.get_models(t, 1)
+            best.index = t
+            best.E[:] = tuple(E_t.reshape(9))
+            eng.set_winner(t)
+            m2, sed = eng.inlier_mask(threshold)
+            mask = m2.astype(np.uint8)
+            best.count_extra = int(m2.sum() - m2[table[t]].sum())
+            best.err = e
+            if _tail is not None:
+                _tail["out"] = list(eng.pose_and_triangulate(threshold, _tail["distance_threshold"]))
+        else:
+            eng.set_winner(int(best.index))
 
     mask = mask.astype(bool)
-    local = int(best.index)
-    sample = np.array(best.sample, dtype=np.int32) if sampler == "device" else table[local]
-    is_sample = np.zeros(n, dtype=bool)
-    is_sample[sample] = True
-    if sampler == "reference":
-        # inliers in the reference's order: samples, then the rest of that iteration's permutation
-        _, perm = ref_sampler.after(int(best.index))  # replayed from the nearest snapshot
-        rest = perm[8:].astype(np.int64)
-        extra = rest[mask[rest]]
-    else:
-        extra = np.nonzero(mask & ~is_sample)[0]
-    inliers = np.concatenate([np.asarray(sample, dtype=np.int64), extra])
+    sample, inliers = _inlier_order(best, sampler, table, ref, mask, 8)
     return RansacResult(
         E=np.array(best.E, dtype=np.float64).reshape(3, 3),
         best_index=int(best.index) + (hyp_offset if sampler == "device" else 0),
@@ -218,7 +256,7 @@ def ransac_essential_arrays(
         inlier_indices=inliers,
         mask=mask,
         sed=sed,
-        sample=np.asarray(sample, dtype=np.int32),
+        sample=sample,
         num_invalid=int(best.num_invalid),
         first_invalid=int(best.first_invalid),
     )
@@ -453,12 +491,11 @@ def _device_result(eng, mask, sed, min_extra, copy: bool) -> "TwoViewResult":
     counts = np.array(p.counts, dtype=np.int64)
     if 0 == np.count_nonzero(counts):
         raise EightPointCalculationError("None of the transformations pass the cheirality check.")
-    sample = np.array(best.sample, dtype=np.int32)
-    extra = idx[~np.isin(idx, sample)]  # the tail's compacted list = sed <= thr plus the samples, ascending
+    sample, inliers = _tail_inliers(best, idx, 8)
     b = int(p.best)
     res = RansacResult(E=np.array(best.E, dtype=np.float64).reshape(3, 3), best_index=int(best.index),
                        error=float(best.err), count_extra=int(best.count_extra),
-                       inlier_indices=np.concatenate([sample.astype(np.int64), extra]), mask=mask.astype(bool),
+                       inlier_indices=inliers, mask=mask.astype(bool),
                        sed=sed.copy() if copy else sed, sample=sample, num_invalid=int(best.num_invalid),
                        first_invalid=int(best.first_invalid))
     R = np.array(p.R, dtype=np.float64).reshape(4, 3, 3)[b].copy()

@@ -384,3 +384,58 @@ def test_near_tie_replay_with_a_scripted_engine():
     seds[9] = base.copy()
     t, e = two_view._resolve_near_ties(Fake(seds), [3, 7, 9], thr, "rms", rows, after)
     assert t == 3  # exact ties keep the earliest iteration
+
+
+def test_near_tie_replay_and_inlier_order_for_4_point_samples():
+    """The shared replay and inlier-order helpers at the homography path's sample size: the list order is the first
+    four table columns, then the rest (columns 4-7 are not part of the sample); the replay runs only for 2..64 near-ties
+    of min_error on a host-side sampler."""
+    import types
+
+    from structure_from_motion_b200 import two_view
+
+    class Fake:
+        def __init__(self, ties, total):
+            self.ties, self.total = ties, total
+
+        def near_ties(self, rel_tol, cap):
+            return np.array(self.ties), self.total
+
+    class Ref:  # ReferenceSampler.after(t) -> (state, permutation of iteration t); it starts with table[t][:4]
+        def after(self, t):
+            return None, np.array({1: [1, 2, 3, 4, 9, 8, 7, 6, 5, 0], 2: [2, 3, 4, 5, 9, 0, 7, 1, 6, 8]}[t])
+
+    n, thr = 10, 1.0
+    table = np.array([[t, t + 1, t + 2, t + 3, 9, 9, 9, 9] for t in range(4)], dtype=np.int32)
+    errs = {1: np.full(n, 0.5), 2: np.array([0.5, 2.0, 0.25, 0.5, 0.5, 0.5, 0.125, 0.5, 3.0, 0.0625])}
+    errs[1][9] = 0.0625 * (1 + 2 ** -45)
+    score = lambda t: (errs[t] <= thr, errs[t])  # noqa: E731
+
+    def list_order_error(t, rest):
+        e, inl = errs[t], errs[t] <= thr
+        return sum([float(v) for v in e[table[t][:4]]] + [float(v) for v in e[rest][inl[rest]]])
+
+    eng = Fake([1, 2], 2)
+    for ref, sampler in ((None, "table"), ((Ref(), 3, None), "reference")):
+        t, e = two_view._replay_near_ties(eng, sampler, "min_error", table, ref, n, 4, thr, "sum", score)
+        rest = {1: np.array([0, 5, 6, 7, 8, 9]), 2: np.array([0, 1, 6, 7, 8, 9])}
+        if ref is not None:
+            rest = {1: np.array([9, 8, 7, 6, 5, 0]), 2: np.array([9, 0, 7, 1, 6, 8])}
+        want = min((1, 2), key=lambda u: (list_order_error(u, rest[u]), u))
+        assert t == want and e == list_order_error(want, rest[want])
+    assert two_view._replay_near_ties(eng, "device", "min_error", table, None, n, 4, thr, "sum", score) is None
+    assert two_view._replay_near_ties(eng, "table", "max_inliers", table, None, n, 4, thr, "sum", score) is None
+    for total in (1, 65):
+        assert two_view._replay_near_ties(Fake([1], total), "table", "min_error", table, None, n, 4, thr, "sum",
+                                          score) is None
+
+    mask = errs[2] <= thr
+    best = types.SimpleNamespace(index=2, sample=[7, 0, 3, 5, 1, 2, 4, 6])
+    sample, inl = two_view._inlier_order(best, "table", table, None, mask, 4)
+    assert sample.dtype == np.int32 and sample.tolist() == [2, 3, 4, 5] and inl.tolist() == [2, 3, 4, 5, 0, 6, 7, 9]
+    sample, inl = two_view._inlier_order(best, "reference", table, (Ref(), 3, None), mask, 4)
+    assert sample.tolist() == [2, 3, 4, 5] and inl.tolist() == [2, 3, 4, 5, 9, 0, 7, 6]
+    sample, inl = two_view._inlier_order(best, "device", table, None, mask, 4)
+    assert sample.tolist() == [7, 0, 3, 5] and inl.tolist() == [7, 0, 3, 5, 2, 4, 6, 9]
+    sample, inl = two_view._tail_inliers(best, np.array([0, 2, 3, 5, 7, 9], dtype=np.int64), 4)
+    assert sample.tolist() == [7, 0, 3, 5] and inl.dtype == np.int64 and inl.tolist() == [7, 0, 3, 5, 2, 9]
