@@ -10,6 +10,10 @@ Every numeric stage runs in libsfm_b200.so on the GPU (no CPU fallback).
     python apps/sfm.py --synthetic 0                      # rendered image pair with known pose
     python apps/sfm.py --image1 a.npy --image2 b.npy --camera-matrix K.npy [--config apps/config/config.yaml]
     python apps/sfm.py --dataset-dir data/temple --index1 170 --index2 172      # Middlebury layout, as the reference
+
+--model auto estimates both the essential matrix and a homography from the filtered matches and keeps the pose of the
+one that ORB-SLAM's score ratio picks (structure_from_motion_b200.model_selection), so that planar scenes and
+rotation-only pairs get a pose too; --synthetic SEED --planar renders a scene that is one plane.
 """
 from __future__ import annotations
 
@@ -45,7 +49,9 @@ DEFAULT_CONFIG = {
     "ncc_window_size": 9,
     "ratio_test_threshold": 0.7,
     "match_score_threshold": 0.3,
-    "ransac": {"sed_inlier_threshold": 1.5e-6, "min_num_extra_inliers": 10, "max_iterations": 2000},
+    # homography_inlier_threshold: symmetric transfer error in px^2 (--model auto only; not a key of the reference)
+    "ransac": {"sed_inlier_threshold": 1.5e-6, "min_num_extra_inliers": 10, "max_iterations": 2000,
+               "homography_inlier_threshold": 4.0},
 }
 
 
@@ -62,6 +68,9 @@ class SfmResult:
     cam2_T_cam1: Transform3D
     world_points: np.ndarray
     seconds: dict
+    model: str = "essential"          # "homography" when --model auto picked it; e then holds H
+    homography_score_ratio: float = None  # S_H / (S_H + S_E) (--model auto)
+    rotation_only: bool = False
 
 
 def load_config(path=None, **overrides):
@@ -95,8 +104,34 @@ def _filter_matches(matches: List[matching.Match], score_threshold: float) -> Li
     return [m for m in matches if not (m.match_score > score_threshold)]
 
 
+def _run_selected(image_1_corners, image_2_corners, matches, camera_matrix, cfg, secs) -> SfmResult:
+    """--model auto: both models on the filtered matches, the pose and points of the one the score ratio picks."""
+    from structure_from_motion_b200.model_selection import two_view_select_arrays
+
+    logging.info("Estimating the Essential Matrix and a Homography")
+    t0 = time.perf_counter()
+    pts_a = np.array([[image_1_corners[m.a_index].x, image_1_corners[m.a_index].y] for m in matches],
+                     dtype=np.float64).reshape(-1, 2)
+    pts_b = np.array([[image_2_corners[m.b_index].x, image_2_corners[m.b_index].y] for m in matches],
+                     dtype=np.float64).reshape(-1, 2)
+    rc = cfg["ransac"]
+    sel = two_view_select_arrays(camera_matrix, pts_a, pts_b, rc["sed_inlier_threshold"],
+                                 rc["homography_inlier_threshold"], rc["min_num_extra_inliers"],
+                                 ErrorAggregationMethod.RMS, rc["max_iterations"])
+    secs["two_view"] = time.perf_counter() - t0
+    logging.info("Model: %s (homography score ratio %.3f)", sel.model, sel.scores.ratio_h)
+    model = sel.essential.ransac.E if sel.model == "essential" else sel.homography.ransac.H
+    pairs = [(image_1_corners[matches[int(i)].a_index], image_2_corners[matches[int(i)].b_index])
+             for i in sel.inlier_indices]
+    return SfmResult(image_1_corners, image_2_corners, matches, model, pairs, sel.R, sel.t, np.flatnonzero(sel.passing),
+                     Transform3D.from_rmat_t(sel.R, sel.t), sel.points[sel.passing], secs, model=sel.model,
+                     homography_score_ratio=sel.scores.ratio_h, rotation_only=sel.rotation_only)
+
+
 def run_sfm(image_1_gray: np.ndarray, image_2_gray: np.ndarray, camera_matrix: np.ndarray, cfg=None,
-            check_opencv: bool = False) -> SfmResult:
+            check_opencv: bool = False, model: str = "essential") -> SfmResult:
+    """model "essential": the reference's path.  "auto": the essential matrix and a homography, the pose of the one the
+    score ratio picks (the OpenCV cross-checks belong to the essential path and are not run)."""
     cfg = cfg or load_config()
     secs = {}
 
@@ -119,6 +154,8 @@ def run_sfm(image_1_gray: np.ndarray, image_2_gray: np.ndarray, camera_matrix: n
         ratio_test_threshold=cfg["ratio_test_threshold"])
     matches = _filter_matches(matches, cfg["match_score_threshold"])
     timed("matching", t0)
+    if model == "auto":
+        return _run_selected(image_1_corners, image_2_corners, matches, camera_matrix, cfg, secs)
 
     logging.info("Estimating Essential Matrix")
     t0 = time.perf_counter()
@@ -204,6 +241,9 @@ def main(argv=None):
     ap.add_argument("--config", default=os.path.join(ROOT, "apps", "config", "config.yaml"))
     ap.add_argument("--seed", type=int, default=None, help="random.seed() for the RANSAC sampler")
     ap.add_argument("--check-opencv", action="store_true")
+    ap.add_argument("--model", choices=["essential", "auto"], default="essential",
+                    help="essential: the essential matrix only; auto: pick between it and a homography")
+    ap.add_argument("--planar", action="store_true", help="with --synthetic: render one plane only")
     args = ap.parse_args(argv)
     logging.basicConfig(level=logging.INFO, format="%(message)s")
     cfg = load_config(args.config)
@@ -211,7 +251,7 @@ def main(argv=None):
     if args.synthetic is not None:
         from structure_from_motion_b200.scenes import make_image_pair
 
-        img1, img2, K, R, t = make_image_pair(args.synthetic)
+        img1, img2, K, R, t = make_image_pair(args.synthetic, planar=args.planar)
         truth = (R, t)
         cfg["ransac"].update(sed_inlier_threshold=1e-5, min_num_extra_inliers=60)  # integer-pixel corners at f = 520
     elif args.dataset_dir:
@@ -224,14 +264,17 @@ def main(argv=None):
         import random
 
         random.seed(args.seed)
-    res = run_sfm(img1, img2, K, cfg, check_opencv=args.check_opencv)
+    res = run_sfm(img1, img2, K, cfg, check_opencv=args.check_opencv, model=args.model)
     out = dict(corners=[len(res.corners_1), len(res.corners_2)], matches=len(res.matches),
                ransac_inliers=len(res.inlier_feature_pairs), cheirality_inliers=int(len(res.inlier_mask)),
                R=res.r.tolist(), t=res.t.tolist(), seconds=res.seconds)
+    if args.model == "auto":
+        out.update(model=res.model, homography_score_ratio=res.homography_score_ratio, rotation_only=res.rotation_only)
     if truth is not None:
         R, t = truth
         out["rotation_error_deg"] = float(np.degrees(np.arccos(np.clip((np.trace(res.r.T @ R) - 1) / 2, -1, 1))))
-        out["translation_angle_deg"] = float(np.degrees(np.arccos(np.clip(res.t @ t / np.linalg.norm(t) / np.linalg.norm(res.t), -1, 1))))
+        if not res.rotation_only:
+            out["translation_angle_deg"] = float(np.degrees(np.arccos(np.clip(res.t @ t / np.linalg.norm(t) / np.linalg.norm(res.t), -1, 1))))
     print(json.dumps(out))
     return res
 

@@ -283,6 +283,28 @@ int sfm_two_view_homography(sfm_ctx *ctx, const double *K, double threshold, dou
                             sfm_hposes *poses, int64_t cap, int64_t *num_inliers, int64_t *inlier_idx, uint8_t *pass,
                             double *X, uint8_t *mask, double *err);
 
+/* ---- essential matrix or homography for one pair ---------------------------------------
+ * The score ratio of ORB-SLAM (Mur-Artal, Montiel & Tardos, 2015, section IV) over the pixel correspondences of the
+ * current single-pair upload, whatever K that upload used.  E becomes F = K^-T E K^-1 (b^T E a = 0 as the SED uses it).
+ * One-way errors in px^2 per correspondence and image: for E the squared distance to the epipolar line (F a in image B,
+ * F^T b in image A), for H the transfer terms of the homography scorer (|x_b - pi(H x_a)|^2 and |x_a - pi(adj(H) x_b)|^2).
+ * rho(d2) = 5.99 - d2/sigma^2 when d2/sigma^2 < T (T_E = 3.84, T_H = 5.99), else 0 (also for NaN / inf errors); each rho is
+ * rounded to a multiple of 2^-32 and summed exactly: fixed_* are those sums, score_* = fixed_* * 2^-32.
+ * ratio_h = score_h / (score_h + score_e) (0 when both are 0); model = 1 (H) iff ratio_h > homography_ratio, and when only
+ * one of E and H is given (the other may be NULL) that one is chosen.  count_* = correspondences whose two errors both
+ * pass T (a diagnostic).  per_point (optional) double[n][4] = (d2_A,E, d2_B,E, d2_A,H, d2_B,H), NaN for a model not
+ * given.  SFM_ERR_ARG: E and H both NULL, a non-finite E or H, a singular or non-finite K, sigma not finite and > 0, a
+ * non-finite homography_ratio.  SFM_ERR_STATE: a batched context or no correspondences. */
+typedef struct sfm_model_scores {
+    double score_e, score_h, ratio_h;
+    uint64_t fixed_e, fixed_h;
+    int64_t count_e, count_h;
+    int32_t model;       /* 0 = E, 1 = H */
+    int32_t reserved;
+} sfm_model_scores;
+int sfm_score_models(sfm_ctx *ctx, const double *E, const double *H, const double *K, double sigma,
+                     double homography_ratio, sfm_model_scores *out, double *per_point);
+
 /* ---- batched image pairs (pair-sharded workloads) ------------------------------------ */
 /* P independent pairs; pair p owns correspondences [offsets[p], offsets[p+1]) of the
  * concatenated arrays, its own K (Ks[p][9]) and h hypotheses drawn by the device sampler

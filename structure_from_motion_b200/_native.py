@@ -44,6 +44,12 @@ class HPoses(C.Structure):
                 ("rotation_only", C.c_int32)]
 
 
+class ModelScores(C.Structure):
+    _fields_ = [("score_e", C.c_double), ("score_h", C.c_double), ("ratio_h", C.c_double), ("fixed_e", C.c_uint64),
+                ("fixed_h", C.c_uint64), ("count_e", C.c_int64), ("count_h", C.c_int64), ("model", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
 _P = C.c_void_p
 _SIGNATURES = {
     "sfm_version": (C.c_int, []),
@@ -97,6 +103,7 @@ _SIGNATURES = {
     "sfm_two_view_homography": (C.c_int, [_P, _P, C.c_double, C.c_double, C.c_int, C.c_int, C.c_double, C.c_double,
                                           C.POINTER(Best), C.POINTER(HPoses), C.c_int64, C.POINTER(C.c_int64), _P, _P,
                                           _P, _P, _P]),
+    "sfm_score_models": (C.c_int, [_P, _P, _P, _P, C.c_double, C.c_double, C.POINTER(ModelScores), _P]),
     "sfm_score_async": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.POINTER(_P)]),
     "sfm_sharded_tail": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_double, C.c_double]),
     "sfm_sharded_fetch": (C.c_int, [_P, C.POINTER(Best), C.POINTER(C.c_int32), C.POINTER(Poses), C.c_int64,
@@ -440,6 +447,19 @@ class Engine:
                                                   _ptr(mask), _ptr(err)), "sfm_two_view_homography")
         m = min(int(num.value), cap)
         return b, mask, err, p, int(num.value), idx[:m], ok[:m], X[:m]
+
+    # -- essential matrix or homography -------------------------------------------------------
+    def model_scores(self, E, H, K, sigma=1.0, homography_ratio=0.45, per_point=False):
+        """Scores of E and / or H (3x3 or None) on the current single-pair upload -> (ModelScores, per-point
+        [n,4] errors (d2_A,E, d2_B,E, d2_A,H, d2_B,H) in px^2 or None)."""
+        Ea = None if E is None else _f64(E).reshape(9)
+        Ha = None if H is None else _f64(H).reshape(9)
+        Ka = _f64(K).reshape(9)
+        s = ModelScores()
+        pp = np.empty((self.n, 4), dtype=np.float64) if per_point else None
+        self._ck(self.lib.sfm_score_models(self.h, _ptr(Ea), _ptr(Ha), _ptr(Ka), float(sigma), float(homography_ratio),
+                                           C.byref(s), _ptr(pp)), "sfm_score_models")
+        return s, pp
 
     # -- pose / triangulation ---------------------------------------------------------------
     def decompose_essential(self, E):

@@ -22,12 +22,14 @@
 #include "sfm_misc.cuh"
 #include "sfm_match.cuh"
 #include "sfm_harris.cuh"
+#include "sfm_select.cuh"
 
 using namespace sfm;
 
 static_assert(sizeof(Corr) == 32, "Corr must be 32 bytes");
 static_assert(sizeof(PoseSet) == sizeof(sfm_poses), "PoseSet/sfm_poses layout mismatch");
 static_assert(sizeof(SelectRecord) == SFM_RECORD_BYTES, "SelectRecord / SFM_RECORD_BYTES mismatch");
+static_assert(sizeof(ModelScores) == sizeof(sfm_model_scores), "ModelScores / sfm_model_scores layout mismatch");
 
 namespace {
 
@@ -99,6 +101,7 @@ struct sfm_ctx {
     Buf h_img, h_gx, h_gy, h_corner, h_alive, h_key, h_idx, h_small, h_xy;
     Buf mask, sed, poses, pass, X, idx, scan, tmp, tailstate, num, winrec, bout;
     Buf planes, hK;  // the homography tail's HPlane and the K it was called with (the upload's K stays in Ks)
+    Buf selstate, selpp;  // k_score_models: self-cleaning sums + result + E, H, K; the per-correspondence errors
     long long n = 0, h = 0, npairs = 1;
     long long first_len = 0;  // batched: correspondences of the first pair (what the AUTO pilot samples)
     long long raw_stride = 1;
@@ -112,6 +115,7 @@ struct sfm_ctx {
     size_t acc_planes_for = 0;  // hypotheses (all pairs) the cleared accumulators were laid out for
     double Kstage[9] = {0};
     double hstage[18] = {0};  // H and K of sfm_decompose_homography, K of the homography tail, staged for async copies
+    double sstage[27] = {0};  // E, H and K of sfm_score_models, staged for the async copy
     const void* occ_fn[4] = {nullptr, nullptr, nullptr, nullptr};  // scoring kernels whose launch configuration is cached
     int occ_blocks[4] = {0, 0, 0, 0};
     int occ_next = 0;
@@ -293,7 +297,7 @@ int sfm_destroy(sfm_ctx* c) {
     Buf* bufs[] = {&c->raw, &c->pts, &c->offsets, &c->Ks, &c->table, &c->E, &c->valid, &c->eig, &c->acc,
                    &c->count_extra, &c->S1, &c->S2, &c->err, &c->blocks, &c->best,
                    &c->invalid, &c->winnerE, &c->record, &c->merged, &c->rows, &c->blockinv, &c->mask, &c->sed, &c->poses, &c->pass, &c->X, &c->idx,
-                   &c->planes, &c->hK,
+                   &c->planes, &c->hK, &c->selstate, &c->selpp,
                    &c->scan, &c->tmp, &c->gathered, &c->tailstate, &c->num, &c->winrec, &c->bout, &c->spts, &c->bounds, &c->fitflag,
                    &c->m_img, &c->m_feat, &c->m_W, &c->m_ss, &c->m_ok, &c->m_S, &c->m_out,
                    &c->h_img, &c->h_gx, &c->h_gy, &c->h_corner, &c->h_alive, &c->h_key, &c->h_idx, &c->h_small, &c->h_xy};
@@ -450,6 +454,14 @@ static int stage_coords(sfm_ctx* c, double* d, const double* xa, const double* y
         return fail(SFM_ERR_ARG, "unsupported layout: stride must be 1 (four arrays) or 2 (two interleaved [n][2] arrays)");
     }
     return 0;
+}
+
+// the device addresses of xa, ya, xb, yb of the current single-pair upload in c->raw (element i at [i * raw_stride])
+static void raw_coords(const sfm_ctx* c, const double* s[4]) {
+    const double* d = c->raw.as<double>();
+    const long long n = c->n;
+    if (c->raw_stride == 1) { s[0] = d; s[1] = d + n; s[2] = d + 2 * n; s[3] = d + 3 * n; }
+    else { s[0] = d; s[1] = d + 1; s[2] = d + 2 * n; s[3] = d + 2 * n + 1; }
 }
 
 // the uploaded pixel coordinates, kept on the device for the triangulation tail
@@ -1289,9 +1301,9 @@ static int pose_tail_launch(sfm_ctx* c, double thr, double dist_thr, const Selec
     a.done = a.ticket + P;
     a.poses = c->poses.as<PoseSet>();
     a.pass = c->pass.as<uint8_t>();
-    const double* d = c->raw.as<double>();
-    if (c->raw_stride == 1) { a.xa = d; a.ya = d + n; a.xb = d + 2 * n; a.yb = d + 3 * n; }
-    else { a.xa = d; a.ya = d + 1; a.xb = d + 2 * n; a.yb = d + 2 * n + 1; }
+    const double* s[4];
+    raw_coords(c, s);
+    a.xa = s[0]; a.ya = s[1]; a.xb = s[2]; a.yb = s[3];
     a.stride = c->raw_stride;
     a.Ks = c->Ks.as<double>();
     a.X = c->X.as<double>();
@@ -1433,13 +1445,19 @@ static int hpose_tail_fetch(sfm_ctx* c, sfm_hposes* poses, int64_t cap, int64_t*
     return 0;
 }
 
-static int hpose_args(const double* K, double rot_tol) {
+// a camera matrix the homography pose and the model scores can invert
+static int check_camera(const double* K) {
     if (!K) return fail(SFM_ERR_ARG, "null camera matrix");
     for (int i = 0; i < 9; ++i)
         if (!std::isfinite(K[i])) return fail(SFM_ERR_ARG, "the camera matrix is not finite");
     const double det = K[0] * (K[4] * K[8] - K[5] * K[7]) - K[1] * (K[3] * K[8] - K[5] * K[6]) +
                        K[2] * (K[3] * K[7] - K[4] * K[6]);
     if (det == 0.0 || K[0] == 0.0 || K[4] == 0.0) return fail(SFM_ERR_ARG, "the camera matrix is singular");
+    return 0;
+}
+
+static int hpose_args(const double* K, double rot_tol) {
+    if (int r = check_camera(K)) return r;
     if (std::isnan(rot_tol)) return fail(SFM_ERR_ARG, "rotation_tolerance is NaN");
     return 0;
 }
@@ -1507,6 +1525,54 @@ int sfm_two_view_homography(sfm_ctx* c, const double* K, double thr, double min_
     if (int r = pose_tail_launch(c, thr, dist_thr, c->record.as<SelectRecord>(), c->n, mask, err, MODEL_H, rotation_tolerance))
         return r;
     return hpose_tail_fetch(c, poses, cap, num_inliers, inlier_idx, pass, X, best);
+}
+
+// ---- essential matrix or homography (sfm_select.cuh) --------------------------------------------
+int sfm_score_models(sfm_ctx* c, const double* E, const double* H, const double* K, double sigma, double homography_ratio,
+                     sfm_model_scores* out, double* per_point) {
+    if (int r = use(c)) return r;
+    if (!out) return fail(SFM_ERR_ARG, "out is null");
+    if (!E && !H) return fail(SFM_ERR_ARG, "give E, H or both");
+    for (int i = 0; i < 9; ++i) {
+        if (E && !std::isfinite(E[i])) return fail(SFM_ERR_ARG, "E is not finite");
+        if (H && !std::isfinite(H[i])) return fail(SFM_ERR_ARG, "H is not finite");
+    }
+    if (int r = check_camera(K)) return r;
+    if (!(sigma > 0.0) || !std::isfinite(sigma)) return fail(SFM_ERR_ARG, "sigma must be finite and > 0");
+    if (!std::isfinite(homography_ratio)) return fail(SFM_ERR_ARG, "homography_ratio is not finite");
+    if (c->batched) return fail(SFM_ERR_STATE, "single-pair call on a batched context");
+    if (!c->has_pts) return fail(SFM_ERR_STATE, "no correspondences loaded");
+    // selstate: +0 the kernel's sums and ticket (zero between launches), +64 the result, +128 E, H, K
+    if (int r = reserve_zeroed(c, c->selstate, 128 + sizeof c->sstage)) return r;
+    if (per_point)
+        if (int r = c->selpp.reserve((size_t)c->n * 32)) return r;
+    memset(c->sstage, 0, sizeof c->sstage);
+    if (E) memcpy(c->sstage, E, 72);
+    if (H) memcpy(c->sstage + 9, H, 72);
+    memcpy(c->sstage + 18, K, 72);
+    char* base = c->selstate.as<char>();
+    CU(cudaMemcpyAsync(base + 128, c->sstage, sizeof c->sstage, cudaMemcpyHostToDevice, c->stream));
+    SelectArgs a;
+    const double* s[4];
+    raw_coords(c, s);
+    a.xa = s[0]; a.ya = s[1]; a.xb = s[2]; a.yb = s[3];
+    a.stride = c->raw_stride;
+    a.n = c->n;
+    a.mats = reinterpret_cast<const double*>(base + 128);
+    a.have_e = E ? 1 : 0;
+    a.have_h = H ? 1 : 0;
+    a.sigma = sigma;
+    a.ratio = homography_ratio;
+    a.state = reinterpret_cast<unsigned long long*>(base);
+    a.out = reinterpret_cast<ModelScores*>(base + 64);
+    a.per_point = per_point ? c->selpp.as<double>() : nullptr;
+    const long long blocks = (c->n + kSelectBlock - 1) / kSelectBlock, cap = 4ll * c->sm_count;
+    k_score_models<<<(unsigned)(blocks < cap ? blocks : cap), kSelectBlock, 0, c->stream>>>(a);
+    if (int r = check_launch(c, "k_score_models")) return r;
+    CU(cudaMemcpyAsync(out, a.out, sizeof(ModelScores), cudaMemcpyDeviceToHost, c->stream));
+    if (per_point) CU(cudaMemcpyAsync(per_point, c->selpp.p, (size_t)c->n * 32, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
 }
 
 int sfm_two_view_async(sfm_ctx* c, double thr, double min_extra, int agg, int mode, double dist_thr, uint8_t* mask,

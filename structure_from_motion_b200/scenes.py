@@ -42,13 +42,15 @@ def make_scene(n: int, outlier_frac: float, seed: int, noise_px: float = 0.5,
     return K, np.ascontiguousarray(x1), np.ascontiguousarray(x2), R, t, idx
 
 
-def make_image_pair(seed: int = 0, h: int = 480, w: int = 640, f: float = 520.0, noise: float = 1.5):
+def make_image_pair(seed: int = 0, h: int = 480, w: int = 640, f: float = 520.0, noise: float = 1.5,
+                    planar: bool = False):
     """A synthetic grayscale image pair for the whole pipeline (detector -> matcher -> two-view geometry).
 
     The scene is three textured fronto-parallel layers at depths 8, 6 and 4.5 in front of camera 1 (so the
     correspondences are not coplanar); camera 2 = [R|t] with R = euler XYZ (1, -4, 0.5) deg, t = (-0.5, 0.02,
     0.05).  Image 1 is the texture; image 2 is rendered by inverse mapping through the plane-induced homographies
-    ``H_d = K (R + t n^T / d) K^-1`` (front layer first), bilinear sampling, plus Gaussian noise.
+    ``H_d = K (R + t n^T / d) K^-1`` (front layer first), bilinear sampling, plus Gaussian noise.  ``planar`` renders the
+    back layer (depth 8) over the whole image: every correspondence then lies on one plane.
     Returns (image_1 uint8[h,w], image_2 uint8[h,w], K, R, t).  numpy only."""
     rng = np.random.default_rng(seed)
     tex = np.full((h, w), 110.0)
@@ -64,6 +66,8 @@ def make_image_pair(seed: int = 0, h: int = 480, w: int = 640, f: float = 520.0,
     t = np.array([-0.5, 0.02, 0.05])
     # (depth, region in image-1 pixels [y0, y1, x0, x1]), front to back
     layers = [(4.5, (250, 440, 330, 600)), (6.0, (60, 300, 60, 320)), (8.0, (-10 ** 6, 10 ** 6, -10 ** 6, 10 ** 6))]
+    if planar:
+        layers = layers[-1:]
     ys, xs = np.mgrid[0:h, 0:w]
     p2 = np.stack([xs.ravel(), ys.ravel(), np.ones(h * w)]).astype(np.float64)
     out = np.zeros(h * w)
