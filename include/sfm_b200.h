@@ -253,7 +253,11 @@ int sfm_two_view_fetch(sfm_ctx *ctx, sfm_best *best, sfm_poses *poses, int64_t c
  * "An Invitation to 3-D Vision", Alg. 5.2, in the order (R+, T+, N+), (R+, -T+, -N+), (R-, T-, N-), (R-, -T-, -N-);
  * t = T / |T|, n = N, d = 1 / |T|.  The order of the four depends on eigenvector signs: compare candidate sets.
  * Rotation-only (sv[0] - sv[2] < rotation_tolerance, 1e-2 ~ 0.6 degrees of plane-induced parallax): all four slots hold
- * the rotation nearest to Hn with t = 0, n = NaN, d = inf; no vote, best = -1. */
+ * the rotation nearest to Hn with t = 0, n = NaN, d = inf; no vote, best = -1.
+ * Camera: every step reads pixels through the same K^-1 - the decomposition (K^-1 H K), the vote's rays
+ * (yn = (y - cy) / fy, xn = (x - cx - s yn) / fx with the skew s = K[0,1]) and the triangulation (P = K[R|t]).  K must
+ * therefore be upper triangular with K[2,2] = 1: the three calls below refuse any other K (a scaled one included) with
+ * SFM_ERR_ARG, as they refuse a singular or non-finite K.  The E path's (x - cx) / fx normalisation is unchanged. */
 typedef struct sfm_hposes {
     double R[4][9];
     double t[4][3];      /* unit; 0 when rotation_only                                    */
@@ -285,7 +289,10 @@ int sfm_two_view_homography(sfm_ctx *ctx, const double *K, double threshold, dou
 
 /* ---- essential matrix or homography for one pair ---------------------------------------
  * The score ratio of ORB-SLAM (Mur-Artal, Montiel & Tardos, 2015, section IV) over the pixel correspondences of the
- * current single-pair upload, whatever K that upload used.  E becomes F = K^-T E K^-1 (b^T E a = 0 as the SED uses it).
+ * current single-pair upload, whatever K that upload used.  E becomes F = Kd^-T E Kd^-1 (b^T E a = 0 as the SED uses
+ * it) with Kd = [[fx, 0, cx], [0, fy, cy], [0, 0, 1]] of K: the camera of the E path, whose (x - cx) / fx, (y - cy) / fy
+ * normalisation ignores the skew and the bottom row of K, so an E it estimated is scored in the coordinates it was
+ * fitted in.  H is scored in pixels and does not use K.
  * One-way errors in px^2 per correspondence and image: for E the squared distance to the epipolar line (F a in image B,
  * F^T b in image A), for H the transfer terms of the homography scorer (|x_b - pi(H x_a)|^2 and |x_a - pi(adj(H) x_b)|^2).
  * rho(d2) = 5.99 - d2/sigma^2 when d2/sigma^2 < T (T_E = 3.84, T_H = 5.99), else 0 (also for NaN / inf errors); each rho is

@@ -38,7 +38,7 @@ def _p(a):
 
 
 def fundamental(E, K):
-    """F = K^-T E K^-1 in the kernel's order."""
+    """F = Kd^-T E Kd^-1 (Kd = oracle.model_select.essential_camera(K)) in the kernel's order."""
     E, K = (np.ascontiguousarray(m, dtype=np.float64).reshape(9) for m in (E, K))
     F = np.empty(9, dtype=np.float64)
     lib().oracle_fundamental(_p(E), _p(K), _p(F))

@@ -134,3 +134,33 @@ def ransac_homography(xa, ya, xb, yb, threshold, min_num_extra_inliers=None, met
     if return_all:
         best.update(all_H=all_H, all_valid=all_valid, all_count=all_count, all_err=all_err)
     return best
+
+
+def expected_selection(models, valid, xa, ya, xb, yb, threshold, table, aggregation, selection, min_extra=0.0):
+    """What the GPU estimate must report for the given per-hypothesis models (H[h,3,3], valid[h]) and table: dict of
+    count_extra[h], S1[h], S2[h] (ctransfer.transfer_score_batch: samples never counted, always summed), err[h] (the
+    aggregated error, the MSAC cost sum_i min(value_i, thr) for selection "msac", inf for a non-candidate) and
+    winners: every index whose err (or count for "max_inliers") is the best one or within 1e-12 of it."""
+    valid = np.asarray(valid, dtype=bool)
+    cnt, s1, s2 = ctransfer.transfer_score_batch(models, xa, ya, xb, yb, threshold, table, valid.astype(np.uint8),
+                                                 nthreads=8)
+    n4 = 4.0 + cnt
+    with np.errstate(all="ignore"):
+        err = {"sum": s1, "square": s2, "mean": s1 / n4, "rms": np.sqrt(s2 / n4)}[aggregation].copy()
+    if selection == "msac":
+        for i in np.flatnonzero(valid):
+            m, v = ctransfer.transfer_exact_many(models[i], xa, ya, xb, yb, threshold)
+            err[i] = np.sum(np.where(m, v, threshold))
+    cand = valid & (min_extra <= cnt) & ~np.isnan(err)
+    err = np.where(cand, err, inf)
+    if not cand.any():
+        winners = np.array([-1])
+    elif selection == "max_inliers":
+        best = np.max(cnt[cand])
+        winners = np.array([int(np.flatnonzero(cand & (cnt == best))[0])])
+    else:
+        best = np.min(err)
+        winners = np.flatnonzero(cand & (np.abs(err - best) <= 1e-12 * np.abs(best)))
+        if not len(winners):  # an infinite minimum
+            winners = np.flatnonzero(cand & (err == best))
+    return dict(count_extra=cnt, S1=s1, S2=s2, err=err, winners=winners)

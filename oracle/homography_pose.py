@@ -2,9 +2,11 @@
 
 H (pixel coordinates, image A -> image B) -> Hn = K^-1 H K scaled to sigma_2 = 1 with det(Hn) > 0 -> the four
 (R, t, n, d) candidates of the SVD construction of Ma, Soatto, Kosecka & Sastry, "An Invitation to 3-D Vision",
-Algorithm 5.2 -> cheirality vote of the RANSAC inliers (oracle.restatement.cheirality_check, every passing inlier
-counts) -> DLT triangulation of the inliers that pass the voted candidate, in pixel coordinates.  A pair whose
-sigma_1 - sigma_3 is below the rotation tolerance is rotation-only: R is the rotation nearest to Hn, t = 0, no vote.
+Algorithm 5.2 -> cheirality vote of the RANSAC inliers (oracle.restatement.cheirality_check on K^-1 x, every passing
+inlier counts) -> DLT triangulation of the inliers that pass the voted candidate, in pixel coordinates.  All three
+steps use the same camera K, which must be upper triangular with K[2,2] = 1 (the library refuses any other).  A pair
+whose sigma_1 - sigma_3 is below the rotation tolerance is rotation-only: R is the rotation nearest to Hn, t = 0, no
+vote.
 
 Never imported by the product path.
 """
@@ -12,7 +14,7 @@ from __future__ import annotations
 
 import numpy as np
 
-from oracle.restatement import DEFAULT_DISTANCE_THRESHOLD, cheirality_check, k_normalise, triangulate_one
+from oracle.restatement import DEFAULT_DISTANCE_THRESHOLD, cheirality_check, triangulate_one
 
 ROTATION_TOLERANCE = 1e-2
 
@@ -56,14 +58,23 @@ def decompose_homography(H, K, rotation_tolerance=ROTATION_TOLERANCE):
     return dict(candidates=cands, sv=s, rotation_only=False)
 
 
+def k_inverse(x, y, K):
+    """K^-1 (x, y, 1) of an upper-triangular K with K[2,2] = 1, in the kernel's order: yn = (y - cy) / fy, then
+    xn = (x - cx - s yn) / fx with the skew s = K[0,1].  With s = 0 this is k_normalise, bit for bit."""
+    K = np.asarray(K, dtype=np.float64).reshape(3, 3)
+    fx, s, cx, fy, cy = K[0, 0], K[0, 1], K[0, 2], K[1, 1], K[1, 2]
+    yn = (np.asarray(y, dtype=np.float64) - cy) / fy
+    return ((np.asarray(x, dtype=np.float64) - cx) - s * yn) / fx, yn
+
+
 def vote(candidates, K, xa, ya, xb, yb, distance_threshold=None):
     """(pass bits uint8[m], counts[4], best) of the inliers (pixel coordinates) under the candidates: bit p = inlier
-    passes candidate p (oracle.restatement.cheirality_check on K-normalised coordinates); every passing inlier
+    passes candidate p (oracle.restatement.cheirality_check on the rays K^-1 x, k_inverse); every passing inlier
     counts; best = first maximum."""
     if distance_threshold is None:
         distance_threshold = DEFAULT_DISTANCE_THRESHOLD
-    nxa, nya = k_normalise(xa, ya, K)
-    nxb, nyb = k_normalise(xb, yb, K)
+    nxa, nya = k_inverse(xa, ya, K)
+    nxb, nyb = k_inverse(xb, yb, K)
     bits = np.zeros(len(nxa), dtype=np.uint8)
     for p, (R, t, _, _) in enumerate(candidates):
         for i in range(len(nxa)):

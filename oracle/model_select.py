@@ -1,8 +1,9 @@
 """TEST INFRASTRUCTURE ONLY — plain numpy restatement of the essential-matrix / homography choice.
 
 ORB-SLAM's score ratio (Mur-Artal, Montiel & Tardos, 2015, section IV) with the E winner as the pixel fundamental
-matrix F = K^-T E K^-1, written the way the formulas read, with no attention to evaluation order.  oracle/select_exact.c
-is the bit-exact checker of the kernel; this file checks that one against the formulas.
+matrix F = Kd^-T E Kd^-1 (Kd: K without skew, bottom row (0, 0, 1)), written the way the formulas read, with no
+attention to evaluation order.  oracle/select_exact.c is the bit-exact checker of the kernel; this file checks that one
+against the formulas.
 """
 from __future__ import annotations
 
@@ -11,8 +12,16 @@ import numpy as np
 GAMMA, T_E, T_H = 5.99, 3.84, 5.99
 
 
+def essential_camera(K):
+    """Kd = [[fx, 0, cx], [0, fy, cy], [0, 0, 1]] of K: the camera of the E path, whose normalisation (x - cx) / fx,
+    (y - cy) / fy ignores the skew and the bottom row of K."""
+    K = np.asarray(K, dtype=np.float64).reshape(3, 3)
+    return np.array([[K[0, 0], 0.0, K[0, 2]], [0.0, K[1, 1], K[1, 2]], [0.0, 0.0, 1.0]])
+
+
 def fundamental(E, K):
-    Ki = np.linalg.inv(np.asarray(K, dtype=np.float64))
+    """F = Kd^-T E Kd^-1 with Kd = essential_camera(K)."""
+    Ki = np.linalg.inv(essential_camera(K))
     return Ki.T @ np.asarray(E, dtype=np.float64) @ Ki
 
 

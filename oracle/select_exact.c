@@ -28,11 +28,13 @@ static void adj3(const double *h, double *a) {
     a[8] = fma(h[0], h[4], -(h[1] * h[3]));
 }
 
-/* F = K^-T E K^-1 with K^-1 = adj(K) / det(K) */
+/* F = Kd^-T E Kd^-1 with Kd^-1 = adj(Kd) / det(Kd), Kd = [[fx, 0, cx], [0, fy, cy], [0, 0, 1]] of K: the camera of the
+ * E path's (x - cx) / fx, (y - cy) / fy normalisation */
 void oracle_fundamental(const double *E, const double *K, double *F) {
+    const double kd[9] = {K[0], 0.0, K[2], 0.0, K[4], K[5], 0.0, 0.0, 1.0};
     double adj[9], ki[9], m[9];
-    adj3(K, adj);
-    const double det = fma(K[0], adj[0], fma(K[1], adj[3], K[2] * adj[6]));
+    adj3(kd, adj);
+    const double det = fma(kd[0], adj[0], fma(kd[1], adj[3], kd[2] * adj[6]));
     for (int i = 0; i < 9; ++i) ki[i] = adj[i] / det;
     for (int i = 0; i < 3; ++i)
         for (int j = 0; j < 3; ++j)

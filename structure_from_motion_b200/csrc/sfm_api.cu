@@ -1456,8 +1456,12 @@ static int check_camera(const double* K) {
     return 0;
 }
 
+// The homography pose reads pixels through K^-1 in three places (the decomposition, the vote's rays, the triangulation):
+// only an upper-triangular K with K[2,2] = 1 makes the vote's (x - cx - s yn) / fx the same camera as the other two.
 static int hpose_args(const double* K, double rot_tol) {
     if (int r = check_camera(K)) return r;
+    if (K[3] != 0.0 || K[6] != 0.0 || K[7] != 0.0 || K[8] != 1.0)
+        return fail(SFM_ERR_ARG, "the camera matrix must be upper triangular with K[2,2] = 1");
     if (std::isnan(rot_tol)) return fail(SFM_ERR_ARG, "rotation_tolerance is NaN");
     return 0;
 }

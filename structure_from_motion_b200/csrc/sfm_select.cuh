@@ -1,7 +1,8 @@
 // Choosing between the essential matrix and a homography for one image pair: the score ratio of ORB-SLAM (Mur-Artal,
 // Montiel & Tardos, 2015, section IV) over the uploaded pixel correspondences, in one launch.
 //
-// E is turned into the pixel fundamental matrix F = K^-T E K^-1 (the convention b^T E a = 0 of sed_exact).  Per
+// E is turned into the pixel fundamental matrix F = Kd^-T E Kd^-1 (the convention b^T E a = 0 of sed_exact), Kd = K
+// without its skew and with (0, 0, 1) as the bottom row: the camera E was fitted in.  Per
 // correspondence and image, one-way errors in px^2:
 //   E: r = b^T F a,  d2_B = r^2 / ((F a)_0^2 + (F a)_1^2),  d2_A = r^2 / ((F^T b)_0^2 + (F^T b)_1^2)
 //   H: d2_B = F/P, d2_A = G/Q of transfer_terms (sfm_device.cuh)
@@ -40,11 +41,11 @@ struct SelectArgs {
     double* per_point;           // [n][4] (d2_A,E, d2_B,E, d2_A,H, d2_B,H) or null
 };
 
-// F = K^-T E K^-1 with K^-1 = adj(K) / det(K); one thread
+// F = Kd^-T E Kd^-1 with Kd^-1 = adj(Kd) / det(Kd), Kd = [[fx, 0, cx], [0, fy, cy], [0, 0, 1]]: the camera of the
+// E path, whose (x - cx) / fx, (y - cy) / fy normalisation ignores the skew and the bottom row of K.  One thread.
 __device__ __forceinline__ void fundamental_from_essential(const double* E, const double* K, double (&F)[9]) {
-    double k[9], adj[9], ki[9], m[9];
-#pragma unroll
-    for (int i = 0; i < 9; ++i) k[i] = K[i];
+    const double k[9] = {K[0], 0.0, K[2], 0.0, K[4], K[5], 0.0, 0.0, 1.0};
+    double adj[9], ki[9], m[9];
     homography_adj(k, adj);
     const double det = __fma_rn(k[0], adj[0], __fma_rn(k[1], adj[3], __dmul_rn(k[2], adj[6])));
 #pragma unroll

@@ -232,7 +232,7 @@ __global__ void __launch_bounds__(128) k_tail_cheirality(const TailArgs a) {
     const long long pbase = a.offsets ? a.offsets[pair] : 0;
     const long long m = a.num[pair];
     PoseSet* poses = a.poses + pair;
-    double fx = 1.0, fy = 1.0, cx = 0.0, cy = 0.0;
+    double fx = 1.0, fy = 1.0, cx = 0.0, cy = 0.0, sk = 0.0;
     if constexpr (KIND == MODEL_H) {
         if (a.planes[pair].rotation_only) {  // no vote: nothing passes, best stays -1 and T3 writes NaN points
             for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < m; i += (long long)gridDim.x * blockDim.x)
@@ -240,7 +240,7 @@ __global__ void __launch_bounds__(128) k_tail_cheirality(const TailArgs a) {
             return;
         }
         const double* K = a.Ks + 9 * (long long)pair;
-        fx = K[0]; fy = K[4]; cx = K[2]; cy = K[5];
+        fx = K[0]; fy = K[4]; cx = K[2]; cy = K[5]; sk = K[1];
     }
     if (threadIdx.x < 4) s_cnt[threadIdx.x] = 0;
     __syncthreads();
@@ -253,11 +253,14 @@ __global__ void __launch_bounds__(128) k_tail_cheirality(const TailArgs a) {
         if (i < m) {
             const long long gi = a.idx[pbase + i];
             Corr c = a.pts[pbase + gi];
-            if constexpr (KIND == MODEL_H) {  // pixel records: k_normalise's operations (eight_point.py:127-133)
-                c.xa = __ddiv_rn(__dsub_rn(c.xa, cx), fx);
+            if constexpr (KIND == MODEL_H) {
+                // pixel records through K^-1, the camera the decomposition and T3 use (hpose_args has checked that K
+                // is upper triangular with K[2,2] = 1): y first, then x minus the skew's share.  With no skew this is
+                // k_normalise's (x - cx) / fx (eight_point.py:127-133), bit for bit.
                 c.ya = __ddiv_rn(__dsub_rn(c.ya, cy), fy);
-                c.xb = __ddiv_rn(__dsub_rn(c.xb, cx), fx);
                 c.yb = __ddiv_rn(__dsub_rn(c.yb, cy), fy);
+                c.xa = __ddiv_rn(__dsub_rn(__dsub_rn(c.xa, cx), __dmul_rn(sk, c.ya)), fx);
+                c.xb = __ddiv_rn(__dsub_rn(__dsub_rn(c.xb, cx), __dmul_rn(sk, c.yb)), fx);
             }
             const double P1[12] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0};  // Transform3D.identity() (:473)
             double P2[12];

@@ -18,14 +18,21 @@ def euler_xyz_intrinsic(deg_x: float, deg_y: float, deg_z: float) -> np.ndarray:
     return rx @ ry @ rz
 
 
+def _camera(K, f, w, h):
+    if K is None:
+        return np.array([[f, 0.0, w / 2], [0.0, f, h / 2], [0.0, 0.0, 1.0]])
+    return np.asarray(K, dtype=np.float64).reshape(3, 3).copy()
+
+
 def make_scene(n: int, outlier_frac: float, seed: int, noise_px: float = 0.5,
-               f: float = 800.0, w: int = 1280, h: int = 960):
+               f: float = 800.0, w: int = 1280, h: int = 960, K=None):
     """Return (K, x1[n,2], x2[n,2], R, t, outlier_idx) in pixel coordinates.
 
-    cam1 = [I|0]; cam2 = [R|t] with R = euler XYZ (2, -8, 1) deg, t = (-1, 0.05, 0.1).
+    cam1 = K[I|0]; cam2 = K[R|t] with R = euler XYZ (2, -8, 1) deg, t = (-1, 0.05, 0.1).  K defaults to
+    [[f, 0, w/2], [0, f, h/2], [0, 0, 1]]; any other (skewed, fx != fy) may be given.
     """
     rng = np.random.default_rng(seed)
-    K = np.array([[f, 0.0, w / 2], [0.0, f, h / 2], [0.0, 0.0, 1.0]])
+    K = _camera(K, f, w, h)
     X = np.column_stack([rng.uniform(-2, 2, n), rng.uniform(-1.5, 1.5, n), rng.uniform(4, 8, n)])
     R = euler_xyz_intrinsic(2.0, -8.0, 1.0)
     t = np.array([-1.0, 0.05, 0.1])
@@ -91,15 +98,15 @@ def make_image_pair(seed: int = 0, h: int = 480, w: int = 640, f: float = 520.0,
 
 
 def make_planar_scene(n: int, outlier_frac: float, seed: int, noise_px: float = 0.5, rotation_only: bool = False,
-                      f: float = 800.0, w: int = 1280, h: int = 960):
+                      f: float = 800.0, w: int = 1280, h: int = 960, K=None):
     """Return (K, x1[n,2], x2[n,2], H_true, outlier_idx) in pixel coordinates for points on one plane.
 
     The cameras are those of ``make_scene`` (cam1 = [I|0], cam2 = [R|t]; t = 0 when ``rotation_only``).  The points lie
     on the plane n^T X = d with n = unit(0.15, -0.1, 1), d = 6, tilted against both image planes and in front of both
     cameras; H_true = K (R + t n^T / d) K^-1 maps image-1 pixels to image-2 pixels (the construction of
-    ``make_image_pair``), divided by its [2,2] entry.  Noise and outliers as in ``make_scene``."""
+    ``make_image_pair``), divided by its [2,2] entry.  Noise, outliers and K as in ``make_scene``."""
     rng = np.random.default_rng(seed)
-    K = np.array([[f, 0.0, w / 2], [0.0, f, h / 2], [0.0, 0.0, 1.0]])
+    K = _camera(K, f, w, h)
     nrm = np.array([0.15, -0.1, 1.0])
     nrm /= np.linalg.norm(nrm)
     d = 6.0

@@ -1,5 +1,6 @@
 """CPU checks of the homography pose oracle (oracle/homography_pose.py): the decomposition against OpenCV and the
-truth, the rotation-only rule, t parallel to n, the sign fix, and the vote on a planar scene."""
+truth, the rotation-only rule, t parallel to n, the sign fix, the vote on a planar scene, and one camera K^-1 for
+every step (skewed and scaled K)."""
 import os
 import re
 
@@ -7,6 +8,7 @@ import numpy as np
 import pytest
 
 from oracle import homography_pose as hp
+from oracle.restatement import k_normalise as o_k_normalise
 from structure_from_motion_b200 import _native
 from structure_from_motion_b200.scenes import euler_xyz_intrinsic, make_planar_scene
 
@@ -141,3 +143,49 @@ def test_abi_declares_the_homography_pose_calls():
     declared = set(re.findall(r"\b(sfm_[a-z0-9_]+)\s*\(", re.sub(r"/\*.*?\*/", "", header, flags=re.S)))
     new = {"sfm_decompose_homography", "sfm_homography_pose_and_triangulate", "sfm_two_view_homography"}
     assert new <= declared and new <= set(_native.EXPORTED_SYMBOLS)
+
+
+# a skewed camera (fx != fy, shifted principal point): the decomposition, the vote's rays and the triangulation all
+# read pixels through the same K^-1
+K_SKEW = np.array([[800.0, 40.0, 610.0], [0.0, 790.0, 500.0], [0.0, 0.0, 1.0]])
+
+
+def test_k_inverse_is_k_normalise_without_skew_and_K_inv_with_it():
+    rng = np.random.default_rng(11)
+    x, y = rng.uniform(0, 1280, 1000), rng.uniform(0, 960, 1000)
+    K = K_SKEW.copy()
+    K[0, 1] = 0.0
+    xn, yn = hp.k_inverse(x, y, K)
+    xr, yr = o_k_normalise(x, y, K)
+    assert np.array_equal(xn, xr) and np.array_equal(yn, yr)  # bit for bit
+    xn, yn = hp.k_inverse(x, y, K_SKEW)
+    ray = np.linalg.solve(K_SKEW, np.vstack([x, y, np.ones_like(x)]))
+    assert np.max(np.abs(xn - ray[0])) < 1e-15 and np.max(np.abs(yn - ray[1])) < 1e-15
+
+
+@pytest.mark.parametrize("skew", [5.0, 40.0])
+def test_skewed_camera_truth_is_recovered(skew):
+    K = K_SKEW.copy()
+    K[0, 1] = skew
+    _, x1, x2, H, _ = make_planar_scene(300, 0.0, 3, noise_px=0.0, K=K)
+    ours = hp.decompose_homography(H, K)
+    bits, counts, best = hp.vote(ours["candidates"], K, x1[:, 0], x1[:, 1], x2[:, 0], x2[:, 1])
+    assert counts[best] == 300 and sorted(counts)[-2] < 300
+    R, t, n, d = ours["candidates"][best]
+    assert np.abs(R - euler_xyz_intrinsic(2.0, -8.0, 1.0)).max() < 1e-8
+    assert np.abs(t - T_TRUE / np.linalg.norm(T_TRUE)).max() < 1e-8 and np.abs(n - N_TRUE).max() < 1e-8
+    X = hp.triangulate(K, R, t, x1[:, 0], x1[:, 1], x2[:, 0], x2[:, 1], (bits >> best) & 1)
+    assert np.max(np.abs(X @ n - d)) / d < 1e-8
+
+
+def test_scaled_camera_gives_the_same_decomposition():
+    # K^-1 H K does not see the scale of K; only the vote's (x - cx) / fx would, which is why the library refuses a K
+    # whose K[2,2] is not 1
+    rng = np.random.default_rng(13)
+    for _ in range(20):
+        K, H, R, t, n, d = _random_pose(rng)
+        a = hp.decompose_homography(H, K)
+        b = hp.decompose_homography(H, 2.0 * K)
+        assert np.allclose(a["sv"], b["sv"], rtol=0, atol=1e-12)
+        for (Ra, ta, na, da), (Rb, tb, nb, db) in zip(a["candidates"], b["candidates"]):
+            assert max(np.abs(Ra - Rb).max(), np.abs(ta - tb).max(), np.abs(na - nb).max(), abs(da - db) / da) < 1e-9

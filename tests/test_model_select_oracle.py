@@ -1,5 +1,6 @@
 """CPU checks of the essential-matrix / homography choice: the C scorer (oracle/select_exact.c) against the numpy
-restatement (oracle/model_select.py) and OpenCV, and the rule's choice on scenes with known models."""
+restatement (oracle/model_select.py) and OpenCV, the rule's choice on scenes with known models, and F built from the E
+path's camera (no skew, bottom row (0, 0, 1)) for a skewed K."""
 import numpy as np
 import pytest
 
@@ -113,3 +114,47 @@ def test_one_model_is_chosen_whatever_the_scores():
     assert cselect.score_models(K, x1, x2, H=H, ratio=2.0)["model"] == 1
     assert cselect.score_models(K, x1, x2, E=E, ratio=-1.0)["model"] == 0
     assert ms.score_models(K, x1, x2, H=H, ratio=2.0)["model"] == 1
+
+
+# E is fitted in the E path's (x - cx) / fx, (y - cy) / fy coordinates, i.e. with the camera Kd = essential_camera(K):
+# F must be built from that camera, not from the full K^-1
+K_SKEW = np.array([[800.0, 40.0, 610.0], [0.0, 790.0, 500.0], [0.0, 0.0, 1.0]])
+
+
+def _kd_essential(K, R, t):
+    """The true E expressed in Kd coordinates, where the E path fits it: Kd^T K^-T [t]x R K^-1 Kd."""
+    Kd, Ki = ms.essential_camera(K), np.linalg.inv(K)
+    return Kd.T @ Ki.T @ _skew(t) @ R @ Ki @ Kd
+
+
+@pytest.mark.parametrize("skew", [5.0, 40.0])
+def test_c_scorer_matches_numpy_with_skew(skew):
+    K = K_SKEW.copy()
+    K[0, 1] = skew
+    K, x1, x2, R, t, _ = make_scene(2000, 0.3, 3, K=K)
+    E = _kd_essential(K, R, t)
+    _, H = _true_models(K, R, t)
+    c = cselect.score_models(K, x1, x2, E, H)
+    o = ms.score_models(K, x1, x2, E, H)
+    scale = _term_scales(K, x1, x2, E)
+    for j in range(4):
+        assert _rel_gap(c["per_point"][:, j], o["per_point"][:, j], scale[:, j]) <= 1e-12, j
+    assert c["count_e"] == o["count_e"] and c["count_h"] == o["count_h"]
+    assert abs(c["score_e"] - o["score_e"]) <= 1e-9 * o["score_e"]
+    # the true E scores its inliers: 1400 of 2000 correspondences are inliers, 0.5 px noise
+    assert c["count_e"] >= 0.95 * 1400
+
+
+def test_fundamental_uses_the_essential_camera():
+    K, _, _, E, _ = _scene("general", 0)
+    Kd = ms.essential_camera(K_SKEW)
+    assert np.array_equal(Kd, [[800.0, 0.0, 610.0], [0.0, 790.0, 500.0], [0.0, 0.0, 1.0]])
+    F = cselect.fundamental(E, K_SKEW)
+    Ki = np.linalg.inv(Kd)
+    assert np.max(np.abs(F - Ki.T @ E @ Ki)) <= 1e-12 * np.max(np.abs(F))
+    assert np.array_equal(cselect.fundamental(E, K_SKEW), cselect.fundamental(E, Kd))
+    # skew, K[1,0] and the bottom row are not read; a K that is its own Kd gives the same bits as before
+    Kb = K_SKEW.copy()
+    Kb[1, 0], Kb[2] = 3.0, (1e-3, 2e-3, 2.0)
+    assert np.array_equal(cselect.fundamental(E, Kb), cselect.fundamental(E, Kd))
+    assert np.array_equal(ms.fundamental(E, Kb), ms.fundamental(E, Kd))
