@@ -306,7 +306,7 @@ typedef struct sfm_model_scores {
     double score_e, score_h, ratio_h;
     uint64_t fixed_e, fixed_h;
     int64_t count_e, count_h;
-    int32_t model;       /* 0 = E, 1 = H */
+    int32_t model;       /* 0 = E, 1 = H, -1 = neither given (sfm_batch_score_models only) */
     int32_t reserved;
 } sfm_model_scores;
 int sfm_score_models(sfm_ctx *ctx, const double *E, const double *H, const double *K, double sigma,
@@ -336,6 +336,35 @@ int sfm_batch_two_view(sfm_ctx *ctx, const double *xa, const double *ya, const d
                        int selection, double distance_threshold, double *E, int64_t *best_index, double *best_err,
                        int32_t *count_extra, int64_t *num_invalid, sfm_poses *poses, int64_t *inlier_offsets,
                        int64_t cap, int32_t *inlier_idx, uint8_t *pass, double *X);
+
+/* sfm_batch_two_view for homographies: per pair, RANSAC H over the device sampler's rows (columns 0-3; stream =
+ * pair_id0 + p) in pixel coordinates, then the homography tail of sfm_two_view_homography with that pair's K (the
+ * decomposition of K^-1 H K, the vote, the triangulation).  Every Ks[p] must pass the checks of sfm_two_view_homography
+ * (finite, non-singular, upper triangular, K[2,2] = 1), else SFM_ERR_ARG naming the pair; rotation_tolerance must not be
+ * NaN.  Per pair, bit for bit what sfm_two_view_homography returns on that pair alone (uploaded with K = I, sampled with
+ * stream pair_id0 + p): H[p][9] (zeros without a model), best_index / best_err / count_extra / num_invalid as
+ * sfm_batch_two_view, poses[p] (best = -2: no model, -1: rotation-only), and the inlier list (the transfer decision plus
+ * the 4 sample points), pass bits and points packed as sfm_batch_two_view packs them.  A pair of fewer than 8
+ * correspondences has no model and an empty segment.  One synchronisation for the fixed-size results, one for the
+ * packed arrays. */
+int sfm_batch_two_view_homography(sfm_ctx *ctx, const double *xa, const double *ya, const double *xb, const double *yb,
+                                  int64_t stride, const int64_t *offsets, int64_t npairs, const double *Ks, int64_t h,
+                                  uint64_t seed, uint64_t pair_id0, double threshold, double min_extra, int aggregation,
+                                  int selection, double distance_threshold, double rotation_tolerance, double *H,
+                                  int64_t *best_index, double *best_err, int32_t *count_extra, int64_t *num_invalid,
+                                  sfm_hposes *poses, int64_t *inlier_offsets, int64_t cap, int32_t *inlier_idx,
+                                  uint8_t *pass, double *X);
+
+/* sfm_score_models for every pair of the current batched upload (sfm_batch_ransac, sfm_batch_two_view or
+ * sfm_batch_two_view_homography: all keep the pixel coordinates): E[p][9] / H[p][9], given for pair p when have_e[p] /
+ * have_h[p] is non-zero (a NULL flag array = all given, a NULL model array = none given), scored with the pair's own
+ * Ks[p] of the upload as K_d.  out[P] is bit for bit what sfm_score_models returns on that pair alone; a pair with
+ * neither model reports model = -1 and zero scores.  per_point (optional) double[n_total][4].  SFM_ERR_ARG: E and H both
+ * NULL, a given model not finite, an upload K that is singular or not finite, sigma or homography_ratio as for
+ * sfm_score_models.  SFM_ERR_STATE: no batched upload.  One synchronisation. */
+int sfm_batch_score_models(sfm_ctx *ctx, const double *E, const uint8_t *have_e, const double *H,
+                           const uint8_t *have_h, double sigma, double homography_ratio, sfm_model_scores *out,
+                           double *per_point);
 
 /* ---- hypothesis-sharded estimates without a host round trip (SURVEY.md 8(e)) ---------- */
 /* One rank of a run whose hypotheses are split over `world` GPUs (correspondences replicated):

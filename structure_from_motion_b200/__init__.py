@@ -7,7 +7,8 @@ The reference's import paths (``lib.ransac.ransac``, ``lib.epipolar.*`` ...) are
 the top-level ``lib`` package, which aliases the sub-modules of this package.
 """
 from .errors import EightPointCalculationError  # noqa: F401
-from .model_selection import ModelScores, TwoViewSelection, model_scores_arrays, two_view_select_arrays  # noqa: F401
+from .model_selection import (  # noqa: F401
+    ModelScores, TwoViewSelection, batch_two_view_select_arrays, model_scores_arrays, two_view_select_arrays)
 from .ransac.ransac import ErrorAggregationMethod  # noqa: F401
 
 __version__ = "0.1.0"

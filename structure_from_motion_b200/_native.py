@@ -117,6 +117,10 @@ _SIGNATURES = {
     "sfm_batch_two_view": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, _P, C.c_int64, _P, C.c_int64, C.c_uint64,
                                      C.c_uint64, C.c_double, C.c_double, C.c_int, C.c_int, C.c_double, _P, _P, _P, _P, _P,
                                      _P, _P, C.c_int64, _P, _P, _P]),
+    "sfm_batch_two_view_homography": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, _P, C.c_int64, _P, C.c_int64, C.c_uint64,
+                                                C.c_uint64, C.c_double, C.c_double, C.c_int, C.c_int, C.c_double,
+                                                C.c_double, _P, _P, _P, _P, _P, _P, _P, C.c_int64, _P, _P, _P]),
+    "sfm_batch_score_models": (C.c_int, [_P, _P, _P, _P, _P, C.c_double, C.c_double, _P, _P]),
     "sfm_match_brute_force": (C.c_int, [_P, _P, _P, C.c_int, C.c_int64, C.c_int64, _P, C.c_int64, _P, C.c_int64, C.c_int,
                                         C.c_int, C.c_int, C.c_double, _P, _P, _P, _P]),
     "sfm_match_from_scores": (C.c_int, [_P, _P, C.c_int64, C.c_int64, C.c_int, C.c_double, _P, _P, _P]),
@@ -191,6 +195,7 @@ class Engine:
         self._keep = None  # host arrays an un-synchronised upload still reads from
         self._out_ptr, self._out_cap, self._out = None, 0, None  # pinned landing buffers of the async path
         self.n = 0
+        self.batch_pairs = 0  # pairs of the current batched upload (0: none)
 
     # -- helpers -------------------------------------------------------------------------
     def _ck(self, rc, what):
@@ -259,7 +264,7 @@ class Engine:
         fn = self.lib.sfm_upload_pairs if sync else self.lib.sfm_upload_pairs_async
         self._ck(fn(self.h, _P(base_a), _P(base_a + 8), _P(base_b), _P(base_b + 8), 2, n, _ptr(K)), "sfm_upload_pairs")
         self._keep = None if sync else (pa, pb)
-        self.n = n
+        self.n, self.batch_pairs = n, 0
 
     def upload_pairs_soa(self, xa, ya, xb, yb, K):
         xa, ya, xb, yb = (_f64(v).reshape(-1) for v in (xa, ya, xb, yb))
@@ -267,13 +272,13 @@ class Engine:
         n = xa.shape[0]
         self._ck(self.lib.sfm_upload_pairs(self.h, _ptr(xa), _ptr(ya), _ptr(xb), _ptr(yb), 1, n, _ptr(K)),
                  "sfm_upload_pairs")
-        self.n = n
+        self.n, self.batch_pairs = n, 0
 
     def upload_pairs_device(self, xa_ptr, ya_ptr, xb_ptr, yb_ptr, stride, n, K):
         K = _f64(K).reshape(3, 3)
         self._ck(self.lib.sfm_upload_pairs_d(self.h, _P(xa_ptr), _P(ya_ptr), _P(xb_ptr), _P(yb_ptr), int(stride),
                                              int(n), _ptr(K)), "sfm_upload_pairs_d")
-        self.n = int(n)
+        self.n, self.batch_pairs = int(n), 0
 
     def get_normalised(self):
         out = np.empty((self.n, 4), dtype=np.float64)
@@ -618,6 +623,7 @@ class Engine:
                                            int(h), int(seed), int(pair_id0), float(threshold), float(min_extra),
                                            AGG[aggregation], SELECT[selection], _ptr(E), _ptr(bi), _ptr(be), _ptr(ce),
                                            _ptr(ni)), "sfm_batch_ransac")
+        self.n, self.batch_pairs = int(offsets[-1]), P
         return dict(E=E, best_index=bi, best_err=be, count_extra=ce, num_invalid=ni)
 
     def batch_two_view(self, pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra=0.0, aggregation="rms",
@@ -625,6 +631,12 @@ class Engine:
         """batch_ransac + per pair: inlier list, pose vote, triangulation.  Returns the batch_ransac dict plus
         R [P,3,3], t [P,3] (NaN without a model), counts [P,4], pose_index [P], inlier_offsets [P+1], inlier_idx
         (pair-relative), pass_bits, points [total,3]."""
+        return self._batch_two_view(pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra, aggregation, selection,
+                                    distance_threshold, pair_id0)[0]
+
+    def _batch_two_view(self, pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra, aggregation, selection,
+                        distance_threshold, pair_id0):
+        """batch_two_view's dict and the smallest singular value of every pair's winning E ([P], NaN without one)."""
         pa, pb = _split_xy(pts_a), _split_xy(pts_b)
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         P = offsets.shape[0] - 1
@@ -646,6 +658,7 @@ class Engine:
                                              AGG[aggregation], SELECT[selection], float(distance_threshold), _ptr(E),
                                              _ptr(bi), _ptr(be), _ptr(ce), _ptr(ni), C.cast(poses, _P), _ptr(ioff), cap,
                                              _ptr(idx), _ptr(ok), _ptr(X)), "sfm_batch_two_view")
+        self.n, self.batch_pairs = cap, P
         raw = np.frombuffer(poses, dtype=np.uint8).reshape(P, C.sizeof(Poses))
         dbl = raw[:, :(36 + 12 + 3) * 8].copy().view(np.float64)
         R4, t4 = dbl[:, :36].reshape(P, 4, 3, 3), dbl[:, 36:48].reshape(P, 4, 3)
@@ -656,10 +669,73 @@ class Engine:
         t = t4[np.arange(P), sel].copy()
         R[pose_index < 0] = np.nan
         t[pose_index < 0] = np.nan
+        sv = dbl[:, 48:51].copy()
         total = int(ioff[-1])
         return dict(E=E, best_index=bi, best_err=be, count_extra=ce, num_invalid=ni, R=R, t=t, counts=counts,
                     pose_index=pose_index, inlier_offsets=ioff, inlier_idx=idx[:total], pass_bits=ok[:total],
-                    points=X[:total])
+                    points=X[:total]), np.where(pose_index[:, None] == -2, np.nan, sv)[:, 2]
+
+    def batch_two_view_homography(self, pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra=0.0,
+                                  aggregation="rms", selection="min_error", distance_threshold=50.0,
+                                  rotation_tolerance=1e-2, pair_id0=0):
+        """batch_two_view for homographies (threshold: symmetric transfer error in px^2; Ks: each upper triangular with
+        K[2,2] = 1).  The keys of batch_two_view with H [P,3,3] in place of E, plus n [P,3], d [P] and
+        rotation_only bool[P] of the voted candidate.  R, t, n, d are NaN without a model; on a rotation-only pair R is
+        the nearest rotation, t = 0, n NaN, d inf, pose_index -1 and no inlier passes."""
+        pa, pb = _split_xy(pts_a), _split_xy(pts_b)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        P = offsets.shape[0] - 1
+        Ks = _f64(Ks).reshape(P, 9)
+        H = np.empty((P, 3, 3), dtype=np.float64)
+        bi = np.empty(P, dtype=np.int64)
+        be = np.empty(P, dtype=np.float64)
+        ce = np.empty(P, dtype=np.int32)
+        ni = np.empty(P, dtype=np.int64)
+        poses = (HPoses * P)()
+        ioff = np.empty(P + 1, dtype=np.int64)
+        cap = int(offsets[-1])
+        idx = np.empty(cap, dtype=np.int32)
+        ok = np.empty(cap, dtype=np.uint8)
+        X = np.empty((cap, 3), dtype=np.float64)
+        a, b = pa.ctypes.data, pb.ctypes.data
+        self._ck(self.lib.sfm_batch_two_view_homography(
+            self.h, _P(a), _P(a + 8), _P(b), _P(b + 8), 2, _ptr(offsets), P, _ptr(Ks), int(h), int(seed), int(pair_id0),
+            float(threshold), float(min_extra), AGG[aggregation], SELECT[selection], float(distance_threshold),
+            float(rotation_tolerance), _ptr(H), _ptr(bi), _ptr(be), _ptr(ce), _ptr(ni), C.cast(poses, _P), _ptr(ioff), cap,
+            _ptr(idx), _ptr(ok), _ptr(X)), "sfm_batch_two_view_homography")
+        self.n, self.batch_pairs = cap, P
+        raw = np.frombuffer(poses, dtype=np.uint8).reshape(P, C.sizeof(HPoses))
+        dbl = raw[:, :67 * 8].copy().view(np.float64)  # R 36, t 12, n 12, d 4, sv 3
+        R4, t4 = dbl[:, :36].reshape(P, 4, 3, 3), dbl[:, 36:48].reshape(P, 4, 3)
+        n4, d4 = dbl[:, 48:60].reshape(P, 4, 3), dbl[:, 60:64]
+        counts = raw[:, 67 * 8:71 * 8].copy().view(np.int64).reshape(P, 4)
+        ints = raw[:, 71 * 8:72 * 8].copy().view(np.int32).reshape(P, 2)
+        pose_index, rot = ints[:, 0].copy(), ints[:, 1] != 0
+        sel = np.clip(pose_index, 0, 3)  # a rotation-only pair's one candidate is candidate 0
+        rows = np.arange(P)
+        R, t, n, d = R4[rows, sel].copy(), t4[rows, sel].copy(), n4[rows, sel].copy(), d4[rows, sel].copy()
+        none = pose_index == -2
+        R[none], t[none], n[none], d[none] = np.nan, np.nan, np.nan, np.nan
+        total = int(ioff[-1])
+        return dict(H=H, best_index=bi, best_err=be, count_extra=ce, num_invalid=ni, R=R, t=t, counts=counts,
+                    pose_index=pose_index, inlier_offsets=ioff, inlier_idx=idx[:total], pass_bits=ok[:total],
+                    points=X[:total], n=n, d=d, rotation_only=rot)
+
+    def batch_score_models(self, E, H, have_e=None, have_h=None, sigma=1.0, homography_ratio=0.45, per_point=False):
+        """model_scores for every pair of the current batched upload: E / H [P,3,3] or None, given for pair p where
+        have_e[p] / have_h[p] (None = all), each pair scored with its own K of the upload.  Returns (ModelScores array
+        [P], per-point [n_total,4] errors or None); a pair with neither model has model -1."""
+        P = self.batch_pairs
+        Ea = None if E is None else _f64(E).reshape(P, 9)
+        Ha = None if H is None else _f64(H).reshape(P, 9)
+        fe = None if have_e is None else np.ascontiguousarray(have_e, dtype=np.uint8).reshape(P)
+        fh = None if have_h is None else np.ascontiguousarray(have_h, dtype=np.uint8).reshape(P)
+        out = (ModelScores * max(P, 1))()
+        pp = np.empty((self.n, 4), dtype=np.float64) if per_point else None
+        self._ck(self.lib.sfm_batch_score_models(self.h, _ptr(Ea), _ptr(fe), _ptr(Ha), _ptr(fh), float(sigma),
+                                                 float(homography_ratio), C.cast(out, _P), _ptr(pp)),
+                 "sfm_batch_score_models")
+        return out, pp
 
     # -- front end: brute-force matcher (N1) ---------------------------------------------------
     def match_brute_force(self, image_a, image_b, feats_a, feats_b, kind="ncc", window=None, ratio_test=False,

@@ -101,9 +101,10 @@ struct sfm_ctx {
     Buf h_img, h_gx, h_gy, h_corner, h_alive, h_key, h_idx, h_small, h_xy;
     Buf mask, sed, poses, pass, X, idx, scan, tmp, tailstate, num, winrec, bout;
     Buf planes, hK;  // the homography tail's HPlane and the K it was called with (the upload's K stays in Ks)
-    Buf selstate, selpp;  // k_score_models: self-cleaning sums + result + E, H, K; the per-correspondence errors
+    Buf selstate, selio, selpp;  // k_score_models: self-cleaning sums; models and results; per-correspondence errors
     long long n = 0, h = 0, npairs = 1;
     long long first_len = 0;  // batched: correspondences of the first pair (what the AUTO pilot samples)
+    long long batch_max_len = 0;  // batched: correspondences of the longest pair
     long long raw_stride = 1;
     bool batched = false, has_pts = false, has_table = false, has_models = false, has_score = false;
     bool models_h = false;       // the current models are homographies (sfm_fit_homography), not essential matrices
@@ -115,7 +116,8 @@ struct sfm_ctx {
     size_t acc_planes_for = 0;  // hypotheses (all pairs) the cleared accumulators were laid out for
     double Kstage[9] = {0};
     double hstage[18] = {0};  // H and K of sfm_decompose_homography, K of the homography tail, staged for async copies
-    double sstage[27] = {0};  // E, H and K of sfm_score_models, staged for the async copy
+    std::vector<SelectModels> sstage;  // the models of sfm_score_models / sfm_batch_score_models, staged for the async copy
+    std::vector<double> Kbatch;        // the cameras of the current batched upload, [P][9] (the device copy is Ks)
     const void* occ_fn[4] = {nullptr, nullptr, nullptr, nullptr};  // scoring kernels whose launch configuration is cached
     int occ_blocks[4] = {0, 0, 0, 0};
     int occ_next = 0;
@@ -297,7 +299,7 @@ int sfm_destroy(sfm_ctx* c) {
     Buf* bufs[] = {&c->raw, &c->pts, &c->offsets, &c->Ks, &c->table, &c->E, &c->valid, &c->eig, &c->acc,
                    &c->count_extra, &c->S1, &c->S2, &c->err, &c->blocks, &c->best,
                    &c->invalid, &c->winnerE, &c->record, &c->merged, &c->rows, &c->blockinv, &c->mask, &c->sed, &c->poses, &c->pass, &c->X, &c->idx,
-                   &c->planes, &c->hK, &c->selstate, &c->selpp,
+                   &c->planes, &c->hK, &c->selstate, &c->selio, &c->selpp,
                    &c->scan, &c->tmp, &c->gathered, &c->tailstate, &c->num, &c->winrec, &c->bout, &c->spts, &c->bounds, &c->fitflag,
                    &c->m_img, &c->m_feat, &c->m_W, &c->m_ss, &c->m_ok, &c->m_S, &c->m_out,
                    &c->h_img, &c->h_gx, &c->h_gy, &c->h_corner, &c->h_alive, &c->h_key, &c->h_idx, &c->h_small, &c->h_xy};
@@ -1036,31 +1038,35 @@ int sfm_ransac_essential(sfm_ctx* c, double thr, double min_extra, int agg, int 
 }
 
 // ---- homography (sfm_homography.cuh) -------------------------------------------------------
+// the 4-point fits of h hypotheses in each pair of the upload (a batch: device-sampler rows only)
 static int fit_h_launch(sfm_ctx* c) {
     if (!c->has_pts || !c->has_table) return fail(SFM_ERR_STATE, "fit needs correspondences and a sample table");
-    if (c->batched) return fail(SFM_ERR_STATE, "homography estimation is a single-pair call");
-    const long long h = c->h;
-    if (int r = c->E.reserve((size_t)h * 72)) return r;
-    if (int r = c->valid.reserve((size_t)h)) return r;
-    const size_t acc_tail = acc_tail_bytes(1);
-    if (int r = c->acc.reserve((size_t)h * kAccWords * 8 + acc_tail)) return r;
+    if (c->batched && !c->table_pending) return fail(SFM_ERR_STATE, "a batch is fitted from the device sampler's draw");
+    const long long h = c->h, P = c->npairs;
+    const size_t H = (size_t)h * P;
+    if (int r = c->E.reserve(H * 72)) return r;
+    if (int r = c->valid.reserve(H)) return r;
+    const size_t acc_tail = acc_tail_bytes(P);
+    if (int r = c->acc.reserve(H * kAccWords * 8 + acc_tail)) return r;
     c->tic(T_FIT);
-    CU(chain_launch(c, k_fit_homography, dim3((unsigned)((h + kFitHThreads - 1) / kFitHThreads)), dim3(kFitHThreads), 0,
-                    c->pts.as<Corr>(), c->table.as<int32_t>(), h, c->E.as<double>(), c->valid.as<uint8_t>(),
-                    c->acc.as<unsigned long long>(), kAccWords, (int)((acc_tail + 7) / 8), c->table_pending ? 1 : 0,
-                    c->smp_seed, c->smp_stream, c->smp_offset, c->n));
+    CU(chain_launch(c, k_fit_homography, dim3((unsigned)((h + kFitHThreads - 1) / kFitHThreads), (unsigned)P),
+                    dim3(kFitHThreads), 0, c->pts.as<Corr>(), c->batched ? c->offsets.as<long long>() : nullptr,
+                    c->table.as<int32_t>(), h, c->E.as<double>(), c->valid.as<uint8_t>(), c->acc.as<unsigned long long>(),
+                    kAccWords, (int)((acc_tail + 7) / 8), c->table_pending ? 1 : 0, c->smp_seed, c->smp_stream,
+                    c->smp_offset, c->n));
     if (int r = check_launch(c, "k_fit_homography")) return r;
     c->toc(T_FIT);
     c->table_pending = false;
     c->acc_clean = true;
-    c->acc_planes_for = (size_t)h;
+    c->acc_planes_for = H;
     c->has_models = true;
     c->models_h = true;
     c->has_score = false;
     return 0;
 }
 
-static int score_h_launch(sfm_ctx* c, double thr, double min_extra, int agg, int mode) {
+// K2 + K3 of homographies over every pair of the upload; max_len = the longest pair
+static int score_h_launch(sfm_ctx* c, double thr, double min_extra, int agg, int mode, long long max_len) {
     if (agg < 0 || agg > 3) return fail(SFM_ERR_ARG, "bad aggregation %d", agg);
     if (mode < 0 || mode > 2) return fail(SFM_ERR_ARG, "bad selection %d", mode);
     int sums = (agg == AGG_SUM || agg == AGG_MEAN) ? SUM_S1 : SUM_S2;
@@ -1068,14 +1074,15 @@ static int score_h_launch(sfm_ctx* c, double thr, double min_extra, int agg, int
     // the same threshold ranges as the E path: below 0, NaN and above 1e100 the scorer is skipped and K3 rescores
     const bool skip_k2 = !(thr >= 0.0) || thr > 1e100;
     const int force_rescore = (thr > 1e100) ? 1 : 0;
-    const long long h = c->h, n = c->n;
+    const long long h = c->h, n = c->n, P = c->npairs;
+    const size_t H = (size_t)h * P;
     // an inlier's value F/P + G/Q can exceed thr by a few ulps (the decision is division-free): the fixed-point scale
     // leaves room for that, value < thr (1 + 2^-20) < 2^e2
     int e2 = 0;
     if (thr > 0.0 && !skip_k2) (void)frexp(thr * (1.0 + 0x1p-20), &e2);
     if (e2 < -400) e2 = -400;
-    if (int r = reserve_selection(c, h, 1)) return r;
-    if (int r = c->acc.reserve((size_t)h * kAccWords * 8 + acc_tail_bytes(1))) return r;
+    if (int r = reserve_selection(c, h, P)) return r;
+    if (int r = c->acc.reserve(H * kAccWords * 8 + acc_tail_bytes(P))) return r;
     unsigned long long* acc = c->acc.as<unsigned long long>();
     const size_t smem = kHScoreWarps * sizeof(HScoreWarpSmem);
     if (!c->hscore_occ) {
@@ -1083,16 +1090,18 @@ static int score_h_launch(sfm_ctx* c, double thr, double min_extra, int agg, int
         CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, k_score_homography<kHScoreHpt>, kHScoreThreads, smem));
         c->hscore_occ = o > 0 ? o : 1;
     }
-    // persistent warps over (correspondence split, group of 32 * HPT hypotheses) items
+    // persistent warps over (pair, correspondence split, group of 32 * HPT hypotheses) items
     const long long grid_blocks = (long long)c->sm_count * c->hscore_occ;
     const long long hblocks = (h + 32ll * kHScoreHpt - 1) / (32ll * kHScoreHpt);
-    const ItemSplit sp = split_items(grid_blocks * kHScoreWarps * 32, hblocks, n, kHTile);
+    const ItemSplit sp = split_items(grid_blocks * kHScoreWarps * 32, hblocks * P, max_len, kHTile);
     const long long chunk = sp.chunk, nsplit = sp.nsplit;
     HScoreArgs a;
     a.pts = c->pts.as<Corr>();
+    a.offsets = c->batched ? c->offsets.as<long long>() : nullptr;
     a.H = c->E.as<double>();
     a.n = n;
     a.h = h;
+    a.htotal = (long long)H;
     a.thr = thr;
     a.scale1 = ldexp(1.0, 63 - e2);
     a.scale2 = ldexp(1.0, 63 - 2 * e2);
@@ -1100,11 +1109,11 @@ static int score_h_launch(sfm_ctx* c, double thr, double min_extra, int agg, int
     a.chunk = chunk;
     a.hblocks = (int)hblocks;
     a.nsplit = (int)nsplit;
-    a.total_items = hblocks * nsplit;
-    a.work_counter = reinterpret_cast<unsigned*>(acc + (size_t)h * kAccWords);
+    a.total_items = hblocks * nsplit * P;
+    a.work_counter = reinterpret_cast<unsigned*>(acc + H * kAccWords);
     a.acc = acc;
     c->tic(T_SCORE);
-    if (int r = clear_acc(c, (size_t)h, 1)) return r;
+    if (int r = clear_acc(c, H, P)) return r;
     if (!skip_k2) {
         const long long want = (a.total_items + kHScoreWarps - 1) / kHScoreWarps;
         CU(chain_launch(c, k_score_homography<kHScoreHpt>, dim3((unsigned)(grid_blocks < want ? grid_blocks : want)),
@@ -1128,6 +1137,7 @@ static int hmask_launch(sfm_ctx* c, double thr, const double* H_dev, const Best*
 
 int sfm_fit_homography(sfm_ctx* c, double* H_out, uint8_t* valid_out) {
     if (int r = use(c)) return r;
+    if (c->batched) return fail(SFM_ERR_STATE, "homography estimation is a single-pair call; use sfm_batch_two_view_homography");
     if (int r = fit_h_launch(c)) return r;
     if (H_out) CU(cudaMemcpyAsync(H_out, c->E.p, (size_t)c->h * 72, cudaMemcpyDeviceToHost, c->stream));
     if (valid_out) CU(cudaMemcpyAsync(valid_out, c->valid.p, (size_t)c->h, cudaMemcpyDeviceToHost, c->stream));
@@ -1142,7 +1152,7 @@ int sfm_ransac_homography(sfm_ctx* c, double thr, double min_extra, int agg, int
     if (c->batched) return fail(SFM_ERR_STATE, "single-pair call on a batched context");
     if (c->has_pts && c->n < 8) return fail(SFM_ERR_ARG, "need at least 8 correspondences, got %lld", c->n);
     if (int r = fit_h_launch(c)) return r;
-    if (int r = score_h_launch(c, thr, min_extra, agg, mode)) return r;
+    if (int r = score_h_launch(c, thr, min_extra, agg, mode, c->n)) return r;
     if (mask || err) {
         if (int r = hmask_launch(c, thr, c->E.as<double>(), c->best.as<Best>())) return r;
         if (mask) CU(cudaMemcpyAsync(mask, c->mask.p, (size_t)c->n, cudaMemcpyDeviceToHost, c->stream));
@@ -1268,7 +1278,8 @@ int sfm_triangulate(sfm_ctx* c, const double* P1, const double* P2, const double
 // The tail of apps/sfm.py:133-186 for the winner described by rec_dev (one SelectRecord per pair on the device):
 // T1 inlier mask + ordered compaction + decomposition, T2 4-pose cheirality + vote, T3 triangulation of the passing
 // inliers - three launches, nothing synchronised (see sfm_tail.cuh).  max_len = the longest pair.
-// kind = MODEL_H: the winner is a homography of a single pair; hpose_stage_k has put the caller's K in c->hK.
+// kind = MODEL_H: the winners are homographies; a single pair's K is the one hpose_stage_k put in c->hK, a batch's are
+// the caller's cameras in c->Ks (its records hold pixels).
 static int pose_tail_launch(sfm_ctx* c, double thr, double dist_thr, const SelectRecord* rec_dev, long long max_len,
                             uint8_t* mask_host = nullptr, double* sed_host = nullptr, int kind = MODEL_E,
                             double rot_tol = 0.0) {
@@ -1310,9 +1321,9 @@ static int pose_tail_launch(sfm_ctx* c, double thr, double dist_thr, const Selec
     a.planes = nullptr;
     a.rot_tol = rot_tol;
     if (kind == MODEL_H) {
-        if (int r = c->planes.reserve(sizeof(HPlane))) return r;
+        if (int r = c->planes.reserve((size_t)P * sizeof(HPlane))) return r;
         a.planes = c->planes.as<HPlane>();
-        a.Ks = c->hK.as<double>();
+        if (!c->batched) a.Ks = c->hK.as<double>();
     }
     c->tic(T_MASK);
     if (kind == MODEL_H) CU(chain_launch(c, k_tail_mask<MODEL_H>, dim3((unsigned)nblk, (unsigned)P), dim3(kTailBlock), 0, a));
@@ -1524,7 +1535,7 @@ int sfm_two_view_homography(sfm_ctx* c, const double* K, double thr, double min_
     // the device and the host synchronises once, at the fetch
     if (int r = hpose_stage_k(c, K)) return r;
     if (int r = fit_h_launch(c)) return r;
-    if (int r = score_h_launch(c, thr, min_extra, agg, mode)) return r;
+    if (int r = score_h_launch(c, thr, min_extra, agg, mode, c->n)) return r;
     // T1's mask / err are those of sfm_homography_mask for the winner
     if (int r = pose_tail_launch(c, thr, dist_thr, c->record.as<SelectRecord>(), c->n, mask, err, MODEL_H, rotation_tolerance))
         return r;
@@ -1532,51 +1543,108 @@ int sfm_two_view_homography(sfm_ctx* c, const double* K, double thr, double min_
 }
 
 // ---- essential matrix or homography (sfm_select.cuh) --------------------------------------------
-int sfm_score_models(sfm_ctx* c, const double* E, const double* H, const double* K, double sigma, double homography_ratio,
-                     sfm_model_scores* out, double* per_point) {
-    if (int r = use(c)) return r;
-    if (!out) return fail(SFM_ERR_ARG, "out is null");
-    if (!E && !H) return fail(SFM_ERR_ARG, "give E, H or both");
-    for (int i = 0; i < 9; ++i) {
-        if (E && !std::isfinite(E[i])) return fail(SFM_ERR_ARG, "E is not finite");
-        if (H && !std::isfinite(H[i])) return fail(SFM_ERR_ARG, "H is not finite");
-    }
-    if (int r = check_camera(K)) return r;
-    if (!(sigma > 0.0) || !std::isfinite(sigma)) return fail(SFM_ERR_ARG, "sigma must be finite and > 0");
-    if (!std::isfinite(homography_ratio)) return fail(SFM_ERR_ARG, "homography_ratio is not finite");
-    if (c->batched) return fail(SFM_ERR_STATE, "single-pair call on a batched context");
-    if (!c->has_pts) return fail(SFM_ERR_STATE, "no correspondences loaded");
-    // selstate: +0 the kernel's sums and ticket (zero between launches), +64 the result, +128 E, H, K
-    if (int r = reserve_zeroed(c, c->selstate, 128 + sizeof c->sstage)) return r;
+// k_score_models over the P pairs of the upload with the models staged in c->sstage; out[P], per_point [n][4] or null.
+// selstate: the kernel's sums and tickets [P][kSelectStateWords], zero between launches (only the kernel writes it);
+// selio: the models [P], then the results [P].
+static int score_models_launch(sfm_ctx* c, double sigma, double homography_ratio, long long max_len,
+                               sfm_model_scores* out, double* per_point) {
+    const long long P = c->npairs;
+    const size_t o_out = (size_t)P * sizeof(SelectModels);
+    if (int r = reserve_zeroed(c, c->selstate, (size_t)P * kSelectStateWords * 8)) return r;
+    if (int r = c->selio.reserve(o_out + (size_t)P * sizeof(ModelScores))) return r;
     if (per_point)
         if (int r = c->selpp.reserve((size_t)c->n * 32)) return r;
-    memset(c->sstage, 0, sizeof c->sstage);
-    if (E) memcpy(c->sstage, E, 72);
-    if (H) memcpy(c->sstage + 9, H, 72);
-    memcpy(c->sstage + 18, K, 72);
-    char* base = c->selstate.as<char>();
-    CU(cudaMemcpyAsync(base + 128, c->sstage, sizeof c->sstage, cudaMemcpyHostToDevice, c->stream));
+    char* base = c->selio.as<char>();
+    CU(cudaMemcpyAsync(base, c->sstage.data(), (size_t)P * sizeof(SelectModels), cudaMemcpyHostToDevice, c->stream));
     SelectArgs a;
     const double* s[4];
     raw_coords(c, s);
     a.xa = s[0]; a.ya = s[1]; a.xb = s[2]; a.yb = s[3];
     a.stride = c->raw_stride;
     a.n = c->n;
-    a.mats = reinterpret_cast<const double*>(base + 128);
-    a.have_e = E ? 1 : 0;
-    a.have_h = H ? 1 : 0;
+    a.offsets = c->batched ? c->offsets.as<long long>() : nullptr;
+    a.models = reinterpret_cast<const SelectModels*>(base);
     a.sigma = sigma;
     a.ratio = homography_ratio;
-    a.state = reinterpret_cast<unsigned long long*>(base);
-    a.out = reinterpret_cast<ModelScores*>(base + 64);
+    a.state = c->selstate.as<unsigned long long>();
+    a.out = reinterpret_cast<ModelScores*>(base + o_out);
     a.per_point = per_point ? c->selpp.as<double>() : nullptr;
-    const long long blocks = (c->n + kSelectBlock - 1) / kSelectBlock, cap = 4ll * c->sm_count;
-    k_score_models<<<(unsigned)(blocks < cap ? blocks : cap), kSelectBlock, 0, c->stream>>>(a);
+    // about 4 blocks per SM in all: a pair gets its share of them, at least one
+    const long long blocks = (max_len + kSelectBlock - 1) / kSelectBlock, cap = (4ll * c->sm_count + P - 1) / P;
+    const long long gx = blocks < cap ? blocks : cap;
+    c->tic(T_SCORE);
+    k_score_models<<<dim3((unsigned)(gx > 0 ? gx : 1), (unsigned)P), kSelectBlock, 0, c->stream>>>(a);
     if (int r = check_launch(c, "k_score_models")) return r;
-    CU(cudaMemcpyAsync(out, a.out, sizeof(ModelScores), cudaMemcpyDeviceToHost, c->stream));
+    c->toc(T_SCORE);
+    CU(cudaMemcpyAsync(out, a.out, (size_t)P * sizeof(ModelScores), cudaMemcpyDeviceToHost, c->stream));
     if (per_point) CU(cudaMemcpyAsync(per_point, c->selpp.p, (size_t)c->n * 32, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     return 0;
+}
+
+// the checks of sigma and the ratio shared by both scoring calls
+static int score_models_args(double sigma, double homography_ratio) {
+    if (!(sigma > 0.0) || !std::isfinite(sigma)) return fail(SFM_ERR_ARG, "sigma must be finite and > 0");
+    if (!std::isfinite(homography_ratio)) return fail(SFM_ERR_ARG, "homography_ratio is not finite");
+    return 0;
+}
+
+static int models_finite(const double* E, const double* H, const char* pair) {
+    for (int i = 0; i < 9; ++i) {
+        if (E && !std::isfinite(E[i])) return fail(SFM_ERR_ARG, "E%s is not finite", pair);
+        if (H && !std::isfinite(H[i])) return fail(SFM_ERR_ARG, "H%s is not finite", pair);
+    }
+    return 0;
+}
+
+// one pair's models into the staging record; E / H null = not given
+static void stage_models(SelectModels& m, const double* E, const double* H, const double* K) {
+    memset(&m, 0, sizeof m);
+    if (E) memcpy(m.E, E, 72);
+    if (H) memcpy(m.H, H, 72);
+    memcpy(m.K, K, 72);
+    m.have_e = E ? 1 : 0;
+    m.have_h = H ? 1 : 0;
+}
+
+int sfm_score_models(sfm_ctx* c, const double* E, const double* H, const double* K, double sigma, double homography_ratio,
+                     sfm_model_scores* out, double* per_point) {
+    if (int r = use(c)) return r;
+    if (!out) return fail(SFM_ERR_ARG, "out is null");
+    if (!E && !H) return fail(SFM_ERR_ARG, "give E, H or both");
+    if (int r = models_finite(E, H, "")) return r;
+    if (int r = check_camera(K)) return r;
+    if (int r = score_models_args(sigma, homography_ratio)) return r;
+    if (c->batched) return fail(SFM_ERR_STATE, "single-pair call on a batched context");
+    if (!c->has_pts) return fail(SFM_ERR_STATE, "no correspondences loaded");
+    c->sstage.resize(1);
+    stage_models(c->sstage[0], E, H, K);
+    return score_models_launch(c, sigma, homography_ratio, c->n, out, per_point);
+}
+
+int sfm_batch_score_models(sfm_ctx* c, const double* E, const uint8_t* have_e, const double* H, const uint8_t* have_h,
+                           double sigma, double homography_ratio, sfm_model_scores* out, double* per_point) {
+    if (int r = use(c)) return r;
+    if (!out) return fail(SFM_ERR_ARG, "out is null");
+    if (!E && !H) return fail(SFM_ERR_ARG, "give E, H or both");
+    if (int r = score_models_args(sigma, homography_ratio)) return r;
+    if (!c->batched || !c->has_pts) return fail(SFM_ERR_STATE, "no batched upload: run a batch call first");
+    const long long P = c->npairs;
+    c->sstage.resize((size_t)P);
+    for (long long p = 0; p < P; ++p) {
+        char which[48];
+        snprintf(which, sizeof which, " of pair %lld", p);
+        const double* K = c->Kbatch.data() + 9 * p;
+        const double* Ep = (E && (!have_e || have_e[p])) ? E + 9 * p : nullptr;
+        const double* Hp = (H && (!have_h || have_h[p])) ? H + 9 * p : nullptr;
+        if (int r = models_finite(Ep, Hp, which)) return r;
+        if (int r = check_camera(K)) {
+            const std::string why = g_err;
+            return fail(r, "pair %lld: %s", p, why.c_str());
+        }
+        stage_models(c->sstage[(size_t)p], Ep, Hp, K);
+    }
+    return score_models_launch(c, sigma, homography_ratio, c->batch_max_len, out, per_point);
 }
 
 int sfm_two_view_async(sfm_ctx* c, double thr, double min_extra, int agg, int mode, double dist_thr, uint8_t* mask,
@@ -1764,10 +1832,12 @@ int sfm_two_view_sharded(sfm_ctx* c, uint64_t seed, int64_t hyps_per_rank, doubl
 extern "C" {
 
 // ---- batched pairs ------------------------------------------------------------------------
-// upload -> device sampler -> fit -> score + select of P independent pairs (nothing synchronised)
-static int batch_core(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb, int64_t stride,
-                      const int64_t* offsets, int64_t npairs, const double* Ks, int64_t h, uint64_t seed, uint64_t pair_id0,
-                      double thr, double min_extra, int agg, int mode, long long* max_len_out) {
+// The upload of P independent pairs: offsets, the caller's cameras (c->Ks, and c->Kbatch on the host) and the raw
+// coordinates (c->raw), from which the records are built - K-normalised with each pair's K for essential matrices, in
+// pixels (an identity camera) for homographies.  Nothing synchronised.
+static int batch_upload(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
+                        int64_t stride, const int64_t* offsets, int64_t npairs, const double* Ks, int64_t h, bool pixels,
+                        long long* max_len_out) {
     if (!xa || !ya || !xb || !yb || !offsets || !Ks) return fail(SFM_ERR_ARG, "null argument");
     if (npairs <= 0 || npairs > 65535) return fail(SFM_ERR_ARG, "need 1 <= npairs <= 65535 per call");
     if (h <= 0) return fail(SFM_ERR_ARG, "need h > 0");
@@ -1788,11 +1858,35 @@ static int batch_core(sfm_ctx* c, const double* xa, const double* ya, const doub
     if (int r = c->Ks.reserve((size_t)npairs * 72)) return r;
     CU(cudaMemcpyAsync(c->offsets.p, offsets, (size_t)(npairs + 1) * 8, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(c->Ks.p, Ks, (size_t)npairs * 72, cudaMemcpyHostToDevice, c->stream));
+    c->Kbatch.assign(Ks, Ks + 9 * npairs);
+    c->batch_max_len = max_len;
     const double* s[4];
     if (int r = stage_raw(c, xa, ya, xb, yb, stride, n, s)) return r;
-    if (int r = normalise_from(c, s[0], s[1], s[2], s[3], stride, n, max_len)) return r;
+    if (pixels) {  // one identity camera for all records: x / 1 = x
+        const double I[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
+        if (int r = hpose_stage_k(c, I)) return r;
+        if (int r = c->pts.reserve((size_t)n * sizeof(Corr))) return r;
+        k_normalise<<<dim3((unsigned)((n + 255) / 256), 1), 256, 0, c->stream>>>(s[0], s[1], s[2], s[3], stride, n, nullptr,
+                                                                                c->hK.as<double>(), c->pts.as<Corr>(), nullptr);
+        if (int r = check_launch(c, "k_normalise")) return r;
+    } else if (int r = normalise_from(c, s[0], s[1], s[2], s[3], stride, n, max_len)) {
+        return r;
+    }
     c->toc(T_UPLOAD);
     c->has_pts = true;
+    c->has_table = c->has_models = c->has_score = false;
+    c->table_pending = false;
+    c->winner_set = false;
+    *max_len_out = max_len;
+    return 0;
+}
+
+// upload -> device sampler -> fit -> score + select of P independent pairs (nothing synchronised)
+static int batch_core(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb, int64_t stride,
+                      const int64_t* offsets, int64_t npairs, const double* Ks, int64_t h, uint64_t seed, uint64_t pair_id0,
+                      double thr, double min_extra, int agg, int mode, long long* max_len_out) {
+    long long max_len = 0;
+    if (int r = batch_upload(c, xa, ya, xb, yb, stride, offsets, npairs, Ks, h, false, &max_len)) return r;
     if (int r = sample_device(c, seed, pair_id0, 0, h)) return r;
     if (int r = fit_launch(c, false)) return r;
     if (int r = score_launch(c, thr, min_extra, agg, mode, true, 0, max_len)) return r;
@@ -1839,23 +1933,11 @@ int sfm_batch_ransac(sfm_ctx* c, const double* xa, const double* ya, const doubl
     return 0;
 }
 
-// The whole path per pair (apps/sfm.py:110-186 for every pair of the batch): RANSAC E, then for each pair's winner the
-// inlier list, the 4-pose cheirality vote and the triangulation of the passing inliers - the same three tail kernels as
-// the single-pair call, with the pair as blockIdx.y.  Per-inlier results come back densely packed:
-// inlier_offsets[p] .. inlier_offsets[p+1] index inlier_idx (pair-relative, ascending), pass and X.
-int sfm_batch_two_view(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
-                       int64_t stride, const int64_t* offsets, int64_t npairs, const double* Ks, int64_t h,
-                       uint64_t seed, uint64_t pair_id0, double thr, double min_extra, int agg, int mode,
-                       double dist_thr, double* E, int64_t* best_index, double* best_err, int32_t* count_extra,
-                       int64_t* num_invalid, sfm_poses* poses, int64_t* inlier_offsets, int64_t cap,
-                       int32_t* inlier_idx, uint8_t* pass, double* X) {
-    if (int r = use(c)) return r;
-    if (!poses || !inlier_offsets) return fail(SFM_ERR_ARG, "null argument");
-    long long max_len = 0;
-    if (int r = batch_core(c, xa, ya, xb, yb, stride, offsets, npairs, Ks, h, seed, pair_id0, thr, min_extra, agg, mode,
-                           &max_len)) return r;
-    if (int r = pose_tail_launch(c, thr, dist_thr, c->record.as<SelectRecord>(), max_len)) return r;
-    // dense packing of the per-pair inlier segments
+// After a batch tail: dense packing of the per-pair inlier segments, then winners, poses (and planes) and offsets with
+// one synchronisation, the packed per-inlier arrays with a second one.
+static int batch_tail_fetch(sfm_ctx* c, int64_t npairs, long long max_len, double* E, int64_t* best_index,
+                            double* best_err, int32_t* count_extra, int64_t* num_invalid, PoseSet* poses, HPlane* planes,
+                            int64_t* inlier_offsets, int64_t cap, int32_t* inlier_idx, uint8_t* pass, double* X) {
     const long long n = c->n;
     const size_t o_off = 0, o_idx = ((size_t)(npairs + 1) * 8 + 63) / 64 * 64, o_pass = o_idx + ((size_t)n * 4 + 63) / 64 * 64,
                  o_X = o_pass + ((size_t)n + 63) / 64 * 64;
@@ -1874,6 +1956,8 @@ int sfm_batch_two_view(sfm_ctx* c, const double* xa, const double* ya, const dou
     const size_t pose_bytes = (size_t)npairs * sizeof(PoseSet);
     if (int r = batch_fetch_winners(c, npairs, pose_bytes, &extra)) return r;
     CU(cudaMemcpyAsync(poses, c->poses.p, pose_bytes, cudaMemcpyDeviceToHost, c->stream));
+    if (planes)
+        CU(cudaMemcpyAsync(planes, c->planes.p, (size_t)npairs * sizeof(HPlane), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(inlier_offsets, d_off, (size_t)(npairs + 1) * 8, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     batch_unpack_winners((const char*)c->hpin, npairs, E, best_index, best_err, count_extra, num_invalid);
@@ -1887,6 +1971,59 @@ int sfm_batch_two_view(sfm_ctx* c, const double* xa, const double* ya, const dou
     }
     c->has_score = false;
     c->winner_set = false;
+    return 0;
+}
+
+// The whole path per pair (apps/sfm.py:110-186 for every pair of the batch): RANSAC E, then for each pair's winner the
+// inlier list, the 4-pose cheirality vote and the triangulation of the passing inliers - the same three tail kernels as
+// the single-pair call, with the pair as blockIdx.y.  Per-inlier results come back densely packed:
+// inlier_offsets[p] .. inlier_offsets[p+1] index inlier_idx (pair-relative, ascending), pass and X.
+int sfm_batch_two_view(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
+                       int64_t stride, const int64_t* offsets, int64_t npairs, const double* Ks, int64_t h,
+                       uint64_t seed, uint64_t pair_id0, double thr, double min_extra, int agg, int mode,
+                       double dist_thr, double* E, int64_t* best_index, double* best_err, int32_t* count_extra,
+                       int64_t* num_invalid, sfm_poses* poses, int64_t* inlier_offsets, int64_t cap,
+                       int32_t* inlier_idx, uint8_t* pass, double* X) {
+    if (int r = use(c)) return r;
+    if (!poses || !inlier_offsets) return fail(SFM_ERR_ARG, "null argument");
+    long long max_len = 0;
+    if (int r = batch_core(c, xa, ya, xb, yb, stride, offsets, npairs, Ks, h, seed, pair_id0, thr, min_extra, agg, mode,
+                           &max_len)) return r;
+    if (int r = pose_tail_launch(c, thr, dist_thr, c->record.as<SelectRecord>(), max_len)) return r;
+    return batch_tail_fetch(c, npairs, max_len, E, best_index, best_err, count_extra, num_invalid,
+                            reinterpret_cast<PoseSet*>(poses), nullptr, inlier_offsets, cap, inlier_idx, pass, X);
+}
+
+// sfm_batch_two_view for homographies: the pixel records of every pair, the device sampler's rows (columns 0-3), the 4-point
+// fits, K2 and K3 over (pair, split, group) items, then the homography tail of every pair's winner with that pair's K.
+int sfm_batch_two_view_homography(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
+                                  int64_t stride, const int64_t* offsets, int64_t npairs, const double* Ks, int64_t h,
+                                  uint64_t seed, uint64_t pair_id0, double thr, double min_extra, int agg, int mode,
+                                  double dist_thr, double rotation_tolerance, double* H, int64_t* best_index,
+                                  double* best_err, int32_t* count_extra, int64_t* num_invalid, sfm_hposes* poses,
+                                  int64_t* inlier_offsets, int64_t cap, int32_t* inlier_idx, uint8_t* pass, double* X) {
+    if (int r = use(c)) return r;
+    if (!poses || !inlier_offsets || !Ks) return fail(SFM_ERR_ARG, "null argument");
+    if (npairs <= 0 || npairs > 65535) return fail(SFM_ERR_ARG, "need 1 <= npairs <= 65535 per call");
+    for (int64_t p = 0; p < npairs; ++p)
+        if (int r = hpose_args(Ks + 9 * p, rotation_tolerance)) {
+            const std::string why = g_err;
+            return fail(r, "pair %lld: %s", (long long)p, why.c_str());
+        }
+    long long max_len = 0;
+    if (int r = batch_upload(c, xa, ya, xb, yb, stride, offsets, npairs, Ks, h, true, &max_len)) return r;
+    if (int r = sample_device(c, seed, pair_id0, 0, h)) return r;
+    if (int r = fit_h_launch(c)) return r;
+    if (int r = score_h_launch(c, thr, min_extra, agg, mode, max_len)) return r;
+    if (int r = pose_tail_launch(c, thr, dist_thr, c->record.as<SelectRecord>(), max_len, nullptr, nullptr, MODEL_H,
+                                 rotation_tolerance))
+        return r;
+    std::vector<PoseSet> ps((size_t)npairs);
+    std::vector<HPlane> pl((size_t)npairs);
+    if (int r = batch_tail_fetch(c, npairs, max_len, H, best_index, best_err, count_extra, num_invalid, ps.data(), pl.data(),
+                                 inlier_offsets, cap, inlier_idx, pass, X))
+        return r;
+    for (int64_t p = 0; p < npairs; ++p) pack_hposes(ps[(size_t)p], pl[(size_t)p], poses + p);
     return 0;
 }
 

@@ -109,25 +109,45 @@ __device__ __forceinline__ bool homography_fit4(const Corr (&c)[4], double (&H)[
 }
 
 // K1 for homographies, one thread per hypothesis, everything in registers (the shape of k_fit_qr): clears this
-// hypothesis's accumulator column (and, thread 0, the tail words), reads its row from the table or draws it with the
-// device sampler (recording all 8 columns, as k_fit_qr does), fits columns 0-3.  Single pair.
+// hypothesis's accumulator column (and, thread 0 of pair 0, the tail words), reads its row from the table or draws it
+// with the device sampler (stream stream0 + pair, recording all 8 columns, as k_fit_qr does), fits columns 0-3.
+// Batched form as k_fit_qr: blockIdx.y = image pair, pair p owns records [offsets[p], offsets[p+1]) and table rows,
+// models and accumulator columns [p h, (p+1) h); its indices are pair-relative.  A pair of fewer than 8 records gets
+// invalid models (and zero rows when drawing).  offsets == nullptr: one pair of n records.
 constexpr int kFitHThreads = 64;
 __global__ void __launch_bounds__(kFitHThreads)
-k_fit_homography(const Corr* __restrict__ pts, const int32_t* __restrict__ table, long long h, double* __restrict__ H_out,
-                 uint8_t* __restrict__ valid_out, unsigned long long* __restrict__ acc, int acc_planes, int acc_tail_words,
-                 int draw, unsigned long long seed, unsigned long long stream0, long long hyp_offset, long long n) {
+k_fit_homography(const Corr* __restrict__ pts, const long long* __restrict__ offsets, const int32_t* __restrict__ table,
+                 long long h, double* __restrict__ H_out, uint8_t* __restrict__ valid_out,
+                 unsigned long long* __restrict__ acc, int acc_planes, int acc_tail_words, int draw,
+                 unsigned long long seed, unsigned long long stream0, long long hyp_offset, long long n) {
     chain_enter();
-    const long long i = blockIdx.x * (long long)kFitHThreads + threadIdx.x;
-    if (i >= h) return;
+    const long long li = blockIdx.x * (long long)kFitHThreads + threadIdx.x;
+    if (li >= h) return;
+    const long long i = (long long)blockIdx.y * h + li;
     if (acc) {
-        for (int k = 0; k < acc_planes; ++k) acc[(long long)k * h + i] = 0ull;
+        const long long htotal = (long long)gridDim.y * h;
+        for (int k = 0; k < acc_planes; ++k) acc[(long long)k * htotal + i] = 0ull;
         if (i == 0)
-            for (int k = 0; k < acc_tail_words; ++k) acc[(long long)acc_planes * h + k] = 0ull;
+            for (int k = 0; k < acc_tail_words; ++k) acc[(long long)acc_planes * htotal + k] = 0ull;
+    }
+    if (offsets) {
+        n = offsets[blockIdx.y + 1] - offsets[blockIdx.y];
+        if (n < 8) {
+            for (int k = 0; k < 9; ++k) H_out[9 * i + k] = 0.0;
+            valid_out[i] = FIT_INVALID;
+            if (draw) {
+                int4* t = reinterpret_cast<int4*>(const_cast<int32_t*>(table) + 8 * i);
+                t[0] = make_int4(0, 0, 0, 0);
+                t[1] = make_int4(0, 0, 0, 0);
+            }
+            return;
+        }
+        pts += offsets[blockIdx.y];
     }
     int idx[4];
     if (draw) {
         int32_t row[8];
-        philox_sample8(seed, stream0, (unsigned long long)(hyp_offset + i), (unsigned)n, row);
+        philox_sample8(seed, stream0 + blockIdx.y, (unsigned long long)(hyp_offset + li), (unsigned)n, row);
         int4* t = reinterpret_cast<int4*>(const_cast<int32_t*>(table) + 8 * i);
         t[0] = make_int4(row[0], row[1], row[2], row[3]);
         t[1] = make_int4(row[4], row[5], row[6], row[7]);
@@ -158,6 +178,9 @@ k_fit_homography(const Corr* __restrict__ pts, const int32_t* __restrict__ table
 // 32-bit chunk registers - a lane owns its hypothesis within the item, so neither atomics nor shared memory are needed
 // until the item ends and the words are folded into the [kAccWords][h] global accumulators.  Integer sums: counts and
 // sums are independent of scheduling and of the split, exactly as on the E path, and K3 reads them unchanged.
+// Batches: items are (pair, split, group) as K2's are.  A split is cut within the pair's own records, the pair's models
+// are H[p h, (p+1) h) and its sums go to accumulator columns p h + hypothesis, so each pair's counts and sums are those
+// of the single-pair call on that pair alone.
 // ------------------------------------------------------------------------------------
 constexpr int kHScoreThreads = 128;
 constexpr int kHScoreWarps = kHScoreThreads / 32;
@@ -167,8 +190,9 @@ constexpr int kHScoreHpt = 2;
 
 struct HScoreArgs {
     const Corr* pts;          // pixel coordinates (K = I)
-    const double* H;          // [h][9]
-    long long n, h;
+    const long long* offsets; // [P+1] or null (one pair of n records)
+    const double* H;          // [P][h][9]
+    long long n, h, htotal;   // htotal = P h: the stride of the accumulator planes
     double thr;
     double scale1, scale2;    // 2^(63-e), 2^(63-2e): every inlier's value < 2^e
     int sums;                 // SUM_S1 | SUM_S2
@@ -176,7 +200,7 @@ struct HScoreArgs {
     int hblocks, nsplit;
     long long total_items;
     unsigned* work_counter;
-    unsigned long long* acc;  // [kAccWords][h], cleared by k_fit_homography
+    unsigned long long* acc;  // [kAccWords][htotal], cleared by k_fit_homography
 };
 
 struct alignas(128) HScoreWarpSmem {
@@ -205,10 +229,15 @@ __global__ void __launch_bounds__(kHScoreThreads, 3) k_score_homography(const HS
         item = __shfl_sync(full, item, 0);
         if (item >= a.total_items) break;
         const int hw = (int)(item % (unsigned)a.hblocks);
-        const int split = (int)(item / (unsigned)a.hblocks);
+        const unsigned rest = item / (unsigned)a.hblocks;
+        const int split = (int)(rest % (unsigned)a.nsplit);
+        const int pair = (int)(rest / (unsigned)a.nsplit);
+        const long long pbase = a.offsets ? a.offsets[pair] : 0;
+        const long long plen = a.offsets ? a.offsets[pair + 1] - pbase : a.n;
         long long begin = (long long)split * a.chunk;
-        if (begin > a.n) begin = a.n;
-        const long long end = (begin + a.chunk < a.n) ? begin + a.chunk : a.n;
+        if (begin > plen) begin = plen;
+        const long long end = pbase + ((begin + a.chunk < plen) ? begin + a.chunk : plen);
+        begin += pbase;
         const int ntiles = (int)((end - begin + kHTile - 1) / kHTile);
         auto issue = [&](int t) {  // lane 0 only
             const int s = (int)((gt + (unsigned)t) % kHStages);
@@ -223,13 +252,14 @@ __global__ void __launch_bounds__(kHScoreThreads, 3) k_score_homography(const HS
 
         // this lane's hypotheses hyp_w + 32 j + lane; padding lanes hold H = 0 (p2 = 0: never an inlier)
         const long long hyp_w = (long long)hw * (32 * HPT);
+        const double* Hp = a.H + 9 * (long long)pair * a.h;
         double hm[HPT][9], am[HPT][9];
         unsigned cw[HPT][kAccWords];
 #pragma unroll
         for (int j = 0; j < HPT; ++j) {
             const long long hyp = hyp_w + 32 * j + lane;
 #pragma unroll
-            for (int k = 0; k < 9; ++k) hm[j][k] = hyp < a.h ? a.H[9 * hyp + k] : 0.0;
+            for (int k = 0; k < 9; ++k) hm[j][k] = hyp < a.h ? Hp[9 * hyp + k] : 0.0;
             homography_adj(hm[j], am[j]);
 #pragma unroll
             for (int k = 0; k < kAccWords; ++k) cw[j][k] = 0u;
@@ -270,11 +300,11 @@ __global__ void __launch_bounds__(kHScoreThreads, 3) k_score_homography(const HS
         gt += (unsigned)ntiles;
 #pragma unroll
         for (int j = 0; j < HPT; ++j) {
-            const long long hyp = hyp_w + 32 * j + lane;
+            const long long hyp = (long long)pair * a.h + hyp_w + 32 * j + lane;
             if (cw[j][0]) {  // only real hypotheses can have inliers
 #pragma unroll
                 for (int k = 0; k < kAccWords; ++k)
-                    if (cw[j][k]) atomicAdd(a.acc + (long long)k * a.h + hyp, (unsigned long long)cw[j][k]);
+                    if (cw[j][k]) atomicAdd(a.acc + (long long)k * a.htotal + hyp, (unsigned long long)cw[j][k]);
             }
         }
     }

@@ -1,5 +1,5 @@
-// Choosing between the essential matrix and a homography for one image pair: the score ratio of ORB-SLAM (Mur-Artal,
-// Montiel & Tardos, 2015, section IV) over the uploaded pixel correspondences, in one launch.
+// Choosing between the essential matrix and a homography for each image pair: the score ratio of ORB-SLAM (Mur-Artal,
+// Montiel & Tardos, 2015, section IV) over the uploaded pixel correspondences, in one launch for one pair or a batch.
 //
 // E is turned into the pixel fundamental matrix F = Kd^-T E Kd^-1 (the convention b^T E a = 0 of sed_exact), Kd = K
 // without its skew and with (0, 0, 1) as the bottom row: the camera E was fitted in.  Per
@@ -30,15 +30,23 @@ struct ModelScores {
     int model, reserved;
 };
 
+// the models of one pair, row-major; a model not given is never read
+struct SelectModels {
+    double E[9], H[9], K[9];
+    int have_e, have_h;
+};
+
+constexpr int kSelectStateWords = 8;  // per pair: fixed_e, fixed_h, count_e, count_h, ticket, 3 unused
+
 struct SelectArgs {
     const double* xa; const double* ya; const double* xb; const double* yb;  // pixel coordinates, element i at [i*stride]
     long long stride, n;
-    const double* mats;          // E[9], H[9], K[9], row-major
-    int have_e, have_h;
+    const long long* offsets;    // [P+1] or null (one pair of n)
+    const SelectModels* models;  // [P]
     double sigma, ratio;
-    unsigned long long* state;   // [5]: fixed_e, fixed_h, count_e, count_h, ticket; zero on entry and on exit
-    ModelScores* out;
-    double* per_point;           // [n][4] (d2_A,E, d2_B,E, d2_A,H, d2_B,H) or null
+    unsigned long long* state;   // [P][kSelectStateWords], zero on entry and on exit
+    ModelScores* out;            // [P]
+    double* per_point;           // [n_total][4] (d2_A,E, d2_B,E, d2_A,H, d2_B,H) or null
 };
 
 // F = Kd^-T E Kd^-1 with Kd^-1 = adj(Kd) / det(Kd), Kd = [[fx, 0, cx], [0, fy, cy], [0, 0, 1]]: the camera of the
@@ -69,20 +77,25 @@ __device__ __forceinline__ unsigned long long select_rho(double d2, double s2, d
     return pass ? __double2ull_rn(__dmul_rn(__dsub_rn(kSelectGamma, x), kSelectFixed)) : 0ull;
 }
 
+// Grid (blocks, P): blockIdx.y = image pair; the blocks of a pair stride over its records and the last of them to
+// finish writes the pair's result.
 __global__ void __launch_bounds__(kSelectBlock) k_score_models(const SelectArgs a) {
     __shared__ double s_f[9], s_h[9], s_adj[9];
     __shared__ unsigned long long s_part[kSelectBlock / 32][4];
     __shared__ unsigned s_last;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int pair = blockIdx.y;
+    const SelectModels& m = a.models[pair];
+    const int have_e = m.have_e, have_h = m.have_h;
     if (tid == 0) {  // the same operations in every block: every block sees the same F and adj(H)
         double f[9], h[9], adj[9];
-        if (a.have_e) fundamental_from_essential(a.mats, a.mats + 18, f);
+        if (have_e) fundamental_from_essential(m.E, m.K, f);
 #pragma unroll
-        for (int i = 0; i < 9; ++i) h[i] = a.mats[9 + i];
+        for (int i = 0; i < 9; ++i) h[i] = m.H[i];
         homography_adj(h, adj);
 #pragma unroll
         for (int i = 0; i < 9; ++i) {
-            s_f[i] = a.have_e ? f[i] : 0.0;
+            s_f[i] = have_e ? f[i] : 0.0;
             s_h[i] = h[i];
             s_adj[i] = adj[i];
         }
@@ -98,11 +111,13 @@ __global__ void __launch_bounds__(kSelectBlock) k_score_models(const SelectArgs 
     const double s2 = __dmul_rn(a.sigma, a.sigma);
     const double nan = __longlong_as_double(0x7ff8000000000000LL);
     unsigned long long se = 0, sh = 0, ce = 0, ch = 0;
-    for (long long i = blockIdx.x * (long long)blockDim.x + tid; i < a.n; i += (long long)gridDim.x * blockDim.x) {
+    const long long pbase = a.offsets ? a.offsets[pair] : 0;
+    const long long pend = a.offsets ? a.offsets[pair + 1] : a.n;
+    for (long long i = pbase + blockIdx.x * (long long)blockDim.x + tid; i < pend; i += (long long)gridDim.x * blockDim.x) {
         const long long g = i * a.stride;
         const double xa = a.xa[g], ya = a.ya[g], xb = a.xb[g], yb = a.yb[g];
         double dae = nan, dbe = nan, dah = nan, dbh = nan;
-        if (a.have_e) {
+        if (have_e) {
             const double la0 = __fma_rn(f[0], xa, __fma_rn(f[1], ya, f[2]));
             const double la1 = __fma_rn(f[3], xa, __fma_rn(f[4], ya, f[5]));
             const double la2 = __fma_rn(f[6], xa, __fma_rn(f[7], ya, f[8]));
@@ -116,7 +131,7 @@ __global__ void __launch_bounds__(kSelectBlock) k_score_models(const SelectArgs 
             se += select_rho(dae, s2, kSelectTE, pa) + select_rho(dbe, s2, kSelectTE, pb);
             ce += (pa && pb) ? 1ull : 0ull;
         }
-        if (a.have_h) {
+        if (have_h) {
             const TransferTerms t = transfer_terms(h, adj, xa, ya, xb, yb);
             dbh = __ddiv_rn(t.F, t.P);
             dah = __ddiv_rn(t.G, t.Q);
@@ -140,21 +155,23 @@ __global__ void __launch_bounds__(kSelectBlock) k_score_models(const SelectArgs 
         s_part[warp][0] = se; s_part[warp][1] = sh; s_part[warp][2] = ce; s_part[warp][3] = ch;
     }
     __syncthreads();
+    unsigned long long* state = a.state + (long long)pair * kSelectStateWords;
     if (tid < 4) {  // integer sums: the order of the blocks' atomics does not matter
         unsigned long long v = 0;
         for (int w = 0; w < kSelectBlock / 32; ++w) v += s_part[w][tid];
-        if (v) atomicAdd(&a.state[tid], v);
+        if (v) atomicAdd(&state[tid], v);
     }
     __syncthreads();
     if (tid == 0) {
         __threadfence();
-        s_last = (atomicAdd(&a.state[4], 1ull) == (unsigned long long)(gridDim.x - 1)) ? 1u : 0u;
+        s_last = (atomicAdd(&state[4], 1ull) == (unsigned long long)(gridDim.x - 1)) ? 1u : 0u;
     }
     __syncthreads();
     if (!s_last || tid != 0) return;
-    // the last block: every other block's sums are visible; write the result and leave the state zero for the next call
+    // the pair's last block: its other blocks' sums are visible; write the result and leave the state zero for the next
+    // call
     __threadfence();
-    volatile unsigned long long* st = a.state;
+    volatile unsigned long long* st = state;
     const unsigned long long fe = st[0], fh = st[1], ne = st[2], nh = st[3];
     st[0] = 0; st[1] = 0; st[2] = 0; st[3] = 0; st[4] = 0;
     ModelScores r;
@@ -166,9 +183,9 @@ __global__ void __launch_bounds__(kSelectBlock) k_score_models(const SelectArgs 
     r.score_h = __dmul_rn(__ull2double_rn(fh), 1.0 / kSelectFixed);
     const double tot = __dadd_rn(r.score_h, r.score_e);
     r.ratio_h = tot > 0.0 ? __ddiv_rn(r.score_h, tot) : 0.0;
-    r.model = !a.have_e ? 1 : (!a.have_h ? 0 : (r.ratio_h > a.ratio ? 1 : 0));
+    r.model = !have_e ? (have_h ? 1 : -1) : (!have_h ? 0 : (r.ratio_h > a.ratio ? 1 : 0));
     r.reserved = 0;
-    *a.out = r;
+    a.out[pair] = r;
 }
 
 }  // namespace sfm

@@ -167,6 +167,24 @@ def shard_pairs(offsets: Sequence[int], rank: int, world: int):
     return p0, p1, offsets[p0:p1 + 1] - offsets[p0]
 
 
+def _merge_chunks(parts: list) -> dict:
+    """The dicts of consecutive chunks of pairs as one dict: arrays concatenated, ``inlier_offsets`` re-based, nested
+    dicts merged alike."""
+    out = {}
+    for key, v in parts[0].items():
+        if isinstance(v, dict):
+            out[key] = _merge_chunks([p[key] for p in parts])
+        elif key == "inlier_offsets":
+            base, segs = 0, [np.zeros(1, dtype=np.int64)]
+            for p in parts:
+                segs.append(p[key][1:] + base)
+                base += int(p[key][-1])
+            out[key] = np.concatenate(segs)
+        else:
+            out[key] = np.concatenate([p[key] for p in parts])
+    return out
+
+
 class PairPipeline:
     """Pair-sharded batches from HOST buffers with the H2D copy of one chunk hidden behind the kernels of another:
     the pairs are cut into chunks that alternate between ``depth`` contexts on the same GPU (each with its own
@@ -219,10 +237,10 @@ class PairPipeline:
         keys = parts[0].keys()
         return {key: np.concatenate([parts[k][key] for k in range(len(bounds) - 1)]) for key in keys}
 
-    def batch_two_view(self, pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra=0.0, aggregation="rms",
-                       selection="min_error", distance_threshold=50.0, pair_id0=0, chunk_pairs: Optional[int] = None):
-        """``Engine.batch_two_view`` (RANSAC E + inlier list + pose vote + triangulation per pair) over chunks of
-        pairs that alternate between the contexts; identical to one call over all pairs."""
+    def _chunked(self, call, pts_a, pts_b, offsets, Ks, pair_id0, chunk_pairs):
+        """call(engine, pts_a, pts_b, offsets, Ks, pair_id0) over chunks of pairs that alternate between the contexts,
+        merged into the dict of one call over all pairs: per-pair and per-inlier arrays are concatenated,
+        ``inlier_offsets`` re-based, nested dicts merged the same way."""
         offsets = np.asarray(offsets, dtype=np.int64)
         P = len(offsets) - 1
         Ks = np.asarray(Ks, dtype=np.float64).reshape(P, 3, 3)
@@ -234,26 +252,41 @@ class PairPipeline:
         def run(k):
             p0, p1 = bounds[k], bounds[k + 1]
             lo, hi = int(offsets[p0]), int(offsets[p1])
-            return self.engines[k % depth].batch_two_view(pts_a[lo:hi], pts_b[lo:hi], offsets[p0:p1 + 1] - lo, Ks[p0:p1],
-                                                          h, seed, threshold, min_extra, aggregation, selection,
-                                                          distance_threshold, pair_id0=pair_id0 + p0)
+            return call(self.engines[k % depth], pts_a[lo:hi], pts_b[lo:hi], offsets[p0:p1 + 1] - lo, Ks[p0:p1],
+                        pair_id0 + p0)
 
         def worker(e):
             return [(k, run(k)) for k in range(e, len(bounds) - 1, depth)]
 
         parts = dict(kv for res in self.pool.map(worker, range(depth)) for kv in res)
-        nchunks = len(bounds) - 1
-        out = {}
-        for key in parts[0].keys():
-            if key == "inlier_offsets":
-                base, segs = 0, [np.zeros(1, dtype=np.int64)]
-                for k in range(nchunks):
-                    segs.append(parts[k][key][1:] + base)
-                    base += int(parts[k][key][-1])
-                out[key] = np.concatenate(segs)
-            else:
-                out[key] = np.concatenate([parts[k][key] for k in range(nchunks)])
-        return out
+        return _merge_chunks([parts[k] for k in range(len(bounds) - 1)])
+
+    def batch_two_view(self, pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra=0.0, aggregation="rms",
+                       selection="min_error", distance_threshold=50.0, pair_id0=0, chunk_pairs: Optional[int] = None):
+        """``Engine.batch_two_view`` (RANSAC E + inlier list + pose vote + triangulation per pair) over chunks of
+        pairs that alternate between the contexts; identical to one call over all pairs."""
+        return self._chunked(lambda e, a, b, o, K, p0: e.batch_two_view(a, b, o, K, h, seed, threshold, min_extra,
+                                                                         aggregation, selection, distance_threshold,
+                                                                         pair_id0=p0),
+                             pts_a, pts_b, offsets, Ks, pair_id0, chunk_pairs)
+
+    def batch_two_view_homography(self, pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra=0.0, aggregation="rms",
+                                  selection="min_error", distance_threshold=50.0, rotation_tolerance=1e-2, pair_id0=0,
+                                  chunk_pairs: Optional[int] = None):
+        """``Engine.batch_two_view_homography`` over chunks of pairs; identical to one call over all pairs."""
+        return self._chunked(lambda e, a, b, o, K, p0: e.batch_two_view_homography(
+            a, b, o, K, h, seed, threshold, min_extra, aggregation, selection, distance_threshold, rotation_tolerance,
+            pair_id0=p0), pts_a, pts_b, offsets, Ks, pair_id0, chunk_pairs)
+
+    def batch_two_view_select(self, pts_a, pts_b, offsets, Ks, essential_threshold, homography_threshold, h, seed,
+                              pair_id0=0, chunk_pairs: Optional[int] = None, **kw):
+        """``model_selection.batch_two_view_select_arrays`` (keyword arguments passed on) over chunks of pairs;
+        identical to one call over all pairs."""
+        from .model_selection import batch_two_view_select_arrays
+
+        return self._chunked(lambda e, a, b, o, K, p0: batch_two_view_select_arrays(
+            a, b, o, K, essential_threshold, homography_threshold, h, seed, pair_id0=p0, engine=e, **kw),
+            pts_a, pts_b, offsets, Ks, pair_id0, chunk_pairs)
 
     def close(self):
         self.pool.shutdown()

@@ -1,4 +1,4 @@
-"""Essential matrix or homography for one image pair (numpy in, numpy out).
+"""Essential matrix or homography for one image pair or a batch of pairs (numpy in, numpy out).
 
 On a planar scene E is not determined by the data, on a rotation-only pair it vanishes, and on a general scene a
 homography fits one depth layer at best: a two-view initialiser estimates both models and keeps one.  The rule is
@@ -136,3 +136,107 @@ def two_view_select_arrays(
                             essential_failure=ess_fail, homography_failure=hom_fail, R=win.R, t=win.t,
                             inlier_indices=win.inlier_indices, passing=win.passing, points=win.points,
                             rotation_only=bool(scores.model == "homography" and hom.rotation_only))
+
+
+_SCORE_FIELDS = ("score_e", "score_h", "ratio_h", "fixed_e", "fixed_h", "count_e", "count_h")
+
+
+def _essential_status(r, sv2) -> np.ndarray:
+    """Per pair, why two_view_arrays would fail on it (None when it would not): no model (a pair of fewer than 8
+    correspondences has none), an E whose smallest singular value is not ~0, or no inlier passing any pose."""
+    st = np.full(len(r["best_index"]), None, dtype=object)
+    for p in range(len(st)):
+        if r["best_index"][p] < 0:
+            st[p] = "no model"
+        elif not np.isclose(0.0, sv2[p]):
+            st[p] = "degenerate essential matrix"
+        elif np.count_nonzero(r["counts"][p]) == 0:
+            st[p] = "no passing inlier"
+    return st
+
+
+def _homography_status(r) -> np.ndarray:
+    """Per pair, why two_view_homography_arrays would fail on it (None when it would not).  A rotation-only pair is
+    kept: it has no vote."""
+    st = np.full(len(r["best_index"]), None, dtype=object)
+    for p in range(len(st)):
+        if r["best_index"][p] < 0:
+            st[p] = "no model"
+        elif not r["rotation_only"][p] and np.count_nonzero(r["counts"][p]) == 0:
+            st[p] = "no passing inlier"
+    return st
+
+
+def batch_two_view_select_arrays(
+    pts_a,
+    pts_b,
+    offsets,
+    Ks,
+    essential_threshold: float,
+    homography_threshold: float,
+    h: int,
+    seed: int,
+    *,
+    min_extra: float = 0.0,
+    aggregation: str = "rms",
+    selection: str = "min_error",
+    distance_threshold: float = 50.0,
+    sigma: float = 1.0,
+    homography_ratio: float = 0.45,
+    rotation_tolerance: float = 1e-2,
+    pair_id0: int = 0,
+    engine: Optional[_native.Engine] = None,
+) -> dict:
+    """``two_view_select_arrays(sampler="device")`` for every pair of a batch: pair p owns rows
+    [offsets[p], offsets[p+1]) of the [n,2] pixel arrays and the camera Ks[p] (upper triangular, K[2,2] = 1).
+
+    Runs ``Engine.batch_two_view`` (E, ``essential_threshold``) and ``Engine.batch_two_view_homography`` (H,
+    ``homography_threshold`` in px^2) with the same h, seed and pair_id0, then ``Engine.batch_score_models`` on the
+    homography call's upload.  A side is given to the scorer for pair p exactly when the single-pair rule keeps it: it
+    has a winner and its vote has a passing inlier (an essential matrix also needs a smallest singular value ~0); a
+    rotation-only homography is kept.  Returns a dict:
+      essential, homography   the two batch dicts, each equal to its standalone call
+      essential_status, homography_status   object[P]: None where the side is kept, else why it is left out
+      model                   object[P]: "essential", "homography" or None (neither side kept)
+      score_e ... count_h     the scores of batch_score_models [P] (zero for a side left out)
+      R [P,3,3], t [P,3], rotation_only [P]   the chosen side's pose (NaN without a model)
+      inlier_offsets [P+1], inlier_idx, passing, points   the chosen side's inlier segments (empty without a model)
+    """
+    eng = engine or _native.get_engine()
+    offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+    P = len(offsets) - 1
+    Ks = np.asarray(Ks, dtype=np.float64).reshape(P, 3, 3)
+    ess, sv2 = eng._batch_two_view(pts_a, pts_b, offsets, Ks, h, seed, essential_threshold, min_extra, aggregation,
+                                   selection, distance_threshold, pair_id0)
+    hom = eng.batch_two_view_homography(pts_a, pts_b, offsets, Ks, h, seed, homography_threshold, min_extra, aggregation,
+                                        selection, distance_threshold, rotation_tolerance, pair_id0)
+    e_st, h_st = _essential_status(ess, sv2), _homography_status(hom)
+    keep_e, keep_h = np.equal(e_st, None), np.equal(h_st, None)
+    s, _ = eng.batch_score_models(ess["E"], hom["H"], keep_e, keep_h, sigma, homography_ratio)
+    out = dict(essential=ess, homography=hom, essential_status=e_st, homography_status=h_st)
+    for f in _SCORE_FIELDS:
+        out[f] = np.array([getattr(x, f) for x in s[:P]], dtype=np.float64 if f[:5] in ("score", "ratio") else np.int64)
+    code = np.array([x.model for x in s[:P]], dtype=np.int64)
+    out["model"] = np.array([_MODEL.get(int(m)) for m in code], dtype=object)
+    R = np.full((P, 3, 3), np.nan)
+    t = np.full((P, 3), np.nan)
+    rot = np.zeros(P, dtype=bool)
+    ioff, idx, passing, pts = [0], [], [], []
+    for p in range(P):
+        side = hom if code[p] == 1 else ess if code[p] == 0 else None
+        if side is None:
+            ioff.append(ioff[-1])
+            continue
+        lo, hi = side["inlier_offsets"][p], side["inlier_offsets"][p + 1]
+        b = int(side["pose_index"][p])
+        R[p], t[p] = side["R"][p], side["t"][p]
+        rot[p] = bool(code[p] == 1 and hom["rotation_only"][p])
+        idx.append(side["inlier_idx"][lo:hi])
+        passing.append(np.zeros(hi - lo, dtype=bool) if b < 0 else ((side["pass_bits"][lo:hi] >> b) & 1).astype(bool))
+        pts.append(side["points"][lo:hi])
+        ioff.append(ioff[-1] + (hi - lo))
+    out.update(R=R, t=t, rotation_only=rot, inlier_offsets=np.array(ioff, dtype=np.int64),
+               inlier_idx=np.concatenate(idx) if idx else np.zeros(0, dtype=np.int32),
+               passing=np.concatenate(passing) if passing else np.zeros(0, dtype=bool),
+               points=np.concatenate(pts) if pts else np.zeros((0, 3)))
+    return out
