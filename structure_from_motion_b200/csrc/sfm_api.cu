@@ -12,6 +12,8 @@
 #include <string>
 #include <vector>
 
+#include <cub/device/device_radix_sort.cuh>
+
 #include "sfm_device.cuh"
 #include "sfm_fit.cuh"
 #include "sfm_linalg.cuh"
@@ -101,6 +103,7 @@ struct sfm_ctx {
     Buf h_img, h_gx, h_gy, h_corner, h_alive, h_key, h_idx, h_small, h_xy;
     Buf mask, sed, poses, pass, X, idx, scan, tmp, tailstate, num, winrec, bout;
     Buf planes, hK;  // the homography tail's HPlane and the K it was called with (the upload's K stays in Ks)
+    Buf k2pts, k2box, k2sort;  // K2's copy of pts in image-B Morton order, its tile boxes, the sort's scratch
     Buf selstate, selio, selpp;  // k_score_models: self-cleaning sums; models and results; per-correspondence errors
     long long n = 0, h = 0, npairs = 1;
     long long first_len = 0;  // batched: correspondences of the first pair (what the AUTO pilot samples)
@@ -108,6 +111,7 @@ struct sfm_ctx {
     long long raw_stride = 1;
     bool batched = false, has_pts = false, has_table = false, has_models = false, has_score = false;
     bool models_h = false;       // the current models are homographies (sfm_fit_homography), not essential matrices
+    bool k2_ready = false;       // k2pts / k2box belong to the current upload (K-normalised records only)
     int hscore_occ = 0;          // resident blocks per SM of k_score_homography (queried once)
     bool table_pending = false;  // sfm_sample_device was called: the table is drawn by the fit kernel (or on demand)
     unsigned long long smp_seed = 0, smp_stream = 0;
@@ -216,25 +220,32 @@ inline cudaError_t chain_launch_ptr(sfm_ctx* c, const void* fn, dim3 grid, dim3 
     return cudaLaunchKernelExC(&cfg, fn, kargs);
 }
 
-// per-warp shared memory of a scoring body (the two-sided one has its own layout for hpt <= 2)
-size_t score_warp_smem(int hpt, bool full) {
+// per-warp shared memory of a scoring body (the two-sided one has its own layout for hpt <= 2, the 9-slot one adds
+// its boxes and kappa: tiles)
+template <int HPT>
+size_t score_warp_smem_h(bool full, bool tiles) {
+    return full ? score_warp_bytes<HPT, MODE_FULL>() : tiles ? score_warp_bytes<HPT, MODE_SCREEN>() : sizeof(ScoreWarpSmem<HPT>);
+}
+size_t score_warp_smem(int hpt, bool full, bool tiles) {
     switch (hpt) {
-        case 1: return full ? score_warp_bytes<1, MODE_FULL>() : sizeof(ScoreWarpSmem<1>);
-        case 2: return full ? score_warp_bytes<2, MODE_FULL>() : sizeof(ScoreWarpSmem<2>);
-        case 4: return full ? score_warp_bytes<4, MODE_FULL>() : sizeof(ScoreWarpSmem<4>);
-        default: return sizeof(ScoreWarpSmem<8>);
+        case 1: return score_warp_smem_h<1>(full, tiles);
+        case 2: return score_warp_smem_h<2>(full, tiles);
+        case 4: return score_warp_smem_h<4>(full, tiles);
+        default: return sizeof(ScoreWarpSmem<8>);  // SCREEN32 only
     }
 }
 
-const void* score_kernel(int variant, int hpt, int group) {
+// tiles: the upload holds K2's sorted copy and its boxes (k2_order), so SCREEN is the 9-slot body; else the 11-slot one
+const void* score_kernel(int variant, int hpt, int group, bool tiles) {
     if (variant == SFM_SCORE_SCREEN32) {
 #define SFM_K32(H, G) if (hpt == H && group == G) return reinterpret_cast<const void*>(&k_score<H, G, MODE_SCREEN32>)
         SFM_K32(2, 16); SFM_K32(4, 8); SFM_K32(8, 4);
 #undef SFM_K32
         return nullptr;
     }
-#define SFM_K(H, G) if (hpt == H && group == G) return scr ? reinterpret_cast<const void*>(&k_score<H, G, MODE_SCREEN>) \
-                                                           : reinterpret_cast<const void*>(&k_score<H, G, MODE_FULL>)
+#define SFM_K(H, G) if (hpt == H && group == G) return !scr ? reinterpret_cast<const void*>(&k_score<H, G, MODE_FULL>) \
+                                                    : tiles ? reinterpret_cast<const void*>(&k_score<H, G, MODE_SCREEN>) \
+                                                            : reinterpret_cast<const void*>(&k_score<H, G, MODE_SCREEN11>)
     const bool scr = variant == SFM_SCORE_SCREEN;
     SFM_K(1, 16); SFM_K(1, 32);
     SFM_K(2, 4); SFM_K(2, 8); SFM_K(2, 16);
@@ -299,7 +310,7 @@ int sfm_destroy(sfm_ctx* c) {
     Buf* bufs[] = {&c->raw, &c->pts, &c->offsets, &c->Ks, &c->table, &c->E, &c->valid, &c->eig, &c->acc,
                    &c->count_extra, &c->S1, &c->S2, &c->err, &c->blocks, &c->best,
                    &c->invalid, &c->winnerE, &c->record, &c->merged, &c->rows, &c->blockinv, &c->mask, &c->sed, &c->poses, &c->pass, &c->X, &c->idx,
-                   &c->planes, &c->hK, &c->selstate, &c->selio, &c->selpp,
+                   &c->planes, &c->hK, &c->selstate, &c->selio, &c->selpp, &c->k2pts, &c->k2box, &c->k2sort,
                    &c->scan, &c->tmp, &c->gathered, &c->tailstate, &c->num, &c->winrec, &c->bout, &c->spts, &c->bounds, &c->fitflag,
                    &c->m_img, &c->m_feat, &c->m_W, &c->m_ss, &c->m_ok, &c->m_S, &c->m_out,
                    &c->h_img, &c->h_gx, &c->h_gy, &c->h_corner, &c->h_alive, &c->h_key, &c->h_idx, &c->h_small, &c->h_xy};
@@ -343,8 +354,8 @@ int sfm_set_score_variant(sfm_ctx* c, int variant, int hpt, int group) {
         nh = variant == SFM_SCORE_SCREEN32 ? 4 : 2;
         ng = variant == SFM_SCORE_SCREEN32 ? 8 : 16;
     }
-    if (!score_kernel(variant == SFM_SCORE_AUTO ? SFM_SCORE_SCREEN : variant, nh, ng) ||
-        (variant == SFM_SCORE_AUTO && !score_kernel(SFM_SCORE_FULL, nh, ng)))
+    if (!score_kernel(variant == SFM_SCORE_AUTO ? SFM_SCORE_SCREEN : variant, nh, ng, true) ||
+        (variant == SFM_SCORE_AUTO && !score_kernel(SFM_SCORE_FULL, nh, ng, true)))
         return fail(SFM_ERR_ARG, "unsupported combination: hyps_per_thread %d, group %d", nh, ng);
     c->variant = variant;
     c->hpt = nh;
@@ -427,6 +438,53 @@ int sfm_get_table(sfm_ctx* c, int32_t* table, int64_t first, int64_t h) {
 }
 
 // ---- correspondences --------------------------------------------------------------------
+// K2's copy of c->pts (sfm_score.cuh, K2 header): the records of a single pair stably sorted by the Morton code of
+// (xb, yb) quantised to 16 bits per axis inside the pair's B bounding box, and the box of every tile of kTile records.
+// Only K2 reads it; every other kernel keeps the input order, and K2's integer sums do not depend on the order.
+// Single pairs of at least kK2SortMin correspondences get it, and K2 then screens in 9 slots against the tile bounds.
+// The sort is paid once per upload and costs 60-75 us below 100 000 correspondences, mostly launches; K2 saves about 7 %
+// of its time per estimate, so the trade depends on N x H, which the upload does not know.  Measured for one upload plus
+// one estimate (tools/sort_threshold.py, profiles/tile_screen_ab.txt): at 32 768 x 16 384 the sort cost 8.7 % end to
+// end and at 65 536 x 16 384 2.8 %, while 65 536 x 65 536 gained 4.3 %, 131 072 x 16 384 1.8 % and config3
+// (100 000 x 65 536) 0.36 ms.  So pairs below 65 536 keep the parent's path; single estimates just above it with few
+// hypotheses pay up to ~3 %, and everything with more correspondences, more hypotheses or several estimates per upload
+// gains.  Batches do not get
+// the sorted copy: at 512 pairs x 2 000 (bench config4) a sort of the whole batch cost 0.19 ms per 1M records at upload
+// and the 9-slot body was 1.5 % slower on K2 than the 11-slot one (the boxes of 2 000-point pairs are wide).
+#ifndef SFM_K2_SORT_MIN
+#define SFM_K2_SORT_MIN 65536
+#endif
+constexpr long long kK2SortMin = SFM_K2_SORT_MIN;
+static int k2_order(sfm_ctx* c, long long n) {
+    size_t cub_bytes = 0;
+    CU(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, (const unsigned*)nullptr, (unsigned*)nullptr, (const int*)nullptr,
+                                       (int*)nullptr, (int)n, 0, 32, c->stream));
+    const size_t vb = ((size_t)n * 4 + 255) & ~(size_t)255;  // one array of n keys or indices
+    if (int r = c->k2sort.reserve(4 * vb + 256 + cub_bytes)) return r;
+    char* w = c->k2sort.as<char>();
+    auto* keys = reinterpret_cast<unsigned*>(w);
+    auto* keys2 = reinterpret_cast<unsigned*>(w + vb);
+    int* idx = reinterpret_cast<int*>(w + 2 * vb);
+    int* idx2 = reinterpret_cast<int*>(w + 3 * vb);
+    auto* bb = reinterpret_cast<unsigned long long*>(w + 4 * vb);
+    void* tmp = w + 4 * vb + 256;
+    const long long tiles = (n + kTile - 1) / kTile;
+    if (int r = c->k2pts.reserve((size_t)n * sizeof(Corr))) return r;
+    if (int r = c->k2box.reserve((size_t)tiles * sizeof(double4))) return r;
+    CU(cudaMemsetAsync(bb, 0, 32, c->stream));
+    const unsigned grid = (unsigned)((n + 255) / 256);
+    k2_order_bbox<<<grid, 256, 0, c->stream>>>(c->pts.as<Corr>(), n, bb);
+    if (int r = check_launch(c, "k2_order_bbox")) return r;
+    k2_order_keys<<<grid, 256, 0, c->stream>>>(c->pts.as<Corr>(), n, bb, keys, idx);
+    if (int r = check_launch(c, "k2_order_keys")) return r;
+    CU(cub::DeviceRadixSort::SortPairs(tmp, cub_bytes, keys, keys2, idx, idx2, (int)n, 0, 32, c->stream));
+    k2_order_gather<<<(unsigned)((tiles + kOrderWarps - 1) / kOrderWarps), 32 * kOrderWarps, 0, c->stream>>>(
+        c->pts.as<Corr>(), n, idx2, c->k2pts.as<Corr>(), c->k2box.as<double4>());
+    if (int r = check_launch(c, "k2_order_gather")) return r;
+    c->k2_ready = true;
+    return 0;
+}
+
 static int normalise_from(sfm_ctx* c, const double* xa, const double* ya, const double* xb, const double* yb,
                           int64_t stride, int64_t n, int64_t max_len) {
     if (int r = c->pts.reserve((size_t)n * sizeof(Corr))) return r;
@@ -436,7 +494,9 @@ static int normalise_from(sfm_ctx* c, const double* xa, const double* ya, const 
     k_normalise<<<grid, 256, 0, c->stream>>>(xa, ya, xb, yb, stride, n,
                                              c->batched ? c->offsets.as<long long>() : nullptr,
                                              c->Ks.as<double>(), c->pts.as<Corr>(), c->bounds.as<unsigned long long>());
-    return check_launch(c, "k_normalise");
+    if (int r = check_launch(c, "k_normalise")) return r;
+    c->k2_ready = false;
+    return (!c->batched && n >= kK2SortMin) ? k2_order(c, n) : 0;
 }
 
 // Host coordinates to the device buffer d (room for 4 n doubles) in the caller's layout: four arrays (stride 1) or two
@@ -763,18 +823,19 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
     // SCREEN: relative guard here, absolute guard = kappa_h inside the kernel (see sfm_score.cuh);
     // SCREEN32: thr32 = 1.0316 thr, kappa32; FULL: relative guard + an absolute term that covers a
     // cancelling residual at the 1-ulp level
-    double thr_pre = f32 ? thr * kThr32Factor : (screen ? thr * (1.0 + 1e-9) : thr * (1.0 + 1e-9) + 1e-22);
+    double thr_pre = f32 ? thr * kThr32Factor : (screen ? thr * kThrScreenFactor : thr * (1.0 + 1e-9) + 1e-22);
     if (f32 && thr_pre < 1e-24) thr_pre = 1e-24;  // keeps s and 1/s comfortably inside fp32; only widens the screen
-    if (screen && thr_pre < 1e-280) thr_pre = 1e-280;  // keeps s = sqrt(thr') and 1/s normal; only widens the screen
+    if (screen && thr_pre < 1e-280) thr_pre = 1e-280;  // keeps thr' NB+ clear of underflow; only widens the screen
     const double s_scale = sqrt(thr_pre);
     const double scale1 = ldexp(1.0, 63 - e2), scale2 = ldexp(1.0, 63 - 2 * e2);
     unsigned long long* acc_dev = nullptr;
     {
         // persistent blocks over (pair, split, hypothesis block) items
-        const void* fn = score_kernel(variant, hpt, G);
+        const bool tiles = c->k2_ready;
+        const void* fn = score_kernel(variant, hpt, G, tiles);
         if (!fn) return fail(SFM_ERR_ARG, "unsupported scoring configuration (variant %d, hpt %d, group %d)", variant, hpt, G);
-        const size_t smem_one = (size_t)kScoreWarps * score_warp_smem(hpt, false);
-        const size_t smem_two = (size_t)kScoreWarps * score_warp_smem(hpt, true);
+        const size_t smem_one = (size_t)kScoreWarps * score_warp_smem(hpt, false, tiles && !f32);
+        const size_t smem_two = (size_t)kScoreWarps * score_warp_smem(hpt, true, false);
         const size_t smem_both = smem_one > smem_two ? smem_one : smem_two;  // AUTO in one launch holds either body
         const size_t smem = screen ? smem_one : smem_two;
         // attribute set and occupancy queried once per kernel instantiation (small cache)
@@ -799,12 +860,16 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
         // AUTO: one kernel holding both screens (shapes 2x16 and 4x8), else the two-launch scheme
         const void* fn_auto = nullptr;
         if (autov && SFM_AUTO_SINGLE) {
-            if (hpt == 2 && G == 16) fn_auto = reinterpret_cast<const void*>(&k_score_auto<2, 16>);
-            if (hpt == 4 && G == 8) fn_auto = reinterpret_cast<const void*>(&k_score_auto<4, 8>);
+            if (hpt == 2 && G == 16)
+                fn_auto = tiles ? reinterpret_cast<const void*>(&k_score_auto<2, 16, MODE_SCREEN>)
+                                : reinterpret_cast<const void*>(&k_score_auto<2, 16, MODE_SCREEN11>);
+            if (hpt == 4 && G == 8)
+                fn_auto = tiles ? reinterpret_cast<const void*>(&k_score_auto<4, 8, MODE_SCREEN>)
+                                : reinterpret_cast<const void*>(&k_score_auto<4, 8, MODE_SCREEN11>);
         }
         if (fn_auto)
             if (int r = occupancy(fn_auto, smem_both, &occ)) return r;
-        const void* fn_full = (autov && !fn_auto) ? score_kernel(SFM_SCORE_FULL, hpt, G) : nullptr;
+        const void* fn_full = (autov && !fn_auto) ? score_kernel(SFM_SCORE_FULL, hpt, G, tiles) : nullptr;
         int occ_full = 0;
         if (fn_full)
             if (int r = occupancy(fn_full, smem_two, &occ_full)) return r;
@@ -815,11 +880,16 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
         const long long total_items = hblocks * nsplit * P;
         if (int r = c->acc.reserve(H * kAccWords * 8 + acc_tail_bytes(P))) return r;
         const long long npts = c->n;  // total records (all pairs)
+        const bool scaled = screen && !f32 && !tiles;  // the 11-slot screen streams a scaled copy
         if (f32) { if (int r = c->spts.reserve((size_t)npts * sizeof(Corr32))) return r; }
-        else if (screen) { if (int r = c->spts.reserve((size_t)npts * sizeof(Corr))) return r; }
+        else if (scaled) { if (int r = c->spts.reserve((size_t)npts * sizeof(Corr))) return r; }
+        // only the 9-slot body streams the sorted copy; the others keep the input order (sorting by image-B position
+        // clusters a hypothesis' survivors into the same batches, which the two-sided body's rounds pay for)
+        const Corr* kpts = (tiles && screen && !f32) ? c->k2pts.as<Corr>() : c->pts.as<Corr>();
         ScoreArgs a;
-        a.pts = c->pts.as<Corr>();
-        a.spts = screen ? c->spts.p : c->pts.p;
+        a.pts = kpts;
+        a.spts = (f32 || scaled) ? c->spts.p : (const void*)kpts;
+        a.boxes = tiles ? c->k2box.as<double4>() : nullptr;
         a.bounds = c->bounds.as<double>();
         a.s = s_scale;
         a.kappa_coef = kKappaCoef * (1.0 + thr);
@@ -847,21 +917,31 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
         c->tic(T_SCORE);
         if (int r = clear_acc(c, H, P)) return r;
         if (f32 && !skip_k2) {
-            k_screen_pts32<<<(unsigned)((npts + 255) / 256), 256, 0, c->stream>>>(c->pts.as<Corr>(), npts, 1.0 / s_scale,
+            k_screen_pts32<<<(unsigned)((npts + 255) / 256), 256, 0, c->stream>>>(kpts, npts, 1.0 / s_scale,
                                                                                   reinterpret_cast<Corr32*>(c->spts.p));
             if (int r = check_launch(c, "k_screen_pts32")) return r;
         }
-        else if (screen && !skip_k2) {
+        else if ((scaled || autov) && !skip_k2) {
             PilotArgs pa;
             pa.E = c->E.as<double>();
             pa.h = h;
             pa.plen = c->batched ? c->first_len : c->n;  // batches: the pilot looks at the first pair
             pa.thr_pre = thr_pre;
+            pa.bounds = a.bounds;
+            pa.kappa_coef = a.kappa_coef;
+            pa.boxes = a.boxes;
             pa.counters = reinterpret_cast<unsigned*>(tailp + 16);
             pa.mode_flag = autov ? reinterpret_cast<int*>(tailp + 32) : nullptr;
-            CU(chain_launch(c, k_screen_pts64, dim3((unsigned)((npts + 255) / 256)), dim3(256), 0, c->pts.as<Corr>(), npts,
-                            1.0 / s_scale, reinterpret_cast<Corr*>(c->spts.p), pa));
-            if (int r = check_launch(c, "k_screen_pts64")) return r;
+            const long long copy_blocks = (npts + 255) / 256;
+            if (scaled) {  // the copy carries the pilot
+                CU(chain_launch(c, k_screen_pts64, dim3((unsigned)copy_blocks), dim3(256), 0, kpts, npts, 1.0 / s_scale,
+                                reinterpret_cast<Corr*>(c->spts.p), pa));
+                if (int r = check_launch(c, "k_screen_pts64")) return r;
+            } else {
+                CU(chain_launch(c, k_pilot, dim3((unsigned)(copy_blocks < kPilotBlocks ? copy_blocks : kPilotBlocks)), dim3(256),
+                                0, kpts, pa));
+                if (int r = check_launch(c, "k_pilot")) return r;
+            }
         }
         const long long want_blocks = (total_items + kScoreWarps - 1) / kScoreWarps;
         const long long launch_blocks = grid_blocks < want_blocks ? grid_blocks : want_blocks;
@@ -869,7 +949,8 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
         if (!skip_k2 && fn_auto) {
             ScoreArgs a2 = a;
             a2.thr_pre = thr * (1.0 + 1e-9) + 1e-22;
-            a2.spts = c->pts.p;
+            a2.pts = c->pts.as<Corr>();
+            a2.spts = a2.pts;
             void* kargs2[] = {(void*)&a, (void*)&a2};
             CU(chain_launch_ptr(c, fn_auto, dim3((unsigned)launch_blocks), dim3(kScoreThreads), smem_both, kargs2));
             if (int r = check_launch(c, "k_score_auto")) return r;
@@ -879,7 +960,8 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
             if (fn_full) {  // AUTO: the two-sided screen on the unscaled records; exits at once unless the pilot chose it
                 ScoreArgs a2 = a;
                 a2.thr_pre = thr * (1.0 + 1e-9) + 1e-22;
-                a2.spts = c->pts.p;
+                a2.pts = c->pts.as<Corr>();
+                a2.spts = a2.pts;
                 const long long gb2 = (long long)c->sm_count * occ_full;
                 const long long lb2 = gb2 < want_blocks ? gb2 : want_blocks;
                 void* kargs2[] = {(void*)&a2};
@@ -1869,6 +1951,7 @@ static int batch_upload(sfm_ctx* c, const double* xa, const double* ya, const do
         k_normalise<<<dim3((unsigned)((n + 255) / 256), 1), 256, 0, c->stream>>>(s[0], s[1], s[2], s[3], stride, n, nullptr,
                                                                                 c->hK.as<double>(), c->pts.as<Corr>(), nullptr);
         if (int r = check_launch(c, "k_normalise")) return r;
+        c->k2_ready = false;  // pixel records: the essential-matrix scorer does not run on them
     } else if (int r = normalise_from(c, s[0], s[1], s[2], s[3], stride, n, max_len)) {
         return r;
     }

@@ -70,20 +70,6 @@ __device__ __forceinline__ double sed_exact(const double (&e)[9], double xa, dou
     return __dmul_rn(__dadd_rn(__drcp_rn(na), __drcp_rn(nb)), __dmul_rn(r, r));
 }
 
-// Screening form: 12 FP64 issue slots.  Returns d = r^2 - thr_pre * nb; a correspondence
-// can only be an inlier (sed <= thr) if r^2/nb <= thr, so d < 0 (with thr_pre carrying a
-// rounding guard) is a necessary condition and everything with d >= 0 is rejected without
-// evaluating the image-A side.
-__device__ __forceinline__ double sed_screen(const double (&e)[9], double xa, double ya, double xb,
-                                             double yb, double thr_pre) {
-    const double lb0 = fma(xb, e[0], fma(yb, e[3], e[6]));
-    const double lb1 = fma(xb, e[1], fma(yb, e[4], e[7]));
-    const double lb2 = fma(xb, e[2], fma(yb, e[5], e[8]));
-    const double r = fma(xa, lb0, fma(ya, lb1, lb2));
-    const double nb = fma(lb0, lb0, lb1 * lb1);
-    return fma(r, r, -(thr_pre * nb));
-}
-
 // Full division-free decision, 21 FP64 issue slots: d = r^2 (na+nb) - thr_pre na nb.
 __device__ __forceinline__ double sed_full_decision(const double (&e)[9], double xa, double ya,
                                                     double xb, double yb, double thr_pre) {

@@ -70,22 +70,43 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
 // the records and process them 32 at a time (dense, no divergence): the exact reference-order
 // SED is evaluated and compared with thr.
 //
-//   SCREEN (default), 11 FP64 issue slots per evaluation.  sed <= thr implies
+//   SCREEN (default), 9 FP64 issue slots per evaluation.  sed <= thr implies
 //   r^2 <= thr * nb  (drop the image-A term), nb = lb0^2 + lb1^2, lb = E^T b, r = lb . a.
-//   With s = sqrt(thr'), the kernel keeps E with columns 0 and 1 pre-multiplied by s and
-//   streams a copy of the correspondences with (xa, ya) pre-divided by s (k_screen_pts64; scaling the
-//   tiles inside this kernel instead costs 5 %: profiles/r2_scale_modes.txt), so that
-//       lb0' = s lb0, lb1' = s lb1, lb2   (6 DFMA)      r = lb0' xa' + lb1' ya' + lb2   (2 DFMA)
-//       m = lb1'^2 + kappa ; m = lb0'^2 + m   (2 DFMA)  d = r^2 - m                      (1 DFMA)
-//   and "d < 0" (sign bit) is the test.  thr' = thr (1 + 1e-9) and
-//   kappa_h = 4e-20 (1 + thr) |E_h|_F^2 A^2 B^2  (A, B = max |(x, y, 1)| over each image)
-//   bound every rounding difference between this evaluation order and the reference's:
-//   |r_screen - r_ref| <= 32 u |E| A B =: eps and 2 |r| eps <= 1e-9 r^2 + 1e9 eps^2 (AM-GM), the
-//   same for the absolute errors of lb0, lb1 inside nb — so an inlier of the exact scorer
-//   can never be screened out, at any threshold.  The screen is written
+//   nb depends on the image-B point only.  K2 streams its own copy of a single pair's correspondences,
+//   sorted by a Morton key of (xb, yb) at upload (k2_order_*, sfm_api.cu: k2_order), and every tile of kTile
+//   records comes with the box of its B points: centre (cx, cy), half-widths (wx, wy) with
+//   |xb - cx| <= wx and |yb - cy| <= wy for every record of the tile.  Once per (tile, hypothesis):
+//       l_i = lb_i(cx, cy),  m_i = |l_i| + |E_0i| wx + |E_1i| wy  (i = 0, 1)      (8 DFMA)
+//       T = thr' (m0^2 + m1^2) + kappa                                             (3 DFMA)
+//   and per test
+//       lb0, lb1, lb2   (6 DFMA)      r = lb0 xa + lb1 ya + lb2   (2 DFMA)      d = r^2 - T   (1 DFMA)
+//   with "d < 0" (sign bit) as the test.  thr' = thr (1 + 3e-9) and
+//   kappa_h = 4.2e-20 (1 + thr) |E_h|_F^2 A^2 B^2  (A, B = max |(x, y, 1)| over each image).
+//   Why no inlier of the exact scorer is ever screened out, at any threshold:
+//   (a) the reference's r and nb against the exact ones: |r_screen - r_ref| <= 32 u |E| A B =: eps
+//       and 2 |r| eps <= 1e-9 r^2 + 1e9 eps^2 (AM-GM), the same for the absolute errors of the
+//       reference's lb0, lb1 inside its nb: 4e-20 (1 + thr) |E|^2 A^2 B^2 of kappa and a relative
+//       1e-9 of thr' (the bound of the 11-slot screen this body replaced, which had the larger
+//       screen-side rounding: it also rounded (xa, ya) / sqrt(thr')).
+//   (b) the box bound against the exact nb of every record of the tile: lb_i is affine in b, so
+//       |lb_i(b)| <= |lb_i(c)| + |E_0i| wx + |E_1i| wy exactly.  The computed l_i is within
+//       delta_i <= 2.0001 u |E_.i| |(cx, cy, 1)| of lb_i(c), and |(cx, cy, 1)|^2 <= 2 B^2, so
+//       (|l_i| + delta_i + w_i)^2 <= (1 + 1e-9) (|l_i| + w_i)^2 + 1.000001e9 delta_i^2 leaves
+//       1e-22 thr |E|^2 B^2 <= 0.0025 * 4e-20 (1 + thr) |E|^2 A^2 B^2 absolute and 1e-9 relative;
+//       the seven roundings of m_i, m0^2 + m1^2 and T are downward by at most (1 - 8u) on sums of
+//       non-negative terms, covered by the remaining 1e-9 of thr'.  kappa's 0.2e-20 covers both.
+//   A T that is NaN (an inf/NaN model or coordinate bound) becomes +inf: every test of that tile
+//   survives and the exact scorer decides, as the 11-slot screen did.  Padding lanes have E = 0
+//   and kappa = -1, so T = -1 and d = 1 > 0 (boxes are finite: a tile with a non-finite B
+//   coordinate gets centre 0 and half-widths DBL_MAX).  The screen is written
 //   hypothesis-innermost so that consecutive DFMAs share the correspondence operand (a DFMA
 //   with three fresh 64-bit register operands issues at 2/3 rate on sm_100, measured by
 //   tools/fp64_micro.cu).
+//   SCREEN11: the 11-slot one-sided screen for uploads without the sorted copy (batches, short pairs: their boxes
+//   are wide, see k2_order in sfm_api.cu).  With s = sqrt(thr'), E has columns 0 and 1 pre-multiplied by s and the
+//   records are a copy with (xa, ya) pre-divided by s (k_screen_pts64), so that
+//       lb0' = s lb0, lb1' = s lb1, lb2 (6 DFMA)   r (2 DFMA)   m = lb1'^2 + kappa; m = lb0'^2 + m (2)   d = r^2 - m (1)
+//   with the same thr' and kappa ((a) above covers it: its nb is the computed one).
 //   FULL: the 21-slot two-sided division-free decision on the unscaled data (survivors ~
 //   inliers); identical results; the like-for-like arithmetic baseline AND the body the AUTO
 //   variant switches to above 9 % survivors.  Its survivor path differs: one ring ENTRY per
@@ -126,10 +147,12 @@ constexpr int kChunkBits = 21;
 constexpr int kAccWords = 1 + 2 * kChunks;  // count, sum(sed), sum(sed^2)
 constexpr long long kMaxItemPoints = 1ll << 11;  // 2^11 adds of < 2^21 cannot overflow a 32-bit word
 enum { SUM_S1 = 1, SUM_S2 = 2 };       // which sums a launch accumulates
-enum { MODE_FULL = 0, MODE_SCREEN = 1, MODE_SCREEN32 = 2 };
-constexpr double kKappaCoef = 4e-20;
+enum { MODE_FULL = 0, MODE_SCREEN = 1, MODE_SCREEN32 = 2, MODE_SCREEN11 = 3 };
+constexpr double kKappaCoef = 4.2e-20;
+constexpr double kThrScreenFactor = 1.0 + 3e-9;  // thr' of the fp64 screen, see the K2 header
 constexpr double kKappa32Coef = 1.2e-10;   // fp32 pre-filter, see the K2 header
 constexpr double kThr32Factor = 1.0316;   // (1 + 1/64)^2 (1 + 1e-4)
+
 
 __global__ void __launch_bounds__(256) k_pad_models(const double* __restrict__ E, long long htotal, ModelRow* __restrict__ rows) {
     const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
@@ -143,15 +166,15 @@ __global__ void __launch_bounds__(256) k_pad_models(const double* __restrict__ E
 }
 
 struct ScoreArgs {
-    const Corr* pts;           // K-normalised correspondences (exact scorer)
-    const void* spts;          // screening copy: Corr (xa/s, ya/s, xb, yb) for the fp64 screen, Corr32 for the fp32 pre-filter
+    const Corr* pts;           // K-normalised correspondences: K2's sorted copy (the 9-slot SCREEN), else in input order
+    const void* spts;          // streamed records: pts, or its scaled copy (SCREEN11: Corr, SCREEN32: Corr32)
     const double* bounds;      // [2]: max (xa^2+ya^2+1), max (xb^2+yb^2+1) over all correspondences
     long long n;
     const long long* offsets;  // [npairs+1] or null (single pair of n records)
     const double* E;           // [npairs][h][9]
     const ModelRow* rows;      // [npairs][h] padded copies of E for the survivor path
     long long h;
-    double thr, thr_pre, s;    // s = sqrt(thr_pre) (SCREEN)
+    double thr, thr_pre, s;    // s = sqrt(thr_pre) (SCREEN32)
     double kappa_coef;         // kKappaCoef * (1 + thr)
     double kappa32_coef;       // kKappa32Coef * (1 + thr)
     double scale1, scale2;     // 2^(63-e), 2^(63-2e) with thr < 2^e
@@ -163,6 +186,7 @@ struct ScoreArgs {
     unsigned* work_counter;
     unsigned long long* acc;   // [kAccWords][htotal] exact integer accumulators (pre-zeroed)
     const int* mode_flag;      // AUTO variant: the MODE the pilot selected (the other kernel exits at once); else null
+    const double4* boxes;      // SCREEN (single pairs only): (cx, cy, wx, wy) of the B points of tile t of pts at [t]
 };
 
 __device__ __forceinline__ unsigned atom_add_acq_rel_shared(unsigned* p, unsigned v) {
@@ -201,60 +225,184 @@ struct __align__(16) Corr32 {
     float xa, ya, xb, yb;
 };
 
-// fp64 screening copy (xa / s, ya / s, xb, yb) written at the head of every SCREEN scoring call - and, for the AUTO
-// variant, the PILOT that chooses between the two fp64 screens: the first kPilotBlocks blocks also run the one-sided
-// test on a sample (64 hypotheses spread over the range x ~1 000 correspondences of the first pair, 8 tests per thread) and the last of
-// them to finish turns the pass rate into the MODE the scoring kernels check.  Above ~9 % survivors the exact
-// evaluation of the survivors dominates and the 21-slot two-sided screen (survivors = inliers) wins; below, the
-// 11-slot one-sided screen does (DESIGN.md, table against the threshold).
+// T = thr' NB+ + kappa of one hypothesis over one tile: NB+ >= lb0^2 + lb1^2 at every B point of the box (K2 header);
+// a NaN bound becomes +inf, so that every test of the tile survives and the exact scorer decides
+__device__ __forceinline__ double tile_bound(const double (&e)[9], double4 box, double thr_pre, double kap) {
+    const double l0 = fma(box.x, e[0], fma(box.y, e[3], e[6]));
+    const double l1 = fma(box.x, e[1], fma(box.y, e[4], e[7]));
+    const double m0 = fma(fabs(e[0]), box.z, fma(fabs(e[3]), box.w, fabs(l0)));
+    const double m1 = fma(fabs(e[1]), box.z, fma(fabs(e[4]), box.w, fabs(l1)));
+    const double t = fma(thr_pre, fma(m0, m0, m1 * m1), kap);
+    return t == t ? t : __longlong_as_double(0x7ff0000000000000LL);
+}
+
+// ---- K2's copy of the correspondences (at upload; it depends on nothing else) ----------------------------------
+// Order-preserving 64-bit image of a double (NaN excluded by the callers): unsigned order = numeric order.
+__device__ __forceinline__ unsigned long long k2_ordered(double x) {
+    const unsigned long long b = (unsigned long long)__double_as_longlong(x);
+    return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+}
+__device__ __forceinline__ double k2_unordered(unsigned long long k) {
+    return __longlong_as_double((long long)((k >> 63) ? (k & 0x7fffffffffffffffull) : ~k));
+}
+
+// Bounding box of the pair's B points: bb = {~min xb, ~min yb, max xb, max yb} as ordered keys (zero on entry; minima
+// complemented so that every word is an atomicMax).  NaN coordinates are left out.
+__global__ void __launch_bounds__(256) k2_order_bbox(const Corr* __restrict__ pts, long long n,
+                                                     unsigned long long* __restrict__ bb) {
+    const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    unsigned long long v[4] = {0ull, 0ull, 0ull, 0ull};
+    if (i < n) {
+        const Corr c = pts[i];
+        if (c.xb == c.xb) { v[0] = ~k2_ordered(c.xb); v[2] = k2_ordered(c.xb); }
+        if (c.yb == c.yb) { v[1] = ~k2_ordered(c.yb); v[3] = k2_ordered(c.yb); }
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) {
+            const unsigned long long o = __shfl_xor_sync(0xffffffffu, v[k], d);
+            v[k] = o > v[k] ? o : v[k];
+        }
+    }
+    if ((threadIdx.x & 31) == 0 && i < n)
+#pragma unroll
+        for (int k = 0; k < 4; ++k) atomicMax(bb + k, v[k]);
+}
+
+// one axis quantised to 16 bits inside [lo, hi]; a degenerate or non-finite range (or a NaN coordinate) maps to 0
+__device__ __forceinline__ unsigned k2_quantise(double x, double lo, double hi) {
+    const double sc = 65535.0 / (hi - lo);
+    const double q = (sc > 0.0 && sc < 1e308) ? (x - lo) * sc : 0.0;
+    return (unsigned)fmin(fmax(q, 0.0), 65535.0);  // fmax(NaN, 0) = 0
+}
+__device__ __forceinline__ unsigned k2_spread16(unsigned v) {  // bit k -> bit 2k
+    v = (v | (v << 8)) & 0x00ff00ffu;
+    v = (v | (v << 4)) & 0x0f0f0f0fu;
+    v = (v | (v << 2)) & 0x33333333u;
+    return (v | (v << 1)) & 0x55555555u;
+}
+// sort keys (Morton code of (xb, yb) in the pair's box) and the identity permutation
+__global__ void __launch_bounds__(256) k2_order_keys(const Corr* __restrict__ pts, long long n,
+                                                     const unsigned long long* __restrict__ bb,
+                                                     unsigned* __restrict__ keys, int* __restrict__ idx) {
+    const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const Corr c = pts[i];
+    const unsigned qx = k2_quantise(c.xb, k2_unordered(~bb[0]), k2_unordered(bb[2]));
+    const unsigned qy = k2_quantise(c.yb, k2_unordered(~bb[1]), k2_unordered(bb[3]));
+    keys[i] = (k2_spread16(qy) << 1) | k2_spread16(qx);
+    idx[i] = (int)i;
+}
+
+// One warp per tile: gather the tile's records in sorted order and write its box (K2 header).  cx is the rounded
+// midpoint and wx = max(hi - cx, cx - lo) rounded up, so |xb - cx| <= wx holds exactly for every record.
+constexpr int kOrderWarps = 4;
+__global__ void __launch_bounds__(32 * kOrderWarps) k2_order_gather(const Corr* __restrict__ pts, long long n,
+                                                                   const int* __restrict__ idx, Corr* __restrict__ out,
+                                                                   double4* __restrict__ boxes) {
+    const long long t = (long long)blockIdx.x * kOrderWarps + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (t * kTile >= n) return;
+    double lo[2] = {__longlong_as_double(0x7ff0000000000000LL), __longlong_as_double(0x7ff0000000000000LL)};
+    double hi[2] = {-lo[0], -lo[1]};
+#pragma unroll
+    for (int k = lane; k < kTile; k += 32) {
+        const long long i = t * kTile + k;
+        if (i < n) {
+            const Corr c = pts[idx[i]];
+            out[i] = c;
+            lo[0] = fmin(lo[0], c.xb); hi[0] = fmax(hi[0], c.xb);  // fmin/fmax drop NaN
+            lo[1] = fmin(lo[1], c.yb); hi[1] = fmax(hi[1], c.yb);
+        }
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1)
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            lo[k] = fmin(lo[k], __shfl_xor_sync(0xffffffffu, lo[k], d));
+            hi[k] = fmax(hi[k], __shfl_xor_sync(0xffffffffu, hi[k], d));
+        }
+    if (lane == 0) {
+        double cw[4];
+        bool finite = true;
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            cw[k] = 0.5 * lo[k] + 0.5 * hi[k];
+            cw[2 + k] = fmax(__dsub_ru(hi[k], cw[k]), __dsub_ru(cw[k], lo[k]));
+            finite = finite && fabs(cw[k]) <= 1.7976931348623157e308 && fabs(cw[2 + k]) <= 1.7976931348623157e308;
+        }
+        // a tile with an infinite B coordinate (or only NaN ones): the box of every finite point
+        boxes[t] = finite ? make_double4(cw[0], cw[1], cw[2], cw[3])
+                          : make_double4(0.0, 0.0, 1.7976931348623157e308, 1.7976931348623157e308);
+    }
+}
+
+// For the AUTO variant, the PILOT that chooses between the one-sided and the two-sided fp64 screen: kPilotBlocks blocks
+// run the one-sided test that K2 will run (9-slot against the tile bounds, or 11-slot) on a sample (64 hypotheses spread
+// over the range x ~1 000 correspondences of the first pair, 8 tests per thread) and the last of them to finish turns
+// the pass rate into the MODE the scoring kernel checks.  Above ~9 % survivors the exact evaluation of the survivors
+// dominates and the 21-slot two-sided screen (survivors = inliers) wins; below, the one-sided screen does (DESIGN.md,
+// table against the threshold).
 constexpr int kPilotBlocks = 32;
 constexpr int kPilotHyps = 64;
 constexpr int kPilotPts = 1024;
-constexpr double kPilotFullAbove = 0.09;  // measured crossover of the two bodies (tools/auto_crossover.py): 9.2 % on config 3
+constexpr double kPilotFullAbove = 0.09;  // measured crossover of the two bodies (tools/auto_crossover.py)
 struct PilotArgs {
     const double* E;      // models of the first pair
     long long h;          // hypotheses per pair
     long long plen;       // correspondences of the first pair
     double thr_pre;
+    const double* bounds; // [2] A^2, B^2 (k_normalise)
+    double kappa_coef;    // kKappaCoef * (1 + thr)
+    const double4* boxes; // the tile boxes of K2's sorted copy (BOXES pilot only)
     unsigned* counters;   // [0] passes, [1] ticket (zero on entry)
     int* mode_flag;       // out
 };
-__global__ void __launch_bounds__(256) k_screen_pts64(const Corr* __restrict__ pts, long long n, double inv_s,
-                                                      Corr* __restrict__ spts, const PilotArgs pa) {
-    chain_enter();
-    const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (i < n) {
-        Corr c = pts[i];
-        c.xa *= inv_s;
-        c.ya *= inv_s;
-        spts[i] = c;
-    }
-    if (!pa.mode_flag || blockIdx.x >= kPilotBlocks) return;
-    // pilot: thread t of block b -> hypothesis (t % 64) of the sample, correspondences (b * 4 + t / 64) + 32 k
-    const int nb = gridDim.x < kPilotBlocks ? gridDim.x : kPilotBlocks;
+// the pilot's work in one of nb blocks (block-uniform: every thread of the block calls it); BOXES: the 9-slot test
+// against the tile bounds, else the 11-slot one
+template <bool BOXES>
+__device__ __forceinline__ void pilot_block(const Corr* __restrict__ pts, const PilotArgs& pa, int nb) {
+    // thread t of block b -> hypothesis (t % 64) of the sample, correspondences (b * 4 + t / 64) + 32 k
     const long long nh = pa.h < kPilotHyps ? pa.h : kPilotHyps;
     const int hs = threadIdx.x % kPilotHyps;
     int pass = 0, tests = 0;
     if (hs < nh && pa.plen > 0) {
         const long long hyp = (pa.h / nh) * hs;
-        double e[9];
+        double e[9], f2 = 0.0;
 #pragma unroll
-        for (int k = 0; k < 9; ++k) e[k] = pa.E[9 * hyp + k];
+        for (int k = 0; k < 9; ++k) {
+            e[k] = pa.E[9 * hyp + k];
+            f2 = fma(e[k], e[k], f2);
+        }
+        const double kap = f2 * (pa.bounds[0] * pa.bounds[1] * pa.kappa_coef);  // as K2's kappa
         const long long np = pa.plen < kPilotPts ? pa.plen : kPilotPts;
         const long long step = pa.plen / np;
         const int lanes = nb * (256 / kPilotHyps);
         // at most 8 correspondences per thread, loads issued back to back (the kernel is pure latency otherwise)
         Corr cs[8];
+        double4 bx[8];
         int got = 0;
 #pragma unroll
         for (int u = 0; u < 8; ++u) {
             const long long q = blockIdx.x * (256 / kPilotHyps) + threadIdx.x / kPilotHyps + (long long)u * lanes;
-            if (q < np) { cs[u] = pts[q * step]; got = u + 1; }
+            if (q < np) {
+                cs[u] = pts[q * step];
+                if constexpr (BOXES) bx[u] = pa.boxes[q * step / kTile];
+                got = u + 1;
+            }
         }
 #pragma unroll
         for (int u = 0; u < 8; ++u)
             if (u < got) {
-                pass += sed_screen(e, cs[u].xa, cs[u].ya, cs[u].xb, cs[u].yb, pa.thr_pre) < 0.0 ? 1 : 0;
+                const double lb0 = fma(cs[u].xb, e[0], fma(cs[u].yb, e[3], e[6]));
+                const double lb1 = fma(cs[u].xb, e[1], fma(cs[u].yb, e[4], e[7]));
+                const double lb2 = fma(cs[u].xb, e[2], fma(cs[u].yb, e[5], e[8]));
+                const double r = fma(cs[u].xa, lb0, fma(cs[u].ya, lb1, lb2));
+                double t;
+                if constexpr (BOXES) t = tile_bound(e, bx[u], pa.thr_pre, kap);
+                else t = pa.thr_pre * fma(lb0, lb0, lb1 * lb1);
+                pass += fma(r, r, -t) < 0.0 ? 1 : 0;
                 tests += 1;
             }
     }
@@ -281,6 +429,28 @@ __global__ void __launch_bounds__(256) k_screen_pts64(const Corr* __restrict__ p
         }
     }
 }
+// the 9-slot screen's pilot on its own (K2's sorted copy needs no per-call copy)
+__global__ void __launch_bounds__(256) k_pilot(const Corr* __restrict__ pts, const PilotArgs pa) {
+    chain_enter();
+    pilot_block<true>(pts, pa, gridDim.x);
+}
+
+// 11-slot screen only: Corr copy with (xa, ya) pre-divided by s = sqrt(thr') (thr-dependent, so it runs at the head of
+// every such scoring call; scaling the tiles inside K2 instead costs 5 %: profiles/r2_scale_modes.txt).  AUTO: its
+// first kPilotBlocks blocks also run the pilot of the 11-slot screen (pa.mode_flag set).
+__global__ void __launch_bounds__(256) k_screen_pts64(const Corr* __restrict__ pts, long long n, double inv_s,
+                                                      Corr* __restrict__ spts, const PilotArgs pa) {
+    chain_enter();
+    const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (i < n) {
+        Corr c = pts[i];
+        c.xa *= inv_s;
+        c.ya *= inv_s;
+        spts[i] = c;
+    }
+    if (!pa.mode_flag || blockIdx.x >= kPilotBlocks) return;
+    pilot_block<false>(pts, pa, gridDim.x < kPilotBlocks ? gridDim.x : kPilotBlocks);
+}
 
 // fp32 pre-filter only: Corr32 copy of the correspondences with (xa, ya) pre-divided by s (thr-dependent, so it runs
 // at the head of every SCREEN32 scoring call).  The coordinate bounds used by kappa come from k_normalise.
@@ -304,6 +474,13 @@ struct alignas(128) ScoreWarpSmem {
     unsigned short own[32];
     unsigned long long full_bar[kStages];
 };
+// The 9-slot body's layout: the same, plus the tile boxes and kappa.  Only it pays for them: the other one-sided
+// bodies keep the smaller layout and with it their blocks per SM (SCREEN32 at hpt 4 fits 5 blocks only without them).
+template <int HPT>
+struct alignas(128) ScoreWarpSmemBox : ScoreWarpSmem<HPT> {
+    double4 box[kStages];  // the box of the tile in the same stage, delivered by the same mbarrier
+    double kap[HPT][32];   // kappa of (slot, lane), read once per tile (registers are the screen's)
+};
 
 // Two-sided body, HPT <= 2 (the survivor-rich regime: AUTO sends > 9 % survivors here): the drain gathers nothing
 // from global memory.  Its models sit in shared memory (component-major: a gather of 32 models is nine LDS.64) and
@@ -325,7 +502,9 @@ struct alignas(128) ScoreWarpSmemFS {
 __host__ __device__ constexpr bool score_full_in_smem(int hpt) { return hpt <= 2; }
 template <int HPT, int MODE>
 constexpr size_t score_warp_bytes() {
-    return (MODE == MODE_FULL && score_full_in_smem(HPT)) ? sizeof(ScoreWarpSmemFS<HPT>) : sizeof(ScoreWarpSmem<HPT>);
+    return (MODE == MODE_FULL && score_full_in_smem(HPT)) ? sizeof(ScoreWarpSmemFS<HPT>)
+           : MODE == MODE_SCREEN                          ? sizeof(ScoreWarpSmemBox<HPT>)
+                                                          : sizeof(ScoreWarpSmem<HPT>);
 }
 
 // resident blocks per SM the register budget is shaped for (HPT 4 / 2 / 1): 16 / 20 / 32 warps.  Measured on
@@ -347,22 +526,27 @@ template <int HPT, int G, int MODE>
 __device__ __forceinline__ void score_body(const ScoreArgs& a) {
     constexpr bool SCREEN = MODE != MODE_FULL;
     constexpr bool F32 = MODE == MODE_SCREEN32;
+    constexpr bool SCALED = F32 || MODE == MODE_SCREEN11;  // columns 0, 1 of E times s, records (xa, ya) / s
     using T = typename std::conditional<F32, float, double>::type;       // arithmetic of the per-test work
     using P = typename std::conditional<F32, Corr32, Corr>::type;       // record streamed through shared memory
     constexpr int NB = HPT * G;  // tests per lane and batch = survivor bits per vote
     constexpr bool FS = MODE == MODE_FULL && score_full_in_smem(HPT);  // drain gathers from shared memory only
     constexpr bool ENTRY = MODE == MODE_FULL;  // survivor ring of per-survivor entries instead of per-lane records
+    constexpr bool BOX = MODE == MODE_SCREEN;  // 9-slot screen against the tile's bound
     constexpr int TILE = FS ? kTileFS : kTile;
     constexpr int STAGES = FS ? kStagesFS : kStages;
     constexpr int AHEAD = FS ? STAGES - 1 : STAGES;  // tiles in flight; FS keeps the previous tile's stage for the drain
-    using WS = typename std::conditional<FS, ScoreWarpSmemFS<HPT>, ScoreWarpSmem<HPT>>::type;
+    using WS = typename std::conditional<FS, ScoreWarpSmemFS<HPT>,
+                                         typename std::conditional<BOX, ScoreWarpSmemBox<HPT>, ScoreWarpSmem<HPT>>::type>::type;
     static_assert(NB <= 32 && (TILE % G) == 0 && (kTile % TILE) == 0, "a batch is at most 32 tests and divides a tile");
     extern __shared__ __align__(128) unsigned char score_smem[];
     const unsigned full = 0xffffffffu;
     const int lane = threadIdx.x & 31;
     const int warp = __shfl_sync(full, (int)(threadIdx.x >> 5), 0);  // tells the compiler it is warp-uniform
     const unsigned lt = lanemask_lt();
-    if (a.mode_flag && *a.mode_flag != MODE) return;  // AUTO in two launches: the pilot chose the other screen
+    // AUTO in two launches: the pilot chose the other screen (its flag is MODE_FULL or MODE_SCREEN, the one-sided body
+    // of either kind)
+    if (a.mode_flag && (*a.mode_flag == MODE_FULL) != (MODE == MODE_FULL)) return;
     WS& ws = reinterpret_cast<WS*>(score_smem)[warp];
 
     if (lane == 0) {
@@ -402,23 +586,26 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
         const double* Ep = a.E + 9 * (long long)pair * a.h;
         const ModelRow* Rw = a.rows + (long long)pair * a.h + hyp_w;  // this warp's models, padded (survivor path)
         const Corr* pbeg = a.pts + begin;    // this item's correspondences (exact copies)
-        const P* src = reinterpret_cast<const P*>(SCREEN ? a.spts : (const void*)a.pts);
+        const P* src = reinterpret_cast<const P*>(a.spts);
+        const int box0 = (int)(begin / kTile);  // BOX: a single pair (pbase = 0), items start on tiles
 
         auto issue = [&](int t) {  // lane 0 only
             const int s = (int)((gt + (unsigned)t) % STAGES);
             const long long first = begin + (long long)t * TILE;
             const long long rem = end - first;
             const uint32_t bytes = (uint32_t)((rem < TILE ? rem : TILE) * sizeof(P));
-            mbar_expect_tx(&ws.full_bar[s], bytes);
+            mbar_expect_tx(&ws.full_bar[s], bytes + (BOX ? (uint32_t)sizeof(double4) : 0u));
             bulk_g2s(&ws.tile[s][0], src + first, bytes, &ws.full_bar[s]);
+            if constexpr (BOX) bulk_g2s(&ws.box[s], a.boxes + box0 + t, (uint32_t)sizeof(double4), &ws.full_bar[s]);
         };
         if (lane == 0) {
             for (int t = 0; t < AHEAD && t < ntiles; ++t) issue(t);
         }
 
-        // register-resident models; SCREEN: columns 0 and 1 scaled by s, kappa per hypothesis;
-        // SCREEN32: additionally normalised to |E|_F = 1 (sed is scale-invariant in E) and rounded to fp32
-        T e[HPT][9], kap[HPT];
+        // register-resident models; SCREEN: kappa per hypothesis, the tile's bound T per hypothesis;
+        // SCREEN11: columns 0 and 1 scaled by s, kappa per hypothesis;
+        // SCREEN32: as SCREEN11, normalised to |E|_F = 1 (sed is scale-invariant in E) and rounded to fp32
+        T e[HPT][9], kap[HPT], tb[HPT];
 #pragma unroll
         for (int j = 0; j < HPT; ++j) {
             const long long hyp = hyp_w + 32 * j + lane;
@@ -439,11 +626,12 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
             }
             const double nrm = F32 ? rsqrt(f2) : 1.0;  // inf/NaN models screen nothing out wrongly: see below
 #pragma unroll
-            for (int k = 0; k < 9; ++k) e[j][k] = (T)((SCREEN && (k % 3) != 2) ? v[k] * nrm * a.s : v[k] * nrm);
-            // padding lanes can never produce a survivor: m = -1, d = r^2 + 1 > 0.  A model whose norm
+            for (int k = 0; k < 9; ++k) e[j][k] = (T)((SCALED && (k % 3) != 2) ? v[k] * nrm * a.s : v[k] * nrm);
+            // padding lanes can never produce a survivor: m = T = -1, d = r^2 + 1 > 0.  A model whose norm
             // is 0, inf or NaN gets kappa = +inf in fp32 mode: every test survives and the exact scorer decides.
             if (F32) kap[j] = (T)(real ? ((f2 > 0.0 && f2 < 1e300) ? ab2 : __longlong_as_double(0x7ff0000000000000LL)) : -1.0);
             else kap[j] = (T)(real ? f2 * ab2 : -1.0);
+            if constexpr (BOX) ws.kap[j][lane] = kap[j];  // the previous item's tiles are done with it
         }
 
         // Exact evaluation of <= 32 survivors, one per lane (the reference's arithmetic, sed_exact), and the sums.
@@ -591,13 +779,39 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
             const long long first = begin + (long long)t * TILE;
             const int np = (int)((end - first < TILE) ? (end - first) : TILE);
             const P* tp = reinterpret_cast<const P*>(&ws.tile[s][0]);
+            if constexpr (BOX) {
+                const double4 bx = ws.box[s];
+#pragma unroll
+                for (int j = 0; j < HPT; ++j) tb[j] = tile_bound(e[j], bx, a.thr_pre, ws.kap[j][lane]);
+            }
             for (int p = 0; p < np; p += G) {
                 unsigned pm = 0;
 #pragma unroll
                 for (int g = 0; g < G; ++g) {
                     const P c = tp[p + g];
                     T d[HPT];
-                    if (SCREEN) {
+                    if constexpr (BOX) {
+                        // hypothesis-innermost: consecutive FMAs share c.yb / c.xb / c.ya / c.xa
+                        double t0[HPT], t1[HPT], t2[HPT];
+#pragma unroll
+                        for (int j = 0; j < HPT; ++j) {
+                            t0[j] = fma(c.yb, e[j][3], e[j][6]);
+                            t1[j] = fma(c.yb, e[j][4], e[j][7]);
+                            t2[j] = fma(c.yb, e[j][5], e[j][8]);
+                        }
+#pragma unroll
+                        for (int j = 0; j < HPT; ++j) {
+                            t0[j] = fma(c.xb, e[j][0], t0[j]);  // lb0
+                            t1[j] = fma(c.xb, e[j][1], t1[j]);  // lb1
+                            t2[j] = fma(c.xb, e[j][2], t2[j]);  // lb2
+                        }
+#pragma unroll
+                        for (int j = 0; j < HPT; ++j) t2[j] = fma(c.ya, t1[j], t2[j]);
+#pragma unroll
+                        for (int j = 0; j < HPT; ++j) t2[j] = fma(c.xa, t0[j], t2[j]);  // r
+#pragma unroll
+                        for (int j = 0; j < HPT; ++j) d[j] = fma(t2[j], t2[j], -tb[j]);
+                    } else if (SCREEN) {
                         // hypothesis-innermost: consecutive FMAs share c.yb / c.xb / c.ya / c.xa
                         T t0[HPT], t1[HPT], t2[HPT];
 #pragma unroll
@@ -608,8 +822,8 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
                         }
 #pragma unroll
                         for (int j = 0; j < HPT; ++j) {
-                            t0[j] = fma(c.xb, e[j][0], t0[j]);  // s lb0
-                            t1[j] = fma(c.xb, e[j][1], t1[j]);  // s lb1
+                            t0[j] = fma(c.xb, e[j][0], t0[j]);  // s lb0 / |E|
+                            t1[j] = fma(c.xb, e[j][1], t1[j]);  // s lb1 / |E|
                             t2[j] = fma(c.xb, e[j][2], t2[j]);  // lb2
                         }
 #pragma unroll
@@ -681,13 +895,13 @@ k_score(const ScoreArgs a) {
     score_body<HPT, G, MODE>(a);
 }
 
-// AUTO variant, one launch: the pilot's verdict (k_screen_pts64) picks the body.  Both bodies live in one kernel, so
+// AUTO variant, one launch: the pilot's verdict (k_pilot) picks the body.  Both bodies live in one kernel, so
 // no second (empty) launch is needed; the register budget is the larger of the two.
-template <int HPT, int G>
+template <int HPT, int G, int SMODE>
 __global__ void __launch_bounds__(kScoreThreads, score_min_blocks(HPT)) k_score_auto(const ScoreArgs a, const ScoreArgs a_full) {
     chain_enter();
     if (*a.mode_flag == MODE_FULL) score_body<HPT, G, MODE_FULL>(a_full);
-    else score_body<HPT, G, MODE_SCREEN>(a);
+    else score_body<HPT, G, SMODE>(a);
 }
 
 // ------------------------------------------------------------------------------------
