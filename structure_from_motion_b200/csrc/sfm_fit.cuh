@@ -32,13 +32,16 @@ __global__ void k_normalise(const double* __restrict__ xa, const double* __restr
         c.xb = __ddiv_rn(__dsub_rn(xb[i * stride], cx), fx);
         c.yb = __ddiv_rn(__dsub_rn(yb[i * stride], cy), fy);
         out[i] = c;
-        a2 = fma(c.xa, c.xa, fma(c.ya, c.ya, 1.0));
-        b2 = fma(c.xb, c.xb, fma(c.yb, c.yb, 1.0));
+        if (isfinite(c.xa) && isfinite(c.ya) && isfinite(c.xb) && isfinite(c.yb)) {
+            a2 = fma(c.xa, c.xa, fma(c.ya, c.ya, 1.0));
+            b2 = fma(c.xb, c.xb, fma(c.yb, c.yb, 1.0));
+        }
     }
     if (!bounds) return;
-    // max |(x, y, 1)|^2 per image over all correspondences: the rounding bound kappa of the K2 screen (sfm_score.cuh).
-    // Non-negative doubles order like their bit patterns; NaN coordinates poison the bound (kappa = NaN => d = NaN,
-    // sign clear) exactly like they poison the reference's score (NaN <= thr is False)
+    // max |(x, y, 1)|^2 per image over the correspondences with four finite coordinates: the rounding bound kappa of
+    // the K2 screens (sfm_score.cuh).  A record with a NaN or infinite coordinate is left out: its sed is inf or NaN
+    // (every product with an infinite coordinate is inf or NaN and reaches r or a line norm), so it is never an inlier
+    // at the thresholds K2 scores (<= 1e100), whatever its test decides.  Non-negative doubles order like their bits.
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) {
         a2 = fmax(a2, __shfl_xor_sync(0xffffffffu, a2, d));

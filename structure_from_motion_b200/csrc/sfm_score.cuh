@@ -95,8 +95,8 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
 //       1e-22 thr |E|^2 B^2 <= 0.0025 * 4e-20 (1 + thr) |E|^2 A^2 B^2 absolute and 1e-9 relative;
 //       the seven roundings of m_i, m0^2 + m1^2 and T are downward by at most (1 - 8u) on sums of
 //       non-negative terms, covered by the remaining 1e-9 of thr'.  kappa's 0.2e-20 covers both.
-//   A T that is NaN (an inf/NaN model or coordinate bound) becomes +inf: every test of that tile
-//   survives and the exact scorer decides, as the 11-slot screen did.  Padding lanes have E = 0
+//   A T that is NaN becomes +inf, a second line behind the range guard below (only a NaN model can make one: T's
+//   terms are non-negative and thr' >= 1e-280, so an infinite box gives T = +inf).  Padding lanes have E = 0
 //   and kappa = -1, so T = -1 and d = 1 > 0 (boxes are finite: a tile with a non-finite B
 //   coordinate gets centre 0 and half-widths DBL_MAX).  The screen is written
 //   hypothesis-innermost so that consecutive DFMAs share the correspondence operand (a DFMA
@@ -119,6 +119,27 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
 //   (|r| + eps)^2 <= (1+l) r^2 + (1+1/l) eps^2 and the same for nb with l = 1/64 give the test
 //   r32^2 < thr32 nb32 + kappa32, thr32 = 1.0316 thr, kappa32 = 1.2e-10 (1+thr) A^2 B^2
 //   (>= u^2 [2113 thr B^2 + 16640 A^2 B^2]); ~2 % more survivors than the fp64 screen.
+//
+// Range guard, every body.  The arguments above model each rounding as relative (1 + delta, |delta| <= u); they hold
+// while no quantity of a screen or of the reference leaves the normal range.  With F = |E_h|_F^2 and A^2, B^2 >= 1 (the
+// bounds of k_normalise, over records with four finite coordinates; a non-finite record has sed = inf or NaN and is
+// never an inlier at thr <= 1e100, the largest threshold K2 scores):
+//   |lb_i| <= |E| B, |la_i| <= |E| A, |r| <= |E| A B, so na, nb, r^2 <= F A^2 B^2 and na nb <= (F A^2 B^2)^2.
+//   Over:  FULL's largest terms are r^2 (na + nb) <= 2 (F A^2 B^2)^2 and thr' na nb <= 1.01e100 (F A^2 B^2)^2; the
+//          one-sided T <= 1.01e100 * 8 F B^2 + kappa.  F A^2 B^2 <= 2^200 keeps all of them below 2^740, clear of
+//          overflow - and keeps the reference's na, nb finite, so it has none of the sed = 0 "inliers" it reports when
+//          na and nb overflow while r^2 does not (|E| near 1e154 on unit coordinates).
+//   Under: an underflowing operation adds an absolute error of at most 2^-1075 instead.  In the one-sided bodies such
+//          errors reach d as at most ~1e3 (1 + thr) 2^-1075 (through thr' NB+ and the squares; through r and lb only
+//          as squares, by the AM-GM step of (a)), covered by kappa's spare 0.2e-20 (1 + thr) F A^2 B^2 once F >= 2^-200.
+//          FULL's decision is homogeneous of degree 4 in E with the same absolute slack 1e-22 na nb, so it decides as
+//          at unit scale while na nb stays normal: F >= 2^-200 keeps na nb ~ F^2 |a|^2 |b|^2 above 2^-400 for records
+//          off the epipoles (below the range, at |E| ~ 1e-80 on unit coordinates, both r^2 (na + nb) and thr' na nb
+//          underflow to 0, d = +0 and inliers were screened out).  SCREEN32 normalises E by rsqrt(F),
+//          which needs F normal.
+// A model outside kRangeLo = 2^-200 <= F, F A^2 B^2 <= kRangeHi = 2^200 (an inf or NaN one included) gets every test
+// survive: one OR of a per-item mask into each batch's survivor bits, no work per test.  Models of the eight-point
+// fit (e_22 = 1 on coordinates of order 1) sit far inside; the guard costs only hypotheses that are degenerate anyway.
 //
 // Order-independent accumulation.  An inlier's sed (or sed^2 — only the sum the aggregation
 // method needs is accumulated unless both are requested) is converted to an 84-bit fixed-point
@@ -152,6 +173,8 @@ constexpr double kKappaCoef = 4.2e-20;
 constexpr double kThrScreenFactor = 1.0 + 3e-9;  // thr' of the fp64 screen, see the K2 header
 constexpr double kKappa32Coef = 1.2e-10;   // fp32 pre-filter, see the K2 header
 constexpr double kThr32Factor = 1.0316;   // (1 + 1/64)^2 (1 + 1e-4)
+constexpr double kRangeLo = 0x1p-200;      // range guard on |E|_F^2, see the K2 header
+constexpr double kRangeHi = 0x1p200;       // range guard on |E|_F^2 A^2 B^2
 
 
 __global__ void __launch_bounds__(256) k_pad_models(const double* __restrict__ E, long long htotal, ModelRow* __restrict__ rows) {
@@ -226,7 +249,7 @@ struct __align__(16) Corr32 {
 };
 
 // T = thr' NB+ + kappa of one hypothesis over one tile: NB+ >= lb0^2 + lb1^2 at every B point of the box (K2 header);
-// a NaN bound becomes +inf, so that every test of the tile survives and the exact scorer decides
+// a NaN bound (a NaN model) becomes +inf, so that every test of the tile survives and the exact scorer decides
 __device__ __forceinline__ double tile_bound(const double (&e)[9], double4 box, double thr_pre, double kap) {
     const double l0 = fma(box.x, e[0], fma(box.y, e[3], e[6]));
     const double l1 = fma(box.x, e[1], fma(box.y, e[4], e[7]));
@@ -562,7 +585,8 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
     uint2* q = ws.ring;
     unsigned head = 0, tail = 0;  // ring positions (records): warp-uniform, monotone, tail - head < 64
     unsigned gt = 0;              // tiles consumed so far by this warp (drives stage + parity)
-    const double ab2 = SCREEN ? a.bounds[0] * a.bounds[1] * (F32 ? a.kappa32_coef : a.kappa_coef) : 0.0;
+    const double abnd = a.bounds[0] * a.bounds[1];  // A^2 B^2
+    const double ab2 = SCREEN ? abnd * (F32 ? a.kappa32_coef : a.kappa_coef) : 0.0;
 
     for (;;) {
         unsigned item = 0;
@@ -606,6 +630,7 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
         // SCREEN11: columns 0 and 1 scaled by s, kappa per hypothesis;
         // SCREEN32: as SCREEN11, normalised to |E|_F = 1 (sed is scale-invariant in E) and rounded to fp32
         T e[HPT][9], kap[HPT], tb[HPT];
+        unsigned fpat = 0u;  // bit HPT-1-j: slot j holds a model outside the range guard, every one of its tests survives
 #pragma unroll
         for (int j = 0; j < HPT; ++j) {
             const long long hyp = hyp_w + 32 * j + lane;
@@ -624,15 +649,21 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
                 mp[3] = make_double2(v[6], v[7]);
                 ws.model[32 * j + lane][8] = v[8];
             }
-            const double nrm = F32 ? rsqrt(f2) : 1.0;  // inf/NaN models screen nothing out wrongly: see below
+            // range guard (K2 header): the bodies are sound for kRangeLo <= |E|^2 and |E|^2 A^2 B^2 <= kRangeHi; outside
+            // (a 0, inf or NaN norm included) the model's tests all survive and the exact scorer decides
+            if (real && !(f2 >= kRangeLo && f2 * abnd <= kRangeHi)) fpat |= 1u << (HPT - 1 - j);
+            const double nrm = F32 ? rsqrt(f2) : 1.0;
 #pragma unroll
             for (int k = 0; k < 9; ++k) e[j][k] = (T)((SCALED && (k % 3) != 2) ? v[k] * nrm * a.s : v[k] * nrm);
-            // padding lanes can never produce a survivor: m = T = -1, d = r^2 + 1 > 0.  A model whose norm
-            // is 0, inf or NaN gets kappa = +inf in fp32 mode: every test survives and the exact scorer decides.
-            if (F32) kap[j] = (T)(real ? ((f2 > 0.0 && f2 < 1e300) ? ab2 : __longlong_as_double(0x7ff0000000000000LL)) : -1.0);
-            else kap[j] = (T)(real ? f2 * ab2 : -1.0);
+            // padding lanes can never produce a survivor: m = T = -1, d = r^2 + 1 > 0
+            kap[j] = (T)(real ? (F32 ? ab2 : f2 * ab2) : -1.0);
             if constexpr (BOX) ws.kap[j][lane] = kap[j];  // the previous item's tiles are done with it
         }
+        // the guard's bits in every group of a batch (bit NB-1-i <-> test i = g * HPT + j, see the one-sided bodies)
+        unsigned frep = 0u;
+#pragma unroll
+        for (int g = 0; g < G; ++g) frep |= 1u << (HPT * g);
+        const unsigned fmask = fpat * frep;
 
         // Exact evaluation of <= 32 survivors, one per lane (the reference's arithmetic, sed_exact), and the sums.
         auto accumulate = [&](bool act, double sv, int slot, int owner) {
@@ -843,6 +874,7 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
 #pragma unroll
                     for (int j = 0; j < HPT; ++j) pm = __funnelshift_l((unsigned)sign_word(d[j]), pm, 1);
                 }
+                pm |= fmask;
                 const int v = np - p;  // a partial last batch evaluated stale records: drop their bits
                 if (v < G) pm &= 0xffffffffu << (NB - v * HPT);
                 const unsigned vote = __ballot_sync(full, pm != 0u);

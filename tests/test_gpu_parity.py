@@ -7,6 +7,7 @@ Tolerances (BASELINE.json north_star):
 All fp64.  The scorer is additionally required to be *bit-exact* against oracle/sed_exact.c
 (which is bit-exact against the reference's numpy evaluation, tests/test_oracle.py).
 """
+import functools
 import random
 
 import numpy as np
@@ -16,6 +17,7 @@ from oracle import csed
 from oracle import restatement as o
 from structure_from_motion_b200 import two_view
 from structure_from_motion_b200.scenes import make_scene
+from test_gpu_score_range import check_against_oracle
 
 pytestmark = pytest.mark.gpu
 
@@ -96,13 +98,15 @@ def test_scorer_bit_exact_against_oracle(engine, variant, hpt, group):
     assert np.array_equal(mask, sed_o <= THR)
 
 
-@pytest.mark.parametrize("thr", [0.0, 1e-30, 1e-18, 1e-12, 1e-9, 1.5e-6, 1e-3, 0.5, 40.0])
-@pytest.mark.parametrize("escale", [1.0, 1e6, 1e-7])
-@pytest.mark.parametrize("variant", ["screen", "screen32"])
-def test_screen_never_drops_an_inlier(engine, thr, escale, variant):
-    """The 11-slot screen is a necessary condition at EVERY threshold and model scale: counts and
-    masks equal the exact oracle scorer's (sed.py is scale-invariant in E; the screen's guard
-    kappa_h scales with |E_h|^2)."""
+# model scales past the underflow knee of the reference's na, nb (|E| ~ 1e-154 on unit coordinates), the knee of the
+# two-sided body's degree-4 terms (~1e-77) and the overflow knee (~1e154), where the reference reports sed = 0 inliers
+RANGE_SCALES = (1e-160, 1e-154, 1e-153, 1e-100, 1e-80, 1e-78, 1e-60, 1e60, 1e77, 1e78, 1e150, 1e154, 1e155, 1e160)
+SCALE_CASES = ([(e, t) for e in (1.0, 1e6, 1e-7) for t in (0.0, 1e-30, 1e-18, 1e-12, 1e-9, 1.5e-6, 1e-3, 0.5, 40.0)]
+               + [(e, t) for e in RANGE_SCALES for t in (0.0, 1e-12, 1.5e-6, 1e-3, 0.5)])
+
+
+@functools.lru_cache(maxsize=None)
+def _scale_case(escale, thr):
     n, h = 1500, 256
     K, x1, x2, *_ = make_scene(n, 0.3, seed=11)
     nxa, nya, nxb, nyb = _norm(K, x1, x2)
@@ -110,18 +114,31 @@ def test_screen_never_drops_an_inlier(engine, thr, escale, variant):
     table = np.stack([rng.choice(n, 8, replace=False) for _ in range(h)]).astype(np.int32)
     ca, cb = np.stack([nxa, nya], 1), np.stack([nxb, nyb], 1)
     E = np.stack([o.eight_point(ca[s], cb[s]) for s in table]) * escale
-    cnt_o, s1_o, s2_o = csed.score_batch(E, nxa, nya, nxb, nyb, thr, table=table, nthreads=8)
+    oracle = csed.score_batch(E, nxa, nya, nxb, nyb, thr, table=table, nthreads=8)
+    return K, x1, x2, (nxa, nya, nxb, nyb), table, E, oracle
+
+
+@pytest.mark.parametrize("escale,thr", SCALE_CASES)
+@pytest.mark.parametrize("variant", ["screen", "screen32", "full", "auto"])
+def test_screen_never_drops_an_inlier(engine, thr, escale, variant):
+    """Every body of the 11-slot upload is a necessary condition at EVERY threshold and model scale: counts, sums,
+    K3's errors and winner and K4's mask and SED equal the exact oracle scorer's (sed.py is scale-invariant in E
+    while it stays in range; the screens' guard kappa_h scales with |E_h|^2, and models outside the range guard of
+    the K2 header have all their tests decided exactly).  At thr 1e-3 AUTO runs the two-sided body."""
+    K, x1, x2, cols, table, E, oracle = _scale_case(escale, thr)
     engine.upload_pairs(x1, x2, K)
     engine.set_table(table)
     engine.set_models(E)
     engine.set_score_variant(variant)
     try:
-        cnt, s1, s2, err = engine.score(thr, min_extra=0, aggregation="sum")
+        got = engine.score(thr, min_extra=0, aggregation="sum")
     finally:
         engine.set_score_variant("auto")
-    assert np.array_equal(cnt, cnt_o)
-    np.testing.assert_allclose(s1, s1_o, rtol=1e-12, atol=0)
-    np.testing.assert_allclose(s2, s2_o, rtol=1e-12, atol=0)
+    check_against_oracle(engine, got, E, cols, thr, oracle)
+    if thr == 1.5e-6 and 1e-153 <= escale <= 1e150:  # the reference's range: there are inliers to drop
+        assert oracle[0].sum() > 0
+    if escale == 1e154 and thr <= 1.5e-6:  # the sed = 0 regime: na, nb overflow, r^2 does not
+        assert oracle[0].sum() > _scale_case(1.0, thr)[-1][0].sum()
 
 
 @pytest.mark.parametrize("thr", [0.0, 1e-12, 1.5e-6, 1e-4, 1e-3, 0.03, 0.5, 40.0])

@@ -2,12 +2,16 @@
 image-B positions at upload, and every test is made against one bound on the line norm per (hypothesis, tile).  The
 bound must never drop an inlier of the exact scorer, the sort must change no output, and padding must never survive.
 Shorter pairs and batches keep the 11-slot screen on the scaled copy (tests/test_gpu_parity.py covers it at 1 500)."""
+import functools
+
 import numpy as np
 import pytest
 
 from oracle import csed
 from oracle import restatement as o
 from structure_from_motion_b200.scenes import make_scene
+from test_gpu_parity import SCALE_CASES
+from test_gpu_score_range import check_against_oracle
 
 pytestmark = pytest.mark.gpu
 THR = 1.5e-6
@@ -144,19 +148,67 @@ def test_adversarial_tiles_match_exact_scorer(engine, kind, thr):
     np.testing.assert_allclose(s2, s2_o, rtol=1e-12, atol=0)
 
 
-@pytest.mark.parametrize("thr", [0.0, 1e-30, 1e-18, 1e-12, 1e-9, 1.5e-6, 1e-3, 0.5, 40.0])
-@pytest.mark.parametrize("escale", [1.0, 1e6, 1e-7])
-def test_tile_screen_never_drops_an_inlier(engine, thr, escale):
-    """The 9-slot screen is a necessary condition at every threshold and model scale (the grid of
-    test_gpu_parity.py::test_screen_never_drops_an_inlier, whose 1 500 correspondences run the 11-slot screen): T's
-    kappa scales with |E_h|^2 and its thr' with the threshold."""
+@functools.lru_cache(maxsize=1)
+def _sweep_scene():
     n, h = SORT_MIN + 7_000, 256
     K, x1, x2, *_ = make_scene(n, 0.3, seed=11)
     nxa, nya, nxb, nyb = _norm(K, x1, x2)
     table, E = _models(nxa, nya, nxb, nyb, h, seed=9)
+    return K, x1, x2, (nxa, nya, nxb, nyb), table, E
+
+
+@functools.lru_cache(maxsize=None)
+def _sweep_oracle(escale, thr):
+    K, x1, x2, cols, table, E = _sweep_scene()
+    return csed.score_batch(E * escale, *cols, thr, table=table, nthreads=8)
+
+
+@pytest.mark.parametrize("escale,thr", SCALE_CASES)
+def test_tile_screen_never_drops_an_inlier(engine, thr, escale):
+    """Every body of the 9-slot upload is a necessary condition at every threshold and model scale (the grid of
+    test_gpu_parity.py::test_screen_never_drops_an_inlier, whose 1 500 correspondences run the 11-slot screen): T's
+    kappa scales with |E_h|^2 and its thr' with the threshold; outside the range guard every test is decided exactly.
+    Counts, sums, K3's errors and winner and K4's mask and SED against the exact oracle, for every variant."""
+    K, x1, x2, cols, table, E = _sweep_scene()
     E = E * escale
-    cnt, s1, s2, _ = _score(engine, x1, x2, K, table, E, thr, aggregation="sum", min_extra=0)
-    cnt_o, s1_o, s2_o = csed.score_batch(E, nxa, nya, nxb, nyb, thr, table=table, nthreads=8)
-    assert np.array_equal(cnt, cnt_o)
-    np.testing.assert_allclose(s1, s1_o, rtol=1e-12, atol=0)
-    np.testing.assert_allclose(s2, s2_o, rtol=1e-12, atol=0)
+    oracle = _sweep_oracle(escale, thr)
+    for variant in ("screen", "full", "screen32", "auto"):
+        engine.upload_pairs(x1, x2, K)
+        engine.set_table(table)
+        engine.set_models(E)
+        engine.set_score_variant(variant)
+        try:
+            got = engine.score(thr, min_extra=0, aggregation="sum")
+        finally:
+            engine.set_score_variant("auto")
+        check_against_oracle(engine, got, E, cols, thr, oracle)
+    if thr == 1.5e-6 and 1e-153 <= escale <= 1e150:
+        assert oracle[0].sum() > 0
+    if escale == 1e154 and thr <= 1.5e-6:
+        assert oracle[0].sum() > _sweep_oracle(1.0, thr)[0].sum()
+
+
+@pytest.mark.parametrize("variant,hpt,group,thr", [("screen", 1, 16, THR), ("screen", 1, 32, THR), ("screen", 2, 4, THR),
+                                                   ("screen", 2, 8, THR), ("screen", 2, 16, THR), ("screen", 4, 2, THR),
+                                                   ("screen", 4, 4, THR), ("screen", 4, 8, THR),
+                                                   ("screen", 2, 16, 1e-3), ("screen", 4, 8, 1e-3),
+                                                   ("auto", 2, 16, THR), ("auto", 2, 16, 1e-3),
+                                                   ("auto", 4, 8, THR), ("auto", 4, 8, 1e-3)])
+def test_every_tiled_shape_matches_exact_scorer(engine, variant, hpt, group, thr):
+    """Every shape of the 9-slot body (ScoreWarpSmemBox<HPT>: boxes and per-lane kappa in shared memory), and AUTO on
+    either side of its pilot's decision (1.5e-6: the 9-slot body; 1e-3: the two-sided one), against the exact oracle:
+    72 573 records (a partial last tile) and 300 hypotheses (not a multiple of 32 HPT), with K3 and the K4 mask."""
+    n, h = SORT_MIN + 7_037, 300
+    K, x1, x2, *_ = make_scene(n, 0.3, seed=13)
+    cols = _norm(K, x1, x2)
+    table, E = _models(*cols, h, seed=14)
+    oracle = csed.score_batch(E, *cols, thr, table=table, nthreads=8)
+    engine.upload_pairs(x1, x2, K)
+    engine.set_table(table)
+    engine.set_models(E)
+    engine.set_score_variant(variant, hpt, group)
+    try:
+        got = engine.score(thr, min_extra=0, aggregation="sum")
+    finally:
+        engine.set_score_variant("auto")
+    check_against_oracle(engine, got, E, cols, thr, oracle)

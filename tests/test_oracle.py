@@ -127,6 +127,47 @@ def test_c_scorer_batch_matches_restatement():
         np.testing.assert_allclose(s2[h], (sed[samp | extra] ** 2).sum(), rtol=1e-13)
 
 
+RANGE_SCALES = (1e-160, 1e-155, 1e-154, 1e-153, 1e-100, 1e-80, 1e-78, 1e-60, 1.0, 1e60, 1e77, 1e78, 1e150, 1e154,
+                1e155, 1e160)
+
+
+def test_c_scorer_matches_restatement_at_range_edges():
+    """The C scorer, which every GPU range test compares against, must follow sed.py itself where the arithmetic leaves
+    the normal range: NaN and +-inf in each coordinate, models scaled from 1e-160 to 1e160 (past the underflow knee of
+    na, nb near 1e-154 and the overflow knee near 1e154), and records whose norms overflow while r^2 does not, so that
+    the reference reports sed = 0."""
+    K, x1, x2, R, t, _ = make_scene(48, 0.25, seed=21)
+    nxa, nya = o.k_normalise(x1[:, 0], x1[:, 1], K)
+    nxb, nyb = o.k_normalise(x2[:, 0], x2[:, 1], K)
+    E = np.array([[0.0, -t[2], t[1]], [t[2], 0.0, -t[0]], [-t[1], t[0], 0.0]]) @ R  # the scene's own E = [t]x R
+    E /= E[2, 2]
+    cols = [nxa, nya, nxb, nyb]
+    for c in range(4):  # one NaN, +inf and -inf record in each coordinate, and a record entirely non-finite
+        for k, v in enumerate((np.nan, np.inf, -np.inf)):
+            cols = [np.append(a, v if j == c else a[8 + 3 * c + k]) for j, a in enumerate(cols)]
+    cols = [np.append(a, v) for a, v in zip(cols, (np.inf, np.nan, -np.inf, np.nan))]
+    xa, ya, xb, yb = cols
+    finite = np.isfinite(xa) & np.isfinite(ya) & np.isfinite(xb) & np.isfinite(yb)
+    assert (~finite).sum() == 13
+    seds = {}
+    with np.errstate(all="ignore"):
+        for s in RANGE_SCALES:
+            Es = E * s
+            c = csed.sed_exact_many(Es, xa, ya, xb, yb)
+            ref = np.array([o.sed_scalar(xa[i], ya[i], xb[i], yb[i], Es) for i in range(len(xa))])
+            assert np.array_equal(c, ref, equal_nan=True), s
+            for thr in (0.0, 1e-12, 1.5e-6, 1e-3, 0.5, 1e100):
+                assert np.array_equal(c <= thr, ref <= thr), (s, thr)
+            assert not (c[~finite] <= 1e100).any(), s  # a non-finite record is never an inlier below thr = 1e100
+            seds[s] = c
+    # the regimes are really reached: finite inliers at unit scale, sed = 0 once na and nb overflow (while r^2 stays
+    # finite), and no finite sed at all once they underflow
+    assert ((seds[1.0] <= 1.5e-6) & finite).sum() >= 10
+    assert ((seds[1e154] == 0.0) & finite).sum() > ((seds[1.0] <= 1.5e-6) & finite).sum()
+    assert not np.isfinite(seds[1e-160][finite]).any()
+    assert np.array_equal(seds[1e-100] <= 1.5e-6, seds[1.0] <= 1.5e-6)
+
+
 def test_restatement_matches_live_reference():
     """The restatement against what the unmodified reference returned on the same 150 correspondences
     (tests/golden/make_golden.py): E, the inlier pairs in order and the global RNG state after the run for every
