@@ -104,6 +104,24 @@ def _load_samples(eng, sampler, n, h, table, seed, hyp_offset):
     return table, ref
 
 
+def _degenerate_sample_error(pts_a, pts_b, K) -> Exception:
+    """The exception the reference raises for one degenerate 8-point sample (pixel coordinates [8,2]).  When the
+    Hartley-normalised coordinates are not finite (a coordinate is NaN or infinite, or all eight points of one image
+    coincide and their mean rounds back to the point, so that the scale is sqrt(2)/0), np.linalg.eig refuses Y^T Y
+    (eight_point.py:410) with numpy's LinAlgError; otherwise the validity test raises EightPointCalculationError
+    (:414-421).  The normalisation repeats the reference's numpy calls (:127-133, :319-326), so both decide alike."""
+    K = np.asarray(K, dtype=np.float64)
+    with np.errstate(all="ignore"):
+        for pts in (pts_a, pts_b):
+            pts = np.asarray(pts, dtype=np.float64)
+            coords = np.stack([(pts[:, 0] - K[0][2]) / K[0][0], (pts[:, 1] - K[1][2]) / K[1][1]], axis=1)
+            centered = coords - np.mean(coords, axis=0)
+            scale = np.sqrt(2.0) / np.mean(np.linalg.norm(centered, axis=1))
+            if not np.isfinite(centered * scale).all():
+                return np.linalg.LinAlgError("Array must not contain infs or NaNs")
+    return EightPointCalculationError(EIGHT_POINT_ERROR_MESSAGE)
+
+
 def _restore_random_state(ref, iteration=None):
     """Leave the global random state where the reference's loop does: after every shuffle, or after the shuffle of
     ``iteration`` when the loop stops there."""
@@ -222,8 +240,10 @@ def ransac_essential_arrays(
 
     if best.num_invalid > 0 and on_degenerate == "raise":
         # the reference aborts inside iteration first_invalid: only that many shuffles happened
-        _restore_random_state(ref, int(best.first_invalid))
-        raise EightPointCalculationError(EIGHT_POINT_ERROR_MESSAGE)  # eight_point.py:417-421
+        first = int(best.first_invalid)
+        row = eng.get_table(1, first)[0] if sampler == "device" else np.asarray(table[first], dtype=np.int64)
+        _restore_random_state(ref, first)
+        raise _degenerate_sample_error(pts_a[row], pts_b[row], camera_matrix)
     _restore_random_state(ref)
     if best.index < 0:
         raise no_model()
@@ -316,7 +336,7 @@ def eight_point_arrays(pts_a, pts_b, camera_matrix=None, engine=None) -> np.ndar
     eng.set_table(np.arange(8, dtype=np.int32).reshape(1, 8))
     E, valid, _ = eng.fit()
     if not valid[0]:
-        raise EightPointCalculationError(EIGHT_POINT_ERROR_MESSAGE)
+        raise _degenerate_sample_error(pts_a, pts_b, K)
     return E[0]
 
 

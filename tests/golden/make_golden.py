@@ -240,6 +240,7 @@ def main():
                                                state_after=list(random.getstate()[1])))
     front_end_golden()
     reference_outputs_golden()
+    nonfinite_golden()
 
 
 def synthetic_image_pair(seed, h=72, w=96):
@@ -378,8 +379,58 @@ def reference_outputs_golden():
                                                                     corners=[[float(c.x), float(c.y)] for c in corners])))
 
 
+def nonfinite_golden():
+    """What the reference raises when a sample's Hartley-normalised coordinates are not finite (a coordinate is NaN,
+    or all eight points of one image coincide and their mean rounds back to the point: scale sqrt(2)/0):
+    np.linalg.eig refuses Y^T Y (eight_point.py:410) with numpy's LinAlgError, which nothing in ransac.py catches.
+    Coincident points whose mean does not round back to the point leave tiny finite offsets, a finite scale and a
+    rank-deficient Y: EightPointCalculationError.  For the RANSAC cases the global random state after the exception
+    is recorded too: the loop stops inside the iteration of the first such sample."""
+    K = camera_matrix(800.0, 1280, 960)
+    _, x1, x2, _, _, _ = make_scene(30, 0.0, seed=4)
+
+    def outcome(call):
+        try:
+            call()
+        except Exception as exc:  # the exception's type and message are the fixture
+            return dict(raises=type(exc).__module__ + "." + type(exc).__qualname__, message=str(exc))
+        return dict(raises=None, message=None)
+
+    def feats(pts):
+        return [F(x=float(p[0]), y=float(p[1])) for p in pts]
+
+    eight = []
+    coincident = np.repeat(x1[:1], 8, axis=0)
+    exact = np.repeat([[K[0, 2] + 0.5 * K[0, 0], K[1, 2] - 0.25 * K[1, 1]]], 8, axis=0)  # K-normalised (0.5, -0.25)
+    nan_rec = x1[:8].copy()
+    nan_rec[3, 1] = np.nan
+    for name, pa, pb in (("coincident_a", coincident, x2[:8]), ("coincident_b", x1[:8], coincident[:, ::-1]),
+                         ("exact_coincident_a", exact, x2[:8]), ("exact_coincident_b", x1[:8], exact),
+                         ("nan", nan_rec, x2[:8])):
+        res = outcome(lambda: ref.eight_point.estimate_essential_mat(
+            camera_matrix=K, features_a=feats(pa), features_b=feats(pb), matches=ref.eight_point.create_trivial_matches(8)))
+        eight.append(dict(name=name, pts_a=pa, pts_b=pb, **res))
+
+    ransac = []
+    nan_scene = x1.copy()
+    nan_scene[17, 0] = np.nan
+    all_same = np.repeat(x1[:1], len(x1), axis=0)
+    all_exact = np.repeat(exact[:1], len(x1), axis=0)
+    for name, pa, pb in (("nan_record", nan_scene, x2), ("coincident_a", all_same, x2),
+                         ("exact_coincident_b", x1, all_exact)):
+        random.seed(5)
+        res = outcome(lambda: ref.epipolar_ransac.estimate_essential_mat_with_ransac(
+            K, feats(pa), feats(pb), [M(a_index=i, b_index=i) for i in range(len(pa))], 1.5e-6,
+            error_aggregation_method=ref.ransac.ErrorAggregationMethod.RMS, max_iterations=50))
+        ransac.append(dict(name=name, pts_a=pa, pts_b=pb, seed=5, max_iterations=50, threshold=1.5e-6,
+                           state_after=list(random.getstate()[1]), **res))
+    dump("nonfinite_sample_fixture.json", dict(K=K, eight_point=eight, ransac=ransac))
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "front_end":
+    if len(sys.argv) > 1 and sys.argv[1] == "nonfinite":
+        nonfinite_golden()
+    elif len(sys.argv) > 1 and sys.argv[1] == "front_end":
         front_end_golden()
     elif len(sys.argv) > 1 and sys.argv[1] == "harris":
         harris_golden()
