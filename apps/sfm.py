@@ -14,6 +14,10 @@ Every numeric stage runs in libsfm_b200.so on the GPU (no CPU fallback).
 --model auto estimates both the essential matrix and a homography from the filtered matches and keeps the pose of the
 one that ORB-SLAM's score ratio picks (structure_from_motion_b200.model_selection), so that planar scenes and
 rotation-only pairs get a pose too; --synthetic SEED --planar renders a scene that is one plane.
+
+--refine N polishes the RANSAC winner (both winners with --model auto) by least squares over its inliers, at most N
+Levenberg-Marquardt iterations on the device, before the pose; the essential path then runs through the array API
+(two_view_arrays) on the same matches and the same global random stream.  The JSON output gains a "refinement" record.
 """
 from __future__ import annotations
 
@@ -71,6 +75,7 @@ class SfmResult:
     model: str = "essential"          # "homography" when --model auto picked it; e then holds H
     homography_score_ratio: float = None  # S_H / (S_H + S_E) (--model auto)
     rotation_only: bool = False
+    refinement: dict = None           # --refine: the report of the refined winner (the chosen one with --model auto)
 
 
 def load_config(path=None, **overrides):
@@ -104,34 +109,74 @@ def _filter_matches(matches: List[matching.Match], score_threshold: float) -> Li
     return [m for m in matches if not (m.match_score > score_threshold)]
 
 
-def _run_selected(image_1_corners, image_2_corners, matches, camera_matrix, cfg, secs) -> SfmResult:
+def _match_arrays(image_1_corners, image_2_corners, matches):
+    pts_a = np.array([[image_1_corners[m.a_index].x, image_1_corners[m.a_index].y] for m in matches],
+                     dtype=np.float64).reshape(-1, 2)
+    pts_b = np.array([[image_2_corners[m.b_index].x, image_2_corners[m.b_index].y] for m in matches],
+                     dtype=np.float64).reshape(-1, 2)
+    return pts_a, pts_b
+
+
+def _report(refinement):
+    if refinement is None:
+        return None
+    return dict(status=refinement.status, iterations=refinement.iterations, rejected=refinement.rejected,
+                num=refinement.num, cost_ransac=refinement.cost_ransac, cost_start=refinement.cost_start,
+                cost_final=refinement.cost_final)
+
+
+def _run_selected(image_1_corners, image_2_corners, matches, camera_matrix, cfg, secs, refine=0) -> SfmResult:
     """--model auto: both models on the filtered matches, the pose and points of the one the score ratio picks."""
     from structure_from_motion_b200.model_selection import two_view_select_arrays
 
     logging.info("Estimating the Essential Matrix and a Homography")
     t0 = time.perf_counter()
-    pts_a = np.array([[image_1_corners[m.a_index].x, image_1_corners[m.a_index].y] for m in matches],
-                     dtype=np.float64).reshape(-1, 2)
-    pts_b = np.array([[image_2_corners[m.b_index].x, image_2_corners[m.b_index].y] for m in matches],
-                     dtype=np.float64).reshape(-1, 2)
+    pts_a, pts_b = _match_arrays(image_1_corners, image_2_corners, matches)
     rc = cfg["ransac"]
     sel = two_view_select_arrays(camera_matrix, pts_a, pts_b, rc["sed_inlier_threshold"],
                                  rc["homography_inlier_threshold"], rc["min_num_extra_inliers"],
-                                 ErrorAggregationMethod.RMS, rc["max_iterations"])
+                                 ErrorAggregationMethod.RMS, rc["max_iterations"], refine_iterations=refine)
     secs["two_view"] = time.perf_counter() - t0
     logging.info("Model: %s (homography score ratio %.3f)", sel.model, sel.scores.ratio_h)
-    model = sel.essential.ransac.E if sel.model == "essential" else sel.homography.ransac.H
+    win = sel.essential if sel.model == "essential" else sel.homography
+    model = win.ransac.E if sel.model == "essential" else win.ransac.H
+    if win.refinement is not None:
+        model = win.refinement.model
     pairs = [(image_1_corners[matches[int(i)].a_index], image_2_corners[matches[int(i)].b_index])
              for i in sel.inlier_indices]
     return SfmResult(image_1_corners, image_2_corners, matches, model, pairs, sel.R, sel.t, np.flatnonzero(sel.passing),
                      Transform3D.from_rmat_t(sel.R, sel.t), sel.points[sel.passing], secs, model=sel.model,
-                     homography_score_ratio=sel.scores.ratio_h, rotation_only=sel.rotation_only)
+                     homography_score_ratio=sel.scores.ratio_h, rotation_only=sel.rotation_only,
+                     refinement=_report(win.refinement))
+
+
+def _run_refined_essential(image_1_corners, image_2_corners, matches, camera_matrix, cfg, secs, refine) -> SfmResult:
+    """--refine with the essential path: RANSAC E (reference sampler on the global random state, as the list API),
+    least-squares refinement over its inliers, then the pose vote and triangulation of the refined E."""
+    from structure_from_motion_b200.two_view import two_view_arrays
+
+    logging.info("Estimating and refining the Essential Matrix")
+    t0 = time.perf_counter()
+    pts_a, pts_b = _match_arrays(image_1_corners, image_2_corners, matches)
+    rc = cfg["ransac"]
+    tv = two_view_arrays(camera_matrix, pts_a, pts_b, rc["sed_inlier_threshold"], rc["min_num_extra_inliers"],
+                         ErrorAggregationMethod.RMS, rc["max_iterations"], refine_iterations=refine)
+    secs["two_view"] = time.perf_counter() - t0
+    logging.info("Refinement: %s after %d iterations, cost %.3e -> %.3e", tv.refinement.status, tv.refinement.iterations,
+                 tv.refinement.cost_start, tv.refinement.cost_final)
+    pairs = [(image_1_corners[matches[int(i)].a_index], image_2_corners[matches[int(i)].b_index])
+             for i in tv.inlier_indices]
+    return SfmResult(image_1_corners, image_2_corners, matches, tv.refinement.model, pairs, tv.R, tv.t,
+                     np.flatnonzero(tv.passing), Transform3D.from_rmat_t(tv.R, tv.t), tv.points[tv.passing], secs,
+                     refinement=_report(tv.refinement))
 
 
 def run_sfm(image_1_gray: np.ndarray, image_2_gray: np.ndarray, camera_matrix: np.ndarray, cfg=None,
-            check_opencv: bool = False, model: str = "essential") -> SfmResult:
+            check_opencv: bool = False, model: str = "essential", refine: int = 0) -> SfmResult:
     """model "essential": the reference's path.  "auto": the essential matrix and a homography, the pose of the one the
-    score ratio picks (the OpenCV cross-checks belong to the essential path and are not run)."""
+    score ratio picks (the OpenCV cross-checks belong to the essential path and are not run).  refine > 0: the winner
+    is refined over its inliers before the pose (the essential path then goes through two_view_arrays; the OpenCV
+    cross-checks are not run)."""
     cfg = cfg or load_config()
     secs = {}
 
@@ -155,7 +200,9 @@ def run_sfm(image_1_gray: np.ndarray, image_2_gray: np.ndarray, camera_matrix: n
     matches = _filter_matches(matches, cfg["match_score_threshold"])
     timed("matching", t0)
     if model == "auto":
-        return _run_selected(image_1_corners, image_2_corners, matches, camera_matrix, cfg, secs)
+        return _run_selected(image_1_corners, image_2_corners, matches, camera_matrix, cfg, secs, refine)
+    if refine > 0:
+        return _run_refined_essential(image_1_corners, image_2_corners, matches, camera_matrix, cfg, secs, refine)
 
     logging.info("Estimating Essential Matrix")
     t0 = time.perf_counter()
@@ -244,7 +291,11 @@ def main(argv=None):
     ap.add_argument("--model", choices=["essential", "auto"], default="essential",
                     help="essential: the essential matrix only; auto: pick between it and a homography")
     ap.add_argument("--planar", action="store_true", help="with --synthetic: render one plane only")
+    ap.add_argument("--refine", type=int, default=0, metavar="N",
+                    help="refine the winner over its inliers (at most N Levenberg-Marquardt iterations) before the pose")
     args = ap.parse_args(argv)
+    if args.refine < 0:
+        ap.error("--refine must be >= 0")
     logging.basicConfig(level=logging.INFO, format="%(message)s")
     cfg = load_config(args.config)
     truth = None
@@ -264,12 +315,14 @@ def main(argv=None):
         import random
 
         random.seed(args.seed)
-    res = run_sfm(img1, img2, K, cfg, check_opencv=args.check_opencv, model=args.model)
+    res = run_sfm(img1, img2, K, cfg, check_opencv=args.check_opencv, model=args.model, refine=args.refine)
     out = dict(corners=[len(res.corners_1), len(res.corners_2)], matches=len(res.matches),
                ransac_inliers=len(res.inlier_feature_pairs), cheirality_inliers=int(len(res.inlier_mask)),
                R=res.r.tolist(), t=res.t.tolist(), seconds=res.seconds)
     if args.model == "auto":
         out.update(model=res.model, homography_score_ratio=res.homography_score_ratio, rotation_only=res.rotation_only)
+    if res.refinement is not None:
+        out["refinement"] = res.refinement
     if truth is not None:
         R, t = truth
         out["rotation_error_deg"] = float(np.degrees(np.arccos(np.clip((np.trace(res.r.T @ R) - 1) / 2, -1, 1))))

@@ -366,6 +366,51 @@ int sfm_batch_score_models(sfm_ctx *ctx, const double *E, const uint8_t *have_e,
                            const uint8_t *have_h, double sigma, double homography_ratio, sfm_model_scores *out,
                            double *per_point);
 
+/* ---- least-squares refinement of the winner (opt-in; csrc/sfm_refine.cuh) ---------------
+ * With max_iterations > 0 (0 = off, the default; a context setting like sfm_set_score_variant) the calls that run a
+ * pose tail - sfm_two_view, sfm_two_view_async / _fetch, sfm_pose_and_triangulate, sfm_two_view_homography,
+ * sfm_homography_pose_and_triangulate, sfm_batch_two_view, sfm_batch_two_view_homography - refine every pair's winner
+ * between the selection and the pose:
+ *   data   the winner's inlier list as the tail compacts it (E: sed <= threshold plus the 8 samples; H: the transfer
+ *          decision plus the 4 samples), fixed during the refinement;
+ *   cost   the sum over that list of the error RANSAC scored: E the symmetric epipolar distance in K-normalised
+ *          coordinates, H the symmetric transfer error in px^2 (4 residuals per correspondence);
+ *   model  E = [t]x R (R <- R exp([w]x), unit t moved in its tangent plane: 5 parameters), started from candidate 0 of
+ *          the decomposition of the RANSAC E (its projection onto the essential manifold); H: h0..h7 with H[2,2] = 1;
+ *   solver Levenberg-Marquardt with Marquardt's diagonal damping: lambda starts at 1e-3, / 10 on an accepted step
+ *          (cost strictly lower), * 10 on a rejected one; converged when an accepted step lowers the cost by a relative
+ *          1e-12 or less, when the cost is at most 1e-24 times the sum of the squared coordinates of the list
+ *          (rounding noise), or when the scaled step |diag(J^T J)^1/2 d| <= 1e-9 sqrt(cost); stalled
+ *          when lambda exceeds 1e16; max_iterations evaluated proposals at most.  The final cost never exceeds the start's.
+ * The RANSAC result is untouched (best, mask, sed / err, the E / H arrays of the batch calls).  The tail then runs on
+ * the refined model as on a caller-supplied one: inliers = the decision under the refined model with no forced samples
+ * (the E vote's index-0 rule applies to list position 0, as after sfm_set_winner(ctx, -1, E)), vote, triangulation.
+ * A pair without a winner, or whose start is not finite, keeps the RANSAC model and its tail.  The refined bits depend on
+ * the pair's inlier list only (fixed-order sums): pair p of a batch equals the single-pair call on that pair.
+ * sfm_two_view_sharded and sfm_sharded_tail refuse with SFM_ERR_STATE while refinement is on. */
+enum sfm_refine_status {
+    SFM_REFINE_CONVERGED = 0,
+    SFM_REFINE_MAX_ITERATIONS = 1,
+    SFM_REFINE_STALLED = 2,      /* lambda reached its cap */
+    SFM_REFINE_NO_MODEL = 3,     /* no winner: nothing refined */
+    SFM_REFINE_NONFINITE = 4     /* the start (model or cost) is not finite: the RANSAC model is kept */
+};
+typedef struct sfm_refinement {
+    double model[9];       /* refined E or H (row-major, model[8] == 1); the RANSAC model when not refined */
+    double cost_ransac;    /* cost of the RANSAC model over the inlier list                              */
+    double cost_start;     /* cost at the start point (E: the projection onto the manifold)              */
+    double cost_final;     /* cost of the refined model, <= cost_start                                   */
+    int64_t num;           /* correspondences in the inlier list                                         */
+    int32_t iterations;    /* proposals evaluated                                                         */
+    int32_t status;        /* sfm_refine_status                                                           */
+    int32_t rejected;      /* of those, proposals rejected (cost not strictly lower)                     */
+    int32_t reserved;
+} sfm_refinement;
+int sfm_set_refinement(sfm_ctx *ctx, int max_iterations);
+/* The reports of the last tail call, one per pair (P = 1 for the single-pair calls); SFM_ERR_STATE when that call did
+ * not refine, SFM_ERR_ARG when P is not its number of pairs. */
+int sfm_get_refinement(sfm_ctx *ctx, sfm_refinement *out, int64_t P);
+
 /* ---- hypothesis-sharded estimates without a host round trip (SURVEY.md 8(e)) ---------- */
 /* One rank of a run whose hypotheses are split over `world` GPUs (correspondences replicated):
  *   1. sfm_score_async  : fit + score + select of this rank's hypotheses, nothing synchronised; *record_dev is the

@@ -50,6 +50,14 @@ class ModelScores(C.Structure):
                 ("reserved", C.c_int32)]
 
 
+class Refinement(C.Structure):
+    _fields_ = [("model", C.c_double * 9), ("cost_ransac", C.c_double), ("cost_start", C.c_double),
+                ("cost_final", C.c_double), ("num", C.c_int64), ("iterations", C.c_int32), ("status", C.c_int32),
+                ("rejected", C.c_int32), ("reserved", C.c_int32)]
+
+
+REFINE_STATUS = {0: "converged", 1: "max_iterations", 2: "stalled", 3: "no_model", 4: "nonfinite"}
+
 _P = C.c_void_p
 _SIGNATURES = {
     "sfm_version": (C.c_int, []),
@@ -104,6 +112,8 @@ _SIGNATURES = {
                                           C.POINTER(Best), C.POINTER(HPoses), C.c_int64, C.POINTER(C.c_int64), _P, _P,
                                           _P, _P, _P]),
     "sfm_score_models": (C.c_int, [_P, _P, _P, _P, C.c_double, C.c_double, C.POINTER(ModelScores), _P]),
+    "sfm_set_refinement": (C.c_int, [_P, C.c_int]),
+    "sfm_get_refinement": (C.c_int, [_P, C.POINTER(Refinement), C.c_int64]),
     "sfm_score_async": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.POINTER(_P)]),
     "sfm_sharded_tail": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_double, C.c_double]),
     "sfm_sharded_fetch": (C.c_int, [_P, C.POINTER(Best), C.POINTER(C.c_int32), C.POINTER(Poses), C.c_int64,
@@ -250,6 +260,20 @@ class Engine:
     def set_score_variant(self, variant="auto", hyps_per_thread=0, group=0):
         self._ck(self.lib.sfm_set_score_variant(self.h, VARIANT[variant], int(hyps_per_thread), int(group)),
                  "sfm_set_score_variant")
+
+    def set_refinement(self, max_iterations=0):
+        """Refine the winner over its inliers before the pose in every later tail call (0 = off).  The calls below
+        take ``refine_iterations`` and set this for themselves, because engines are shared."""
+        n = int(max_iterations)
+        if n < 0:
+            raise ValueError(f"refine_iterations must be >= 0, got {n}")
+        self._ck(self.lib.sfm_set_refinement(self.h, n), "sfm_set_refinement")
+
+    def get_refinement(self, pairs=1):
+        """The refinement reports of the last tail call (a ctypes array of ``pairs`` Refinement)."""
+        out = (Refinement * max(int(pairs), 1))()
+        self._ck(self.lib.sfm_get_refinement(self.h, C.cast(out, C.POINTER(Refinement)), int(pairs)), "sfm_get_refinement")
+        return out
 
     # -- correspondences ------------------------------------------------------------------
     def upload_pairs(self, pts_a, pts_b, K, sync=True):
@@ -417,8 +441,11 @@ class Engine:
                  "sfm_decompose_homography")
         return p
 
-    def homography_pose_and_triangulate(self, K, threshold, distance_threshold=50.0, rotation_tolerance=1e-2, cap=None):
-        """Tail of the current homography winner -> (HPoses, num_inliers, inlier_idx, pass_bits, X)."""
+    def homography_pose_and_triangulate(self, K, threshold, distance_threshold=50.0, rotation_tolerance=1e-2, cap=None,
+                                        refine_iterations=0):
+        """Tail of the current homography winner -> (HPoses, num_inliers, inlier_idx, pass_bits, X).  With
+        refine_iterations > 0 the winner is refined first and the tail describes the refined H (get_refinement())."""
+        self.set_refinement(refine_iterations)
         cap = self.n if cap is None else int(cap)
         Ka = _f64(K).reshape(9)
         p = HPoses()
@@ -434,9 +461,10 @@ class Engine:
         return p, int(num.value), idx[:m], ok[:m], X[:m]
 
     def two_view_homography(self, K, threshold, min_extra=0.0, aggregation="rms", selection="min_error",
-                            distance_threshold=50.0, rotation_tolerance=1e-2, cap=None):
+                            distance_threshold=50.0, rotation_tolerance=1e-2, cap=None, refine_iterations=0):
         """ransac_homography + homography_pose_and_triangulate in one C call (one synchronisation for the fixed-size
         results).  Returns (best, mask, err, HPoses, num_inliers, inlier_idx, pass_bits, X)."""
+        self.set_refinement(refine_iterations)
         cap = self.n if cap is None else int(cap)
         Ka = _f64(K).reshape(9)
         b, p = Best(), HPoses()
@@ -503,7 +531,8 @@ class Engine:
                                           _ptr(X)), "sfm_triangulate")
         return X
 
-    def pose_and_triangulate(self, threshold, distance_threshold=50.0, cap=None):
+    def pose_and_triangulate(self, threshold, distance_threshold=50.0, cap=None, refine_iterations=0):
+        self.set_refinement(refine_iterations)
         cap = self.n if cap is None else int(cap)
         p = Poses()
         num = C.c_int64(0)
@@ -517,9 +546,10 @@ class Engine:
         return p, int(num.value), idx[:m], ok[:m], X[:m]
 
     def two_view(self, threshold, min_extra=0.0, aggregation="rms", selection="min_error", distance_threshold=50.0,
-                 cap=None, want_mask=True, want_sed=True):
+                 cap=None, want_mask=True, want_sed=True, refine_iterations=0):
         """ransac_essential + pose_and_triangulate in one C call (one synchronisation for the fixed-size results).
         Returns (best, mask, sed, poses, num_inliers, inlier_idx, pass_bits, X)."""
+        self.set_refinement(refine_iterations)
         cap = self.n if cap is None else int(cap)
         b, p = Best(), Poses()
         num = C.c_int64(0)
@@ -535,10 +565,11 @@ class Engine:
         return b, mask, sed, p, int(num.value), idx[:m], ok[:m], X[:m]
 
     def two_view_async(self, threshold, min_extra=0.0, aggregation="rms", selection="min_error", distance_threshold=50.0,
-                       want_mask=True, want_sed=True, out=None):
+                       want_mask=True, want_sed=True, out=None, refine_iterations=0):
         """Enqueue fit -> score -> select -> tail; nothing synchronises.  Returns the (mask, sed) arrays that the
         enqueued copies will fill - valid after two_view_fetch().  ``out``: (uint8[n], float64[n]) to fill, ideally
         pinned and reused (page-locking fresh memory per call costs more than the estimate's transfers)."""
+        self.set_refinement(refine_iterations)
         mask, sed = out if out is not None else self.pinned_out(self.n)
         if not want_mask:
             mask = None
@@ -627,16 +658,32 @@ class Engine:
         return dict(E=E, best_index=bi, best_err=be, count_extra=ce, num_invalid=ni)
 
     def batch_two_view(self, pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra=0.0, aggregation="rms",
-                       selection="min_error", distance_threshold=50.0, pair_id0=0):
+                       selection="min_error", distance_threshold=50.0, pair_id0=0, refine_iterations=0):
         """batch_ransac + per pair: inlier list, pose vote, triangulation.  Returns the batch_ransac dict plus
         R [P,3,3], t [P,3] (NaN without a model), counts [P,4], pose_index [P], inlier_offsets [P+1], inlier_idx
-        (pair-relative), pass_bits, points [total,3]."""
+        (pair-relative), pass_bits, points [total,3].  With refine_iterations > 0 the pose and everything after it
+        describe the refined E, and the dict gains refined_E and the refine_* reports (_refine_keys)."""
         return self._batch_two_view(pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra, aggregation, selection,
-                                    distance_threshold, pair_id0)[0]
+                                    distance_threshold, pair_id0, refine_iterations)[0]
+
+    def _refine_keys(self, out, P, model_key):
+        """The per-pair refinement reports of the last batch tail as dict entries."""
+        rep = self.get_refinement(P)
+        raw = np.frombuffer(rep, dtype=np.uint8).reshape(P, C.sizeof(Refinement))
+        dbl = raw[:, :12 * 8].copy().view(np.float64)
+        out[model_key] = dbl[:, :9].reshape(P, 3, 3).copy()
+        out["refine_cost_ransac"], out["refine_cost_start"], out["refine_cost_final"] = (dbl[:, 9].copy(), dbl[:, 10].copy(),
+                                                                                        dbl[:, 11].copy())
+        out["refine_num"] = raw[:, 96:104].copy().view(np.int64).reshape(P)
+        ints = raw[:, 104:116].copy().view(np.int32).reshape(P, 3)
+        out["refine_iterations"], out["refine_status"], out["refine_rejected"] = (ints[:, 0].copy(), ints[:, 1].copy(),
+                                                                                  ints[:, 2].copy())
+        return out
 
     def _batch_two_view(self, pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra, aggregation, selection,
-                        distance_threshold, pair_id0):
+                        distance_threshold, pair_id0, refine_iterations=0):
         """batch_two_view's dict and the smallest singular value of every pair's winning E ([P], NaN without one)."""
+        self.set_refinement(refine_iterations)
         pa, pb = _split_xy(pts_a), _split_xy(pts_b)
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         P = offsets.shape[0] - 1
@@ -671,17 +718,22 @@ class Engine:
         t[pose_index < 0] = np.nan
         sv = dbl[:, 48:51].copy()
         total = int(ioff[-1])
-        return dict(E=E, best_index=bi, best_err=be, count_extra=ce, num_invalid=ni, R=R, t=t, counts=counts,
-                    pose_index=pose_index, inlier_offsets=ioff, inlier_idx=idx[:total], pass_bits=ok[:total],
-                    points=X[:total]), np.where(pose_index[:, None] == -2, np.nan, sv)[:, 2]
+        out = dict(E=E, best_index=bi, best_err=be, count_extra=ce, num_invalid=ni, R=R, t=t, counts=counts,
+                   pose_index=pose_index, inlier_offsets=ioff, inlier_idx=idx[:total], pass_bits=ok[:total],
+                   points=X[:total])
+        if int(refine_iterations) > 0:
+            self._refine_keys(out, P, "refined_E")
+        return out, np.where(pose_index[:, None] == -2, np.nan, sv)[:, 2]
 
     def batch_two_view_homography(self, pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra=0.0,
                                   aggregation="rms", selection="min_error", distance_threshold=50.0,
-                                  rotation_tolerance=1e-2, pair_id0=0):
+                                  rotation_tolerance=1e-2, pair_id0=0, refine_iterations=0):
         """batch_two_view for homographies (threshold: symmetric transfer error in px^2; Ks: each upper triangular with
         K[2,2] = 1).  The keys of batch_two_view with H [P,3,3] in place of E, plus n [P,3], d [P] and
         rotation_only bool[P] of the voted candidate.  R, t, n, d are NaN without a model; on a rotation-only pair R is
-        the nearest rotation, t = 0, n NaN, d inf, pose_index -1 and no inlier passes."""
+        the nearest rotation, t = 0, n NaN, d inf, pose_index -1 and no inlier passes.  refine_iterations > 0: as in
+        batch_two_view, with refined_H."""
+        self.set_refinement(refine_iterations)
         pa, pb = _split_xy(pts_a), _split_xy(pts_b)
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         P = offsets.shape[0] - 1
@@ -717,9 +769,12 @@ class Engine:
         none = pose_index == -2
         R[none], t[none], n[none], d[none] = np.nan, np.nan, np.nan, np.nan
         total = int(ioff[-1])
-        return dict(H=H, best_index=bi, best_err=be, count_extra=ce, num_invalid=ni, R=R, t=t, counts=counts,
-                    pose_index=pose_index, inlier_offsets=ioff, inlier_idx=idx[:total], pass_bits=ok[:total],
-                    points=X[:total], n=n, d=d, rotation_only=rot)
+        out = dict(H=H, best_index=bi, best_err=be, count_extra=ce, num_invalid=ni, R=R, t=t, counts=counts,
+                   pose_index=pose_index, inlier_offsets=ioff, inlier_idx=idx[:total], pass_bits=ok[:total],
+                   points=X[:total], n=n, d=d, rotation_only=rot)
+        if int(refine_iterations) > 0:
+            self._refine_keys(out, P, "refined_H")
+        return out
 
     def batch_score_models(self, E, H, have_e=None, have_h=None, sigma=1.0, homography_ratio=0.45, per_point=False):
         """model_scores for every pair of the current batched upload: E / H [P,3,3] or None, given for pair p where

@@ -25,6 +25,7 @@
 #include "sfm_match.cuh"
 #include "sfm_harris.cuh"
 #include "sfm_select.cuh"
+#include "sfm_refine.cuh"
 
 using namespace sfm;
 
@@ -32,6 +33,7 @@ static_assert(sizeof(Corr) == 32, "Corr must be 32 bytes");
 static_assert(sizeof(PoseSet) == sizeof(sfm_poses), "PoseSet/sfm_poses layout mismatch");
 static_assert(sizeof(SelectRecord) == SFM_RECORD_BYTES, "SelectRecord / SFM_RECORD_BYTES mismatch");
 static_assert(sizeof(ModelScores) == sizeof(sfm_model_scores), "ModelScores / sfm_model_scores layout mismatch");
+static_assert(sizeof(RefineReport) == sizeof(sfm_refinement), "RefineReport / sfm_refinement layout mismatch");
 
 namespace {
 
@@ -105,6 +107,7 @@ struct sfm_ctx {
     Buf planes, hK;  // the homography tail's HPlane and the K it was called with (the upload's K stays in Ks)
     Buf k2pts, k2box, k2sort;  // K2's copy of pts in image-B Morton order, its tile boxes, the sort's scratch
     Buf selstate, selio, selpp;  // k_score_models: self-cleaning sums; models and results; per-correspondence errors
+    Buf refstate, refpart, reftick, refrec, refrep;  // refinement: LM state, chunk partials, tickets, records, reports
     long long n = 0, h = 0, npairs = 1;
     long long first_len = 0;  // batched: correspondences of the first pair (what the AUTO pilot samples)
     long long batch_max_len = 0;  // batched: correspondences of the longest pair
@@ -135,6 +138,8 @@ struct sfm_ctx {
     double Khost[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
     // config
     int variant = SFM_SCORE_AUTO, hpt = 2, group = 16;  // AUTO: a pilot on the device picks SCREEN or FULL per call
+    int refine_iters = 0;          // sfm_set_refinement: 0 = off
+    long long refined_pairs = 0;   // pairs whose reports the last tail call left in refrep (0: it did not refine)
     // timing
     bool timing = false;
     cudaEvent_t ev0[T_COUNT], ev1[T_COUNT];
@@ -310,7 +315,7 @@ int sfm_destroy(sfm_ctx* c) {
     Buf* bufs[] = {&c->raw, &c->pts, &c->offsets, &c->Ks, &c->table, &c->E, &c->valid, &c->eig, &c->acc,
                    &c->count_extra, &c->S1, &c->S2, &c->err, &c->blocks, &c->best,
                    &c->invalid, &c->winnerE, &c->record, &c->merged, &c->rows, &c->blockinv, &c->mask, &c->sed, &c->poses, &c->pass, &c->X, &c->idx,
-                   &c->planes, &c->hK, &c->selstate, &c->selio, &c->selpp, &c->k2pts, &c->k2box, &c->k2sort,
+                   &c->planes, &c->hK, &c->selstate, &c->selio, &c->selpp, &c->refstate, &c->refpart, &c->reftick, &c->refrec, &c->refrep, &c->k2pts, &c->k2box, &c->k2sort,
                    &c->scan, &c->tmp, &c->gathered, &c->tailstate, &c->num, &c->winrec, &c->bout, &c->spts, &c->bounds, &c->fitflag,
                    &c->m_img, &c->m_feat, &c->m_W, &c->m_ss, &c->m_ok, &c->m_S, &c->m_out,
                    &c->h_img, &c->h_gx, &c->h_gy, &c->h_corner, &c->h_alive, &c->h_key, &c->h_idx, &c->h_small, &c->h_xy};
@@ -360,6 +365,23 @@ int sfm_set_score_variant(sfm_ctx* c, int variant, int hpt, int group) {
     c->variant = variant;
     c->hpt = nh;
     c->group = ng;
+    return 0;
+}
+
+int sfm_set_refinement(sfm_ctx* c, int max_iterations) {
+    if (!c) return fail(SFM_ERR_ARG, "null context");
+    if (max_iterations < 0) return fail(SFM_ERR_ARG, "max_iterations must be >= 0, got %d", max_iterations);
+    c->refine_iters = max_iterations;
+    return 0;
+}
+
+int sfm_get_refinement(sfm_ctx* c, sfm_refinement* out, int64_t P) {
+    if (int r = use(c)) return r;
+    if (!out) return fail(SFM_ERR_ARG, "null argument");
+    if (c->refined_pairs == 0) return fail(SFM_ERR_STATE, "the last tail call did not refine (sfm_set_refinement)");
+    if (P != c->refined_pairs) return fail(SFM_ERR_ARG, "the last call refined %lld pairs, not %lld", c->refined_pairs, (long long)P);
+    CU(cudaMemcpyAsync(out, c->refrep.p, (size_t)P * sizeof(RefineReport), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
     return 0;
 }
 
@@ -1357,6 +1379,51 @@ int sfm_triangulate(sfm_ctx* c, const double* P1, const double* P2, const double
     return 0;
 }
 
+// The refinement of sfm_refine.cuh behind T1: init, refine_iters + 1 LM steps (the first evaluates the start), finish -
+// all enqueued without a round trip.  *rec_out: the refined records for the rest of the tail.
+static int refine_launch(sfm_ctx* c, int kind, const SelectRecord* rec_dev, long long max_len, const SelectRecord** rec_out) {
+    const long long P = c->npairs;
+    const long long maxch = (max_len + kRefineChunk - 1) / kRefineChunk;
+    const int nv = kind == MODEL_H ? refine_nv<MODEL_H>() : refine_nv<MODEL_E>();
+    if (int r = c->refstate.reserve((size_t)P * sizeof(RefineState))) return r;
+    // chunk partials by total length (refine_chunk_base): n / kRefineChunk + P + 1 slots cover every pair's chunks
+    if (int r = c->refpart.reserve((size_t)(c->n / kRefineChunk + P + 1) * nv * 8)) return r;
+    if (int r = reserve_zeroed(c, c->reftick, (size_t)P * 4)) return r;
+    if (int r = c->refrec.reserve((size_t)P * sizeof(SelectRecord))) return r;
+    if (int r = c->refrep.reserve((size_t)P * sizeof(RefineReport))) return r;
+    RefineArgs a;
+    a.pts = c->pts.as<Corr>();
+    a.offsets = c->batched ? c->offsets.as<long long>() : nullptr;
+    a.rec = rec_dev;
+    a.idx = c->idx.as<long long>();
+    a.num = c->num.as<long long>();
+    a.state = c->refstate.as<RefineState>();
+    a.partial = c->refpart.as<double>();
+    a.ticket = c->reftick.as<unsigned>();
+    a.npairs = (int)P;
+    a.max_iter = c->refine_iters;
+    a.out_rec = c->refrec.as<SelectRecord>();
+    a.report = c->refrep.as<RefineReport>();
+    const dim3 gp((unsigned)((P + 127) / 128));
+    // about 4 blocks per SM in all: a pair gets its share, at least one; blocks grid-stride over the pair's chunks, and
+    // the blocks beyond a pair's own chunk count leave at once
+    const long long cap = (4ll * c->sm_count + P - 1) / P;
+    const dim3 gs((unsigned)(maxch < 1 ? 1 : (maxch < cap ? maxch : cap)), (unsigned)P);
+    if (kind == MODEL_H) CU(chain_launch(c, k_refine_init<MODEL_H>, gp, dim3(128), 0, a));
+    else CU(chain_launch(c, k_refine_init<MODEL_E>, gp, dim3(128), 0, a));
+    if (int r = check_launch(c, "k_refine_init")) return r;
+    for (int it = 0; it <= c->refine_iters; ++it) {
+        if (kind == MODEL_H) CU(chain_launch(c, k_refine_step<MODEL_H>, gs, dim3(kRefineBlock), 0, a));
+        else CU(chain_launch(c, k_refine_step<MODEL_E>, gs, dim3(kRefineBlock), 0, a));
+        if (int r = check_launch(c, "k_refine_step")) return r;
+    }
+    if (kind == MODEL_H) CU(chain_launch(c, k_refine_finish<MODEL_H>, gp, dim3(128), 0, a));
+    else CU(chain_launch(c, k_refine_finish<MODEL_E>, gp, dim3(128), 0, a));
+    if (int r = check_launch(c, "k_refine_finish")) return r;
+    *rec_out = a.out_rec;
+    return 0;
+}
+
 // The tail of apps/sfm.py:133-186 for the winner described by rec_dev (one SelectRecord per pair on the device):
 // T1 inlier mask + ordered compaction + decomposition, T2 4-pose cheirality + vote, T3 triangulation of the passing
 // inliers - three launches, nothing synchronised (see sfm_tail.cuh).  max_len = the longest pair.
@@ -1415,6 +1482,18 @@ static int pose_tail_launch(sfm_ctx* c, double thr, double dist_thr, const Selec
     // the caller's mask is "sed <= thr" (the forced sample points live in the compacted list only)
     if (mask_host) CU(cudaMemcpyAsync(mask_host, c->mask.p, (size_t)n, cudaMemcpyDeviceToHost, c->stream));
     if (sed_host) CU(cudaMemcpyAsync(sed_host, c->sed.p, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream));
+    c->refined_pairs = 0;
+    if (c->refine_iters > 0) {
+        // refine over the list T1 just compacted, then T1 again from the refined records (mask and sed stay those of
+        // the RANSAC winner)
+        if (int r = refine_launch(c, kind, rec_dev, max_len, &a.rec)) return r;
+        a.mask = nullptr;
+        a.sed = nullptr;
+        if (kind == MODEL_H) CU(chain_launch(c, k_tail_mask<MODEL_H>, dim3((unsigned)nblk, (unsigned)P), dim3(kTailBlock), 0, a));
+        else CU(chain_launch(c, k_tail_mask<MODEL_E>, dim3((unsigned)nblk, (unsigned)P), dim3(kTailBlock), 0, a));
+        if (int r = check_launch(c, "k_tail_mask")) return r;
+        c->refined_pairs = P;
+    }
     c->tic(T_POSE);
     // grids sized for the machine (grid-stride inside): the number of inliers is only known on the device
     const long long cap_blocks = P >= 64 ? 8 : 2ll * c->sm_count;
@@ -1771,6 +1850,7 @@ int sfm_sharded_tail(sfm_ctx* c, const void* gathered_records_dev, int world, in
     if (int r = use(c)) return r;
     if (!gathered_records_dev || world < 1 || rank < 0 || rank >= world) return fail(SFM_ERR_ARG, "bad gather arguments");
     if (!c->has_score) return fail(SFM_ERR_STATE, "sfm_score_async first");
+    if (c->refine_iters > 0) return fail(SFM_ERR_STATE, "refinement is not supported on hypothesis-sharded runs");
     if (mode < 0 || mode > 2) return fail(SFM_ERR_ARG, "bad selection %d", mode);
     if (int r = c->winnerE.reserve(72)) return r;
     if (int r = c->merged.reserve(sizeof(SelectRecord) + sizeof(Best) + 16)) return r;
@@ -1900,6 +1980,7 @@ int sfm_two_view_sharded(sfm_ctx* c, uint64_t seed, int64_t hyps_per_rank, doubl
                          int mode, double dist_thr) {
     if (int r = use(c)) return r;
     if (!c->nccl_comm) return fail(SFM_ERR_STATE, "sfm_nccl_init first");
+    if (c->refine_iters > 0) return fail(SFM_ERR_STATE, "refinement is not supported on hypothesis-sharded runs");
     if (c->batched) return fail(SFM_ERR_STATE, "single-pair call on a batched context");
     if (int r = sample_device(c, seed, 0, (int64_t)c->nccl_rank * hyps_per_rank, hyps_per_rank)) return r;
     if (int r = fit_launch(c, false)) return r;

@@ -262,21 +262,23 @@ class PairPipeline:
         return _merge_chunks([parts[k] for k in range(len(bounds) - 1)])
 
     def batch_two_view(self, pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra=0.0, aggregation="rms",
-                       selection="min_error", distance_threshold=50.0, pair_id0=0, chunk_pairs: Optional[int] = None):
+                       selection="min_error", distance_threshold=50.0, pair_id0=0, chunk_pairs: Optional[int] = None,
+                       refine_iterations=0):
         """``Engine.batch_two_view`` (RANSAC E + inlier list + pose vote + triangulation per pair) over chunks of
-        pairs that alternate between the contexts; identical to one call over all pairs."""
+        pairs that alternate between the contexts; identical to one call over all pairs (refinement included: a pair's
+        refined model depends on its inliers only)."""
         return self._chunked(lambda e, a, b, o, K, p0: e.batch_two_view(a, b, o, K, h, seed, threshold, min_extra,
                                                                          aggregation, selection, distance_threshold,
-                                                                         pair_id0=p0),
+                                                                         pair_id0=p0, refine_iterations=refine_iterations),
                              pts_a, pts_b, offsets, Ks, pair_id0, chunk_pairs)
 
     def batch_two_view_homography(self, pts_a, pts_b, offsets, Ks, h, seed, threshold, min_extra=0.0, aggregation="rms",
                                   selection="min_error", distance_threshold=50.0, rotation_tolerance=1e-2, pair_id0=0,
-                                  chunk_pairs: Optional[int] = None):
+                                  chunk_pairs: Optional[int] = None, refine_iterations=0):
         """``Engine.batch_two_view_homography`` over chunks of pairs; identical to one call over all pairs."""
         return self._chunked(lambda e, a, b, o, K, p0: e.batch_two_view_homography(
             a, b, o, K, h, seed, threshold, min_extra, aggregation, selection, distance_threshold, rotation_tolerance,
-            pair_id0=p0), pts_a, pts_b, offsets, Ks, pair_id0, chunk_pairs)
+            pair_id0=p0, refine_iterations=refine_iterations), pts_a, pts_b, offsets, Ks, pair_id0, chunk_pairs)
 
     def batch_two_view_select(self, pts_a, pts_b, offsets, Ks, essential_threshold, homography_threshold, h, seed,
                               pair_id0=0, chunk_pairs: Optional[int] = None, **kw):

@@ -24,8 +24,8 @@ import numpy as np
 
 from . import _native
 from .errors import EightPointCalculationError
-from .two_view import (_agg_name, _inlier_order, _load_samples, _replay_near_ties, _restore_random_state,
-                       _tail_inliers)
+from .two_view import (Refinement, _agg_name, _inlier_order, _load_samples, _ransac_list, _refine_count, _refinement,
+                       _replay_near_ties, _restore_random_state, _tail_inliers)
 
 _SAMPLE = 4  # points per minimal sample
 
@@ -200,6 +200,8 @@ class HomographyTwoViewResult:
     inlier_indices: np.ndarray    # ascending indices of the winner's inliers (samples included)
     passing: np.ndarray           # bool per inlier: passes the voted candidate (all False when rotation_only)
     points: np.ndarray            # [m,3] triangulated points (NaN where not passing)
+    refinement: Optional[Refinement] = None  # with refine_iterations > 0: everything above but ``ransac`` describes
+                                             # the refined H
 
 
 def two_view_homography_arrays(
@@ -218,6 +220,7 @@ def two_view_homography_arrays(
     selection: str = "min_error",
     engine: Optional[_native.Engine] = None,
     table: Optional[np.ndarray] = None,
+    refine_iterations: int = 0,
 ) -> HomographyTwoViewResult:
     """RANSAC homography -> pose and plane candidates -> cheirality vote -> triangulation, for [n,2] pixel arrays.
 
@@ -226,7 +229,10 @@ def two_view_homography_arrays(
     passes when both depths are >= -1e-8 and |X| <= ``distance_threshold`` (default 50), every passing inlier counts,
     and the first maximum wins.  The passing inliers are triangulated in pixel coordinates (P1 = K[I|0], P2 = K[R|t]).
     Raises EightPointCalculationError when no inlier passes any candidate.  With ``sampler="device"`` the estimate and
-    the tail are one library call."""
+    the tail are one library call.  refine_iterations > 0 refines the winning H over its inliers (Levenberg-Marquardt
+    on the symmetric transfer error, at most that many iterations, on the device) before the decomposition; the pose,
+    inliers and points then describe the refined H and ``refinement`` reports it."""
+    refine_iterations = _refine_count(refine_iterations)
     if distance_threshold is None:
         distance_threshold = 50.0
     K = np.asarray(camera_matrix, dtype=np.float64)
@@ -243,10 +249,10 @@ def two_view_homography_arrays(
         eng.sample_device(seed, iterations)
         best, mask, err, p, _, idx, ok, X = eng.two_view_homography(
             K, threshold, float(min_extra), _agg_name(error_aggregation_method), selection, distance_threshold,
-            rotation_tolerance)
+            rotation_tolerance, refine_iterations=refine_iterations)
         if best.index < 0:
             raise ValueError(f"No model could be found with at least {min_extra + _SAMPLE} inliers.")
-        sample, inliers = _tail_inliers(best, idx, _SAMPLE)
+        sample, inliers = _tail_inliers(best, _ransac_list(best, mask, _SAMPLE) if refine_iterations else idx, _SAMPLE)
         res = HomographyResult(H=np.array(best.E, dtype=np.float64).reshape(3, 3), best_index=int(best.index),
                                error=float(best.err), count_extra=int(best.count_extra),
                                inlier_indices=inliers, mask=mask.astype(bool),
@@ -256,7 +262,8 @@ def two_view_homography_arrays(
         res = ransac_homography_arrays(pa, pb, threshold, min_num_extra_inliers, error_aggregation_method, max_iterations,
                                        sampler=sampler, seed=seed, selection=selection, engine=eng, table=table)
         eng.set_winner(res.best_index)  # the host's winner (a near-tie replay may have moved it)
-        p, _, idx, ok, X = eng.homography_pose_and_triangulate(K, threshold, distance_threshold, rotation_tolerance)
+        p, _, idx, ok, X = eng.homography_pose_and_triangulate(K, threshold, distance_threshold, rotation_tolerance,
+                                                               refine_iterations=refine_iterations)
     cands = _candidates(p)
     counts = np.array(p.counts, dtype=np.int64)
     if p.rotation_only:
@@ -269,4 +276,5 @@ def two_view_homography_arrays(
         passing = ((ok >> int(p.best)) & 1).astype(bool)
     return HomographyTwoViewResult(ransac=res, R=R.copy(), t=t.copy(), n=n.copy(), d=d,
                                    rotation_only=bool(p.rotation_only), candidates=cands, counts=counts,
-                                   inlier_indices=idx, passing=passing, points=X)
+                                   inlier_indices=idx, passing=passing, points=X,
+                                   refinement=_refinement(eng) if refine_iterations else None)

@@ -101,6 +101,7 @@ def two_view_select_arrays(
     seed: int = 0,
     selection: str = "min_error",
     engine: Optional[_native.Engine] = None,
+    refine_iterations: int = 0,
 ) -> TwoViewSelection:
     """Both two-view paths on one pair, then the ratio rule on their winners.
 
@@ -109,10 +110,11 @@ def two_view_select_arrays(
     and with the same remaining arguments: each sub-result equals the standalone call, and with the reference sampler
     the global ``random`` state ends where the E call followed by the H call leaves it.  A call that raises ValueError
     or EightPointCalculationError leaves its model out (its message is kept) and the other one is chosen; when both
-    fail, ValueError carries both messages."""
+    fail, ValueError carries both messages.  With refine_iterations > 0 both winners are refined over their inliers
+    before their poses, and the ratio rule scores the refined models."""
     eng = engine or _native.get_engine()
     K = np.asarray(camera_matrix, dtype=np.float64)
-    common = dict(sampler=sampler, seed=seed, selection=selection, engine=eng)
+    common = dict(sampler=sampler, seed=seed, selection=selection, engine=eng, refine_iterations=refine_iterations)
     ess = hom = None
     ess_fail = hom_fail = None
     try:
@@ -129,8 +131,9 @@ def two_view_select_arrays(
     if ess is None and hom is None:
         raise ValueError(f"neither model could be estimated: essential matrix: {ess_fail}; homography: {hom_fail}")
     # both calls uploaded these correspondences: the context's pixel coordinates are this pair's
-    scores = _scores(eng, None if ess is None else ess.ransac.E, None if hom is None else hom.ransac.H, K, sigma,
-                     homography_ratio, False)
+    E = None if ess is None else (ess.refinement.model if ess.refinement else ess.ransac.E)
+    H = None if hom is None else (hom.refinement.model if hom.refinement else hom.ransac.H)
+    scores = _scores(eng, E, H, K, sigma, homography_ratio, False)
     win = hom if scores.model == "homography" else ess
     return TwoViewSelection(model=scores.model, scores=scores, essential=ess, homography=hom,
                             essential_failure=ess_fail, homography_failure=hom_fail, R=win.R, t=win.t,
@@ -186,6 +189,7 @@ def batch_two_view_select_arrays(
     rotation_tolerance: float = 1e-2,
     pair_id0: int = 0,
     engine: Optional[_native.Engine] = None,
+    refine_iterations: int = 0,
 ) -> dict:
     """``two_view_select_arrays(sampler="device")`` for every pair of a batch: pair p owns rows
     [offsets[p], offsets[p+1]) of the [n,2] pixel arrays and the camera Ks[p] (upper triangular, K[2,2] = 1).
@@ -201,18 +205,21 @@ def batch_two_view_select_arrays(
       score_e ... count_h     the scores of batch_score_models [P] (zero for a side left out)
       R [P,3,3], t [P,3], rotation_only [P]   the chosen side's pose (NaN without a model)
       inlier_offsets [P+1], inlier_idx, passing, points   the chosen side's inlier segments (empty without a model)
+    With refine_iterations > 0 both batch calls refine their winners (refined_E / refined_H and the refine_* keys in
+    their dicts) and the scorer reads the refined models.
     """
     eng = engine or _native.get_engine()
     offsets = np.ascontiguousarray(offsets, dtype=np.int64)
     P = len(offsets) - 1
     Ks = np.asarray(Ks, dtype=np.float64).reshape(P, 3, 3)
     ess, sv2 = eng._batch_two_view(pts_a, pts_b, offsets, Ks, h, seed, essential_threshold, min_extra, aggregation,
-                                   selection, distance_threshold, pair_id0)
+                                   selection, distance_threshold, pair_id0, refine_iterations)
     hom = eng.batch_two_view_homography(pts_a, pts_b, offsets, Ks, h, seed, homography_threshold, min_extra, aggregation,
-                                        selection, distance_threshold, rotation_tolerance, pair_id0)
+                                        selection, distance_threshold, rotation_tolerance, pair_id0, refine_iterations)
     e_st, h_st = _essential_status(ess, sv2), _homography_status(hom)
     keep_e, keep_h = np.equal(e_st, None), np.equal(h_st, None)
-    s, _ = eng.batch_score_models(ess["E"], hom["H"], keep_e, keep_h, sigma, homography_ratio)
+    s, _ = eng.batch_score_models(ess.get("refined_E", ess["E"]), hom.get("refined_H", hom["H"]), keep_e, keep_h, sigma,
+                                  homography_ratio)
     out = dict(essential=ess, homography=hom, essential_status=e_st, homography_status=h_st)
     for f in _SCORE_FIELDS:
         out[f] = np.array([getattr(x, f) for x in s[:P]], dtype=np.float64 if f[:5] in ("score", "ratio") else np.int64)

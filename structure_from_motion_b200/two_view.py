@@ -34,6 +34,35 @@ class RansacResult:
     first_invalid: int
 
 
+@dataclasses.dataclass
+class Refinement:
+    """The least-squares refinement of a winner over its inliers (include/sfm_b200.h, sfm_set_refinement)."""
+    model: np.ndarray     # (3,3) refined E or H, [2,2] == 1; the RANSAC model when status is no_model / nonfinite
+    cost_ransac: float    # sum of the RANSAC model's errors over the inlier list
+    cost_start: float     # at the start point (E: the RANSAC E projected onto the essential manifold)
+    cost_final: float     # at the refined model, <= cost_start
+    num: int              # correspondences in the inlier list
+    iterations: int       # proposals evaluated
+    status: str           # converged | max_iterations | stalled | no_model | nonfinite
+    rejected: int = 0     # of those, proposals rejected (cost not strictly lower)
+
+
+def _refinement(eng) -> Refinement:
+    """The report of the last single-pair tail call that refined."""
+    r = eng.get_refinement(1)[0]
+    return Refinement(model=np.array(r.model, dtype=np.float64).reshape(3, 3), cost_ransac=float(r.cost_ransac),
+                      cost_start=float(r.cost_start), cost_final=float(r.cost_final), num=int(r.num),
+                      iterations=int(r.iterations), status=_native.REFINE_STATUS[int(r.status)],
+                      rejected=int(r.rejected))
+
+
+def _refine_count(refine_iterations) -> int:
+    n = int(refine_iterations)
+    if n < 0:
+        raise ValueError(f"refine_iterations must be >= 0, got {n}")
+    return n
+
+
 def _agg_name(method) -> str:
     if method is None:
         return "rms"  # ransac.py:50-51
@@ -172,6 +201,13 @@ def _inlier_order(best, sampler, table, ref, mask, k):
     return sample, np.concatenate([sample.astype(np.int64), extra])
 
 
+def _ransac_list(best, mask, k):
+    """The list T1 compacts for the RANSAC winner (decision or sample, ascending), rebuilt from its mask."""
+    keep = np.asarray(mask).astype(bool).copy()
+    keep[np.array(best.sample[:k], dtype=np.int64)] = True
+    return np.flatnonzero(keep)
+
+
 def _tail_inliers(best, idx, k):
     """(sample int32[k], inlier indices int64) of a winner selected on the device: the sample, then the rest of the
     tail's compacted list (decision | sample, ascending)."""
@@ -235,7 +271,7 @@ def ransac_essential_arrays(
         best, mask, sed = eng.ransac_essential(threshold, float(min_num_extra_inliers), agg, selection)
     else:  # two_view_arrays: selection, inlier mask, pose vote and triangulation in one C call
         best, mask, sed, *rest = eng.two_view(threshold, float(min_num_extra_inliers), agg, selection,
-                                              _tail["distance_threshold"])
+                                              _tail["distance_threshold"], refine_iterations=_tail["refine_iterations"])
         _tail["out"] = rest
 
     if best.num_invalid > 0 and on_degenerate == "raise":
@@ -261,8 +297,9 @@ def ransac_essential_arrays(
             mask = m2.astype(np.uint8)
             best.count_extra = int(m2.sum() - m2[table[t]].sum())
             best.err = e
-            if _tail is not None:
-                _tail["out"] = list(eng.pose_and_triangulate(threshold, _tail["distance_threshold"]))
+            if _tail is not None:  # the tail (and the refinement) of the replayed winner
+                _tail["out"] = list(eng.pose_and_triangulate(threshold, _tail["distance_threshold"],
+                                                             refine_iterations=_tail["refine_iterations"]))
         else:
             eng.set_winner(int(best.index))
 
@@ -428,14 +465,19 @@ class TwoViewResult:
     passing: np.ndarray          # bool per inlier: passed the cheirality vote
     points: np.ndarray           # [m,3] triangulated points (NaN where not passing)
     counts: np.ndarray
+    refinement: Optional[Refinement] = None  # with refine_iterations > 0: R, t and the inlier arrays are those of the
+                                             # refined E; ``ransac`` is the RANSAC result, unchanged
 
 
 def two_view_arrays(camera_matrix, pts_a, pts_b, threshold, min_num_extra_inliers=None,
                     error_aggregation_method=None, max_iterations=None, distance_threshold=None,
-                    **kw) -> TwoViewResult:
+                    refine_iterations: int = 0, **kw) -> TwoViewResult:
     """The whole hot path of apps/sfm.py:110-186 in one call: RANSAC E -> cheirality vote ->
     triangulation of the passing inliers.  Correspondences are uploaded once; only results
-    come back."""
+    come back.  refine_iterations > 0 refines the winning E over its inliers (Levenberg-Marquardt on the essential
+    manifold, at most that many iterations, on the device) before the vote; the pose, inliers and points then describe
+    the refined E and ``refinement`` reports it."""
+    refine_iterations = _refine_count(refine_iterations)
     if distance_threshold is None:
         distance_threshold = 50.0
     eng = kw.get("engine") or _native.get_engine()
@@ -446,8 +488,8 @@ def two_view_arrays(camera_matrix, pts_a, pts_b, threshold, min_num_extra_inlier
         # whole estimate is enqueued in one go (un-synchronised upload included) and fetched once
         return _two_view_device(eng, camera_matrix, pts_a, pts_b, threshold, min_num_extra_inliers or 0,
                                 _agg_name(error_aggregation_method), int(max_iterations or 100), float(distance_threshold),
-                                int(kw.get("seed", 0)), kw.get("selection", "min_error"))
-    tail = {"distance_threshold": float(distance_threshold)}
+                                int(kw.get("seed", 0)), kw.get("selection", "min_error"), refine_iterations)
+    tail = {"distance_threshold": float(distance_threshold), "refine_iterations": refine_iterations}
     res = ransac_essential_arrays(camera_matrix, pts_a, pts_b, threshold, min_num_extra_inliers,
                                   error_aggregation_method, max_iterations, _tail=tail, **kw)
     p, num, idx, ok, X = tail["out"]
@@ -459,7 +501,7 @@ def two_view_arrays(camera_matrix, pts_a, pts_b, threshold, min_num_extra_inlier
     R = np.array(p.R, dtype=np.float64).reshape(4, 3, 3)[b].copy()
     t = np.array(p.t, dtype=np.float64).reshape(4, 3)[b].copy()
     return TwoViewResult(ransac=res, R=R, t=t, inlier_indices=idx, passing=((ok >> b) & 1).astype(bool),
-                         points=X, counts=counts)
+                         points=X, counts=counts, refinement=_refinement(eng) if refine_iterations else None)
 
 
 @dataclasses.dataclass
@@ -497,13 +539,14 @@ def image_pair_arrays(image_a, image_b, camera_matrix, *, num_harris_corners: in
 
 
 def _device_submit(eng, out, camera_matrix, pts_a, pts_b, threshold, min_extra, agg, max_iterations, distance_threshold,
-                   seed, selection):
+                   seed, selection, refine_iterations=0):
     eng.upload_pairs(pts_a, pts_b, camera_matrix, sync=False)
     eng.sample_device(seed, max_iterations)
-    return eng.two_view_async(threshold, float(min_extra), agg, selection, distance_threshold, out=out)
+    return eng.two_view_async(threshold, float(min_extra), agg, selection, distance_threshold, out=out,
+                              refine_iterations=refine_iterations)
 
 
-def _device_result(eng, mask, sed, min_extra, copy: bool) -> "TwoViewResult":
+def _device_result(eng, mask, sed, min_extra, copy: bool, refine_iterations=0) -> "TwoViewResult":
     best, p, num, idx, ok, X = eng.two_view_fetch()
     if best.index < 0:
         raise ValueError(f"No model could be found with at least {min_extra + 8} inliers.")
@@ -511,7 +554,8 @@ def _device_result(eng, mask, sed, min_extra, copy: bool) -> "TwoViewResult":
     counts = np.array(p.counts, dtype=np.int64)
     if 0 == np.count_nonzero(counts):
         raise EightPointCalculationError("None of the transformations pass the cheirality check.")
-    sample, inliers = _tail_inliers(best, idx, 8)
+    # with refinement the tail's list is the refined model's: the RANSAC list is the mask plus the sample
+    sample, inliers = _tail_inliers(best, _ransac_list(best, mask, 8) if refine_iterations else idx, 8)
     b = int(p.best)
     res = RansacResult(E=np.array(best.E, dtype=np.float64).reshape(3, 3), best_index=int(best.index),
                        error=float(best.err), count_extra=int(best.count_extra),
@@ -521,16 +565,16 @@ def _device_result(eng, mask, sed, min_extra, copy: bool) -> "TwoViewResult":
     R = np.array(p.R, dtype=np.float64).reshape(4, 3, 3)[b].copy()
     t = np.array(p.t, dtype=np.float64).reshape(4, 3)[b].copy()
     return TwoViewResult(ransac=res, R=R, t=t, inlier_indices=idx, passing=((ok >> b) & 1).astype(bool), points=X,
-                         counts=counts)
+                         counts=counts, refinement=_refinement(eng) if refine_iterations else None)
 
 
 def _two_view_device(eng, camera_matrix, pts_a, pts_b, threshold, min_extra, agg, max_iterations, distance_threshold, seed,
-                     selection):
+                     selection, refine_iterations=0):
     n = np.asarray(pts_a).reshape(-1, 2).shape[0]
     out = eng.pinned_out(n)  # engine-owned pinned landing buffers: page-locking per call would dominate the transfers
     mask, sed = _device_submit(eng, out, camera_matrix, pts_a, pts_b, threshold, min_extra, agg, max_iterations,
-                               distance_threshold, seed, selection)
-    return _device_result(eng, mask, sed, min_extra, copy=True)
+                               distance_threshold, seed, selection, refine_iterations)
+    return _device_result(eng, mask, sed, min_extra, copy=True, refine_iterations=refine_iterations)
 
 
 class TwoViewStream:
