@@ -66,8 +66,9 @@ int sfm_set_stream(sfm_ctx *ctx, void *cuda_stream);
  * when the context's work has to be ordered with that stream's work (NCCL collectives, timing events). */
 int sfm_use_default_stream(sfm_ctx *ctx);
 int sfm_synchronize(sfm_ctx *ctx);
-/* hyps_per_thread: essential matrices per thread (1, 2, 4; fp32 pre-filter: 2, 4, 8); group:
- * correspondences per vote (hyps_per_thread * group <= 32 tests per lane and vote); 0 keeps the
+/* hyps_per_thread: essential matrices per thread; group: correspondences per vote.  The shapes
+ * (hyps_per_thread x group) with a kernel are 2 x 16 for the fp64 variants, and 4 x 8 (the default)
+ * and 2 x 16 for SCREEN32; any other shape fails with SFM_ERR_ARG.  hyps_per_thread 0 keeps the
  * current shape, or selects the variant's default when switching to/from SCREEN32. */
 int sfm_set_score_variant(sfm_ctx *ctx, int variant, int hyps_per_thread, int group);
 /* Pinned host memory for the caller's buffers (so that H2D/D2H copies are true async DMA). */

@@ -209,7 +209,7 @@ inline void chain_config(sfm_ctx* c, dim3 grid, dim3 block, size_t smem, cudaLau
     at->id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at->val.programmaticStreamSerializationAllowed = 1;
     cfg->attrs = at;
-    cfg->numAttrs = SFM_PDL ? 1 : 0;
+    cfg->numAttrs = 1;
 }
 template <typename... KArgs, typename... Args>
 cudaError_t chain_launch(sfm_ctx* c, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, Args&&... args) {
@@ -225,38 +225,34 @@ inline cudaError_t chain_launch_ptr(sfm_ctx* c, const void* fn, dim3 grid, dim3 
     return cudaLaunchKernelExC(&cfg, fn, kargs);
 }
 
-// per-warp shared memory of a scoring body (the two-sided one has its own layout for hpt <= 2, the 9-slot one adds
-// its boxes and kappa: tiles)
-template <int HPT>
-size_t score_warp_smem_h(bool full, bool tiles) {
-    return full ? score_warp_bytes<HPT, MODE_FULL>() : tiles ? score_warp_bytes<HPT, MODE_SCREEN>() : sizeof(ScoreWarpSmem<HPT>);
+// K2's kernel for a variant and shape, and the dynamic shared memory it takes per warp; fn is null for a shape without
+// a kernel.  fp64: 2 x 16 only.  The fp32 pre-filter: 4 x 8 (its default) and 2 x 16.  tiles: the upload holds K2's
+// sorted copy and its boxes (k2_order), so SCREEN is the 9-slot body; else the 11-slot one.  AUTO holds a one-sided
+// body and the two-sided one.
+struct ScoreKernel {
+    const void* fn;
+    size_t warp_bytes;
+};
+template <typename K>
+ScoreKernel score_kernel_of(K* kernel, size_t warp_bytes) {
+    return {reinterpret_cast<const void*>(kernel), warp_bytes};
 }
-size_t score_warp_smem(int hpt, bool full, bool tiles) {
-    switch (hpt) {
-        case 1: return score_warp_smem_h<1>(full, tiles);
-        case 2: return score_warp_smem_h<2>(full, tiles);
-        case 4: return score_warp_smem_h<4>(full, tiles);
-        default: return sizeof(ScoreWarpSmem<8>);  // SCREEN32 only
-    }
-}
-
-// tiles: the upload holds K2's sorted copy and its boxes (k2_order), so SCREEN is the 9-slot body; else the 11-slot one
-const void* score_kernel(int variant, int hpt, int group, bool tiles) {
+ScoreKernel score_kernel(int variant, int hpt, int group, bool tiles) {
     if (variant == SFM_SCORE_SCREEN32) {
-#define SFM_K32(H, G) if (hpt == H && group == G) return reinterpret_cast<const void*>(&k_score<H, G, MODE_SCREEN32>)
-        SFM_K32(2, 16); SFM_K32(4, 8); SFM_K32(8, 4);
-#undef SFM_K32
-        return nullptr;
+        if (hpt == 4 && group == 8) return score_kernel_of(&k_score<4, 8, MODE_SCREEN32>, sizeof(ScoreWarpSmem<4>));
+        if (hpt == 2 && group == 16) return score_kernel_of(&k_score<2, 16, MODE_SCREEN32>, sizeof(ScoreWarpSmem<2>));
+        return {nullptr, 0};
     }
-#define SFM_K(H, G) if (hpt == H && group == G) return !scr ? reinterpret_cast<const void*>(&k_score<H, G, MODE_FULL>) \
-                                                    : tiles ? reinterpret_cast<const void*>(&k_score<H, G, MODE_SCREEN>) \
-                                                            : reinterpret_cast<const void*>(&k_score<H, G, MODE_SCREEN11>)
-    const bool scr = variant == SFM_SCORE_SCREEN;
-    SFM_K(1, 16); SFM_K(1, 32);
-    SFM_K(2, 4); SFM_K(2, 8); SFM_K(2, 16);
-    SFM_K(4, 2); SFM_K(4, 4); SFM_K(4, 8);
-#undef SFM_K
-    return nullptr;
+    if (hpt != 2 || group != 16) return {nullptr, 0};
+    const size_t one = tiles ? sizeof(ScoreWarpSmemBox<2>) : sizeof(ScoreWarpSmem<2>), two = sizeof(ScoreWarpSmemFS<2>);
+    switch (variant) {
+        case SFM_SCORE_FULL: return score_kernel_of(&k_score<2, 16, MODE_FULL>, two);
+        case SFM_SCORE_SCREEN:
+            return tiles ? score_kernel_of(&k_score<2, 16, MODE_SCREEN>, one) : score_kernel_of(&k_score<2, 16, MODE_SCREEN11>, one);
+        default:  // SFM_SCORE_AUTO
+            return tiles ? score_kernel_of(&k_score_auto<2, 16, MODE_SCREEN>, one > two ? one : two)
+                         : score_kernel_of(&k_score_auto<2, 16, MODE_SCREEN11>, one > two ? one : two);
+    }
 }
 
 }  // namespace
@@ -359,8 +355,7 @@ int sfm_set_score_variant(sfm_ctx* c, int variant, int hpt, int group) {
         nh = variant == SFM_SCORE_SCREEN32 ? 4 : 2;
         ng = variant == SFM_SCORE_SCREEN32 ? 8 : 16;
     }
-    if (!score_kernel(variant == SFM_SCORE_AUTO ? SFM_SCORE_SCREEN : variant, nh, ng, true) ||
-        (variant == SFM_SCORE_AUTO && !score_kernel(SFM_SCORE_FULL, nh, ng, true)))
+    if (!score_kernel(variant, nh, ng, true).fn)
         return fail(SFM_ERR_ARG, "unsupported combination: hyps_per_thread %d, group %d", nh, ng);
     c->variant = variant;
     c->hpt = nh;
@@ -473,10 +468,7 @@ int sfm_get_table(sfm_ctx* c, int32_t* table, int64_t first, int64_t h) {
 // gains.  Batches do not get
 // the sorted copy: at 512 pairs x 2 000 (bench config4) a sort of the whole batch cost 0.19 ms per 1M records at upload
 // and the 9-slot body was 1.5 % slower on K2 than the 11-slot one (the boxes of 2 000-point pairs are wide).
-#ifndef SFM_K2_SORT_MIN
-#define SFM_K2_SORT_MIN 65536
-#endif
-constexpr long long kK2SortMin = SFM_K2_SORT_MIN;
+constexpr long long kK2SortMin = 65536;
 static int k2_order(sfm_ctx* c, long long n) {
     size_t cub_bytes = 0;
     CU(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, (const unsigned*)nullptr, (unsigned*)nullptr, (const int*)nullptr,
@@ -835,8 +827,8 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
     // rounding guard of the screening tests: relative slack + an absolute term that covers a
     // cancelling residual r at the 1-ulp level (only matters for thr -> 0)
     // the fp32 pre-filter needs s = sqrt(thr32) and 1/s inside the fp32 range: huge thresholds use the fp64 screen
-    // AUTO: the one-sided screen is prepared and launched as usual, the two-sided one right behind it; a pilot that
-    // rides on the screening-copy kernel measures the survivor rate and one of the two scoring kernels exits at once
+    // AUTO: the one-sided screen is prepared as usual; a pilot (k_pilot, or riding on the screening-copy kernel)
+    // measures its survivor rate and k_score_auto runs the one-sided or the two-sided body
     const bool autov = c->variant == SFM_SCORE_AUTO;
     int variant = autov ? SFM_SCORE_SCREEN : c->variant;
     if (variant == SFM_SCORE_SCREEN32 && thr > 1e6) variant = SFM_SCORE_SCREEN;  // with hpt 2 / group 16, see above
@@ -854,47 +846,21 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
     {
         // persistent blocks over (pair, split, hypothesis block) items
         const bool tiles = c->k2_ready;
-        const void* fn = score_kernel(variant, hpt, G, tiles);
-        if (!fn) return fail(SFM_ERR_ARG, "unsupported scoring configuration (variant %d, hpt %d, group %d)", variant, hpt, G);
-        const size_t smem_one = (size_t)kScoreWarps * score_warp_smem(hpt, false, tiles && !f32);
-        const size_t smem_two = (size_t)kScoreWarps * score_warp_smem(hpt, true, false);
-        const size_t smem_both = smem_one > smem_two ? smem_one : smem_two;  // AUTO in one launch holds either body
-        const size_t smem = screen ? smem_one : smem_two;
+        const ScoreKernel sk = score_kernel(autov ? SFM_SCORE_AUTO : variant, hpt, G, tiles);
+        if (!sk.fn) return fail(SFM_ERR_ARG, "unsupported scoring configuration (variant %d, hpt %d, group %d)", variant, hpt, G);
+        const size_t smem = (size_t)kScoreWarps * sk.warp_bytes;
         // attribute set and occupancy queried once per kernel instantiation (small cache)
-        auto occupancy = [&](const void* f, size_t bytes, int* out) -> int {
-            for (int k = 0; k < 4; ++k)
-                if (c->occ_fn[k] == f) { *out = c->occ_blocks[k]; return 0; }
-            int o = 0;
-            CU(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-            CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, f, kScoreThreads, bytes));
-            if (o < 1) o = 1;
-            c->occ_fn[c->occ_next] = f;
-            c->occ_blocks[c->occ_next] = o;
-            c->occ_next = (c->occ_next + 1) & 3;
-            *out = o;
-            return 0;
-        };
         int occ = 0;
-        if (int r = occupancy(fn, smem, &occ)) return r;
-#ifndef SFM_AUTO_SINGLE
-#define SFM_AUTO_SINGLE 1
-#endif
-        // AUTO: one kernel holding both screens (shapes 2x16 and 4x8), else the two-launch scheme
-        const void* fn_auto = nullptr;
-        if (autov && SFM_AUTO_SINGLE) {
-            if (hpt == 2 && G == 16)
-                fn_auto = tiles ? reinterpret_cast<const void*>(&k_score_auto<2, 16, MODE_SCREEN>)
-                                : reinterpret_cast<const void*>(&k_score_auto<2, 16, MODE_SCREEN11>);
-            if (hpt == 4 && G == 8)
-                fn_auto = tiles ? reinterpret_cast<const void*>(&k_score_auto<4, 8, MODE_SCREEN>)
-                                : reinterpret_cast<const void*>(&k_score_auto<4, 8, MODE_SCREEN11>);
+        for (int k = 0; k < 4 && !occ; ++k)
+            if (c->occ_fn[k] == sk.fn) occ = c->occ_blocks[k];
+        if (!occ) {
+            CU(cudaFuncSetAttribute(sk.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, sk.fn, kScoreThreads, smem));
+            if (occ < 1) occ = 1;
+            c->occ_fn[c->occ_next] = sk.fn;
+            c->occ_blocks[c->occ_next] = occ;
+            c->occ_next = (c->occ_next + 1) & 3;
         }
-        if (fn_auto)
-            if (int r = occupancy(fn_auto, smem_both, &occ)) return r;
-        const void* fn_full = (autov && !fn_auto) ? score_kernel(SFM_SCORE_FULL, hpt, G, tiles) : nullptr;
-        int occ_full = 0;
-        if (fn_full)
-            if (int r = occupancy(fn_full, smem_two, &occ_full)) return r;
         const long long grid_blocks = (long long)c->sm_count * occ;
         constexpr int items_per_warp = 32;  // 12 -> 32 shortens the end-of-launch tail (+1 % on config 3)
         const ItemSplit sp = split_items(grid_blocks * kScoreWarps * items_per_warp, hblocks * P, max_len, kTile);
@@ -967,29 +933,18 @@ static int score_launch(sfm_ctx* c, double thr, double min_extra, int agg, int m
         }
         const long long want_blocks = (total_items + kScoreWarps - 1) / kScoreWarps;
         const long long launch_blocks = grid_blocks < want_blocks ? grid_blocks : want_blocks;
-        void* kargs[] = {(void*)&a};
-        if (!skip_k2 && fn_auto) {
-            ScoreArgs a2 = a;
+        if (!skip_k2 && autov) {
+            ScoreArgs a2 = a;  // the two-sided body: its guard, on the unscaled records
             a2.thr_pre = thr * (1.0 + 1e-9) + 1e-22;
             a2.pts = c->pts.as<Corr>();
             a2.spts = a2.pts;
-            void* kargs2[] = {(void*)&a, (void*)&a2};
-            CU(chain_launch_ptr(c, fn_auto, dim3((unsigned)launch_blocks), dim3(kScoreThreads), smem_both, kargs2));
+            void* kargs[] = {(void*)&a, (void*)&a2};
+            CU(chain_launch_ptr(c, sk.fn, dim3((unsigned)launch_blocks), dim3(kScoreThreads), smem, kargs));
             if (int r = check_launch(c, "k_score_auto")) return r;
         } else if (!skip_k2) {
-            CU(chain_launch_ptr(c, fn, dim3((unsigned)launch_blocks), dim3(kScoreThreads), smem, kargs));
+            void* kargs[] = {(void*)&a};
+            CU(chain_launch_ptr(c, sk.fn, dim3((unsigned)launch_blocks), dim3(kScoreThreads), smem, kargs));
             if (int r = check_launch(c, "k_score")) return r;
-            if (fn_full) {  // AUTO: the two-sided screen on the unscaled records; exits at once unless the pilot chose it
-                ScoreArgs a2 = a;
-                a2.thr_pre = thr * (1.0 + 1e-9) + 1e-22;
-                a2.pts = c->pts.as<Corr>();
-                a2.spts = a2.pts;
-                const long long gb2 = (long long)c->sm_count * occ_full;
-                const long long lb2 = gb2 < want_blocks ? gb2 : want_blocks;
-                void* kargs2[] = {(void*)&a2};
-                CU(chain_launch_ptr(c, fn_full, dim3((unsigned)lb2), dim3(kScoreThreads), smem_two, kargs2));
-                if (int r = check_launch(c, "k_score")) return r;
-            }
         }
         c->toc(T_SCORE);
     }

@@ -14,14 +14,9 @@ namespace sfm {
 // wait until the preceding grid has completed and its memory is visible (a no-op for an ordinary launch), then let
 // the NEXT kernel of the chain be launched - its blocks become resident as resources free up and sit in their own
 // wait, so the launch latency of a kernel overlaps the execution of its predecessor.
-#ifndef SFM_PDL
-#define SFM_PDL 1
-#endif
 __device__ __forceinline__ void chain_enter() {
-#if SFM_PDL
     asm volatile("griddepcontrol.wait;" ::: "memory");
     asm volatile("griddepcontrol.launch_dependents;");
-#endif
 }
 
 

@@ -287,11 +287,11 @@ __device__ __forceinline__ int eight_point_fit_qr(const Corr (&c)[8], double (&E
 }
 
 constexpr int kFitQrThreads = 64;
+// 168 registers + 0.5 KB of L1-resident spills: 12 warps/SM hide the sqrt/div latency chains better than 8 warps without
+// spills (222 registers: config 4 0.39 vs 0.34 ms) or 14 warps with 1 KB of spills (144 registers: 0.38 ms)
+constexpr int kFitQrMinBlocks = 6;
 
-#ifndef SFM_FIT_MINB
-#define SFM_FIT_MINB 6  // 168 registers + 0.5 KB of L1-resident spills: 12 warps/SM hide the sqrt/div latency chains better than 8 warps without spills (222 registers: config 4 0.39 vs 0.34 ms) or 14 warps with 1 KB of spills (144 registers: 0.38 ms)
-#endif
-__global__ void __launch_bounds__(kFitQrThreads, SFM_FIT_MINB)
+__global__ void __launch_bounds__(kFitQrThreads, kFitQrMinBlocks)
 k_fit_qr(const Corr* __restrict__ pts, const long long* __restrict__ offsets, const int32_t* __restrict__ table,
          long long h, double* __restrict__ E_out, uint8_t* __restrict__ valid_out,
          unsigned* __restrict__ ambiguous_count, ModelRow* __restrict__ rows,

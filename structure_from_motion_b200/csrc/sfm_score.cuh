@@ -111,7 +111,7 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
 //   inliers); identical results; the like-for-like arithmetic baseline AND the body the AUTO
 //   variant switches to above 9 % survivors.  Its survivor path differs: one ring ENTRY per
 //   survivor (handed out in ballot-compacted rounds) instead of one record per lane and batch,
-//   and - HPT <= 2 - models and correspondences gathered from shared memory (ScoreWarpSmemFS).
+//   and models and correspondences gathered from shared memory (ScoreWarpSmemFS).
 //   SCREEN32 (reported separately, never the fp64 headline): the same 11-slot test in fp32 on
 //   E/|E|_F and fp32 copies of the correspondences — a PRE-FILTER only: every survivor is still
 //   decided and summed by the exact fp64 scorer, so counts, sums and the winner are bit-identical
@@ -152,14 +152,8 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
 // ------------------------------------------------------------------------------------
 constexpr int kScoreThreads = 128;
 constexpr int kScoreWarps = kScoreThreads / 32;
-#ifndef SFM_SCORE_TILE
-#define SFM_SCORE_TILE 64
-#endif
-#ifndef SFM_SCORE_STAGES
-#define SFM_SCORE_STAGES 3
-#endif
-constexpr int kTile = SFM_SCORE_TILE;     // correspondences per stage (2 KB)
-constexpr int kStages = SFM_SCORE_STAGES;
+constexpr int kTile = 64;     // correspondences per stage (2 KB)
+constexpr int kStages = 3;
 constexpr int kRing = 64;     // survivor records per warp: < 32 pending + <= 32 new
 constexpr unsigned kMaxPoints = 1u << 25;
 constexpr int kChunks = 4;             // 21-bit chunks of an 84-bit fixed-point term
@@ -208,7 +202,7 @@ struct ScoreArgs {
     long long htotal;          // npairs * h
     unsigned* work_counter;
     unsigned long long* acc;   // [kAccWords][htotal] exact integer accumulators (pre-zeroed)
-    const int* mode_flag;      // AUTO variant: the MODE the pilot selected (the other kernel exits at once); else null
+    const int* mode_flag;      // AUTO variant: the MODE the pilot selected (k_score_auto runs that body); else null
     const double4* boxes;      // SCREEN (single pairs only): (cx, cy, wx, wy) of the B points of tile t of pts at [t]
 };
 
@@ -505,7 +499,7 @@ struct alignas(128) ScoreWarpSmemBox : ScoreWarpSmem<HPT> {
     double kap[HPT][32];   // kappa of (slot, lane), read once per tile (registers are the screen's)
 };
 
-// Two-sided body, HPT <= 2 (the survivor-rich regime: AUTO sends > 9 % survivors here): the drain gathers nothing
+// Two-sided body (the survivor-rich regime: AUTO sends > 9 % survivors here): the drain gathers nothing
 // from global memory.  Its models sit in shared memory (component-major: a gather of 32 models is nine LDS.64) and
 // its correspondences are read from the tile ring itself - the two-sided screen streams the UNSCALED records, and a
 // stage is refilled only after every record that points into it has been drained (one tile of slack: see the tile
@@ -522,24 +516,11 @@ struct alignas(128) ScoreWarpSmemFS {
     uint2 ring[kRing];
     unsigned long long full_bar[kStagesFS];
 };
-__host__ __device__ constexpr bool score_full_in_smem(int hpt) { return hpt <= 2; }
-template <int HPT, int MODE>
-constexpr size_t score_warp_bytes() {
-    return (MODE == MODE_FULL && score_full_in_smem(HPT)) ? sizeof(ScoreWarpSmemFS<HPT>)
-           : MODE == MODE_SCREEN                          ? sizeof(ScoreWarpSmemBox<HPT>)
-                                                          : sizeof(ScoreWarpSmem<HPT>);
-}
 
-// resident blocks per SM the register budget is shaped for (HPT 4 / 2 / 1): 16 / 20 / 32 warps.  Measured on
-// config 3: HPT 2 at 96 registers (5 blocks) beats 80 registers (6 blocks) by ~1.5 %: the extra registers let
-// ptxas keep more independent DFMA chains in flight, which is what the FP64 pipe's ~25-cycle latency needs.
-#ifndef SFM_SCORE_MINB4
-#define SFM_SCORE_MINB4 4
-#endif
-#ifndef SFM_SCORE_MINB2
-#define SFM_SCORE_MINB2 5
-#endif
-constexpr int score_min_blocks(int hpt) { return hpt >= 4 ? SFM_SCORE_MINB4 : (hpt == 2 ? SFM_SCORE_MINB2 : 8); }
+// resident blocks per SM the register budget is shaped for (HPT 2 / 1): 20 / 32 warps.  Measured on config 3: HPT 2
+// at 96 registers (5 blocks) beats 80 registers (6 blocks) by ~1.5 %: the extra registers let ptxas keep more
+// independent DFMA chains in flight, which is what the FP64 pipe's ~25-cycle latency needs.
+constexpr int score_min_blocks(int hpt) { return hpt == 2 ? 5 : 8; }
 
 
 __device__ __forceinline__ int sign_word(double d) { return __double2hiint(d); }
@@ -553,22 +534,23 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
     using T = typename std::conditional<F32, float, double>::type;       // arithmetic of the per-test work
     using P = typename std::conditional<F32, Corr32, Corr>::type;       // record streamed through shared memory
     constexpr int NB = HPT * G;  // tests per lane and batch = survivor bits per vote
-    constexpr bool FS = MODE == MODE_FULL && score_full_in_smem(HPT);  // drain gathers from shared memory only
-    constexpr bool ENTRY = MODE == MODE_FULL;  // survivor ring of per-survivor entries instead of per-lane records
+    // two-sided: a survivor ring of per-survivor entries instead of per-lane records, drained from shared memory only
+    constexpr bool ENTRY = MODE == MODE_FULL;
     constexpr bool BOX = MODE == MODE_SCREEN;  // 9-slot screen against the tile's bound
-    constexpr int TILE = FS ? kTileFS : kTile;
-    constexpr int STAGES = FS ? kStagesFS : kStages;
-    constexpr int AHEAD = FS ? STAGES - 1 : STAGES;  // tiles in flight; FS keeps the previous tile's stage for the drain
-    using WS = typename std::conditional<FS, ScoreWarpSmemFS<HPT>,
+    constexpr int TILE = ENTRY ? kTileFS : kTile;
+    constexpr int STAGES = ENTRY ? kStagesFS : kStages;
+    constexpr int AHEAD = ENTRY ? STAGES - 1 : STAGES;  // tiles in flight; ENTRY keeps the previous tile's stage for the drain
+    using WS = typename std::conditional<ENTRY, ScoreWarpSmemFS<HPT>,
                                          typename std::conditional<BOX, ScoreWarpSmemBox<HPT>, ScoreWarpSmem<HPT>>::type>::type;
     static_assert(NB <= 32 && (TILE % G) == 0 && (kTile % TILE) == 0, "a batch is at most 32 tests and divides a tile");
+    static_assert(!ENTRY || HPT <= 2, "the two-sided body's bank swizzle of sacc holds two slots");
     extern __shared__ __align__(128) unsigned char score_smem[];
     const unsigned full = 0xffffffffu;
     const int lane = threadIdx.x & 31;
     const int warp = __shfl_sync(full, (int)(threadIdx.x >> 5), 0);  // tells the compiler it is warp-uniform
     const unsigned lt = lanemask_lt();
-    // AUTO in two launches: the pilot chose the other screen (its flag is MODE_FULL or MODE_SCREEN, the one-sided body
-    // of either kind)
+    // The pilot's flag (AUTO only) never disagrees here: k_score_auto branches on it first.  The test stays because
+    // without it ptxas spills 16-28 bytes in both k_score_auto kernels at the same 96 registers (k2_shapes_sass_check).
     if (a.mode_flag && (*a.mode_flag == MODE_FULL) != (MODE == MODE_FULL)) return;
     WS& ws = reinterpret_cast<WS*>(score_smem)[warp];
 
@@ -641,7 +623,7 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
                 v[k] = real ? Ep[9 * hyp + k] : 0.0;
                 f2 = fma(v[k], v[k], f2);
             }
-            if constexpr (FS) {  // the previous item's drains are complete (queue emptied at its end)
+            if constexpr (ENTRY) {  // the previous item's drains are complete (queue emptied at its end)
                 double2* mp = reinterpret_cast<double2*>(&ws.model[32 * j + lane][0]);
                 mp[0] = make_double2(v[0], v[1]);
                 mp[1] = make_double2(v[2], v[3]);
@@ -669,8 +651,8 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
         auto accumulate = [&](bool act, double sv, int slot, int owner) {
             if (act && (sv <= a.thr)) {  // ransac.py:73  score <= threshold
                 unsigned ch[kChunks];
-                // same-address atomics serialise; FS also keeps the two slots of an owner in different banks
-                unsigned* dst = &ws.sacc[slot][0][FS ? (owner ^ (slot << 4)) : owner];
+                // same-address atomics serialise; ENTRY also keeps the two slots of an owner in different banks
+                unsigned* dst = &ws.sacc[slot][0][ENTRY ? (owner ^ (slot << 4)) : owner];
                 atomicAdd(dst, 1u);
                 if (a.sums & SUM_S1) {
                     chunks21(sv, a.scale1, ch);
@@ -684,11 +666,11 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
                 }
             }
         };
-        // candidate's E and correspondence: from global memory (L1/L2 hits) by index, or - FS - from shared memory
+        // candidate's E and correspondence: from global memory (L1/L2 hits) by index, or - ENTRY - from shared memory
         auto survivor_sed = [&](unsigned hl, unsigned pos) -> double {
             double eo[9];
             Corr c;
-            if constexpr (FS) {
+            if constexpr (ENTRY) {
                 const double2* mp = reinterpret_cast<const double2*>(&ws.model[hl][0]);
                 const double2 m0 = mp[0], m1 = mp[1], m2 = mp[2], m3 = mp[3];
                 eo[0] = m0.x; eo[1] = m0.y; eo[2] = m1.x; eo[3] = m1.y;
@@ -707,8 +689,7 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
         };
 
         // ---- two-sided body: one ring ENTRY per survivor ------------------------------------------------------------
-        // {owner lane << 14 | slot << 11 | position}: position = the correspondence's place in the tile ring (FS) or its
-        // item-relative index.  A drain is "lane l takes entry head + l": no prefix sum over record counts, no search
+        // {owner lane << 14 | slot << 11 | position}: position = the correspondence's place in the tile ring.  A drain is "lane l takes entry head + l": no prefix sum over record counts, no search
         // for the n-th set bit, no record straddling a drain.  The bits of a batch are handed out in rounds, one bit per
         // lane and round (ballot-compacted): ~12 instructions per round, as many rounds as the fullest lane has
         // survivors.  ncu of the record scheme below at 17 % inliers: 130 of the drain's 237 instructions were that
@@ -716,7 +697,7 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
         // one-sided body (1 % survivors, 1.3 bits per record) the rounds cost more than they save (-5 %), so it keeps
         // the records.
         unsigned* qe = reinterpret_cast<unsigned*>(ws.ring);
-        constexpr int LH = HPT >= 8 ? 3 : (HPT == 4 ? 2 : (HPT == 2 ? 1 : 0));  // slot bits, kept at the top of an entry
+        constexpr int LH = HPT == 4 ? 2 : (HPT == 2 ? 1 : 0);  // slot bits, kept at the top of an entry
         const unsigned ln = (unsigned)__popc(lt);  // the lane index again, from a live register (ptxas re-reads SR_TID otherwise)
         auto drain_entries = [&]() {
             const unsigned navail = tail - head;  // 1..63
@@ -802,7 +783,7 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
             else drain_records();
         };
 
-        unsigned mark = tail;  // FS: queue position behind the last record of the previous tile
+        unsigned mark = tail;  // ENTRY: queue position behind the last record of the previous tile
         for (int t = 0; t < ntiles; ++t) {
             const unsigned gti = gt + (unsigned)t;
             const int s = (int)(gti % STAGES);
@@ -879,17 +860,17 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
                 if (v < G) pm &= 0xffffffffu << (NB - v * HPT);
                 const unsigned vote = __ballot_sync(full, pm != 0u);
                 if (vote) {
-                    if constexpr (ENTRY) push_entries(pm, FS ? (unsigned)(s * TILE + p) : (unsigned)(first - begin) + (unsigned)p);
+                    if constexpr (ENTRY) push_entries(pm, (unsigned)(s * TILE + p));
                     else push_records(vote, pm, (unsigned)(first - begin) + (unsigned)p);
                 }
             }
-            if constexpr (FS) {
+            if constexpr (ENTRY) {
                 // the stage of tile t - 1 is refilled next: records that still point into it go first (never the case in
                 // the survivor-rich regime - a tile leaves < 32 records behind and they are its own)
                 while ((int)(mark - head) > 0) drain();
                 mark = tail;
             }
-            // every lane is done with the stage: refill it (FS: the previous tile's) with the tile AHEAD tiles on
+            // every lane is done with the stage: refill it (ENTRY: the previous tile's) with the tile AHEAD tiles on
             __syncwarp();
             if (lane == 0 && t + AHEAD < ntiles) issue(t + AHEAD);
         }
@@ -900,7 +881,7 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
 #pragma unroll
         for (int j = 0; j < HPT; ++j) {
             const long long hyp = hyp_w + 32 * j + lane;
-            const int col = FS ? (lane ^ ((j & 1) << 4)) : lane;
+            const int col = ENTRY ? (lane ^ ((j & 1) << 4)) : lane;
             const unsigned cnt = ws.sacc[j][0][col];
             if (cnt) {  // only real hypotheses can have inliers
                 unsigned long long* dst = a.acc + (long long)pair * a.h + hyp;
@@ -927,8 +908,8 @@ k_score(const ScoreArgs a) {
     score_body<HPT, G, MODE>(a);
 }
 
-// AUTO variant, one launch: the pilot's verdict (k_pilot) picks the body.  Both bodies live in one kernel, so
-// no second (empty) launch is needed; the register budget is the larger of the two.
+// AUTO variant: the pilot's verdict (k_pilot, or the one riding on k_screen_pts64) picks the body.  Both bodies live
+// in one kernel; the register budget is the larger of the two.
 template <int HPT, int G, int SMODE>
 __global__ void __launch_bounds__(kScoreThreads, score_min_blocks(HPT)) k_score_auto(const ScoreArgs a, const ScoreArgs a_full) {
     chain_enter();

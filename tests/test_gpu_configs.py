@@ -105,7 +105,7 @@ def config3(engine):
 
 def test_config3_deterministic_and_variant_invariant(engine, config3):
     c = config3
-    for variant, hpt, group in [("screen", 2, 16), ("screen", 4, 8), ("full", 2, 16), ("screen32", 4, 8)]:
+    for variant, hpt, group in [("screen", 2, 16), ("full", 2, 16), ("screen32", 4, 8)]:
         engine.set_score_variant(variant, hpt, group)
         try:
             cnt, s1, s2, err = engine.score(THR, min_extra=10, aggregation="rms")

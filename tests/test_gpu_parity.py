@@ -15,7 +15,7 @@ import pytest
 
 from oracle import csed
 from oracle import restatement as o
-from structure_from_motion_b200 import two_view
+from structure_from_motion_b200 import _native, two_view
 from structure_from_motion_b200.scenes import make_scene
 from test_gpu_score_range import check_against_oracle
 
@@ -60,10 +60,7 @@ def test_sampler_table_roundtrip(engine):
     assert counts.min() > 20 and counts.max() < 130
 
 
-@pytest.mark.parametrize("variant,hpt,group", [("screen", 2, 16), ("screen", 4, 8), ("screen", 1, 32), ("screen", 2, 8),
-                                               ("screen", 4, 4), ("screen", 4, 2), ("screen", 2, 4), ("screen", 1, 16),
-                                               ("full", 4, 8), ("full", 2, 16), ("full", 1, 32),
-                                               ("screen32", 4, 8), ("screen32", 8, 4), ("screen32", 2, 16)])
+@pytest.mark.parametrize("variant,hpt,group", [("screen", 2, 16), ("full", 2, 16), ("screen32", 4, 8), ("screen32", 2, 16)])
 def test_scorer_bit_exact_against_oracle(engine, variant, hpt, group):
     """K2+K3 with oracle-supplied E's: counts equal, sums within 1e-12 (different summation order)."""
     n, h = 3003, 700  # 3003 = 23 tiles + 59: partial last tile, partial last batch for every group size
@@ -142,10 +139,10 @@ def test_screen_never_drops_an_inlier(engine, thr, escale, variant):
 
 
 @pytest.mark.parametrize("thr", [0.0, 1e-12, 1.5e-6, 1e-4, 1e-3, 0.03, 0.5, 40.0])
-@pytest.mark.parametrize("variant,hpt,group", [("full", 2, 16), ("full", 1, 32), ("full", 4, 8), ("auto", 2, 16), ("auto", 4, 8)])
+@pytest.mark.parametrize("variant,hpt,group", [("full", 2, 16), ("auto", 2, 16)])
 def test_two_sided_body_at_every_inlier_rate(engine, thr, variant, hpt, group):
-    """The two-sided body's survivor path (one ring entry per survivor, handed out in rounds; gathers from shared memory
-    for hpt <= 2) from no survivors at all to EVERY test surviving (32 rounds per batch, ring full): counts equal and sums
+    """The two-sided body's survivor path (one ring entry per survivor, handed out in rounds; gathers from shared memory)
+    from no survivors at all to EVERY test surviving (32 rounds per batch, ring full): counts equal and sums
     within 1e-12 of the exact oracle scorer; 1 500 correspondences = partial last tile and partial last batch."""
     n, h = 1500, 200
     K, x1, x2, *_ = make_scene(n, 0.3, seed=12)
@@ -168,6 +165,21 @@ def test_two_sided_body_at_every_inlier_rate(engine, thr, variant, hpt, group):
     np.testing.assert_allclose(s2, s2_o, rtol=1e-12, atol=0)
     if thr >= 40.0:
         assert cnt_o.mean() > 0.99 * (n - 8)  # (nearly) every correspondence is an inlier of every model
+
+
+def test_only_shapes_with_a_kernel_are_accepted(engine):
+    """K2 has kernels for fp64 2 x 16 and for the fp32 pre-filter at 4 x 8 and 2 x 16: set_score_variant refuses every
+    other shape with SFM_ERR_ARG (-1), and accepts the kept shapes and 0 / 0 (the current shape, or the variant's
+    default when switching to or from screen32)."""
+    try:
+        for variant, hpt, group in [("screen", 4, 8), ("full", 1, 32), ("auto", 4, 8), ("screen32", 8, 4)]:
+            with pytest.raises(_native.NativeError, match=r"sfm_set_score_variant -> -1:"):
+                engine.set_score_variant(variant, hpt, group)
+        for variant, hpt, group in [("screen", 2, 16), ("full", 2, 16), ("auto", 2, 16), ("screen32", 4, 8),
+                                    ("screen32", 2, 16), ("auto", 0, 0), ("screen32", 0, 0), ("full", 0, 0)]:
+            engine.set_score_variant(variant, hpt, group)
+    finally:
+        engine.set_score_variant("auto")
 
 
 @pytest.mark.parametrize("agg", ["sum", "square", "mean", "rms"])

@@ -188,14 +188,10 @@ def test_tile_screen_never_drops_an_inlier(engine, thr, escale):
         assert oracle[0].sum() > _sweep_oracle(1.0, thr)[0].sum()
 
 
-@pytest.mark.parametrize("variant,hpt,group,thr", [("screen", 1, 16, THR), ("screen", 1, 32, THR), ("screen", 2, 4, THR),
-                                                   ("screen", 2, 8, THR), ("screen", 2, 16, THR), ("screen", 4, 2, THR),
-                                                   ("screen", 4, 4, THR), ("screen", 4, 8, THR),
-                                                   ("screen", 2, 16, 1e-3), ("screen", 4, 8, 1e-3),
-                                                   ("auto", 2, 16, THR), ("auto", 2, 16, 1e-3),
-                                                   ("auto", 4, 8, THR), ("auto", 4, 8, 1e-3)])
+@pytest.mark.parametrize("variant,hpt,group,thr", [("screen", 2, 16, THR), ("screen", 2, 16, 1e-3),
+                                                   ("auto", 2, 16, THR), ("auto", 2, 16, 1e-3)])
 def test_every_tiled_shape_matches_exact_scorer(engine, variant, hpt, group, thr):
-    """Every shape of the 9-slot body (ScoreWarpSmemBox<HPT>: boxes and per-lane kappa in shared memory), and AUTO on
+    """The 9-slot body (ScoreWarpSmemBox<HPT>: boxes and per-lane kappa in shared memory), and AUTO on
     either side of its pilot's decision (1.5e-6: the 9-slot body; 1e-3: the two-sided one), against the exact oracle:
     72 573 records (a partial last tile) and 300 hypotheses (not a multiple of 32 HPT), with K3 and the K4 mask."""
     n, h = SORT_MIN + 7_037, 300

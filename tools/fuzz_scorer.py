@@ -20,8 +20,7 @@ for k in range(cases):
     h = int(rng.choice([1, 2, 31, 32, 33, 63, 64, 65, 129, 1000, 4097]))
     thr = float(10.0 ** rng.uniform(-9, 1))
     frac = float(rng.choice([0.0, 0.1, 0.4, 0.9]))
-    variant, hpt, g = [("screen", 2, 16), ("screen", 1, 32), ("screen", 4, 8), ("full", 2, 16), ("screen32", 4, 8),
-                       ("auto", 2, 16), ("full", 1, 32), ("full", 4, 8), ("auto", 4, 8)][k % 9]
+    variant, hpt, g = [("screen", 2, 16), ("full", 2, 16), ("screen32", 4, 8), ("auto", 2, 16), ("screen32", 2, 16)][k % 5]
     agg = ["rms", "sum", "mean", "square"][k % 4]
     K, x1, x2, *_ = make_scene(n, frac, seed=100 + k)
     nxa, nya = o.k_normalise(x1[:, 0], x1[:, 1], K)

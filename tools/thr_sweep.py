@@ -23,8 +23,6 @@ for thr in thrs:
     shapes = (("auto", 2, 16), ("screen", 2, 16), ("full", 2, 16), ("screen32", 4, 8))
     if "--cliff" in sys.argv:
         shapes = (("auto", 2, 16), ("full", 2, 16))
-    if "--shapes" in sys.argv:
-        shapes = (("screen", 1, 32), ("screen", 2, 16), ("screen", 4, 8), ("full", 1, 32), ("full", 4, 8))
     for v, hpt, g in shapes:
         eng.set_score_variant(v, hpt, g)
         ts = []

@@ -14,7 +14,7 @@ eng.upload_pairs(x1, x2, K)
 eng.sample_device(0, h)
 eng.fit(want_E=False)
 eng.enable_timing(True)
-cfgs = [("screen32", 4, 8), ("screen32", 8, 4), ("screen32", 2, 16), ("screen", 2, 16), ("screen", 4, 8), ("screen", 1, 32), ("screen", 2, 8), ("screen", 4, 4), ("screen", 4, 2), ("screen", 2, 4), ("full", 4, 8), ("full", 2, 16)]
+cfgs = [("screen32", 4, 8), ("screen32", 2, 16), ("screen", 2, 16), ("full", 2, 16), ("auto", 2, 16)]
 if len(sys.argv) > 2:
     cfgs = [tuple([sys.argv[2], int(sys.argv[3]), int(sys.argv[4])])]
 for thr in (1.5e-6, 1.5e-8, 1e-30):
