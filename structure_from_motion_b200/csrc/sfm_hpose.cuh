@@ -16,7 +16,7 @@
 #pragma once
 #include "sfm_device.cuh"
 #include "sfm_linalg.cuh"
-#include "sfm_pose.cuh"
+#include "sfm_types.h"
 
 namespace sfm {
 

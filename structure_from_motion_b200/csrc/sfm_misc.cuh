@@ -1,7 +1,6 @@
 // Small utility kernels: FP64 peak probe (the tail's compaction lives in sfm_tail.cuh).
 #pragma once
 #include "sfm_device.cuh"
-#include "sfm_score.cuh"
 
 namespace sfm {
 

@@ -39,8 +39,8 @@
 // without a round trip.
 #pragma once
 #include "sfm_device.cuh"
-#include "sfm_score.cuh"
-#include "sfm_pose.cuh"
+#include "sfm_pose_math.cuh"
+#include "sfm_types.h"
 
 namespace sfm {
 

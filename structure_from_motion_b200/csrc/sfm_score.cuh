@@ -3,6 +3,7 @@
 #include <type_traits>
 
 #include "sfm_device.cuh"
+#include "sfm_types.h"
 
 namespace sfm {
 
@@ -73,7 +74,7 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
 //   SCREEN (default), 9 FP64 issue slots per evaluation.  sed <= thr implies
 //   r^2 <= thr * nb  (drop the image-A term), nb = lb0^2 + lb1^2, lb = E^T b, r = lb . a.
 //   nb depends on the image-B point only.  K2 streams its own copy of a single pair's correspondences,
-//   sorted by a Morton key of (xb, yb) at upload (k2_order_*, sfm_api.cu: k2_order), and every tile of kTile
+//   sorted by a Morton key of (xb, yb) at upload (k2_order_*, sfm_ransac.cu: k2_order), and every tile of kTile
 //   records comes with the box of its B points: centre (cx, cy), half-widths (wx, wy) with
 //   |xb - cx| <= wx and |yb - cy| <= wy for every record of the tile.  Once per (tile, hypothesis):
 //       l_i = lb_i(cx, cy),  m_i = |l_i| + |E_0i| wx + |E_1i| wy  (i = 0, 1)      (8 DFMA)
@@ -103,7 +104,7 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
 //   with three fresh 64-bit register operands issues at 2/3 rate on sm_100, measured by
 //   tools/fp64_micro.cu).
 //   SCREEN11: the 11-slot one-sided screen for uploads without the sorted copy (batches, short pairs: their boxes
-//   are wide, see k2_order in sfm_api.cu).  With s = sqrt(thr'), E has columns 0 and 1 pre-multiplied by s and the
+//   are wide, see k2_order in sfm_ransac.cu).  With s = sqrt(thr'), E has columns 0 and 1 pre-multiplied by s and the
 //   records are a copy with (xa, ya) pre-divided by s (k_screen_pts64), so that
 //       lb0' = s lb0, lb1' = s lb1, lb2 (6 DFMA)   r (2 DFMA)   m = lb1'^2 + kappa; m = lb0'^2 + m (2)   d = r^2 - m (1)
 //   with the same thr' and kappa ((a) above covers it: its nb is the computed one).
@@ -932,20 +933,6 @@ __global__ void __launch_bounds__(kScoreThreads, score_min_blocks(HPT)) k_score_
 enum { AGG_SUM = 0, AGG_SQUARE = 1, AGG_MEAN = 2, AGG_RMS = 3 };
 enum { SELECT_MIN_ERROR = 0, SELECT_MAX_INLIERS = 1, SELECT_MSAC = 2 };
 
-struct Best {
-    double err;
-    long long idx;
-    int count;
-    int pad;
-};
-
-struct SelectRecord {
-    Best best;
-    long long num_invalid, first_invalid;
-    double E[9];
-    int32_t sample[8];  // the winner's minimal sample (its table row; ransac.py:63), -1 without a table or a winner
-};
-
 __device__ __forceinline__ bool better(const Best& x, const Best& y, int mode) {
     // is x better than y ?
     if (y.idx < 0) return x.idx >= 0;
@@ -1050,10 +1037,6 @@ struct FinalArgs {
     unsigned* fitflag;             // K1's ambiguous-sample counter: reset here for the next fit (may be null)
 };
 
-// The model K3 selects among: the essential matrix (8-point samples, SED in K-normalised coordinates) or the homography
-// (4-point samples, symmetric transfer error in pixels; sfm_homography.cuh).  The kind fixes the sample size and the
-// exact scorer of the sample rule and of the rescore; the selection rule itself is the same.
-enum { MODEL_E = 0, MODEL_H = 1 };
 template <int KIND> struct ExactModel;
 template <> struct ExactModel<MODEL_E> {
     static constexpr int kSample = 8;

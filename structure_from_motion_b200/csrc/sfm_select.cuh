@@ -13,6 +13,7 @@
 // __fma_rn; the oracle evaluates the same order with fma() under -ffp-contract=off.
 #pragma once
 #include "sfm_device.cuh"
+#include "sfm_types.h"
 
 namespace sfm {
 
@@ -28,12 +29,6 @@ struct ModelScores {
     unsigned long long fixed_e, fixed_h;
     long long count_e, count_h;
     int model, reserved;
-};
-
-// the models of one pair, row-major; a model not given is never read
-struct SelectModels {
-    double E[9], H[9], K[9];
-    int have_e, have_h;
 };
 
 constexpr int kSelectStateWords = 8;  // per pair: fixed_e, fixed_h, count_e, count_h, ticket, 3 unused

@@ -16,8 +16,8 @@
 #pragma once
 #include "sfm_device.cuh"
 #include "sfm_hpose.cuh"
-#include "sfm_pose.cuh"
-#include "sfm_score.cuh"
+#include "sfm_pose_math.cuh"
+#include "sfm_types.h"
 
 namespace sfm {
 

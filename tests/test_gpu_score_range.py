@@ -14,7 +14,7 @@ from oracle import restatement as o
 from structure_from_motion_b200.scenes import make_scene
 
 pytestmark = pytest.mark.gpu
-SORT_MIN = 65_536  # kK2SortMin in csrc/sfm_api.cu: single pairs from here on get the 9-slot screen
+SORT_MIN = 65_536  # kK2SortMin in csrc/sfm_ransac.cu: single pairs from here on get the 9-slot screen
 SIZES = {"11-slot": 3_003, "9-slot": SORT_MIN + 7_000}
 VARIANTS = ("screen", "full", "screen32", "auto")
 THRS = (0.0, 1.5e-6, 1e-3, 0.5)  # at 1e-3 AUTO picks the two-sided body

@@ -16,7 +16,7 @@ from test_gpu_score_range import check_against_oracle
 pytestmark = pytest.mark.gpu
 THR = 1.5e-6
 IDENT = np.eye(3)
-SORT_MIN = 65_536  # kK2SortMin in csrc/sfm_api.cu
+SORT_MIN = 65_536  # kK2SortMin in csrc/sfm_ransac.cu
 
 
 def _norm(K, x1, x2):

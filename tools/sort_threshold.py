@@ -1,5 +1,5 @@
 """One upload plus one estimate (device sampler, fit, K2, K3, tail) of a single pair, against the pair size: the cost
-the upload-time sort of K2's copy adds (kK2SortMin in csrc/sfm_api.cu) against what the 9-slot screen saves.  Run it in
+the upload-time sort of K2's copy adds (kK2SortMin in csrc/sfm_ransac.cu) against what the 9-slot screen saves.  Run it in
 two trees and compare; prints the median wall time of 20 calls per (N, H) after 3 warm-up calls."""
 import os
 import sys
