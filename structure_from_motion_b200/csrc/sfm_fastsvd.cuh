@@ -5,7 +5,8 @@
 //
 //   null_vector4_fast   right singular vector of the smallest singular value of a 4x4 matrix (the DLT system of
 //                       lib/epipolar/triangulation.py:34-35): Householder QR, then inverse iteration on R^T R through
-//                       the triangular factor (never forming A^T A, so the accuracy is that of an SVD: eps * cond(A)).
+//                       the triangular factor (never forming A^T A: backward stable like an SVD, but the absolute stop
+//                       below adds up to ~8e-13 q / (1 - q), q = (sigma4 / sigma3)^4, to the eps * sigma1 / gap of one).
 //                       Convergence is checked; the caller falls back to the Jacobi SVD when 40 steps do not suffice
 //                       (sigma4 close to sigma3: a correspondence whose rays do not meet - never an inlier).
 //   svd3_rank2_frames   U, V of a 3x3 matrix with a (numerically) zero third singular value - what
@@ -209,7 +210,11 @@ __host__ __device__ inline bool svd3_rank2_frames(const double (&A)[9], double (
         U[3 * i] = u0[i]; U[3 * i + 1] = u1[i]; U[3 * i + 2] = u2[i];
         V[3 * i] = va[i]; V[3 * i + 1] = vb[i]; V[3 * i + 2] = v3[i];
     }
-    sv[0] = s0; sv[1] = s1; sv[2] = s2;
+    // the reported sigma3: |A v3| is the null vector's residual of two rows only - for A of rank 3 it overstates
+    // sigma3 by up to sqrt(3) (|A v3| = |det A| / |r_i x r_j| with |r_i x r_j| >= s0 s1 / sqrt(3)).  Its component
+    // along u2, normal to A p and A q, is |det A| / |A p x A q| = sigma3 to rounding (|A p x A q| = s0 s1 up to
+    // O(sigma3^2)), which is what the caller's absolute test against 1e-8 needs
+    sv[0] = s0; sv[1] = s1; sv[2] = fabs(dot3(u2, av3));
     return true;
 }
 

@@ -93,6 +93,8 @@ struct sfm_ctx {
     bool acc_clean = false;  // K2's accumulators (+ tail words) are zero: the fit kernel cleared them
     size_t acc_planes_for = 0;  // hypotheses (all pairs) the cleared accumulators were laid out for
     double Kstage[9] = {0};
+    double Estage[9] = {0};   // caller's E (stand-alone decomposition / pose), prescaled
+    double Pstage[24] = {0};  // caller's P1, P2 (stand-alone triangulation), prescaled
     double hstage[18] = {0};  // H and K of sfm_decompose_homography, K of the homography tail, staged for async copies
     std::vector<sfm::SelectModels> sstage;  // the models of sfm_score_models / sfm_batch_score_models, staged for the async copy
     std::vector<double> Kbatch;        // the cameras of the current batched upload, [P][9] (the device copy is Ks)

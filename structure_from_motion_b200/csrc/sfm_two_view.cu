@@ -26,16 +26,38 @@ int sfm_get_refinement(sfm_ctx* c, sfm_refinement* out, int64_t P) {
 }
 
 // ---- pose + triangulation ---------------------------------------------------------------
+// Caller-supplied E, P1 and P2 may have any scale, but the decomposition and the DLT square their entries (twice, in
+// the cross products of svd3_rank2_frames) and leave the double range from about 2^+-250 on.  Their answers do not
+// depend on the scale: the frames of E and 2^k E are the same, as is the null vector of 2^k A.  So the stand-alone
+// calls bring an input whose largest finite magnitude lies outside [2^-100, 2^100] to [0.5, 1) by a power of two - exact,
+// and no bit changes inside that range - and undo it on the singular values.  Returns the exponent applied (0 = none).
+static int prescale_exponent(const double* a, int n) {
+    double big = 0.0;
+    for (int i = 0; i < n; ++i)
+        if (std::isfinite(a[i])) big = std::fmax(big, std::fabs(a[i]));
+    if (big == 0.0 || (big >= 0x1p-100 && big <= 0x1p100)) return 0;
+    int e = 0;
+    std::frexp(big, &e);  // big = f 2^e, f in [0.5, 1)
+    return -e;
+}
+
+static void prescaled(const double* a, int n, int k, double* out) {
+    for (int i = 0; i < n; ++i) out[i] = std::ldexp(a[i], k);
+}
+
 int sfm_decompose_essential(sfm_ctx* c, const double* E, sfm_poses* out) {
     if (int r = use(c)) return r;
     if (!E || !out) return fail(SFM_ERR_ARG, "null argument");
     if (int r = c->tmp.reserve(72)) return r;
     if (int r = c->poses.reserve(sizeof(PoseSet))) return r;
-    CU(cudaMemcpyAsync(c->tmp.p, E, 72, cudaMemcpyHostToDevice, c->stream));
+    const int k = prescale_exponent(E, 9);
+    prescaled(E, 9, k, c->Estage);  // staged in the context: the async copy must not read caller memory later
+    CU(cudaMemcpyAsync(c->tmp.p, c->Estage, 72, cudaMemcpyHostToDevice, c->stream));
     k_decompose<<<1, 32, 0, c->stream>>>(c->tmp.as<double>(), nullptr, 0, c->poses.as<PoseSet>(), 1);
     if (int r = check_launch(c, "k_decompose")) return r;
     CU(cudaMemcpyAsync(out, c->poses.p, sizeof(PoseSet), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
+    for (int i = 0; i < 3; ++i) out->sv[i] = std::ldexp(out->sv[i], -k);
     return 0;
 }
 
@@ -53,7 +75,9 @@ static int recover_pose_impl(sfm_ctx* c, const double* E, const double* K9, cons
     double* dK = dE + 9;
     double* draw = dK + 9;
     Corr* dpts = reinterpret_cast<Corr*>(((uintptr_t)(draw + 4 * m) + 31) & ~(uintptr_t)31);
-    CU(cudaMemcpyAsync(dE, E, 72, cudaMemcpyHostToDevice, c->stream));
+    const int k = prescale_exponent(E, 9);
+    prescaled(E, 9, k, c->Estage);
+    CU(cudaMemcpyAsync(dE, c->Estage, 72, cudaMemcpyHostToDevice, c->stream));
     k_decompose<<<1, 32, 0, c->stream>>>(dE, nullptr, 0, c->poses.as<PoseSet>(), 1);
     if (int r = check_launch(c, "k_decompose")) return r;
     if (m > 0) {
@@ -76,6 +100,7 @@ static int recover_pose_impl(sfm_ctx* c, const double* E, const double* K9, cons
     CU(cudaMemcpyAsync(out, c->poses.p, sizeof(PoseSet), cudaMemcpyDeviceToHost, c->stream));
     if (pass4 && m > 0) CU(cudaMemcpyAsync(pass4, c->pass.p, (size_t)m, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
+    for (int i = 0; i < 3; ++i) out->sv[i] = std::ldexp(out->sv[i], -k);
     return 0;
 }
 
@@ -103,8 +128,12 @@ int sfm_triangulate(sfm_ctx* c, const double* P1, const double* P2, const double
     c->tic(T_TRI);
     double* dP = c->tmp.as<double>();
     double* draw = dP + 24;
-    CU(cudaMemcpyAsync(dP, P1, 96, cudaMemcpyHostToDevice, c->stream));
-    CU(cudaMemcpyAsync(dP + 12, P2, 96, cudaMemcpyHostToDevice, c->stream));
+    // one power of two for both cameras: the DLT system scales as a whole and its null vector does not change
+    double* Ps = c->Pstage;
+    memcpy(Ps, P1, 96);
+    memcpy(Ps + 12, P2, 96);
+    prescaled(Ps, 24, prescale_exponent(Ps, 24), Ps);
+    CU(cudaMemcpyAsync(dP, Ps, 192, cudaMemcpyHostToDevice, c->stream));
     const double* s[4];
     if (int r = stage_coords(c, draw, xa, ya, xb, yb, stride, m, s)) return r;
     k_triangulate<<<(unsigned)((m + 127) / 128), 128, 0, c->stream>>>(s[0], s[1], s[2], s[3], stride, m, nullptr, dP, dP + 12,

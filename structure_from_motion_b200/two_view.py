@@ -407,9 +407,29 @@ def _check_decomposition(p):
             "The smallest singular value of the Essential matrix is expected to be ~0")
 
 
+def _svd_refuses(*arrays):
+    """np.linalg.svd raises LinAlgError ("SVD did not converge") on a matrix with a NaN, which the device's SVDs would
+    turn into NaN results instead.  A NaN anywhere in E, in P1 / P2 or in a coordinate reaches the reference's SVD input
+    (eight_point.py:254, triangulation.py:34).  So does an infinite coordinate wherever the camera's third row has a
+    zero entry (inf * 0 = NaN in the DLT row): P1 = [I|0] of the cheirality test and K[I|0] of triangulate_points always
+    have one.  Against a third row without zeros the DLT row is infinite but NaN-free, and what numpy's SVD does with it
+    depends on the LAPACK build (tests/golden/pose_nonfinite_fixture.json records one such case); an infinite coordinate
+    is refused with LinAlgError there too, the reference's answer wherever it gives one.  An infinite entry of E or of a
+    camera gives no NaN: the reference goes on (E: EightPointCalculationError from the check of U; a camera: non-finite
+    points), and so does the device."""
+    for a, coords in arrays:
+        a = np.asarray(a, dtype=np.float64)
+        if np.isnan(a).any() or (coords and not np.isfinite(a).all()):
+            return np.linalg.LinAlgError("SVD did not converge")
+    return None
+
+
 def recover_all_r_t_arrays(e, engine=None):
     """_recover_all_r_t (lib/epipolar/eight_point.py:245-280) -> (R1, R2, t1)."""
     eng = engine or _native.get_engine()
+    exc = _svd_refuses((e, False))
+    if exc is not None:
+        raise exc
     p = eng.decompose_essential(e)
     _check_decomposition(p)
     R = np.array(p.R, dtype=np.float64).reshape(4, 3, 3)
@@ -426,6 +446,11 @@ def recover_pose_arrays(e, pts_a, pts_b, distance_threshold=None, engine=None, c
     eng = engine or _native.get_engine()
     na = np.ascontiguousarray(pts_a, dtype=np.float64).reshape(-1, 2)
     nb = np.ascontiguousarray(pts_b, dtype=np.float64).reshape(-1, 2)
+    exc = _svd_refuses((e, False), (na, True), (nb, True))
+    if exc is not None:
+        # the reference decomposes E before it triangulates a point (eight_point.py:207): its errors come first
+        recover_all_r_t_arrays(e, engine=eng)
+        raise exc
     p, pass4 = eng.recover_pose(e, na, nb, distance_threshold, camera_matrix=camera_matrix)
     _check_decomposition(p)
     counts = np.array(p.counts, dtype=np.int64)
@@ -442,6 +467,9 @@ def recover_pose_arrays(e, pts_a, pts_b, distance_threshold=None, engine=None, c
 def triangulate_arrays(pts_a, pts_b, P1, P2, engine=None) -> np.ndarray:
     """triangulate_point_correspondence over arrays (lib/epipolar/triangulation.py:9-39)."""
     eng = engine or _native.get_engine()
+    exc = _svd_refuses((np.asarray(P1)[:3], False), (np.asarray(P2)[:3], False), (pts_a, True), (pts_b, True))
+    if exc is not None:
+        raise exc
     return eng.triangulate(P1, P2, pts_a, pts_b)
 
 

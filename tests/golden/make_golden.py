@@ -427,9 +427,87 @@ def nonfinite_golden():
     dump("nonfinite_sample_fixture.json", dict(K=K, eight_point=eight, ransac=ransac))
 
 
+def pose_nonfinite_golden():
+    """What the reference's pose functions do with a NaN or an infinity in E, in one correspondence, or in P1 / P2:
+    _recover_all_r_t (eight_point.py:245-280), _recover_r_t (:181-242, normalised coordinates) and
+    triangulate_point_correspondence (triangulation.py:9-39) applied to every correspondence.  Recorded: the
+    exception's type and message, or the result (R, t and passing indices; the points)."""
+    rng = np.random.default_rng(11)
+    R = np.array([[0.9950041652780258, -0.09983341664682815, 0.0], [0.09983341664682815, 0.9950041652780258, 0.0],
+                  [0.0, 0.0, 1.0]])
+    t = np.array([1.0, 0.2, 0.1])
+    X = np.stack([rng.uniform(-1, 1, 6), rng.uniform(-1, 1, 6), rng.uniform(2, 8, 6)], 1)
+    na = X[:, :2] / X[:, 2:3]
+    Xb = X @ R.T + t
+    nb = Xb[:, :2] / Xb[:, 2:3]
+    tx = np.array([[0, -t[2], t[1]], [t[2], 0, -t[0]], [-t[1], t[0], 0]])
+    E = tx @ R
+    P1 = np.eye(4)[:3]
+    P2 = np.hstack([R, t[:, None]])
+
+    def outcome(call):
+        try:
+            out = call()
+        except Exception as exc:
+            return dict(raises=type(exc).__module__ + "." + type(exc).__qualname__, message=str(exc), result=None)
+        return dict(raises=None, message=None, result=out)
+
+    def feats(a):
+        return [F(x=float(p[0]), y=float(p[1])) for p in a]
+
+    def recover_all(e):
+        R1, R2, t1 = ref.eight_point._recover_all_r_t(e.copy())
+        return dict(R1=R1, R2=R2, t1=t1)
+
+    def recover(e, a, b):
+        Rr, tr, idx = ref.eight_point._recover_r_t(feats(a), feats(b), e.copy())
+        return dict(R=Rr, t=tr, passing=[int(i) for i in idx])
+
+    def triangulate(a, b, p1, p2):
+        return [ref.triangulation.triangulate_point_correspondence(fa, fb, p1, p2)
+                for fa, fb in zip(feats(a), feats(b))]
+
+    cases = []
+    for val, vname in ((np.nan, "nan"), (np.inf, "inf"), (-np.inf, "-inf")):
+        e = E.copy()
+        e[1, 2] = val
+        cases.append(dict(name=f"E_{vname}", call="recover_all_r_t", E=e, **outcome(lambda: recover_all(e))))
+        cases.append(dict(name=f"E_{vname}", call="recover_r_t", E=e, pts_a=na, pts_b=nb,
+                          **outcome(lambda: recover(e, na, nb))))
+        for side, col in (("a", 0), ("b", 1)):
+            a, b = na.copy(), nb.copy()
+            (a if side == "a" else b)[2, col] = val
+            cases.append(dict(name=f"pts_{side}_{vname}", call="recover_r_t", E=E, pts_a=a, pts_b=b,
+                              **outcome(lambda: recover(E, a, b))))
+            cases.append(dict(name=f"pts_{side}_{vname}", call="triangulate", P1=P1, P2=P2, pts_a=a, pts_b=b,
+                              **outcome(lambda: triangulate(a, b, P1, P2))))
+        for which in ("P1", "P2"):
+            p1, p2 = P1.copy(), P2.copy()
+            (p1 if which == "P1" else p2)[1, 3] = val
+            cases.append(dict(name=f"{which}_{vname}", call="triangulate", P1=p1, P2=p2, pts_a=na, pts_b=nb,
+                              **outcome(lambda: triangulate(na, nb, p1, p2))))
+    # an infinite coordinate against a camera whose third row has no zero: the DLT row is infinite, NaN-free
+    Rg = np.array([[0.936, -0.28, 0.2136], [0.3104, 0.9464, -0.0896], [-0.1770, 0.1608, 0.9710]])
+    Pg = np.hstack([Rg, np.array([[1.0], [0.2], [0.1]])])
+    a, b = na.copy(), nb.copy()
+    b[2, 1] = np.inf
+    cases.append(dict(name="pts_b_inf_generic_camera", call="triangulate", P1=P1, P2=Pg, pts_a=a, pts_b=b,
+                      **outcome(lambda: triangulate(a, b, P1, Pg))))
+    # E of rank 3 with a NaN coordinate: the decomposition's error comes before any point is triangulated
+    e3 = E.copy()
+    e3[2, 2] += 0.5
+    a = na.copy()
+    a[1, 0] = np.nan
+    cases.append(dict(name="E_rank3_pts_a_nan", call="recover_r_t", E=e3, pts_a=a, pts_b=nb,
+                      **outcome(lambda: recover(e3, a, nb))))
+    dump("pose_nonfinite_fixture.json", dict(cases=cases))
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "nonfinite":
         nonfinite_golden()
+    elif len(sys.argv) > 1 and sys.argv[1] == "pose_nonfinite":
+        pose_nonfinite_golden()
     elif len(sys.argv) > 1 and sys.argv[1] == "front_end":
         front_end_golden()
     elif len(sys.argv) > 1 and sys.argv[1] == "harris":
