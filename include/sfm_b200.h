@@ -197,6 +197,34 @@ int sfm_ransac_homography(sfm_ctx *ctx, double threshold, double min_extra, int 
  * last sfm_ransac_homography when H is NULL.  mask uint8[n], err double[n]; either may be NULL. */
 int sfm_homography_mask(sfm_ctx *ctx, const double *H, double threshold, uint8_t *mask, double *err);
 
+/* ---- absolute pose of a new view (PnP) ---------------------------------------------------
+ * Records: n world points X (double[n][3]) and their observed pixels x (double[n][2]) in the new image, with its K
+ * (double[9], row-major): finite, non-singular, upper triangular with K[2,2] = 1, else SFM_ERR_ARG.  The model is
+ * [R | t] (double[12], row-major 3 x 4, x_cam = R X + t); P = K [R | t] and p = P (X, 1) are formed in the pinned order
+ * of csrc/sfm_pnp.cuh.  A record is an inlier iff p2 > 0 && F <= thr p2^2 with F = (p0 - u p2)^2 + (p1 - v p2)^2; its
+ * value is the squared reprojection error F / p2^2 in px^2.  The minimal solver is P3P (Lambda Twist) on columns 0-2
+ * of a sample, with column 3 choosing among the solutions (smallest error at point 3).  A sample with a non-finite
+ * coordinate, three collinear world points, no solution with three positive depths or a non-finite pose is invalid:
+ * never a candidate, counted in sfm_best.num_invalid / first_invalid. */
+/* Replace the context's records with PnP records: the essential-matrix and homography calls refuse until the next
+ * sfm_upload_pairs.  Then load a sample table or call the device sampler (columns 0-3 are the sample). */
+int sfm_upload_pnp(sfm_ctx *ctx, const double *X, const double *x, int64_t n, const double *K);
+/* The P3P fit of every row of the current table or device draw.  Rt_out double[h][12] (zeros for an invalid sample)
+ * or NULL; valid_out uint8[h] or NULL. */
+int sfm_fit_pnp(sfm_ctx *ctx, double *Rt_out, uint8_t *valid_out);
+/* RANSAC absolute pose in one call: fit -> score -> select (fit_with_ransac with 4-point samples: samples never counted,
+ * always in the error; the aggregation and selection rules of sfm_score) -> mask of the winner.  Needs n >= 8.
+ * best->E is unused (zeros); Rt (double[12], may be NULL) receives the winner, zeros without one.  Optional (NULL =
+ * not wanted): mask uint8[n] / err double[n] = decision / reprojection error under the winner; count_extra_h
+ * int32[h] (-1 = invalid), err_h double[h] (+inf = not a candidate).  sfm_near_ties works afterwards. */
+int sfm_ransac_pnp(sfm_ctx *ctx, double threshold, double min_extra, int aggregation, int selection, sfm_best *best,
+                   double *Rt, uint8_t *mask, double *err, int32_t *count_extra_h, double *err_h);
+/* Decision and reprojection error of every record under Rt (double[12]), or under the winner of the last
+ * sfm_ransac_pnp when Rt is NULL.  mask uint8[n], err double[n]; either may be NULL. */
+int sfm_pnp_mask(sfm_ctx *ctx, const double *Rt, double threshold, uint8_t *mask, double *err);
+/* Poses [first, first + count) of the last PnP fit: Rt_out double[count][12], valid_out uint8[count]; either may be NULL. */
+int sfm_get_pnp_models(sfm_ctx *ctx, int64_t first, int64_t count, double *Rt_out, uint8_t *valid_out);
+
 /* ---- pose + triangulation ------------------------------------------------------------ */
 typedef struct sfm_poses {
     double R[4][9];      /* (R1,t) (R1,-t) (R2,t) (R2,-t)  — eight_point.py:210-212 order */

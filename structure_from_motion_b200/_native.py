@@ -94,6 +94,11 @@ _SIGNATURES = {
     "sfm_fit_homography": (C.c_int, [_P, _P, _P]),
     "sfm_ransac_homography": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.POINTER(Best), _P, _P, _P, _P]),
     "sfm_homography_mask": (C.c_int, [_P, _P, C.c_double, _P, _P]),
+    "sfm_upload_pnp": (C.c_int, [_P, _P, _P, C.c_int64, _P]),
+    "sfm_fit_pnp": (C.c_int, [_P, _P, _P]),
+    "sfm_ransac_pnp": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.POINTER(Best), _P, _P, _P, _P, _P]),
+    "sfm_pnp_mask": (C.c_int, [_P, _P, C.c_double, _P, _P]),
+    "sfm_get_pnp_models": (C.c_int, [_P, C.c_int64, C.c_int64, _P, _P]),
     "sfm_decompose_essential": (C.c_int, [_P, _P, C.POINTER(Poses)]),
     "sfm_recover_pose": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_int64, C.c_int64, C.c_double, C.POINTER(Poses), _P]),
     "sfm_recover_pose_pixels": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int64, C.c_int64, C.c_double,
@@ -480,6 +485,56 @@ class Engine:
                                                   _ptr(mask), _ptr(err)), "sfm_two_view_homography")
         m = min(int(num.value), cap)
         return b, mask, err, p, int(num.value), idx[:m], ok[:m], X[:m]
+
+    # -- absolute pose (PnP) ------------------------------------------------------------------
+    def upload_pnp(self, points_3d, pts, K):
+        """points_3d [n,3] world points and pts [n,2] their pixels in the new view, K 3x3.  Replaces the current
+        upload: the essential-matrix and homography calls need a new upload_pairs afterwards."""
+        X = _f64(points_3d).reshape(-1, 3)
+        x = _f64(pts).reshape(-1, 2)
+        if X.shape[0] != x.shape[0]:
+            raise ValueError("points_3d and pts must have the same number of rows")
+        K = _f64(K).reshape(3, 3)
+        self._ck(self.lib.sfm_upload_pnp(self.h, _ptr(X), _ptr(x), X.shape[0], _ptr(K)), "sfm_upload_pnp")
+        self.n, self.batch_pairs = X.shape[0], 0
+
+    def fit_pnp(self):
+        """The P3P fit of every row of the current table / device draw -> ([R|t] [h,3,4], valid bool[h])."""
+        h = self.h_count
+        Rt = np.empty((h, 3, 4), dtype=np.float64)
+        valid = np.empty(h, dtype=np.uint8)
+        self._ck(self.lib.sfm_fit_pnp(self.h, _ptr(Rt), _ptr(valid)), "sfm_fit_pnp")
+        return Rt, valid.astype(bool)
+
+    def get_pnp_models(self, first=0, count=None):
+        count = self.h_count - first if count is None else int(count)
+        Rt = np.empty((count, 3, 4), dtype=np.float64)
+        valid = np.empty(count, dtype=np.uint8)
+        self._ck(self.lib.sfm_get_pnp_models(self.h, int(first), count, _ptr(Rt), _ptr(valid)), "sfm_get_pnp_models")
+        return Rt, valid.astype(bool)
+
+    def ransac_pnp(self, threshold, min_extra=0.0, aggregation="rms", selection="min_error", want_arrays=False):
+        """fit -> score -> select -> mask in one call.  Returns (best, [R|t] of the winner [3,4], mask uint8[n],
+        err[n], count_extra[h], err[h]); the per-hypothesis arrays are None unless want_arrays."""
+        b = Best()
+        Rt = np.empty((3, 4), dtype=np.float64)
+        mask = np.empty(self.n, dtype=np.uint8)
+        err = np.empty(self.n, dtype=np.float64)
+        cnt = np.empty(self.h_count, dtype=np.int32) if want_arrays else None
+        err_h = np.empty(self.h_count, dtype=np.float64) if want_arrays else None
+        self._ck(self.lib.sfm_ransac_pnp(self.h, float(threshold), float(min_extra), AGG[aggregation],
+                                         SELECT[selection], C.byref(b), _ptr(Rt), _ptr(mask), _ptr(err), _ptr(cnt),
+                                         _ptr(err_h)), "sfm_ransac_pnp")
+        return b, Rt, mask, err, cnt, err_h
+
+    def pnp_mask(self, Rt, threshold):
+        """(decision bool[n], squared reprojection error [n]) under [R|t] (3x4), or under the last estimate's winner
+        when Rt is None."""
+        Ra = None if Rt is None else _f64(Rt).reshape(12)
+        mask = np.empty(self.n, dtype=np.uint8)
+        err = np.empty(self.n, dtype=np.float64)
+        self._ck(self.lib.sfm_pnp_mask(self.h, _ptr(Ra), float(threshold), _ptr(mask), _ptr(err)), "sfm_pnp_mask")
+        return mask.astype(bool), err
 
     # -- essential matrix or homography -------------------------------------------------------
     def model_scores(self, E, H, K, sigma=1.0, homography_ratio=0.45, per_point=False):

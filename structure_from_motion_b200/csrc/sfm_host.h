@@ -1,8 +1,8 @@
 // Host side shared by the translation units of the C ABI: the context, device buffers, error reporting, launch helpers
 // and the few internal functions one stage calls in another.  Each stage file owns its kernel headers:
 //   sfm_api.cu          context lifecycle, stream, errors, timing               sfm_misc.cuh
-//   sfm_ransac.cu       upload, sampler, E and H fit, K2 and its shape, K3,     sfm_fit.cuh, sfm_score.cuh, sfm_homography.cuh
-//                       masks, batches, hypothesis-sharded scoring
+//   sfm_ransac.cu       upload, sampler, E, H and PnP fit, K2 and its shape,    sfm_fit.cuh, sfm_score.cuh, sfm_homography.cuh,
+//                       K3, masks, batches, hypothesis-sharded scoring          sfm_pnp.cuh
 //   sfm_two_view.cu     pose/triangulation list API, tail, refinement           sfm_pose.cuh, sfm_hpose.cuh, sfm_tail.cuh,
 //                                                                               sfm_refine.cuh
 //   sfm_model_select.cu essential matrix or homography                          sfm_select.cuh
@@ -79,6 +79,7 @@ struct sfm_ctx {
     sfm_host::Buf k2pts, k2box, k2sort;  // K2's copy of pts in image-B Morton order, its tile boxes, the sort's scratch
     sfm_host::Buf selstate, selio, selpp;  // k_score_models: self-cleaning sums; models and results; per-correspondence errors
     sfm_host::Buf refstate, refpart, reftick, refrec, refrep;  // refinement: LM state, chunk partials, tickets, records, reports
+    sfm_host::Buf ppts, pK, pmodels, pwin;  // PnP: records (PnpRec), K, poses [h][12], the winner or a caller's pose [12]
     long long n = 0, h = 0, npairs = 1;
     long long first_len = 0;  // batched: correspondences of the first pair (what the AUTO pilot samples)
     long long batch_max_len = 0;  // batched: correspondences of the longest pair
@@ -87,6 +88,9 @@ struct sfm_ctx {
     bool models_h = false;       // the current models are homographies (sfm_fit_homography), not essential matrices
     bool k2_ready = false;       // k2pts / k2box belong to the current upload (K-normalised records only)
     int hscore_occ = 0;          // resident blocks per SM of k_score_homography (queried once)
+    bool has_pnp = false;        // the upload holds PnP records (ppts), not correspondences: has_pts is false
+    bool pnp_models = false;     // pmodels holds the poses of the current table
+    int pscore_occ = 0;          // resident blocks per SM of k_score_pnp (queried once)
     bool table_pending = false;  // sfm_sample_device was called: the table is drawn by the fit kernel (or on demand)
     unsigned long long smp_seed = 0, smp_stream = 0;
     long long smp_offset = 0;

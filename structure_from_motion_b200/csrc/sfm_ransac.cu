@@ -1,6 +1,6 @@
-// The C ABI's RANSAC stages: correspondence upload and K2's sorted copy, the sample table, the essential-matrix and
-// homography fits (K1), scoring (K2), finalise + select (K3), inlier masks, the batched estimate and the
-// hypothesis-sharded score, merge and fetch.
+// The C ABI's RANSAC stages: correspondence upload and K2's sorted copy, the sample table, the essential-matrix,
+// homography and absolute-pose fits (K1), scoring (K2), finalise + select (K3), inlier masks, the batched estimate and
+// the hypothesis-sharded score, merge and fetch.
 #include <cmath>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -9,6 +9,7 @@
 #include "sfm_fit.cuh"
 #include "sfm_score.cuh"
 #include "sfm_homography.cuh"
+#include "sfm_pnp.cuh"
 
 using namespace sfm;
 using namespace sfm_host;
@@ -72,7 +73,7 @@ int sfm_set_score_variant(sfm_ctx* c, int variant, int hpt, int group) {
 int sfm_set_table(sfm_ctx* c, const int32_t* table, int64_t h) {
     if (int r = use(c)) return r;
     if (!table || h <= 0) return fail(SFM_ERR_ARG, "bad table");
-    if (!c->has_pts) return fail(SFM_ERR_STATE, "upload correspondences before the sample table");
+    if (!c->has_pts && !c->has_pnp) return fail(SFM_ERR_STATE, "upload correspondences before the sample table");
     for (int64_t i = 0; i < 8 * h; ++i)
         if (table[i] < 0 || table[i] >= c->n) return fail(SFM_ERR_ARG, "table[%lld] = %d out of range", (long long)i, table[i]);
     if (int r = c->table.reserve((size_t)h * 32)) return r;
@@ -91,7 +92,7 @@ int sfm_set_table(sfm_ctx* c, const int32_t* table, int64_t h) {
 // kernel (one launch less per estimate); anything else that needs the table first materialises it with k_sample.
 int sfm_host::sample_device(sfm_ctx* c, uint64_t seed, uint64_t stream, int64_t hyp_offset, int64_t h) {
     if (h <= 0) return fail(SFM_ERR_ARG, "need h > 0");
-    if (!c->has_pts) return fail(SFM_ERR_STATE, "upload correspondences before sampling");
+    if (!c->has_pts && !c->has_pnp) return fail(SFM_ERR_STATE, "upload correspondences before sampling");
     if (!c->batched && c->n < 8) return fail(SFM_ERR_ARG, "need at least 8 correspondences");
     if (int r = c->table.reserve((size_t)h * c->npairs * 32)) return r;
     c->smp_seed = seed;
@@ -266,6 +267,7 @@ static int upload_pairs_impl(sfm_ctx* c, const double* xa, const double* ya, con
     // the coordinate copies read caller memory: finish before returning unless the caller took that on (_async)
     if (sync) CU(cudaStreamSynchronize(c->stream));
     c->has_pts = true;
+    c->has_pnp = c->pnp_models = false;
     c->has_table = c->has_models = c->has_score = false;
     c->table_pending = false;
     c->winner_set = false;
@@ -447,9 +449,10 @@ static int finalise_launch(sfm_ctx* c, int kind, double thr, double min_extra, i
     const int fblocks = (int)((h + 255) / 256);
     c->tic(T_SELECT);
     FinalArgs f;
-    f.pts = c->pts.as<Corr>();
+    f.pts = kind == MODEL_P ? c->ppts.p : c->pts.p;
     f.offsets = c->batched ? c->offsets.as<long long>() : nullptr;
-    f.E = c->E.as<double>();
+    f.E = kind == MODEL_P ? c->pmodels.as<double>() : c->E.as<double>();
+    f.K = c->pK.as<double>();
     f.valid = c->valid.as<uint8_t>();
     f.table = use_table ? c->table.as<int32_t>() : nullptr;
     f.h = h;
@@ -481,6 +484,7 @@ static int finalise_launch(sfm_ctx* c, int kind, double thr, double min_extra, i
     f.record = c->record.as<SelectRecord>();
     f.fitflag = c->fitflag.as<unsigned>();
     if (kind == MODEL_H) CU(chain_launch(c, k_finalise<MODEL_H>, dim3((unsigned)fblocks, (unsigned)P), dim3(256), 0, f));
+    else if (kind == MODEL_P) CU(chain_launch(c, k_finalise<MODEL_P>, dim3((unsigned)fblocks, (unsigned)P), dim3(256), 0, f));
     else CU(chain_launch(c, k_finalise<MODEL_E>, dim3((unsigned)fblocks, (unsigned)P), dim3(256), 0, f));
     if (int r = check_launch(c, "k_finalise")) return r;
     c->toc(T_SELECT);
@@ -934,6 +938,182 @@ int sfm_homography_mask(sfm_ctx* c, const double* H, double thr, uint8_t* mask, 
     return 0;
 }
 
+// ---- absolute pose (sfm_pnp.cuh) --------------------------------------------------------------
+int sfm_upload_pnp(sfm_ctx* c, const double* X, const double* x, int64_t n, const double* K) {
+    if (int r = use(c)) return r;
+    if (!X || !x) return fail(SFM_ERR_ARG, "null argument");
+    if (n <= 0 || (uint64_t)n >= kMaxPoints) return fail(SFM_ERR_ARG, "need 0 < n < 2^25 records, got %lld", (long long)n);
+    if (int r = check_camera(K)) return r;
+    if (K[3] != 0.0 || K[6] != 0.0 || K[7] != 0.0 || K[8] != 1.0)
+        return fail(SFM_ERR_ARG, "the camera matrix must be upper triangular with K[2,2] = 1");
+    std::vector<PnpRec> rec((size_t)n);
+    for (int64_t i = 0; i < n; ++i)
+        rec[(size_t)i] = PnpRec{X[3 * i], X[3 * i + 1], X[3 * i + 2], x[2 * i], x[2 * i + 1], 0.0};
+    if (int r = c->ppts.reserve((size_t)n * sizeof(PnpRec))) return r;
+    if (int r = c->pK.reserve(72)) return r;
+    c->tic(T_UPLOAD);
+    CU(cudaMemcpyAsync(c->ppts.p, rec.data(), (size_t)n * sizeof(PnpRec), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(c->pK.p, K, 72, cudaMemcpyHostToDevice, c->stream));
+    c->toc(T_UPLOAD);
+    CU(cudaStreamSynchronize(c->stream));  // the copies read host memory
+    c->n = n;
+    c->batched = false;
+    c->npairs = 1;
+    c->has_pts = false;  // c->pts no longer describes the upload: the E and H calls refuse
+    c->has_pnp = true;
+    c->pnp_models = false;
+    c->has_table = c->has_models = c->has_score = false;
+    c->table_pending = false;
+    c->winner_set = false;
+    return 0;
+}
+
+// the P3P fits of the h rows of the table or the device draw; clears K2's accumulators as the other fits do
+static int fit_p_launch(sfm_ctx* c) {
+    if (!c->has_pnp || !c->has_table) return fail(SFM_ERR_STATE, "fit needs PnP records and a sample table");
+    const long long h = c->h;
+    if (int r = c->pmodels.reserve((size_t)h * 96)) return r;
+    if (int r = c->valid.reserve((size_t)h)) return r;
+    const size_t acc_tail = acc_tail_bytes(1);
+    if (int r = c->acc.reserve((size_t)h * kAccWords * 8 + acc_tail)) return r;
+    c->tic(T_FIT);
+    CU(chain_launch(c, k_fit_pnp, dim3((unsigned)((h + kFitPThreads - 1) / kFitPThreads)), dim3(kFitPThreads), 0,
+                    c->ppts.as<PnpRec>(), c->pK.as<double>(), c->table.as<int32_t>(), h, c->pmodels.as<double>(),
+                    c->valid.as<uint8_t>(), c->acc.as<unsigned long long>(), kAccWords, (int)((acc_tail + 7) / 8),
+                    c->table_pending ? 1 : 0, c->smp_seed, c->smp_stream, c->smp_offset, c->n));
+    if (int r = check_launch(c, "k_fit_pnp")) return r;
+    c->toc(T_FIT);
+    c->table_pending = false;
+    c->acc_clean = true;
+    c->acc_planes_for = (size_t)h;
+    c->pnp_models = true;
+    c->has_score = false;
+    return 0;
+}
+
+// K2 + K3 of the poses of the last fit
+static int score_p_launch(sfm_ctx* c, double thr, double min_extra, int agg, int mode) {
+    if (agg < 0 || agg > 3) return fail(SFM_ERR_ARG, "bad aggregation %d", agg);
+    if (mode < 0 || mode > 2) return fail(SFM_ERR_ARG, "bad selection %d", mode);
+    int sums = (agg == AGG_SUM || agg == AGG_MEAN) ? SUM_S1 : SUM_S2;
+    if (mode == SELECT_MSAC) sums |= SUM_S1;
+    // the threshold ranges of the E and H paths: below 0, NaN and above 1e100 the scorer is skipped and K3 rescores
+    const bool skip_k2 = !(thr >= 0.0) || thr > 1e100;
+    const int force_rescore = (thr > 1e100) ? 1 : 0;
+    const long long h = c->h, n = c->n;
+    // an inlier's value F / W can exceed thr by a few ulps (the decision is division-free), as on the H path
+    int e2 = 0;
+    if (thr > 0.0 && !skip_k2) (void)frexp(thr * (1.0 + 0x1p-20), &e2);
+    if (e2 < -400) e2 = -400;
+    if (int r = reserve_selection(c, h, 1)) return r;
+    if (int r = c->acc.reserve((size_t)h * kAccWords * 8 + acc_tail_bytes(1))) return r;
+    unsigned long long* acc = c->acc.as<unsigned long long>();
+    const size_t smem = kPScoreWarps * sizeof(PScoreWarpSmem);
+    if (!c->pscore_occ) {
+        int o = 0;
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, k_score_pnp<kPScoreHpt>, kPScoreThreads, smem));
+        c->pscore_occ = o > 0 ? o : 1;
+    }
+    const long long grid_blocks = (long long)c->sm_count * c->pscore_occ;
+    const long long hblocks = (h + 32ll * kPScoreHpt - 1) / (32ll * kPScoreHpt);
+    const ItemSplit sp = split_items(grid_blocks * kPScoreWarps * 32, hblocks, n, kPTile);
+    PScoreArgs a;
+    a.pts = c->ppts.as<PnpRec>();
+    a.K = c->pK.as<double>();
+    a.Rt = c->pmodels.as<double>();
+    a.n = n;
+    a.h = h;
+    a.thr = thr;
+    a.scale1 = ldexp(1.0, 63 - e2);
+    a.scale2 = ldexp(1.0, 63 - 2 * e2);
+    a.sums = sums;
+    a.chunk = sp.chunk;
+    a.hblocks = (int)hblocks;
+    a.nsplit = (int)sp.nsplit;
+    a.total_items = hblocks * sp.nsplit;
+    a.work_counter = reinterpret_cast<unsigned*>(acc + (size_t)h * kAccWords);
+    a.acc = acc;
+    c->tic(T_SCORE);
+    if (int r = clear_acc(c, (size_t)h, 1)) return r;
+    if (!skip_k2) {
+        const long long want = (a.total_items + kPScoreWarps - 1) / kPScoreWarps;
+        CU(chain_launch(c, k_score_pnp<kPScoreHpt>, dim3((unsigned)(grid_blocks < want ? grid_blocks : want)),
+                        dim3(kPScoreThreads), smem, a));
+        if (int r = check_launch(c, "k_score_pnp")) return r;
+    }
+    c->toc(T_SCORE);
+    return finalise_launch(c, MODEL_P, thr, min_extra, agg, mode, true, 0, sums, e2, force_rescore, acc);
+}
+
+// decision and value of every record under the pose at Rt_dev[12 * best->idx] (best != null) or at Rt_dev
+static int pmask_launch(sfm_ctx* c, double thr, const double* Rt_dev, const Best* best_dev, double* winner_out) {
+    if (int r = c->mask.reserve((size_t)c->n)) return r;
+    if (int r = c->sed.reserve((size_t)c->n * 8)) return r;
+    c->tic(T_MASK);
+    CU(chain_launch(c, k_pnp_mask, dim3((unsigned)((c->n + 255) / 256)), dim3(256), 0, c->ppts.as<PnpRec>(), c->n,
+                    c->pK.as<double>(), Rt_dev, best_dev, thr, c->mask.as<uint8_t>(), c->sed.as<double>(), winner_out));
+    if (int r = check_launch(c, "k_pnp_mask")) return r;
+    c->toc(T_MASK);
+    return 0;
+}
+
+int sfm_fit_pnp(sfm_ctx* c, double* Rt_out, uint8_t* valid_out) {
+    if (int r = use(c)) return r;
+    if (int r = fit_p_launch(c)) return r;
+    if (Rt_out) CU(cudaMemcpyAsync(Rt_out, c->pmodels.p, (size_t)c->h * 96, cudaMemcpyDeviceToHost, c->stream));
+    if (valid_out) CU(cudaMemcpyAsync(valid_out, c->valid.p, (size_t)c->h, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int sfm_get_pnp_models(sfm_ctx* c, int64_t first, int64_t count, double* Rt_out, uint8_t* valid_out) {
+    if (int r = use(c)) return r;
+    if (!c->has_pnp || !c->pnp_models || first < 0 || count < 0 || first + count > c->h)
+        return fail(SFM_ERR_STATE, "no poses [%lld, %lld)", (long long)first, (long long)(first + count));
+    if (Rt_out) CU(cudaMemcpyAsync(Rt_out, c->pmodels.as<double>() + 12 * first, (size_t)count * 96, cudaMemcpyDeviceToHost, c->stream));
+    if (valid_out) CU(cudaMemcpyAsync(valid_out, c->valid.as<uint8_t>() + first, (size_t)count, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int sfm_ransac_pnp(sfm_ctx* c, double thr, double min_extra, int agg, int mode, sfm_best* best, double* Rt,
+                   uint8_t* mask, double* err, int32_t* count_extra_h, double* err_h) {
+    if (int r = use(c)) return r;
+    if (!best) return fail(SFM_ERR_ARG, "best is null");
+    if (c->has_pnp && c->n < 8) return fail(SFM_ERR_ARG, "need at least 8 records, got %lld", c->n);
+    if (int r = c->pwin.reserve(96)) return r;
+    if (int r = fit_p_launch(c)) return r;
+    if (int r = score_p_launch(c, thr, min_extra, agg, mode)) return r;
+    // the mask kernel also copies the winner out of the poses (K3's record has no room for 12 doubles)
+    if (int r = pmask_launch(c, thr, c->pmodels.as<double>(), c->best.as<Best>(), c->pwin.as<double>())) return r;
+    if (mask) CU(cudaMemcpyAsync(mask, c->mask.p, (size_t)c->n, cudaMemcpyDeviceToHost, c->stream));
+    if (err) CU(cudaMemcpyAsync(err, c->sed.p, (size_t)c->n * 8, cudaMemcpyDeviceToHost, c->stream));
+    if (Rt) CU(cudaMemcpyAsync(Rt, c->pwin.p, 96, cudaMemcpyDeviceToHost, c->stream));
+    if (count_extra_h) CU(cudaMemcpyAsync(count_extra_h, c->count_extra.p, (size_t)c->h * 4, cudaMemcpyDeviceToHost, c->stream));
+    if (err_h) CU(cudaMemcpyAsync(err_h, c->err.p, (size_t)c->h * 8, cudaMemcpyDeviceToHost, c->stream));
+    return fetch_best(c, best);
+}
+
+int sfm_pnp_mask(sfm_ctx* c, const double* Rt, double thr, uint8_t* mask, double* err) {
+    if (int r = use(c)) return r;
+    if (!c->has_pnp) return fail(SFM_ERR_STATE, "no PnP records loaded");
+    const double* Rt_dev;
+    if (Rt) {
+        if (int r = c->pwin.reserve(96)) return r;
+        CU(cudaMemcpyAsync(c->pwin.p, Rt, 96, cudaMemcpyHostToDevice, c->stream));
+        Rt_dev = c->pwin.as<double>();
+    } else {
+        if (!c->pnp_models || !c->has_score || !c->winner_set || c->winner_local < 0)
+            return fail(SFM_ERR_STATE, "no pose winner: pass Rt or run sfm_ransac_pnp first");
+        Rt_dev = c->pmodels.as<double>() + 12 * c->winner_local;
+    }
+    if (int r = pmask_launch(c, thr, Rt_dev, nullptr, nullptr)) return r;
+    if (mask) CU(cudaMemcpyAsync(mask, c->mask.p, (size_t)c->n, cudaMemcpyDeviceToHost, c->stream));
+    if (err) CU(cudaMemcpyAsync(err, c->sed.p, (size_t)c->n * 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
 // ---- hypothesis-sharded runs without a host round trip (SURVEY.md 8(e)) -----------------------
 int sfm_score_async(sfm_ctx* c, double thr, double min_extra, int agg, int mode, void** record_dev) {
     if (int r = use(c)) return r;
@@ -1035,6 +1215,7 @@ int sfm_host::batch_upload(sfm_ctx* c, const double* xa, const double* ya, const
     }
     c->toc(T_UPLOAD);
     c->has_pts = true;
+    c->has_pnp = c->pnp_models = false;
     c->has_table = c->has_models = c->has_score = false;
     c->table_pending = false;
     c->winner_set = false;

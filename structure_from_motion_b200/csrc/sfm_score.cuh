@@ -1008,9 +1008,9 @@ __device__ __forceinline__ double u128_to_double(unsigned __int128 v) {
 }
 
 struct FinalArgs {
-    const Corr* pts;
+    const void* pts;       // ExactModel<KIND>::Rec records
     const long long* offsets;
-    const double* E;
+    const double* E;       // [npairs][h][ExactModel<KIND>::kStride]
     const uint8_t* valid;
     const int32_t* table;  // may be null: no sample rule
     long long h;
@@ -1035,13 +1035,17 @@ struct FinalArgs {
     SelectRecord* record;    // [npairs]
     unsigned long long* rescored;  // [1] number of hypotheses that went through the exact rescore (diagnostic)
     unsigned* fitflag;             // K1's ambiguous-sample counter: reset here for the next fit (may be null)
+    const double* K;               // MODEL_P: the camera of the new view [9]
 };
 
+// What K3 needs of a model kind: its record type, model stride, sample size and exact scorer (MODEL_P: sfm_pnp.cuh)
 template <int KIND> struct ExactModel;
 template <> struct ExactModel<MODEL_E> {
+    using Rec = Corr;
     static constexpr int kSample = 8;
+    static constexpr int kStride = 9;
     double e[9];
-    __device__ __forceinline__ void load(const double* m) {
+    __device__ __forceinline__ void load(const double* m, const double*) {
 #pragma unroll
         for (int k = 0; k < 9; ++k) e[k] = m[k];
     }
@@ -1051,9 +1055,11 @@ template <> struct ExactModel<MODEL_E> {
     }
 };
 template <> struct ExactModel<MODEL_H> {
+    using Rec = Corr;
     static constexpr int kSample = 4;
+    static constexpr int kStride = 9;
     double h[9], adj[9];
-    __device__ __forceinline__ void load(const double* m) {
+    __device__ __forceinline__ void load(const double* m, const double*) {
 #pragma unroll
         for (int k = 0; k < 9; ++k) h[k] = m[k];
         homography_adj(h, adj);
@@ -1066,16 +1072,16 @@ template <> struct ExactModel<MODEL_H> {
 // the sample rule + aggregation + candidate test of one hypothesis (ransac.py:63-64, 70-76, 96-108), given the count and
 // the sums over ALL correspondences with sed <= thr
 template <int KIND>
-__device__ __forceinline__ bool finalise_one(const FinalArgs& a, const Corr* pts, long long i, long long npts, bool valid,
-                                             long long cnt, double s1, double s2, double& err_out, long long& cnt_out,
-                                             double& s1_out, double& s2_out) {
+__device__ __forceinline__ bool finalise_one(const FinalArgs& a, const typename ExactModel<KIND>::Rec* pts, long long i,
+                                             long long npts, bool valid, long long cnt, double s1, double s2,
+                                             double& err_out, long long& cnt_out, double& s1_out, double& s2_out) {
     constexpr int KS = ExactModel<KIND>::kSample;
     const double msac = __dadd_rn(s1, __dmul_rn(a.thr, (double)(npts - cnt)));  // K2 saw every correspondence
     if (a.table && valid) {
         ExactModel<KIND> m;
-        m.load(a.E + 9 * i);
+        m.load(a.E + ExactModel<KIND>::kStride * i, a.K);
         for (int k = 0; k < KS; ++k) {
-            const Corr c = pts[a.table[8 * i + k]];
+            const typename ExactModel<KIND>::Rec c = pts[a.table[8 * i + k]];
             double sv;
             if (m.eval(c, a.thr, sv)) {
                 cnt -= 1;  // was counted by K2, but samples are not "extra" inliers
@@ -1117,7 +1123,8 @@ __global__ void __launch_bounds__(256) k_finalise(const FinalArgs a) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const long long li = blockIdx.x * (long long)blockDim.x + tid;
     const long long i = (long long)blockIdx.y * a.h + li;  // blockIdx.y = image pair
-    const Corr* pts = a.pts + (a.offsets ? a.offsets[blockIdx.y] : 0);
+    using Rec = typename ExactModel<KIND>::Rec;
+    const Rec* pts = static_cast<const Rec*>(a.pts) + (a.offsets ? a.offsets[blockIdx.y] : 0);
     const long long npts = a.offsets ? a.offsets[blockIdx.y + 1] - a.offsets[blockIdx.y] : a.n;
     const double qnan = __longlong_as_double(0x7ff8000000000000LL);
     const double pinf = __longlong_as_double(0x7ff0000000000000LL);
@@ -1134,8 +1141,9 @@ __global__ void __launch_bounds__(256) k_finalise(const FinalArgs a) {
         const unsigned __int128 need = (unsigned __int128)(unsigned long long)cnt << 53;
         bool coarse = cnt > 0 && (((a.sums & SUM_S1) && v1 < need) || ((a.sums & SUM_S2) && v2 < need));
         // a 4-point fit reproduces its own samples to rounding level, so nearly every homography has a coarse sum (its
-        // samples and little else): those that cannot be candidates (count_extra <= cnt < min_extra) are not rescored
-        if constexpr (KIND == MODEL_H) coarse = coarse && !((double)cnt < a.min_extra);
+        // samples and little else): those that cannot be candidates (count_extra <= cnt < min_extra) are not rescored;
+        // the same holds for a P3P pose and its 4 samples
+        if constexpr (KIND != MODEL_E) coarse = coarse && !((double)cnt < a.min_extra);
         if (valid && (a.force_rescore || coarse)) {
             s_list[atomicAdd(&s_nlist, 1)] = tid;
         } else {
@@ -1158,11 +1166,11 @@ __global__ void __launch_bounds__(256) k_finalise(const FinalArgs a) {
         const int owner = s_list[q];
         const long long hi_ = (long long)blockIdx.y * a.h + blockIdx.x * (long long)blockDim.x + owner;
         ExactModel<KIND> m;
-        m.load(a.E + 9 * hi_);
+        m.load(a.E + ExactModel<KIND>::kStride * hi_, a.K);
         dd p1{0.0, 0.0}, p2{0.0, 0.0};
         long long pc = 0;
         for (long long j = tid; j < npts; j += 256) {
-            const Corr c = pts[j];
+            const Rec c = pts[j];
             double sv;
             if (m.eval(c, a.thr, sv)) {
                 pc += 1;
@@ -1255,7 +1263,8 @@ __global__ void __launch_bounds__(256) k_finalise(const FinalArgs a) {
         r.num_invalid = s_ninv;
         r.first_invalid = s_ninv ? s_first2 : -1;
         const long long w = (long long)blockIdx.y * a.h + (g.idx >= 0 ? g.idx - a.idx_offset : 0);
-        for (int k = 0; k < 9; ++k) r.E[k] = g.idx >= 0 ? a.E[9 * w + k] : 0.0;
+        // a pose does not fit E[9]: its winner is read from the models by the index (k_pnp_mask), E reads zero
+        for (int k = 0; k < 9; ++k) r.E[k] = (KIND != MODEL_P && g.idx >= 0) ? a.E[ExactModel<KIND>::kStride * w + k] : 0.0;
         for (int k = 0; k < 8; ++k)
             r.sample[k] = (a.table && g.idx >= 0 && k < ExactModel<KIND>::kSample) ? a.table[8 * w + k] : -1;
     }

@@ -6,10 +6,12 @@
 
 namespace sfm {
 
-// The model K3 selects among: the essential matrix (8-point samples, SED in K-normalised coordinates) or the homography
-// (4-point samples, symmetric transfer error in pixels; sfm_homography.cuh).  The kind fixes the sample size and the
-// exact scorer of the sample rule and of the rescore; the selection rule itself is the same.
-enum { MODEL_E = 0, MODEL_H = 1 };
+// The model K3 selects among: the essential matrix (8-point samples, SED in K-normalised coordinates), the homography
+// (4-point samples, symmetric transfer error in pixels; sfm_homography.cuh) or the absolute pose [R | t] of a new view
+// (4-point samples of 2-D-3-D records, reprojection error in pixels; sfm_pnp.cuh).  The kind fixes the record type,
+// the model stride, the sample size and the exact scorer of the sample rule and of the rescore; the selection rule
+// itself is the same.
+enum { MODEL_E = 0, MODEL_H = 1, MODEL_P = 2 };
 
 struct Best {
     double err;

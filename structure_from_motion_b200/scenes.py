@@ -127,3 +127,50 @@ def make_planar_scene(n: int, outlier_frac: float, seed: int, noise_px: float = 
     x2[idx] = np.column_stack([rng.uniform(0, w, n_out), rng.uniform(0, h, n_out)])
     H_true = K @ (R + np.outer(t, nrm) / d) @ np.linalg.inv(K)
     return K, np.ascontiguousarray(x1), np.ascontiguousarray(x2), H_true / H_true[2, 2], idx
+
+
+def make_pnp_scene(n: int, outlier_frac: float, seed: int, noise_px: float = 0.5,
+                   f: float = 800.0, w: int = 1280, h: int = 960, K=None):
+    """Return (K, X[n,3], x[n,2], R, t, outlier_idx) for the absolute pose of one camera.
+
+    The world points are those of ``make_scene`` (in front of the world camera [I|0]); the new camera is K[R|t] with
+    R = euler XYZ (-3, 12, 2) deg, t = (0.8, -0.1, 0.3), so every point is in front of it too.  x = the projection plus
+    Gaussian noise; a fraction ``outlier_frac`` of the pixels is replaced by uniform pixels.  K as in ``make_scene``."""
+    rng = np.random.default_rng(seed)
+    K = _camera(K, f, w, h)
+    X = np.column_stack([rng.uniform(-2, 2, n), rng.uniform(-1.5, 1.5, n), rng.uniform(4, 8, n)])
+    R = euler_xyz_intrinsic(-3.0, 12.0, 2.0)
+    t = np.array([0.8, -0.1, 0.3])
+    p = (K @ ((R @ X.T).T + t).T).T
+    x = p[:, :2] / p[:, 2:]
+    x += rng.normal(0, noise_px, x.shape)
+    n_out = int(round(outlier_frac * n))
+    idx = rng.choice(n, n_out, replace=False)
+    x[idx] = np.column_stack([rng.uniform(0, w, n_out), rng.uniform(0, h, n_out)])
+    return K, np.ascontiguousarray(X), np.ascontiguousarray(x), R, t, idx
+
+
+def make_three_view_scene(n: int, outlier_frac: float, seed: int, noise_px: float = 0.5,
+                          f: float = 800.0, w: int = 1280, h: int = 960, K=None):
+    """Return (K, x1, x2, x3 [n,2] each, (R2, t2), (R3, t3), X[n,3]) for one point set seen by three cameras.
+
+    Cameras 1 and 2 and the points are those of ``make_scene`` (cam1 = K[I|0], cam2 = K[R2|t2]); camera 3 is the new
+    view of ``make_pnp_scene`` (K[R3|t3], R3 = euler XYZ (-3, 12, 2) deg, t3 = (0.8, -0.1, 0.3)), all in camera-1
+    coordinates.  Noise on every image; outliers (uniform pixels) in image 2 and, independently drawn, in image 3."""
+    rng = np.random.default_rng(seed)
+    K = _camera(K, f, w, h)
+    X = np.column_stack([rng.uniform(-2, 2, n), rng.uniform(-1.5, 1.5, n), rng.uniform(4, 8, n)])
+    R2, t2 = euler_xyz_intrinsic(2.0, -8.0, 1.0), np.array([-1.0, 0.05, 0.1])
+    R3, t3 = euler_xyz_intrinsic(-3.0, 12.0, 2.0), np.array([0.8, -0.1, 0.3])
+
+    def project(R, t):
+        p = (K @ ((R @ X.T).T + t).T).T
+        return p[:, :2] / p[:, 2:] + rng.normal(0, noise_px, (n, 2))
+
+    x1, x2, x3 = project(np.eye(3), np.zeros(3)), project(R2, t2), project(R3, t3)
+    n_out = int(round(outlier_frac * n))
+    for x in (x2, x3):
+        idx = rng.choice(n, n_out, replace=False)
+        x[idx] = np.column_stack([rng.uniform(0, w, n_out), rng.uniform(0, h, n_out)])
+    return (K, np.ascontiguousarray(x1), np.ascontiguousarray(x2), np.ascontiguousarray(x3), (R2, t2), (R3, t3),
+            np.ascontiguousarray(X))
