@@ -489,7 +489,6 @@ struct alignas(128) ScoreWarpSmem {
     Corr tile[kStages][kTile];
     unsigned sacc[HPT][kAccWords][32];
     uint2 ring[kRing];
-    unsigned short own[32];
     unsigned long long full_bar[kStages];
 };
 // The 9-slot body's layout: the same, plus the tile boxes and kappa.  Only it pays for them: the other one-sided
@@ -728,50 +727,67 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
 
         // ---- one-sided bodies: one ring RECORD per (lane, batch) with survivors ------------------------------------
         // {batch mask pm, owner lane << 27 | item-relative index of the batch's first correspondence}; bit NB-1-i of pm
-        // <-> test i = g*HPT + j.  drain_records() expands the first <= 32 records into <= 32 survivors, one per lane:
-        // prefix sum of the popcounts, then an owner table in shared memory {record, bit position} that every record
-        // fills for the survivor slots it owns (1.3 bits per record at a 1 % survivor rate).
+        // <-> test i = g*HPT + j.  drain_records(), whenever >= 32 records wait: lane l takes record head + l and
+        // evaluates its lowest set bit; the records that keep bits go back to the ring behind tail, ballot-compacted as
+        // in a push, and the 32 drained ones retire.  No scan, no owner table, no record straddling a drain: records
+        // hold 1.3 bits at a 1 % survivor rate, so the write-back is the rare case.  Every record holds at least one bit,
+        // so each such drain removes exactly 32 bits.  The ring cannot overflow: < 32 records wait before a push and
+        // <= 32 arrive, so tail - head <= 63; the write-backs land in [tail, tail + 32), which may wrap onto the records
+        // being read (hence the __syncwarp between read and write) but never onto [head + 32, tail).
+        // drain_tail() empties the m < 32 records left at the end of an item, min(their bits, 32) survivors per pass:
+        // survivor l goes to lane l (prefix sum of the records' bit counts; the first survivor of each record marks its
+        // start in a warp-wide OR), and what a record keeps beyond survivor 31 is written back.  Where items are short
+        // (config 2) or survivors rare, much of the survivor work is done here, and draining lowest bits first would
+        // take one pass per bit of the fullest record.
+        // Survivors are summed in another order than the batches produced them: the sums are integers (order-free).
+        auto evaluate = [&](bool act, unsigned pm, unsigned y) {  // the survivor of pm's lowest bit in record {pm, y}
+            const int i = NB - __ffs(pm);  // test index in the batch: g * HPT + j
+            const int owner = (int)(y >> 27), slot = i % HPT;
+            const unsigned rel = act ? (y & 0x3fffffu) + (unsigned)(i / HPT) : 0u;
+            accumulate(act, survivor_sed(act ? (unsigned)(32 * slot + owner) : 0u, rel), slot, owner);
+        };
         auto drain_records = [&]() {
-            const unsigned nrec = tail - head;  // 1..63
+            const uint2 rec = q[(head + lane) & (kRing - 1)];
+            const unsigned rest = rec.x & (rec.x - 1u);  // the record without its lowest bit
+            const unsigned wb = __ballot_sync(full, rest != 0u);
+            __syncwarp();
+            if (rest) q[(tail + __popc(wb & lt)) & (kRing - 1)] = make_uint2(rest, rec.y);
+            head += 32u;
+            tail += __popc(wb);
+            evaluate(true, rec.x, rec.y);
+            __syncwarp();
+        };
+        auto drain_tail = [&]() {
+            const unsigned m = tail - head;  // 1..31
             uint2 rec = make_uint2(0u, 0u);
-            if ((unsigned)lane < nrec) rec = q[(head + lane) & (kRing - 1)];
+            if ((unsigned)lane < m) rec = q[(head + lane) & (kRing - 1)];
             const int cnt = __popc(rec.x);
             int incl = cnt;
 #pragma unroll
             for (int d = 1; d < 32; d <<= 1) incl = scan_step(incl, d);
-            const int total = __shfl_sync(full, incl, 31);
-            const int m = total < 32 ? total : 32;  // survivors handled now
             const int excl = incl - cnt;
-            // ring bookkeeping: records entirely inside the first 32 survivors are retired
-            const unsigned done_mask = __ballot_sync(full, (unsigned)lane < nrec && incl <= 32);
-            const int ndone = __popc(done_mask);
-            const bool act = lane < m;
-            unsigned o = 0u;  // {record (low byte), bit position of this lane's survivor in it}
-            uint2 rj = make_uint2(0u, 0u);
-            if constexpr (!ENTRY) {
-                // the record's set bits are handed out lowest first, so what is left in pmw afterwards is exactly what a
-                // record that straddles the 32-survivor boundary keeps for the next drain
-                unsigned pmw = rec.x;
-                for (int t = excl; pmw && t < 32; ++t) {
-                    ws.own[t] = (unsigned short)(lane | ((__ffs(pmw) - 1) << 8));
-                    pmw &= pmw - 1u;
-                }
-                __syncwarp();
-                o = act ? ws.own[lane] : 0u;
-                rj = q[(head + (o & 255u)) & (kRing - 1)];
-                __syncwarp();
-                if (lane == ndone && (unsigned)lane < nrec) q[(head + lane) & (kRing - 1)].x = pmw;  // first record not retired
+            const unsigned starts = __reduce_or_sync(full, (cnt != 0 && excl < 32) ? 1u << excl : 0u);
+            const unsigned le = starts & ((lt << 1) | 1u);  // starts at or below this lane (bit 0 is record 0's)
+            const int src = __popc(le) - 1, k = lane - (31 - __clz(le));  // this lane's record and bit within it
+            unsigned pm = __shfl_sync(full, rec.x, src);
+            const unsigned y = __shfl_sync(full, rec.y, src);
+            for (int j = 0; j < k; ++j) pm &= pm - 1u;  // zero past the record's last bit: no survivor here
+            unsigned rest = 0u;  // what this lane's record keeps: its bits from survivor 32 on
+            if (incl > 32) {
+                rest = rec.x;
+                for (int t = excl; t < 32; ++t) rest &= rest - 1u;
             }
-            const int i = NB - 1 - (int)(o >> 8);  // test index in the batch: g * HPT + j
-            const int owner = (int)(rj.y >> 27), slot = i % HPT;
-            const unsigned rel = act ? (rj.y & 0x3fffffu) + (unsigned)(i / HPT) : 0u;
-            accumulate(act, survivor_sed(act ? (unsigned)(32 * slot + owner) : 0u, rel), slot, owner);
-            head += (unsigned)ndone;
+            const unsigned wb = __ballot_sync(full, rest != 0u);
+            __syncwarp();
+            if (rest) q[(tail + __popc(wb & lt)) & (kRing - 1)] = make_uint2(rest, rec.y);
+            head += m;
+            tail += __popc(wb);
+            evaluate(pm != 0u, pm, y);
             __syncwarp();
         };
         // one record per lane with survivors in this batch (ballot-compacted: no atomics, no loop).  The queue is
         // drained whenever 32 RECORDS are waiting - every record holds at least one survivor, so a drain always finds
-        // its 32 survivors, retires at least one record, and the ring (< 32 waiting + <= 32 new) cannot overflow; the
+        // its 32 survivors and retires 32 records, and the ring (< 32 waiting + <= 32 new) cannot overflow; the
         // trigger needs no reduction over the lanes (a REDUX per batch sat on the critical path before)
         auto push_records = [&](unsigned vote, unsigned pm, unsigned rel0) {
             if (pm) q[(tail + __popc(vote & lt)) & (kRing - 1)] = make_uint2(pm, ((unsigned)lane << 27) | rel0);
@@ -781,7 +797,7 @@ __device__ __forceinline__ void score_body(const ScoreArgs& a) {
         };
         auto drain = [&]() {
             if constexpr (ENTRY) drain_entries();
-            else drain_records();
+            else drain_tail();  // only the item's tail: < 32 records
         };
 
         unsigned mark = tail;  // ENTRY: queue position behind the last record of the previous tile
