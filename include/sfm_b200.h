@@ -201,10 +201,12 @@ int sfm_homography_mask(sfm_ctx *ctx, const double *H, double threshold, uint8_t
  * Records: n world points X (double[n][3]) and their observed pixels x (double[n][2]) in the new image, with its K
  * (double[9], row-major): finite, non-singular, upper triangular with K[2,2] = 1, else SFM_ERR_ARG.  The model is
  * [R | t] (double[12], row-major 3 x 4, x_cam = R X + t); P = K [R | t] and p = P (X, 1) are formed in the pinned order
- * of csrc/sfm_pnp.cuh.  A record is an inlier iff p2 > 0 && F <= thr p2^2 with F = (p0 - u p2)^2 + (p1 - v p2)^2; its
- * value is the squared reprojection error F / p2^2 in px^2.  The minimal solver is P3P (Lambda Twist) on columns 0-2
+ * of csrc/sfm_pnp.cuh.  A record is an inlier iff p2 >= 2^-537 && F < inf && F <= thr p2^2 with
+ * F = (p0 - u p2)^2 + (p1 - v p2)^2; its value is the squared reprojection error F / p2^2 in px^2 (always finite for an
+ * inlier).  The minimal solver is P3P (Lambda Twist) on columns 0-2
  * of a sample, with column 3 choosing among the solutions (smallest error at point 3).  A sample with a non-finite
- * coordinate, three collinear world points, no solution with three positive depths or a non-finite pose is invalid:
+ * coordinate, three collinear world points, no solution with three positive depths and an R orthonormal to 1e-6, or a
+ * non-finite pose is invalid:
  * never a candidate, counted in sfm_best.num_invalid / first_invalid. */
 /* Replace the context's records with PnP records: the essential-matrix and homography calls refuse until the next
  * sfm_upload_pairs.  Then load a sample table or call the device sampler (columns 0-3 are the sample). */

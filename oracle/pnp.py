@@ -23,12 +23,13 @@ from oracle import creproj
 from oracle.restatement import AGG_RMS, aggregate_error
 
 COLLINEAR = 1e-6  # csrc/sfm_pnp.cuh kPnpCollinear: sine of the angle at X0
+MIN_DEPTH = 2.0 ** -537  # csrc/sfm_pnp.cuh kPnpMinDepthHi: the smallest p2 of an inlier (its square is not 0)
 _DPS = 50
 
 
 def reproj(Rt, K, X, x, thr):
     """(decision bool[n], value [n]) of every record: p = K [R|t] (X, 1), F = (p0 - u p2)^2 + (p1 - v p2)^2,
-    inlier iff p2 > 0 and F <= thr p2^2, value F / p2^2."""
+    inlier iff p2 >= 2^-537 (W = p2^2 > 0), F < inf and F <= thr p2^2, value F / p2^2."""
     Rt = np.asarray(Rt, dtype=np.float64).reshape(3, 4)
     X = np.asarray(X, dtype=np.float64).reshape(-1, 3)
     x = np.asarray(x, dtype=np.float64).reshape(-1, 2)
@@ -39,7 +40,7 @@ def reproj(Rt, K, X, x, thr):
         d1 = p[:, 1] - x[:, 1] * p[:, 2]
         F = d0 * d0 + d1 * d1
         W = p[:, 2] * p[:, 2]
-        return (p[:, 2] > 0) & (F <= thr * W), F / W
+        return (p[:, 2] >= MIN_DEPTH) & (F < inf) & (F <= thr * W), F / W
 
 
 def bearings(K, x):
@@ -50,7 +51,12 @@ def bearings(K, x):
         yn = (x[:, 1] - K[1, 2]) / K[1, 1]
         xn = ((x[:, 0] - K[0, 2]) - K[0, 1] * yn) / K[0, 0]
         b = np.stack([xn, yn, np.ones_like(xn)], axis=1)
-        return b / np.linalg.norm(b, axis=1, keepdims=True)
+        nrm = np.linalg.norm(b, axis=1, keepdims=True)
+        # np.linalg.norm squares: beyond ~1e154 it overflows, so such rows are divided by their largest entry first
+        big = ~np.isfinite(nrm[:, 0]) & np.isfinite(b).all(axis=1)
+        b[big] /= np.abs(b[big]).max(axis=1, keepdims=True)
+        nrm[big] = np.linalg.norm(b[big], axis=1, keepdims=True)
+        return b / nrm
 
 
 def collinear_ratio(X3):
@@ -166,12 +172,18 @@ def fit_pnp_exact(K, X, x):
     (sine <= COLLINEAR) or no candidate remains."""
     X = np.asarray(X, dtype=np.float64).reshape(4, 3)
     x = np.asarray(x, dtype=np.float64).reshape(4, 2)
-    info = dict(collinear=collinear_ratio(X[:3]), gap=inf, ncand=0)
+    # the sine and the solve are scale-free: they run on the world points scaled by a power of two (exact), so that
+    # float64 norms and mpmath's singularity test see coordinates of order 1 at any world scale; t is scaled back
+    with np.errstate(all="ignore"):
+        spread = np.abs(X[:3, None, :] - X[None, :3, :]).max()
+    e = int(np.frexp(spread)[1]) if np.isfinite(spread) and spread > 0 else 0
+    Xs = np.ldexp(X[:3], -e)
+    info = dict(collinear=collinear_ratio(Xs), gap=inf, ncand=0)
     if not (np.isfinite(X).all() and np.isfinite(x).all()):
         return None, info
     if not info["collinear"] > COLLINEAR:
         return None, info
-    cands = p3p_exact(bearings(K, x[:3]), X[:3])
+    cands = [(R, np.ldexp(t, e)) for R, t in p3p_exact(bearings(K, x[:3]), Xs)]
     info["ncand"] = len(cands)
     best, errs = select_fourth(K, cands, X[3], x[3])
     if best < 0:
@@ -258,3 +270,36 @@ def expected_selection(models, valid, K, X, x, threshold, table, aggregation, se
         if not len(winners):
             winners = np.flatnonzero(cand & (err == best))
     return dict(count_extra=cnt, S1=s1, S2=s2, err=err, winners=winners)
+
+
+def cubic_branch(y, X):
+    """1 or 3: the number of real roots cubic_roots (csrc/sfm_pnp.cuh) takes for the Lambda Twist cubic
+    det(D1 + g D2) of unit bearings y[3,3] and world points X[3,3], restated in float64 (the sign of the depressed
+    cubic's discriminant; a sample within rounding of disc = 0 may fall on either side on the device).  0 when the
+    leading coefficient is 0 or a coefficient is not finite."""
+    y = np.asarray(y, dtype=np.float64)
+    X = np.asarray(X, dtype=np.float64)
+    w1, w2, w12 = X[0] - X[1], X[0] - X[2], X[1] - X[2]
+    a01, a02, a12 = w1 @ w1, w2 @ w2, w12 @ w12
+    b01, b02, b12 = y[0] @ y[1], y[0] @ y[2], y[1] @ y[2]
+    D1 = np.array([[a12, -a12 * b01, 0.0], [-a12 * b01, a12 - a01, a01 * b12], [0.0, a01 * b12, -a01]])
+    D2 = np.array([[a12, 0.0, -a12 * b02], [0.0, -a02, a02 * b12], [-a12 * b02, a02 * b12, a12 - a02]])
+    det = lambda a, b, c: float(np.dot(a, np.cross(b, c)))  # noqa: E731  (columns = rows: both are symmetric)
+    A, B = D1, D2
+    k3 = det(B[0], B[1], B[2])
+    k2 = det(A[0], B[1], B[2]) + det(B[0], A[1], B[2]) + det(B[0], B[1], A[2])
+    k1 = det(A[0], A[1], B[2]) + det(A[0], B[1], A[2]) + det(B[0], A[1], A[2])
+    k0 = det(A[0], A[1], A[2])
+    if not (k3 != 0 and np.isfinite([k3, k2, k1, k0]).all()):
+        return 0
+    p, q, r = k2 / k3, k1 / k3, k0 / k3
+    P = q - p * p / 3.0
+    Q = 2.0 * p * p * p / 27.0 - p * q / 3.0 + r
+    return 1 if 0.25 * Q * Q + P * P * P / 27.0 > 0.0 else 3
+
+
+def bearing_angles(y):
+    """The smallest angle (radians) between two of the unit bearings y[3,3]: the conditioning of a P3P sample."""
+    y = np.asarray(y, dtype=np.float64)
+    ang = [np.arctan2(np.linalg.norm(np.cross(y[i], y[j])), y[i] @ y[j]) for i, j in ((0, 1), (0, 2), (1, 2))]
+    return float(min(ang))

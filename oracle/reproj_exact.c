@@ -1,7 +1,7 @@
 /* TEST INFRASTRUCTURE ONLY — plain-C restatement of the PnP reprojection scorer (csrc/sfm_pnp.cuh).
  *
  * P = K [R | t] and p = P (X, Y, Z, 1), the differences, F = d0^2 + d1^2, W = p2^2, the decision
- * p2 > 0 && F <= thr W and the value F / W, each one IEEE operation or one fma() in the device's pinned order.
+ * p2 >= 2^-537 && F < inf && F <= thr W and the value F / W, each one IEEE operation or one fma() in the device's pinned order.
  * Compiled with -ffp-contract=off so that no product and sum are fused behind our back: decisions and values are
  * bit-identical to the kernels (k_score_pnp, k_finalise<MODEL_P>, k_pnp_mask). */
 #include <math.h>
@@ -24,7 +24,7 @@ static inline int reproj_eval(const double *P, double X, double Y, double Z, dou
     const double F = fma(d0, d0, d1 * d1);
     const double W = p2 * p2;
     *value = F / W;
-    return p2 > 0.0 && F <= thr * W;
+    return p2 >= 0x1p-537 && F < INFINITY && F <= thr * W;
 }
 
 /* decision and value of every record under one [R | t] (row-major 3 x 4) */

@@ -10,9 +10,15 @@
 // once per model load, and then p = P (X, Y, Z, 1) with pnp_terms' pinned order.
 //
 // Error.  With d0 = p0 - u p2, d1 = p1 - v p2 (one fma each), F = d0^2 + d1^2 and W = p2^2:
-//   inlier   <=>  p2 > 0 && F <= thr W                  (every evaluation; division-free; NaN fails)
+//   inlier   <=>  p2 >= 2^-537 && F < inf && F <= thr W   (every evaluation; division-free; NaN fails)
 //   value     =   F / W, the squared reprojection error in px^2   (inliers only; summed)
 // A point on or behind the camera plane is never an inlier.  thr is in px^2 and the test is "<=" (ransac.py:73).
+// The two range terms keep every inlier's value finite: without them a finite record some 1e154 units or pixels out
+// has F = W = inf and would pass with the value NaN, and a record with 0 < p2 < 2^-537 (W = 0) and F = 0 with 0 / 0.
+// A finite record with W = inf but F finite (on its ray, ~1e154 out) passes and is scored 0: its true squared error is
+// somewhere below 1 px^2, so with thr < 1 such a record can be admitted wrongly; its value stays finite.
+// Both are integer tests on the high words and use no FP64 slot; k_score_pnp still measured 2.3 % slower with them
+// on one B200 (DESIGN.md 7f).
 //
 // FP64 issue slots of one evaluation (the scorer's hot loop, counted from the source, one per DFMA/DMUL):
 //   p 9, the two differences 2, F 2, W 1, thr W 1, the compare 1                              = 16
@@ -27,7 +33,15 @@
 // within a plane the smaller root of the quadratic first.  A sample is invalid (never a candidate, counted in num_invalid /
 // first_invalid) when a coordinate is not finite, when the three world points are collinear
 // (|w1 x w2|^2 <= kPnpCollinear^2 |w1|^2 |w2|^2, w1 = X0 - X1, w2 = X0 - X2), when no real solution has three
-// positive depths, or when the chosen [R | t] is not finite.
+// positive depths, or when the chosen [R | t] is not finite or its R is not orthonormal to kPnpOrthonormal
+// (max |R R^T - I|).  The last rule is for near-collinear world points (sine below ~1e-2): the rotation about their
+// line rests on the last bits of the depths, and float64 Lambda Twist then returns solutions that are wrong, not merely
+// imprecise (up to ~1 in R at sine 1e-5), and visibly non-orthonormal.  Such a sample is invalid rather than wrong;
+// well-spread samples, narrow cameras included, stay below 3e-7.
+// Range.  The solver runs on the world points scaled by a power of two taken from their largest coordinate difference
+// and scales t back, so it is exactly equivariant under world x 2^k and works at any world scale whose coordinate
+// differences and pose are finite.  A pixel's bearing takes a power-of-two-scaled norm when xn^2 + yn^2 overflows
+// (more than ~1e154 focal lengths off axis), so every finite pixel has a unit bearing.
 //
 // RANSAC semantics: fit_with_ransac(data, 4, ...) (lib/ransac/ransac.py:19-93) exactly as the homography path applies
 // it: columns 0-3 of the shared int32[H][8] table, samples never extra inliers and always in the error, K3
@@ -46,6 +60,8 @@ struct __align__(16) PnpRec {
 static_assert(sizeof(PnpRec) == 48, "PnpRec must be 48 bytes");
 
 constexpr double kPnpCollinear = 1e-6;  // sine of the angle at X0 below which three world points are collinear
+constexpr double kPnpOrthonormal = 1e-6;  // largest |R R^T - I| entry of a valid sample's chosen R
+constexpr int kPnpMinDepthHi = 0x1e600000;  // high word of 2^-537, the smallest p2 whose square W is not 0
 
 // P = K [R | t] in the pinned order (see the header)
 __device__ __forceinline__ void pnp_projection(const double* K, const double* m, double (&P)[12]) {
@@ -70,8 +86,9 @@ __device__ __forceinline__ PnpTerms pnp_terms(const double (&P)[12], double X, d
     r.p2 = p2;
     return r;
 }
+// p2 >= 2^-537 and F < inf are tested on the high words, as integers: no FP64 issue slot
 __device__ __forceinline__ bool pnp_inlier(const PnpTerms& r, double thr) {
-    return r.p2 > 0.0 && r.F <= __dmul_rn(thr, r.W);
+    return __double2hiint(r.p2) >= kPnpMinDepthHi && __double2hiint(r.F) < 0x7ff00000 && r.F <= __dmul_rn(thr, r.W);
 }
 __device__ __forceinline__ double pnp_value(const PnpTerms& r) { return __ddiv_rn(r.F, r.W); }
 __device__ __forceinline__ bool pnp_exact(const double (&P)[12], const PnpRec& c, double thr, double& value) {
@@ -313,12 +330,39 @@ __device__ __forceinline__ bool pnp_fit4(const PnpRec (&c)[4], const double* K, 
     const double fx = K[0], sk = K[1], cx = K[2], fy = K[4], cy = K[5];
 #pragma unroll
     for (int i = 0; i < 3; ++i) {
-        x[i][0] = c[i].X; x[i][1] = c[i].Y; x[i][2] = c[i].Z;
         const double yn = __ddiv_rn(__dsub_rn(c[i].v, cy), fy);
         const double xn = __ddiv_rn(__dsub_rn(__dsub_rn(c[i].u, cx), __dmul_rn(sk, yn)), fx);
-        const double inv = 1.0 / sqrt(xn * xn + yn * yn + 1.0);
-        y[i][0] = xn * inv; y[i][1] = yn * inv; y[i][2] = inv;
+        const double n2 = xn * xn + yn * yn + 1.0;
+        if (isfinite(n2)) {
+            const double inv = 1.0 / sqrt(n2);
+            y[i][0] = xn * inv; y[i][1] = yn * inv; y[i][2] = inv;
+        } else {  // a pixel ~1e154 focal lengths off axis: (xn, yn, 1) scaled by a power of two before its norm
+            int e;
+            (void)frexp(fmax(fabs(xn), fabs(yn)), &e);
+            const double bx = ldexp(xn, -e), by = ldexp(yn, -e), bz = ldexp(1.0, -e);
+            const double inv = 1.0 / sqrt(bx * bx + by * by + bz * bz);
+            y[i][0] = bx * inv; y[i][1] = by * inv; y[i][2] = bz * inv;
+        }
     }
+    // The solver sees the world points scaled by 2^-we, 2^we the power of two just above the largest coordinate
+    // difference, so that its degree-8 terms (eigvec3) and degree-6 terms (the cubic) neither overflow nor underflow;
+    // t is scaled back.  Every step is homogeneous in the world scale, so this changes no bit where the unscaled
+    // solve stayed in range.
+#pragma unroll
+    for (int i = 0; i < 3; ++i) { x[i][0] = c[i].X; x[i][1] = c[i].Y; x[i][2] = c[i].Z; }
+    int we = 0;
+    {
+        double m = 0.0;
+#pragma unroll
+        for (int k = 0; k < 3; ++k)
+            m = fmax(m, fmax(fabs(x[0][k] - x[1][k]), fmax(fabs(x[0][k] - x[2][k]), fabs(x[1][k] - x[2][k]))));
+        if (!isfinite(m)) return false;
+        (void)frexp(m, &we);
+    }
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+        for (int k = 0; k < 3; ++k) x[i][k] = ldexp(x[i][k], -we);
     {
         double w1[3], w2[3], w3[3];
 #pragma unroll
@@ -332,6 +376,8 @@ __device__ __forceinline__ bool pnp_fit4(const PnpRec (&c)[4], const double* K, 
     int best = -1;
     double be = 0.0;
     for (int s = 0; s < ns; ++s) {
+#pragma unroll
+        for (int r = 0; r < 3; ++r) M[s][4 * r + 3] = ldexp(M[s][4 * r + 3], we);
         double P[12];
         pnp_projection(K, M[s], P);
         const PnpTerms t = pnp_terms(P, c[3].X, c[3].Y, c[3].Z, c[3].u, c[3].v);
@@ -339,6 +385,18 @@ __device__ __forceinline__ bool pnp_fit4(const PnpRec (&c)[4], const double* K, 
         if (e == e && (best < 0 || e < be)) { best = s; be = e; }
     }
     if (best < 0) return false;
+    {
+        // near-collinear world points leave the rotation about their line to the last bits of the depths: the chosen
+        // solution then comes out visibly non-orthonormal and is wrong, not merely imprecise, so the sample is invalid
+        double dev = 0.0;
+#pragma unroll
+        for (int a = 0; a < 3; ++a)
+#pragma unroll
+            for (int b = a; b < 3; ++b)
+                dev = fmax(dev, fabs(M[best][4 * a] * M[best][4 * b] + M[best][4 * a + 1] * M[best][4 * b + 1] +
+                                     M[best][4 * a + 2] * M[best][4 * b + 2] - (a == b ? 1.0 : 0.0)));
+        if (!(dev <= kPnpOrthonormal)) return false;
+    }
 #pragma unroll
     for (int k = 0; k < 12; ++k) {
         Rt[k] = M[best][k];

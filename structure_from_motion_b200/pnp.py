@@ -3,8 +3,8 @@
 Registers a further image against triangulated points: given world points X (for points from ``two_view_arrays`` the
 frame of camera 1, with the baseline |t| = 1) and their pixels x in the new image, find [R | t] with x_cam = R X + t.
 K must be upper triangular with K[2,2] = 1.  The error is the squared reprojection error in px^2, F / p2^2 with
-p = K [R | t] (X, 1) and F = (p0 - u p2)^2 + (p1 - v p2)^2, and a record is an inlier iff p2 > 0 and F <= thr p2^2
-(division-free; csrc/sfm_pnp.cuh pins the evaluation order).  The minimal solver is P3P (Lambda Twist) on the first
+p = K [R | t] (X, 1) and F = (p0 - u p2)^2 + (p1 - v p2)^2, and a record is an inlier iff p2 >= 2^-537, F < inf and
+F <= thr p2^2 (division-free; csrc/sfm_pnp.cuh pins the evaluation order).  The minimal solver is P3P (Lambda Twist) on the first
 three points of a sample, the fourth choosing among its solutions.  The RANSAC loop is the reference's
 ``fit_with_ransac(data, 4, ...)`` (lib/ransac/ransac.py:19-93) as ``ransac_homography_arrays`` applies it.  Everything
 numeric runs in libsfm_b200.so; there is no CPU fallback.

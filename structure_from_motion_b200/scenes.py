@@ -174,3 +174,66 @@ def make_three_view_scene(n: int, outlier_frac: float, seed: int, noise_px: floa
         x[idx] = np.column_stack([rng.uniform(0, w, n_out), rng.uniform(0, h, n_out)])
     return (K, np.ascontiguousarray(x1), np.ascontiguousarray(x2), np.ascontiguousarray(x3), (R2, t2), (R3, t3),
             np.ascontiguousarray(X))
+
+
+def random_rotation(rng) -> np.ndarray:
+    """A rotation drawn uniformly over SO(3) (a normalised Gaussian quaternion)."""
+    q = rng.normal(size=4)
+    w, x, y, z = q / np.linalg.norm(q)
+    return np.array([[1 - 2 * (y * y + z * z), 2 * (x * y - w * z), 2 * (x * z + w * y)],
+                     [2 * (x * y + w * z), 1 - 2 * (x * x + z * z), 2 * (y * z - w * x)],
+                     [2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)]])
+
+
+def _axis_rotations():
+    """Rotations whose optical axis (third row) is each of +-x, +-y, +-z, and three rotations by 180 deg - 1e-6."""
+    out = []
+    for k in range(3):
+        for s in (1.0, -1.0):
+            z = np.zeros(3)
+            z[k] = s
+            x = np.zeros(3)
+            x[(k + 1) % 3] = 1.0
+            out.append(np.stack([x, np.cross(z, x), z]))
+    for axis in np.eye(3):
+        a = np.pi - 1e-6
+        Kx = np.array([[0, -axis[2], axis[1]], [axis[2], 0, -axis[0]], [-axis[1], axis[0], 0]])
+        out.append(np.eye(3) + np.sin(a) * Kx + (1 - np.cos(a)) * Kx @ Kx)
+    return out
+
+
+def make_pnp_samples(m: int, seed: int, noise_px: float = 0.0, K=None, w: int = 1280, h: int = 960):
+    """m random 4-point PnP samples, each (K, X[4,3], x[4,2], R, t) with x_cam = R X + t.
+
+    Pose: R uniform over SO(3) (the first nine samples: optical axis along each of +-x, +-y, +-z, and rotations by
+    180 deg - 1e-6 about each axis), the camera centre uniform in a cube of side 2 D around the origin.  Points: pixels
+    uniform in a disc of radius rho f around a random image point, wrapped into the image (so up to ~75 deg off axis for
+    f = 150), at depths D exp(U(-1, 1) min(rho, 1)); D is log-uniform in [0.5, 100] and the spread rho log-uniform in
+    [1e-3, 10] times the depth.  K: f log-uniform in [150, 20 000], principal point at the image centre, unless given.
+    x is the projection plus Gaussian noise of noise_px."""
+    rng = np.random.default_rng(seed)
+    special = _axis_rotations()
+    out = []
+    for i in range(m):
+        if K is None:
+            f = float(np.exp(rng.uniform(np.log(150.0), np.log(20_000.0))))
+            Ki = np.array([[f, 0.0, w / 2], [0.0, f, h / 2], [0.0, 0.0, 1.0]])
+        else:
+            Ki = np.asarray(K, dtype=np.float64)
+        f = Ki[0, 0]
+        R = special[i] if i < len(special) else random_rotation(rng)
+        D = float(np.exp(rng.uniform(np.log(0.5), np.log(100.0))))
+        rho = float(10.0 ** rng.uniform(-3.0, 1.0))
+        ctr = np.array([rng.uniform(0, w), rng.uniform(0, h)])
+        r = rho * f * np.sqrt(rng.uniform(0, 1, 4))
+        phi = rng.uniform(0, 2 * np.pi, 4)
+        pix = np.mod(ctr + np.column_stack([r * np.cos(phi), r * np.sin(phi)]), [w, h])  # wrapped into the image
+        dep = D * np.exp(rng.uniform(-1.0, 1.0, 4) * min(rho, 1.0))
+        cam = (np.linalg.solve(Ki, np.column_stack([pix, np.ones(4)]).T) * dep).T
+        C = rng.uniform(-D, D, 3)
+        t = -R @ C
+        X = (R.T @ (cam - t).T).T
+        p = (Ki @ ((R @ X.T).T + t).T).T
+        x = p[:, :2] / p[:, 2:] + rng.normal(0, noise_px, (4, 2))
+        out.append((Ki, np.ascontiguousarray(X), np.ascontiguousarray(x), R, t))
+    return out
