@@ -158,7 +158,10 @@ typedef struct sfm_best {
 /* Winner of the last sfm_score (ransac.py:83: minimum error, earliest iteration on ties). */
 int sfm_get_best(sfm_ctx *ctx, sfm_best *out);
 /* Tell the context which hypothesis won (hypothesis-sharded runs: after the cross-rank
- * merge).  local_index < 0 = the winner lives on another rank; E then supplies the model. */
+ * merge).  local_index < 0 = the winner lives on another rank; E then supplies the model, at any scale: an E whose
+ * largest finite entry lies outside [2^-100, 2^100] is brought to [0.5, 1) by a power of two, so the tail and the
+ * refinement of 2^k E equal those of E bit for bit.  Such an E is stored scaled: a refinement report that falls back
+ * to the unrefined model (nonfinite) returns it as 2^j E, the same model. */
 int sfm_set_winner(sfm_ctx *ctx, int64_t local_index, const double *E);
 /* SURVEY.md H1 (ransac.py:83,96-108: strict < on errors summed in LIST order): the local indices of the hypotheses
  * of the last score whose error is <= best * (1 + rel_tol), unordered, at most cap of them; *count is their total
@@ -416,7 +419,9 @@ int sfm_batch_score_models(sfm_ctx *ctx, const double *E, const uint8_t *have_e,
  * The RANSAC result is untouched (best, mask, sed / err, the E / H arrays of the batch calls).  The tail then runs on
  * the refined model as on a caller-supplied one: inliers = the decision under the refined model with no forced samples
  * (the E vote's index-0 rule applies to list position 0, as after sfm_set_winner(ctx, -1, E)), vote, triangulation.
- * A pair without a winner, or whose start is not finite, keeps the RANSAC model and its tail.  The refined bits depend on
+ * A pair without a winner, or whose start is not finite, keeps the RANSAC model and its tail.  An empty list (a
+ * caller's E that explains no correspondence) reports converged at iteration 0 with cost 0, and its model is the start:
+ * the caller's E projected onto the essential manifold.  The refined bits depend on
  * the pair's inlier list only (fixed-order sums): pair p of a batch equals the single-pair call on that pair.
  * sfm_two_view_sharded and sfm_sharded_tail refuse with SFM_ERR_STATE while refinement is on. */
 enum sfm_refine_status {

@@ -222,6 +222,9 @@ int fit_h_launch(sfm_ctx* c);
 int score_h_launch(sfm_ctx* c, double thr, double min_extra, int agg, int mode, long long max_len);
 void unpack_best(const sfm::SelectRecord& r, sfm_best* out);
 const double* winner_E_dev(sfm_ctx* c);
+// a caller's matrix outside [2^-100, 2^100] brought to [0.5, 1) by a power of two (sfm_two_view.cu)
+int prescale_exponent(const double* a, int n);
+void prescaled(const double* a, int n, int k, double* out);
 int batch_fetch_winners(sfm_ctx* c, int64_t npairs, size_t extra_pinned, char** extra);
 void batch_unpack_winners(const char* hp, int64_t npairs, double* E, int64_t* best_index, double* best_err,
                           int32_t* count_extra, int64_t* num_invalid);

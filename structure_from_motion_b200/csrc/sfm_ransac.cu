@@ -739,7 +739,11 @@ int sfm_set_winner(sfm_ctx* c, int64_t local_index, const double* E) {
     } else {
         if (!E) return fail(SFM_ERR_ARG, "need the winning model when it lives on another rank");
         if (int r = c->winnerE.reserve(72)) return r;
-        CU(cudaMemcpyAsync(c->winnerE.p, E, 72, cudaMemcpyHostToDevice, c->stream));
+        // the decomposition of the refinement's start and the tail square E's entries: a power of two keeps them in
+        // range whatever the caller's scale, and every result is the same as for 2^k E
+        double Es[9];
+        prescaled(E, 9, prescale_exponent(E, 9), Es);
+        CU(cudaMemcpyAsync(c->winnerE.p, Es, 72, cudaMemcpyHostToDevice, c->stream));
         CU(cudaStreamSynchronize(c->stream));
         c->winner_local = -1;
     }

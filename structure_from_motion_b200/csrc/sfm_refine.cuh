@@ -13,6 +13,8 @@
 // Parameters.  E = [t]x R on the essential manifold: R <- R exp([w]x), the unit t moves by (b1, b2) in its tangent
 // plane (b1 = t x e_k / |t x e_k|, e_k the axis of t's smallest component, b2 = t x b1), then is renormalised: 5
 // parameters.  The start is candidate 0 of decompose_essential of the RANSAC E (its projection onto the manifold).
+// Which rotation of the twisted pair is candidate 0 matters: [t]x R1 = -[t]x R2, but the tangent moves of t are taken
+// against R, so the two charts give different steps (oracle/refine_exact.py replays from the device's candidate).
 // H: h0..h7 with h8 = 1 held fixed: 8 parameters.
 //
 // Solver (fixed control).  The normal equations J^T J, J^T r of the last accepted point are kept per pair.  A step
@@ -25,7 +27,8 @@
 // through its own 4 samples), or when the scaled step |D d| (D = the square
 // roots of diag(J^T J): the first-order change of the residual vector) is at most kRefineXtol sqrt(cost); stalled when
 // lambda exceeds kRefineLambdaCap; iteration cap after `max_iter` evaluated proposals.  The final cost is the cost of the
-// last accepted point, never above the start's.
+// last accepted point, never above the start's.  An empty list has cost 0 at the floor 0: converged at iteration 0,
+// the start (E: the projected RANSAC or caller E) reported as the refined model.
 //
 // Determinism.  Each launch sums per-correspondence terms over fixed chunks of kRefineChunk list entries (thread t
 // takes entries t and t + 128 of the chunk, in that order; warps reduce with a fixed butterfly and the four warp sums

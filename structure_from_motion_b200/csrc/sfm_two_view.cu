@@ -26,12 +26,12 @@ int sfm_get_refinement(sfm_ctx* c, sfm_refinement* out, int64_t P) {
 }
 
 // ---- pose + triangulation ---------------------------------------------------------------
-// Caller-supplied E, P1 and P2 may have any scale, but the decomposition and the DLT square their entries (twice, in
+// Caller-supplied E (sfm_set_winner too), P1 and P2 may have any scale, but the decomposition and the DLT square their entries (twice, in
 // the cross products of svd3_rank2_frames) and leave the double range from about 2^+-250 on.  Their answers do not
 // depend on the scale: the frames of E and 2^k E are the same, as is the null vector of 2^k A.  So the stand-alone
 // calls bring an input whose largest finite magnitude lies outside [2^-100, 2^100] to [0.5, 1) by a power of two - exact,
 // and no bit changes inside that range - and undo it on the singular values.  Returns the exponent applied (0 = none).
-static int prescale_exponent(const double* a, int n) {
+int sfm_host::prescale_exponent(const double* a, int n) {
     double big = 0.0;
     for (int i = 0; i < n; ++i)
         if (std::isfinite(a[i])) big = std::fmax(big, std::fabs(a[i]));
@@ -41,7 +41,7 @@ static int prescale_exponent(const double* a, int n) {
     return -e;
 }
 
-static void prescaled(const double* a, int n, int k, double* out) {
+void sfm_host::prescaled(const double* a, int n, int k, double* out) {
     for (int i = 0; i < n; ++i) out[i] = std::ldexp(a[i], k);
 }
 
