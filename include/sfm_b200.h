@@ -229,6 +229,35 @@ int sfm_ransac_pnp(sfm_ctx *ctx, double threshold, double min_extra, int aggrega
 int sfm_pnp_mask(sfm_ctx *ctx, const double *Rt, double threshold, uint8_t *mask, double *err);
 /* Poses [first, first + count) of the last PnP fit: Rt_out double[count][12], valid_out uint8[count]; either may be NULL. */
 int sfm_get_pnp_models(sfm_ctx *ctx, int64_t first, int64_t count, double *Rt_out, uint8_t *valid_out);
+/* Least-squares refinement of a pose over its inliers (Levenberg-Marquardt on [R | t], FP64; csrc/sfm_refine.cuh):
+ *   list    fixed while the refinement runs, in ascending record order (which fixes the sums): the records whose
+ *           decision passes under the start pose at threshold, plus the forced indices - with Rt NULL the RANSAC
+ *           winner's 4 samples, else the caller's optional 4 (sample NULL: none);
+ *   cost    the sum over the list of the squared reprojection error, two residuals per record, r0 = p0 / p2 - u and
+ *           r1 = p1 / p2 - v with p = K [R | t] (X, 1) in the scorer's order.  A proposal under which a list record has
+ *           p2 < 2^-537 or a non-finite residual costs +inf and is rejected; at the start that is SFM_REFINE_NONFINITE
+ *           and the start pose is kept;
+ *   model   R <- R exp([w]x), t <- t + dt (6 parameters), started from the rotation nearest to the start's R (det +1:
+ *           a reflection is projected onto a rotation) and its t;
+ *   solver  the control of sfm_set_refinement's (lambda 1e-3, x / 10, Ftol 1e-12, Xtol 1e-9, lambda cap 1e16,
+ *           max_iterations evaluated proposals), with the cost floor 1e-24 sum(u^2 + v^2) over the list.
+ * Rt NULL: the winner of the last sfm_ransac_pnp (SFM_ERR_STATE without one); else a caller pose (double[12]).
+ * sfm_set_refinement does not govern this call, and it changes no RANSAC result: sfm_best, the winner, masks,
+ * sfm_near_ties, sfm_get_pnp_models and sfm_get_refinement read the same afterwards.  mask uint8[n] / err double[n]
+ * (may be NULL): decision and reprojection error under the reported pose at threshold, no forced samples.  The bits
+ * depend only on the list and the start: not on records outside the list, the grid or the run.  An empty list
+ * reports converged at iteration 0 with cost 0 and the projected start.  SFM_ERR_STATE without PnP records;
+ * SFM_ERR_ARG for max_iterations < 1, a non-finite threshold or a sample index outside [0, n). */
+typedef struct sfm_pnp_refinement {
+    double Rt[12];                 /* refined [R | t], row-major 3x4; the RANSAC / caller pose when not refined */
+    double cost_ransac;            /* cost of the start pose as given, F / p2^2 summed over the list            */
+    double cost_start;             /* cost at the start point (its R projected onto the rotations)              */
+    double cost_final;             /* cost of the reported pose, <= cost_start                                  */
+    int64_t num;                   /* records in the list                                                       */
+    int32_t iterations, status, rejected, reserved;   /* status: enum sfm_refine_status                        */
+} sfm_pnp_refinement;
+int sfm_refine_pnp(sfm_ctx *ctx, const double *Rt, const int32_t *sample, double threshold, int max_iterations,
+                   sfm_pnp_refinement *out, uint8_t *mask, double *err);
 
 /* ---- pose + triangulation ------------------------------------------------------------ */
 typedef struct sfm_poses {

@@ -56,6 +56,12 @@ class Refinement(C.Structure):
                 ("rejected", C.c_int32), ("reserved", C.c_int32)]
 
 
+class PnpRefinement(C.Structure):
+    _fields_ = [("Rt", C.c_double * 12), ("cost_ransac", C.c_double), ("cost_start", C.c_double),
+                ("cost_final", C.c_double), ("num", C.c_int64), ("iterations", C.c_int32), ("status", C.c_int32),
+                ("rejected", C.c_int32), ("reserved", C.c_int32)]
+
+
 REFINE_STATUS = {0: "converged", 1: "max_iterations", 2: "stalled", 3: "no_model", 4: "nonfinite"}
 
 _P = C.c_void_p
@@ -99,6 +105,7 @@ _SIGNATURES = {
     "sfm_ransac_pnp": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.POINTER(Best), _P, _P, _P, _P, _P]),
     "sfm_pnp_mask": (C.c_int, [_P, _P, C.c_double, _P, _P]),
     "sfm_get_pnp_models": (C.c_int, [_P, C.c_int64, C.c_int64, _P, _P]),
+    "sfm_refine_pnp": (C.c_int, [_P, _P, _P, C.c_double, C.c_int, C.POINTER(PnpRefinement), _P, _P]),
     "sfm_decompose_essential": (C.c_int, [_P, _P, C.POINTER(Poses)]),
     "sfm_recover_pose": (C.c_int, [_P, _P, _P, _P, _P, _P, C.c_int64, C.c_int64, C.c_double, C.POINTER(Poses), _P]),
     "sfm_recover_pose_pixels": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int64, C.c_int64, C.c_double,
@@ -535,6 +542,19 @@ class Engine:
         err = np.empty(self.n, dtype=np.float64)
         self._ck(self.lib.sfm_pnp_mask(self.h, _ptr(Ra), float(threshold), _ptr(mask), _ptr(err)), "sfm_pnp_mask")
         return mask.astype(bool), err
+
+    def refine_pnp(self, threshold, max_iterations, Rt=None, sample=None, want_arrays=True):
+        """Levenberg-Marquardt refinement of a pose over its inlier list (sfm_refine_pnp): Rt None = the winner of the
+        last ransac_pnp with its sample row, else a caller pose [3,4] with optional forced list entries sample int[4].
+        Returns (PnpRefinement, mask bool[n] or None, err [n] or None) under the reported pose."""
+        Ra = None if Rt is None else _f64(Rt).reshape(12)
+        sa = None if sample is None else np.ascontiguousarray(sample, dtype=np.int32).reshape(4)
+        rep = PnpRefinement()
+        mask = np.empty(self.n, dtype=np.uint8) if want_arrays else None
+        err = np.empty(self.n, dtype=np.float64) if want_arrays else None
+        self._ck(self.lib.sfm_refine_pnp(self.h, _ptr(Ra), _ptr(sa), float(threshold), int(max_iterations), C.byref(rep),
+                                         _ptr(mask), _ptr(err)), "sfm_refine_pnp")
+        return rep, (None if mask is None else mask.astype(bool)), err
 
     # -- essential matrix or homography -------------------------------------------------------
     def model_scores(self, E, H, K, sigma=1.0, homography_ratio=0.45, per_point=False):

@@ -3,8 +3,8 @@
 //   sfm_api.cu          context lifecycle, stream, errors, timing               sfm_misc.cuh
 //   sfm_ransac.cu       upload, sampler, E, H and PnP fit, K2 and its shape,    sfm_fit.cuh, sfm_score.cuh, sfm_homography.cuh,
 //                       K3, masks, batches, hypothesis-sharded scoring          sfm_pnp.cuh
-//   sfm_two_view.cu     pose/triangulation list API, tail, refinement           sfm_pose.cuh, sfm_hpose.cuh, sfm_tail.cuh,
-//                                                                               sfm_refine.cuh
+//   sfm_two_view.cu     pose/triangulation list API, tail, refinement (E, H,    sfm_pose.cuh, sfm_hpose.cuh, sfm_tail.cuh,
+//                       and the PnP pose)                                       sfm_refine.cuh
 //   sfm_model_select.cu essential matrix or homography                          sfm_select.cuh
 //   sfm_front_end.cu    matcher, cross-correlation, Harris                      sfm_match.cuh, sfm_harris.cuh
 //   sfm_nccl.cpp, sfm_sampler.cpp: host only, compiled by the host compiler
@@ -80,6 +80,8 @@ struct sfm_ctx {
     sfm_host::Buf selstate, selio, selpp;  // k_score_models: self-cleaning sums; models and results; per-correspondence errors
     sfm_host::Buf refstate, refpart, reftick, refrec, refrep;  // refinement: LM state, chunk partials, tickets, records, reports
     sfm_host::Buf ppts, pK, pmodels, pwin;  // PnP: records (PnpRec), K, poses [h][12], the winner or a caller's pose [12]
+    sfm_host::Buf prstate, prpart, pridx, przero, prio;  // PnP refinement: LM state, chunk partials, list + length,
+                                                          // self-cleaning tickets, pose / forced indices / report
     long long n = 0, h = 0, npairs = 1;
     long long first_len = 0;  // batched: correspondences of the first pair (what the AUTO pilot samples)
     long long batch_max_len = 0;  // batched: correspondences of the longest pair
@@ -100,6 +102,8 @@ struct sfm_ctx {
     double Estage[9] = {0};   // caller's E (stand-alone decomposition / pose), prescaled
     double Pstage[24] = {0};  // caller's P1, P2 (stand-alone triangulation), prescaled
     double hstage[18] = {0};  // H and K of sfm_decompose_homography, K of the homography tail, staged for async copies
+    double prstage[12] = {0};    // sfm_refine_pnp: the caller's pose and forced list entries, staged for the async copy
+    int32_t prforced[4] = {-1, -1, -1, -1};
     std::vector<sfm::SelectModels> sstage;  // the models of sfm_score_models / sfm_batch_score_models, staged for the async copy
     std::vector<double> Kbatch;        // the cameras of the current batched upload, [P][9] (the device copy is Ks)
     const void* occ_fn[4] = {nullptr, nullptr, nullptr, nullptr};  // scoring kernels whose launch configuration is cached
@@ -225,6 +229,8 @@ const double* winner_E_dev(sfm_ctx* c);
 // a caller's matrix outside [2^-100, 2^100] brought to [0.5, 1) by a power of two (sfm_two_view.cu)
 int prescale_exponent(const double* a, int n);
 void prescaled(const double* a, int n, int k, double* out);
+// k_pnp_mask: decision and value of every record under Rt_dev[12 * best->idx] (best != null) or Rt_dev, into mask / sed
+int pmask_launch(sfm_ctx* c, double thr, const double* Rt_dev, const sfm::Best* best_dev, double* winner_out);
 int batch_fetch_winners(sfm_ctx* c, int64_t npairs, size_t extra_pinned, char** extra);
 void batch_unpack_winners(const char* hp, int64_t npairs, double* E, int64_t* best_index, double* best_err,
                           int32_t* count_extra, int64_t* num_invalid);

@@ -1050,7 +1050,7 @@ static int score_p_launch(sfm_ctx* c, double thr, double min_extra, int agg, int
 }
 
 // decision and value of every record under the pose at Rt_dev[12 * best->idx] (best != null) or at Rt_dev
-static int pmask_launch(sfm_ctx* c, double thr, const double* Rt_dev, const Best* best_dev, double* winner_out) {
+int sfm_host::pmask_launch(sfm_ctx* c, double thr, const double* Rt_dev, const Best* best_dev, double* winner_out) {
     if (int r = c->mask.reserve((size_t)c->n)) return r;
     if (int r = c->sed.reserve((size_t)c->n * 8)) return r;
     c->tic(T_MASK);

@@ -40,8 +40,28 @@
 // launch exit at once), k_refine_finish (the refined selection record - the winner's index, sample row -1 - and the
 // per-pair report).  All are chain kernels (programmatic dependent launch); the host enqueues max_iter + 1 steps
 // without a round trip.
+//
+// MODEL_P, the absolute pose [R | t] of a new view (sfm_refine_pnp; one pose, npairs = 1, PnpRec records):
+//   list   k_refine_list compacts, in ascending record order, the records whose pnp_exact decision passes under the
+//          start pose at thr, plus up to 4 forced indices (the RANSAC winner's sample, or a caller's); decoupled
+//          look-back as in k_tail_mask, so the list - and with it every sum - does not depend on the grid.
+//   cost   the sum over the list of the squared reprojection error, two residuals per record: r0 = p0 / p2 - u,
+//          r1 = p1 / p2 - v, p = P (X, 1), P = K [R | t] formed by pnp_projection and p by pnp_terms' FMA order
+//          (refine_p_residuals).  Cheirality guard: a proposal under which a list record has p2 < 2^-537 (the scorer's
+//          depth rule) or a non-finite residual costs +inf and is rejected; at the start point that is `nonfinite`
+//          and the start pose is kept.  cost_ransac is the scorer's F / W summed under the unprojected start.
+//   model  R <- R exp([w]x) (refine_rotate), t <- t + dt: 6 parameters.  The start is the nearest rotation to the given
+//          R (one-sided Jacobi SVD, U's smallest column replaced so that det = +1) with the given t.  The cost floor
+//          is kRefineCostFloor times the sum of u^2 + v^2 over the list.
+//   report PnpRefineReport: the refined [R | t] (the unprojected start when not refined), the costs, the list length,
+//          iterations, status, rejected.  An empty list is converged at iteration 0 with cost 0 and the projected
+//          start.  The control is refine_control unchanged.
+// Scaling the world by 2^k (t with it) or the pixels and K's first two rows by 2^k changes every sum by an exact power
+// of two, and Marquardt's scaling cancels it: the report is bit-identical after exact rescaling while p2 stays above
+// 2^-537 and no sum overflows.
 #pragma once
 #include "sfm_device.cuh"
+#include "sfm_pnp_model.cuh"
 #include "sfm_pose_math.cuh"
 #include "sfm_types.h"
 
@@ -62,12 +82,13 @@ enum { REFINE_CONVERGED = 0, REFINE_MAX_ITER = 1, REFINE_STALLED = 2, REFINE_NO_
 template <int KIND> struct RefineDims;
 template <> struct RefineDims<MODEL_E> { static constexpr int NP = 5; };
 template <> struct RefineDims<MODEL_H> { static constexpr int NP = 8; };
+template <> struct RefineDims<MODEL_P> { static constexpr int NP = 6; };
 // partial sums: cost, cost of the RANSAC model (first evaluation only), sum of squared coordinates, J^T J upper triangle
 // (row-major), J^T r
 template <int KIND> __host__ __device__ constexpr int refine_nv() { return 3 + RefineDims<KIND>::NP * (RefineDims<KIND>::NP + 1) / 2 + RefineDims<KIND>::NP; }
 
 struct RefineState {
-    double x[12], px[12];   // accepted point, proposal: E: R[9], t[3]; H: h0..h7
+    double x[12], px[12];   // accepted point, proposal: E and P: R[9], t[3]; H: h0..h7
     double A[64], g[8];     // J^T J (full, row-major NP x NP) and J^T r at the accepted point
     double cost, lambda, cost_ransac, cost_start;
     long long num;
@@ -77,6 +98,15 @@ struct RefineState {
 // layout of sfm_refinement (include/sfm_b200.h)
 struct RefineReport {
     double model[9];
+    double cost_ransac, cost_start, cost_final;
+    long long num;
+    int iterations, status;
+    int rejected, reserved;
+};
+
+// layout of sfm_pnp_refinement (include/sfm_b200.h)
+struct PnpRefineReport {
+    double Rt[12];
     double cost_ransac, cost_start, cost_final;
     long long num;
     int iterations, status;
@@ -96,6 +126,25 @@ struct RefineArgs {
     SelectRecord* out_rec;        // [P]
     RefineReport* report;         // [P]
 };
+
+// MODEL_P's arguments: one pose (npairs 1; pts, offsets, rec, out_rec and report unused).  A type of its own, so that
+// the E and H kernels keep their parameter block.
+struct PnpRefineArgs : RefineArgs {
+    const PnpRec* ppts;           // [n] the records
+    long long n;
+    const double* K;              // [9]
+    const double* start;          // [12] the RANSAC winner or the caller's pose, row-major [R | t]
+    const int32_t* forced;        // [4] list entries whatever their decision (-1 = none), or null
+    double thr;
+    unsigned long long* list_agg; // [ceil(n / kListPerBlock)] look-back state of k_refine_list, zero on entry and exit
+    unsigned* list_ticket;        // [2] zero on entry and on exit
+    long long* list_out;          // [n + 1] k_refine_list's list, then its length (what idx and num point at)
+    double* pose_out;             // [12] the reported pose (k_pnp_mask's input)
+    PnpRefineReport* preport;
+};
+
+template <int KIND> struct RefineArgsOf { using type = RefineArgs; };
+template <> struct RefineArgsOf<MODEL_P> { using type = PnpRefineArgs; };
 
 // ---- small 3x3 helpers (row-major) ----
 __host__ __device__ __forceinline__ void refine_skew(const double* v, double (&S)[9]) {
@@ -229,6 +278,66 @@ __host__ __device__ inline void refine_rotate(const double* R, const double* w, 
     refine_mul3(R, X, out);
 }
 
+// The two reprojection residuals of one PnP record under P = K [R | t] (pnp_projection) and their rows of the Jacobian
+// over (w0, w1, w2, t0, t1, t2) of R <- R exp([w]x), t <- t + dt.  p = P (X, 1) in pnp_terms' FMA order; dp/dw_k =
+// K R (e_k x X), and K R is P's left 3 x 3 block; dp/dt_k = K e_k.  Then d(p_i / p2) = (dp_i - (p_i / p2) dp2) / p2.
+// Returns p2 (the cheirality guard tests it).
+__host__ __device__ __forceinline__ double refine_p_residuals(const double* P, const double* K, double X, double Y,
+                                                              double Z, double u, double v, double (&r)[2],
+                                                              double (&J)[2][6]) {
+    const double p0 = fma(P[0], X, fma(P[1], Y, fma(P[2], Z, P[3])));
+    const double p1 = fma(P[4], X, fma(P[5], Y, fma(P[6], Z, P[7])));
+    const double p2 = fma(P[8], X, fma(P[9], Y, fma(P[10], Z, P[11])));
+    const double ip = 1.0 / p2;
+    const double u0 = p0 * ip, u1 = p1 * ip;
+    r[0] = u0 - u;
+    r[1] = u1 - v;
+    double dp[3][6];
+    for (int i = 0; i < 3; ++i) {
+        const double* Pi = P + 4 * i;
+        dp[i][0] = fma(Pi[2], Y, -Pi[1] * Z);  // e_0 x X = (0, -Z, Y)
+        dp[i][1] = fma(Pi[0], Z, -Pi[2] * X);  // e_1 x X = (Z, 0, -X)
+        dp[i][2] = fma(Pi[1], X, -Pi[0] * Y);  // e_2 x X = (-Y, X, 0)
+        dp[i][3] = K[3 * i];
+        dp[i][4] = K[3 * i + 1];
+        dp[i][5] = K[3 * i + 2];
+    }
+    for (int k = 0; k < 6; ++k) {
+        J[0][k] = fma(-u0, dp[2][k], dp[0][k]) * ip;
+        J[1][k] = fma(-u1, dp[2][k], dp[1][k]) * ip;
+    }
+    return p2;
+}
+
+// The rotation nearest to M (3 x 3 row-major) in the Frobenius norm: M = U S V^T by one-sided Jacobi (M V = U S), the
+// columns of U normalised, the one of the smallest singular value replaced by the cross product of the other two (so
+// det U = +1 = det V and a reflection is projected onto a rotation), R = U V^T.
+__device__ inline void refine_nearest_rotation(const double* M, double* R) {
+    double g[9], V[9];
+    for (int k = 0; k < 9; ++k) g[k] = M[k];
+    jacobi_svd_onesided<3, 3>(g, V, 30);
+    double sv[3];
+    for (int c = 0; c < 3; ++c) sv[c] = sqrt(fma(g[c], g[c], fma(g[3 + c], g[3 + c], g[6 + c] * g[6 + c])));
+    int m = 0;
+    if (sv[1] < sv[m]) m = 1;
+    if (sv[2] < sv[m]) m = 2;
+    const int a = (m + 1) % 3, b = (m + 2) % 3;  // (a, b, m) cyclic: u_m = u_a x u_b
+    double ua[3], ub[3], um[3];
+    for (int k = 0; k < 3; ++k) {
+        ua[k] = g[3 * k + a] / sv[a];
+        ub[k] = g[3 * k + b] / sv[b];
+    }
+    refine_cross(ua, ub, um);
+    double U[9];
+    for (int k = 0; k < 3; ++k) {
+        U[3 * k + a] = ua[k];
+        U[3 * k + b] = ub[k];
+        U[3 * k + m] = um[k];
+    }
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) R[3 * i + j] = fma(U[3 * i + 2], V[3 * j + 2], fma(U[3 * i + 1], V[3 * j + 1], U[3 * i] * V[3 * j]));
+}
+
 // First chunk partial of the pair whose records start at pbase: pair q owns at most ceil(len_q / kRefineChunk) chunks,
 // so floor(pbase / kRefineChunk) + pair never overlaps the previous pair's and the buffer grows with the total length,
 // not with the number of pairs times the longest one.
@@ -240,13 +349,131 @@ __device__ __forceinline__ void refine_load_proposal(const RefineState* s, doubl
     for (int k = 0; k < 12; ++k) x[k] = __ldcg(s->px + k);
 }
 
+// ---- MODEL_P: the inlier list of the start pose, ascending (T1's decoupled look-back over PnpRec records) ----
+constexpr int kListBlock = 256;
+constexpr int kListPerBlock = 4 * kListBlock;  // records per block
+
+template <int KIND, class Args = typename RefineArgsOf<KIND>::type>
+__global__ void __launch_bounds__(kListBlock) k_refine_list(const Args a) {
+    static_assert(KIND == MODEL_P, "the E and H lists are T1's (k_tail_mask)");
+    chain_enter();
+    __shared__ unsigned s_bid;
+    __shared__ int warp_cnt[4][kListBlock / 32];
+    __shared__ long long s_prefix;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nblk = gridDim.x;
+    if (tid == 0) s_bid = atomicAdd(&a.list_ticket[0], 1u);  // ticket order = start order: predecessors are running
+    __syncthreads();
+    const int bid = (int)s_bid;
+    double P[12];
+    pnp_projection(a.K, a.start, P);
+    long long forced[4];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) forced[q] = a.forced ? a.forced[q] : -1;
+    const long long base = (long long)bid * kListPerBlock;
+    bool f[4];
+    unsigned b[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const long long i = base + k * kListBlock + tid;
+        f[k] = false;
+        if (i < a.n) {
+            double v;
+            bool in = pnp_exact(P, a.ppts[i], a.thr, v);
+#pragma unroll
+            for (int q = 0; q < 4; ++q) in |= forced[q] == i;
+            f[k] = in;
+        }
+        b[k] = __ballot_sync(0xffffffffu, f[k]);
+        if (lane == 0) warp_cnt[k][warp] = __popc(b[k]);
+    }
+    __syncthreads();
+    int total = 0;
+    if (tid == 0) {
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+            for (int w = 0; w < kListBlock / 32; ++w) total += warp_cnt[k][w];
+        atomicExch(&a.list_agg[bid], (unsigned long long)total | (1ull << 62));  // value and flag in one word
+    }
+    if (warp == 0) {
+        long long sum = 0;
+        for (int j0 = 0; j0 < bid; j0 += 32) {
+            const int j = j0 + lane;
+            long long v = 0;
+            if (j < bid) {
+                unsigned long long w;
+                do { w = *reinterpret_cast<volatile unsigned long long*>(a.list_agg + j); } while (!(w & (1ull << 62)));
+                v = (long long)(w & ~(1ull << 62));
+            }
+#pragma unroll
+            for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
+            sum += v;
+        }
+        if (lane == 0) s_prefix = sum;
+    }
+    __syncthreads();
+    long long off = s_prefix;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        long long o = off;
+        for (int w = 0; w < kListBlock / 32; ++w) {
+            if (w < warp) o += warp_cnt[k][w];
+            off += warp_cnt[k][w];
+        }
+        if (f[k]) a.list_out[o + __popc(b[k] & ((1u << lane) - 1u))] = base + k * kListBlock + tid;
+    }
+    if (bid == nblk - 1 && tid == 0) a.list_out[a.n] = s_prefix + total;
+    // the last block past the look-back clears the state for the next call
+    __syncthreads();
+    if (tid == 0) {
+        __threadfence();
+        if (atomicAdd(&a.list_ticket[1], 1u) == (unsigned)(nblk - 1)) {
+            for (int j = 0; j < nblk; ++j) a.list_agg[j] = 0;
+            a.list_ticket[0] = 0;
+            a.list_ticket[1] = 0;
+        }
+    }
+}
+
 // ---- start point and per-pair state ----
-template <int KIND>
-__global__ void __launch_bounds__(128) k_refine_init(const RefineArgs a) {
+template <int KIND, class Args = typename RefineArgsOf<KIND>::type>
+__global__ void __launch_bounds__(128) k_refine_init(const Args a) {
     chain_enter();
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= a.npairs) return;
     RefineState& s = a.state[p];
+    if constexpr (KIND == MODEL_P) {  // the nearest rotation to the start's R, and its t
+        s.num = a.num[0];
+        s.iter = 0;
+        s.evals = 0;
+        s.rejected = 0;
+        s.pad = 0;
+        s.lambda = kRefineLambda0;
+        s.cost = s.cost_ransac = s.cost_start = __longlong_as_double(0x7ff8000000000000LL);
+        s.status = REFINE_RUNNING;
+        s.done = 0;
+        double m[12];
+        bool finite = true;
+        for (int k = 0; k < 12; ++k) {
+            m[k] = a.start[k];
+            finite = finite && isfinite(m[k]);
+            s.px[k] = s.x[k] = 0.0;
+        }
+        if (finite) {
+            const double M[9] = {m[0], m[1], m[2], m[4], m[5], m[6], m[8], m[9], m[10]};
+            double R[9];
+            refine_nearest_rotation(M, R);
+            for (int k = 0; k < 9; ++k) {
+                s.px[k] = R[k];
+                finite = finite && isfinite(R[k]);
+            }
+            for (int k = 0; k < 3; ++k) s.px[9 + k] = m[4 * k + 3];
+        }
+        if (!finite) {
+            s.status = REFINE_NONFINITE;
+            s.done = 1;
+        }
+        return;
+    }
     const SelectRecord& rec = a.rec[p];
     const double nan = __longlong_as_double(0x7ff8000000000000LL);
     s.num = a.num[p];
@@ -329,7 +556,7 @@ __device__ __noinline__ void refine_control(RefineState& s, const double* tot, i
     bool accept;
     if (s.evals == 0) {  // the start point
         s.cost_start = c;
-        s.cost_ransac = KIND == MODEL_E ? tot[1] : c;
+        s.cost_ransac = (KIND == MODEL_E || KIND == MODEL_P) ? tot[1] : c;
         if (!isfinite(c)) {
             s.status = REFINE_NONFINITE;
             s.done = 1;
@@ -406,21 +633,25 @@ __device__ __noinline__ void refine_control(RefineState& s, const double* tot, i
         for (int k = 0; k < 3; ++k) t[k] = fma(d[3], b1[k], fma(d[4], b2[k], s.x[9 + k]));
         const double inv = 1.0 / sqrt(fma(t[0], t[0], fma(t[1], t[1], t[2] * t[2])));
         for (int k = 0; k < 3; ++k) s.px[9 + k] = t[k] * inv;
-    } else {
+    } else if constexpr (KIND == MODEL_H) {
         for (int k = 0; k < 8; ++k) s.px[k] = s.x[k] + d[k];
+    } else {
+        refine_rotate(s.x, d, s.px);
+        for (int k = 0; k < 3; ++k) s.px[9 + k] = s.x[9 + k] + d[3 + k];
     }
 }
 
 // ---- one LM iteration: evaluate the pair's proposal over its inlier list, then the last block steps ----
-template <int KIND>
-__global__ void __launch_bounds__(kRefineBlock) k_refine_step(const RefineArgs a) {
+template <int KIND, class Args = typename RefineArgsOf<KIND>::type>
+__global__ void __launch_bounds__(kRefineBlock) k_refine_step(const Args a) {
     chain_enter();
     constexpr int NP = RefineDims<KIND>::NP;
     constexpr int NV = refine_nv<KIND>();
     constexpr int NW = kRefineBlock / 32;
-    __shared__ double s_model[9];
-    __shared__ double s_M[45];       // E: dE / dtheta
-    __shared__ double s_ransac[9];   // E: the RANSAC model (first evaluation only)
+    __shared__ double s_model[KIND == MODEL_P ? 12 : 9];   // P: K [R | t] of the proposal
+    __shared__ double s_M[45];                             // E: dE / dtheta; P: K
+    __shared__ double s_ransac[KIND == MODEL_P ? 12 : 9];  // the RANSAC model (E) or K [R | t] of the unprojected
+                                                           // start (P), read by the first evaluation only
     __shared__ double s_warp[NW][NV];
     __shared__ double s_tot[NV];
     __shared__ int s_last;
@@ -444,9 +675,17 @@ __global__ void __launch_bounds__(kRefineBlock) k_refine_step(const RefineArgs a
             for (int k = 0; k < 9; ++k) s_model[k] = E[k];
             for (int k = 0; k < 45; ++k) s_M[k] = M[k];
             for (int k = 0; k < 9; ++k) s_ransac[k] = a.rec[pair].E[k];
-        } else {
+        } else if constexpr (KIND == MODEL_H) {
             for (int k = 0; k < 8; ++k) s_model[k] = x[k];
             s_model[8] = 1.0;
+        } else {
+            const double m[12] = {x[0], x[1], x[2], x[9], x[3], x[4], x[5], x[10], x[6], x[7], x[8], x[11]};
+            double P[12];
+            pnp_projection(a.K, m, P);
+            for (int k = 0; k < 12; ++k) s_model[k] = P[k];
+            for (int k = 0; k < 9; ++k) s_M[k] = a.K[k];
+            pnp_projection(a.K, a.start, P);
+            for (int k = 0; k < 12; ++k) s_ransac[k] = P[k];
         }
     }
     __syncthreads();
@@ -458,7 +697,36 @@ __global__ void __launch_bounds__(kRefineBlock) k_refine_step(const RefineArgs a
 #pragma unroll
         for (int half = 0; half < 2; ++half) {
             const long long i = ch * kRefineChunk + half * kRefineBlock + tid;
-            if (i < num) {
+            if constexpr (KIND == MODEL_P) {
+                if (i < num) {
+                    const PnpRec c = a.ppts[a.idx[i]];
+                    acc[2] += fma(c.u, c.u, c.v * c.v);
+                    double r[2], J[2][6];
+                    const double p2 = refine_p_residuals(s_model, s_M, c.X, c.Y, c.Z, c.u, c.v, r, J);
+                    if (first) {
+                        double pm[12];
+#pragma unroll
+                        for (int k = 0; k < 12; ++k) pm[k] = s_ransac[k];
+                        acc[1] += pnp_value(pnp_terms(pm, c.X, c.Y, c.Z, c.u, c.v));
+                    }
+                    // cheirality guard: the scorer's depth rule and finite residuals, else the proposal costs +inf
+                    if (!(p2 >= 0x1p-537) || !isfinite(r[0]) || !isfinite(r[1])) {
+                        acc[0] = __longlong_as_double(0x7ff0000000000000LL);
+                    } else {
+#pragma unroll
+                        for (int k = 0; k < 2; ++k) {
+                            acc[0] = fma(r[k], r[k], acc[0]);
+                            int q = 3;
+#pragma unroll
+                            for (int p = 0; p < 6; ++p)
+#pragma unroll
+                                for (int m = p; m < 6; ++m, ++q) acc[q] = fma(J[k][p], J[k][m], acc[q]);
+#pragma unroll
+                            for (int p = 0; p < 6; ++p) acc[q + p] = fma(J[k][p], r[k], acc[q + p]);
+                        }
+                    }
+                }
+            } else if (i < num) {
                 const Corr c = a.pts[pbase + a.idx[pbase + i]];
                 acc[2] += fma(c.xa, c.xa, fma(c.ya, c.ya, fma(c.xb, c.xb, c.yb * c.yb)));
                 if constexpr (KIND == MODEL_E) {
@@ -540,12 +808,35 @@ __global__ void __launch_bounds__(kRefineBlock) k_refine_step(const RefineArgs a
 }
 
 // ---- the refined record and the report ----
-template <int KIND>
-__global__ void __launch_bounds__(128) k_refine_finish(const RefineArgs a) {
+template <int KIND, class Args = typename RefineArgsOf<KIND>::type>
+__global__ void __launch_bounds__(128) k_refine_finish(const Args a) {
     chain_enter();
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= a.npairs) return;
     const RefineState& s = a.state[p];
+    if constexpr (KIND == MODEL_P) {  // the report and the pose k_pnp_mask reads
+        PnpRefineReport rep;
+        rep.cost_ransac = s.cost_ransac;
+        rep.cost_start = s.cost_start;
+        rep.cost_final = s.cost;
+        rep.num = s.num;
+        rep.iterations = s.iter;
+        rep.rejected = s.rejected;
+        rep.reserved = 0;
+        rep.status = s.status;
+        if (s.status == REFINE_NONFINITE) {
+            for (int k = 0; k < 12; ++k) rep.Rt[k] = a.start[k];
+            rep.cost_final = rep.cost_start;
+        } else {
+            for (int r = 0; r < 3; ++r) {
+                for (int c = 0; c < 3; ++c) rep.Rt[4 * r + c] = s.x[3 * r + c];
+                rep.Rt[4 * r + 3] = s.x[9 + r];
+            }
+        }
+        for (int k = 0; k < 12; ++k) a.pose_out[k] = rep.Rt[k];
+        *a.preport = rep;
+        return;
+    }
     const SelectRecord& rec = a.rec[p];
     SelectRecord out = rec;
     RefineReport rep;

@@ -14,6 +14,7 @@ using namespace sfm_host;
 
 static_assert(sizeof(PoseSet) == sizeof(sfm_poses), "PoseSet/sfm_poses layout mismatch");
 static_assert(sizeof(RefineReport) == sizeof(sfm_refinement), "RefineReport / sfm_refinement layout mismatch");
+static_assert(sizeof(PnpRefineReport) == sizeof(sfm_pnp_refinement), "PnpRefineReport / sfm_pnp_refinement layout mismatch");
 
 int sfm_get_refinement(sfm_ctx* c, sfm_refinement* out, int64_t P) {
     if (int r = use(c)) return r;
@@ -187,6 +188,86 @@ static int refine_launch(sfm_ctx* c, int kind, const SelectRecord* rec_dev, long
     else CU(chain_launch(c, k_refine_finish<MODEL_E>, gp, dim3(128), 0, a));
     if (int r = check_launch(c, "k_refine_finish")) return r;
     *rec_out = a.out_rec;
+    return 0;
+}
+
+// Least-squares refinement of a pose over its inlier list (sfm_refine.cuh, MODEL_P): list, init, max_iterations + 1
+// LM steps, finish and, when wanted, the mask under the reported pose - enqueued back to back, one synchronisation.
+int sfm_refine_pnp(sfm_ctx* c, const double* Rt, const int32_t* sample, double thr, int max_iterations,
+                   sfm_pnp_refinement* out, uint8_t* mask, double* err) {
+    if (int r = use(c)) return r;
+    if (!out) return fail(SFM_ERR_ARG, "out is null");
+    if (!c->has_pnp) return fail(SFM_ERR_STATE, "no PnP records loaded");
+    if (max_iterations < 1) return fail(SFM_ERR_ARG, "max_iterations must be >= 1, got %d", max_iterations);
+    if (!std::isfinite(thr)) return fail(SFM_ERR_ARG, "the threshold must be finite");
+    if (sample)
+        for (int k = 0; k < 4; ++k)
+            if (sample[k] < 0 || sample[k] >= c->n) return fail(SFM_ERR_ARG, "sample index %d outside [0, %lld)", sample[k], c->n);
+    if (!Rt && (!c->pnp_models || !c->has_score || !c->winner_set || c->winner_local < 0))
+        return fail(SFM_ERR_STATE, "no pose winner: pass Rt or run sfm_ransac_pnp first");
+    const long long n = c->n;
+    const int nv = refine_nv<MODEL_P>();
+    const long long nblk = (n + kListPerBlock - 1) / kListPerBlock;
+    if (int r = c->prstate.reserve(sizeof(RefineState))) return r;
+    if (int r = c->prpart.reserve((size_t)(n / kRefineChunk + 2) * nv * 8)) return r;
+    if (int r = c->pridx.reserve((size_t)n * 8 + 8)) return r;
+    // tickets of the step (1) and of the list (2), then the list's look-back words: zero between calls
+    if (int r = reserve_zeroed(c, c->przero, 16 + (size_t)nblk * 8)) return r;
+    if (int r = c->prio.reserve(96 + 96 + 16 + sizeof(PnpRefineReport))) return r;
+    double* d_start = c->prio.as<double>();
+    double* d_pose = d_start + 12;
+    int32_t* d_forced = reinterpret_cast<int32_t*>(d_pose + 12);
+    PnpRefineReport* d_rep = reinterpret_cast<PnpRefineReport*>(d_pose + 14);
+    PnpRefineArgs a;
+    memset(&a, 0, sizeof a);
+    if (Rt) {
+        memcpy(c->prstage, Rt, 96);  // staged in the context: the async copy must not read caller memory later
+        CU(cudaMemcpyAsync(d_start, c->prstage, 96, cudaMemcpyHostToDevice, c->stream));
+        a.start = d_start;
+        if (sample) {
+            memcpy(c->prforced, sample, 16);
+            CU(cudaMemcpyAsync(d_forced, c->prforced, 16, cudaMemcpyHostToDevice, c->stream));
+            a.forced = d_forced;
+        }
+    } else {  // the winner of the last sfm_ransac_pnp and its sample row (K3's record)
+        a.start = c->pmodels.as<double>() + 12 * c->winner_local;
+        a.forced = c->record.as<SelectRecord>()->sample;
+    }
+    a.list_out = c->pridx.as<long long>();
+    a.idx = a.list_out;
+    a.num = a.list_out + n;
+    a.state = c->prstate.as<RefineState>();
+    a.partial = c->prpart.as<double>();
+    a.ticket = c->przero.as<unsigned>();
+    a.list_ticket = a.ticket + 2;
+    a.list_agg = c->przero.as<unsigned long long>() + 2;
+    a.npairs = 1;
+    a.max_iter = max_iterations;
+    a.ppts = c->ppts.as<PnpRec>();
+    a.n = n;
+    a.K = c->pK.as<double>();
+    a.thr = thr;
+    a.pose_out = d_pose;
+    a.preport = d_rep;
+    const long long maxch = (n + kRefineChunk - 1) / kRefineChunk;  // the list is at most n long
+    const dim3 gs((unsigned)(maxch < 4ll * c->sm_count ? maxch : 4ll * c->sm_count));
+    CU(chain_launch(c, k_refine_list<MODEL_P>, dim3((unsigned)nblk), dim3(kListBlock), 0, a));
+    if (int r = check_launch(c, "k_refine_list")) return r;
+    CU(chain_launch(c, k_refine_init<MODEL_P>, dim3(1), dim3(128), 0, a));
+    if (int r = check_launch(c, "k_refine_init")) return r;
+    for (int it = 0; it <= max_iterations; ++it) {
+        CU(chain_launch(c, k_refine_step<MODEL_P>, gs, dim3(kRefineBlock), 0, a));
+        if (int r = check_launch(c, "k_refine_step")) return r;
+    }
+    CU(chain_launch(c, k_refine_finish<MODEL_P>, dim3(1), dim3(128), 0, a));
+    if (int r = check_launch(c, "k_refine_finish")) return r;
+    if (mask || err) {
+        if (int r = pmask_launch(c, thr, d_pose, nullptr, nullptr)) return r;
+        if (mask) CU(cudaMemcpyAsync(mask, c->mask.p, (size_t)n, cudaMemcpyDeviceToHost, c->stream));
+        if (err) CU(cudaMemcpyAsync(err, c->sed.p, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream));
+    }
+    CU(cudaMemcpyAsync(out, d_rep, sizeof(PnpRefineReport), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
     return 0;
 }
 

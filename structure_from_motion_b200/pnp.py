@@ -23,6 +23,29 @@ _SAMPLE = 4  # points per minimal sample
 
 
 @dataclasses.dataclass
+class PnpRefinement:
+    R: np.ndarray                 # (3,3) refined rotation (the start pose's R when not refined)
+    t: np.ndarray                 # (3,)
+    cost_ransac: float            # the start pose's summed squared reprojection error over the list (px^2)
+    cost_start: float             # the same at the start point (R projected onto the rotations)
+    cost_final: float             # at the reported pose, <= cost_start
+    num: int                      # records in the list
+    iterations: int               # proposals evaluated
+    status: str                   # converged, max_iterations, stalled or nonfinite
+    rejected: int                 # of those, proposals rejected
+    mask: np.ndarray              # bool[n]: inlier decision under the reported pose (no forced samples)
+    err: np.ndarray               # float64[n]: squared reprojection error under the reported pose (px^2)
+
+
+def _refinement(rep, mask, err) -> PnpRefinement:
+    Rt = np.array(rep.Rt[:], dtype=np.float64).reshape(3, 4)
+    return PnpRefinement(R=Rt[:, :3].copy(), t=Rt[:, 3].copy(), cost_ransac=float(rep.cost_ransac),
+                         cost_start=float(rep.cost_start), cost_final=float(rep.cost_final), num=int(rep.num),
+                         iterations=int(rep.iterations), status=_native.REFINE_STATUS[int(rep.status)],
+                         rejected=int(rep.rejected), mask=mask, err=err)
+
+
+@dataclasses.dataclass
 class PnpResult:
     R: np.ndarray                 # (3,3) rotation, world -> camera
     t: np.ndarray                 # (3,) translation: x_cam = R X + t
@@ -36,6 +59,7 @@ class PnpResult:
     sample: np.ndarray            # int32[4] the winner's minimal sample
     num_invalid: int              # degenerate samples (skipped)
     first_invalid: int            # earliest such iteration, -1 if none
+    refinement: Optional[PnpRefinement] = None  # refine_iterations > 0: the winner refined over its inliers
 
 
 def _camera(camera_matrix) -> np.ndarray:
@@ -68,6 +92,7 @@ def ransac_pnp_arrays(
     selection: str = "min_error",
     engine: Optional[_native.Engine] = None,
     table: Optional[np.ndarray] = None,
+    refine_iterations: int = 0,
 ) -> PnpResult:
     """RANSAC absolute pose from world points [n,3] and their pixels [n,2] in the new view (n >= 8).
 
@@ -76,7 +101,13 @@ def ransac_pnp_arrays(
              "device" — Philox sampler on the GPU (``seed``, ``hyp_offset`` for split runs); "table" — the given int
              table, [H,4] or [H,8] (columns 0-3 are the sample).
     threshold: on the squared reprojection error in px^2, finite.  Defaults: 100 iterations, RMS, 0 extra inliers.
+    refine_iterations > 0: the final winner (after the near-tie replay) is refined over its inliers plus its sample by
+             Levenberg-Marquardt on the reprojection error (``refine_pnp_arrays``) into ``refinement``; R, t and
+             everything else stay the RANSAC result.  0 (the default) makes no refinement call.
     """
+    refine_iterations = int(refine_iterations)
+    if refine_iterations < 0:
+        raise ValueError(f"refine_iterations must be >= 0, got {refine_iterations}")
     if max_iterations is None:
         max_iterations = 100  # ransac.py:48-49
     if min_num_extra_inliers is None:
@@ -131,6 +162,9 @@ def ransac_pnp_arrays(
     mask = np.asarray(mask).astype(bool)
     sample, inliers = _inlier_order(best, sampler, table, ref, mask, _SAMPLE)
     Rt = np.array(Rt, dtype=np.float64).reshape(3, 4)
+    refinement = None
+    if refine_iterations > 0:  # the winner as settled above, with its own sample: the reference's tie rule holds
+        refinement = _refinement(*eng.refine_pnp(threshold, refine_iterations, Rt=Rt, sample=sample))
     return PnpResult(
         R=Rt[:, :3].copy(),
         t=Rt[:, 3].copy(),
@@ -143,6 +177,7 @@ def ransac_pnp_arrays(
         sample=sample,
         num_invalid=int(best.num_invalid),
         first_invalid=int(best.first_invalid),
+        refinement=refinement,
     )
 
 
@@ -173,3 +208,24 @@ def reprojection_error_arrays(R, t, camera_matrix, points_3d, pts, threshold: fl
     eng = engine or _native.get_engine()
     eng.upload_pnp(X, x, K)
     return eng.pnp_mask(Rt, threshold)
+
+
+def refine_pnp_arrays(R, t, camera_matrix, points_3d, pts, threshold: float, max_iterations: int = 20, sample=None,
+                      engine: Optional[_native.Engine] = None) -> PnpRefinement:
+    """Refine a caller's pose [R | t] over its inlier list by Levenberg-Marquardt on the squared reprojection error.
+
+    The list is the records whose decision passes under [R | t] at ``threshold`` (px^2), plus the optional forced
+    indices ``sample`` (4 ints), in ascending order; it stays fixed while the refinement runs.  The start is the
+    rotation nearest to R (a reflection is projected onto a rotation) and t.  A start under which a list record lies
+    behind the camera, or with a non-finite entry, reports ``nonfinite`` and keeps the pose."""
+    K = _camera(camera_matrix)
+    X, x = _records(points_3d, pts)
+    if not np.isfinite(threshold):
+        raise ValueError(f"the threshold must be finite, got {threshold}")
+    if int(max_iterations) < 1:
+        raise ValueError(f"max_iterations must be >= 1, got {max_iterations}")
+    Rt = np.concatenate([np.asarray(R, dtype=np.float64).reshape(3, 3),
+                         np.asarray(t, dtype=np.float64).reshape(3, 1)], axis=1)
+    eng = engine or _native.get_engine()
+    eng.upload_pnp(X, x, K)
+    return _refinement(*eng.refine_pnp(threshold, int(max_iterations), Rt=Rt, sample=sample))
