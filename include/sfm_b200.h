@@ -286,6 +286,61 @@ int sfm_recover_pose_pixels(sfm_ctx *ctx, const double *E, const double *K, cons
 int sfm_triangulate(sfm_ctx *ctx, const double *P1, const double *P2, const double *xa,
                     const double *ya, const double *xb, const double *yb, int64_t stride, int64_t m,
                     double *X);
+
+/* ---- multi-view triangulation of tracks (csrc/sfm_tracks.cuh) -----------------------------
+ * One 3-D point per track from its observations in V registered views, outlier observations rejected.
+ *   cameras      K double[V][9] (finite, non-singular, upper triangular with K[2,2] = 1) and Rt double[V][12] (finite,
+ *                world to camera, x_cam = R X + t, the PnP convention); P_c = K_c [R_c | t_c] in the PnP order.
+ *   tracks       CSR: offsets int64[T+1] (offsets[0] = 0, non-decreasing, M = offsets[T]), view int32[M] in [0, V),
+ *                x double[M][2] pixels.  At most SFM_TRACK_MAX_OBSERVATIONS observations per track.
+ *   decision     observation (u, v) of view c under X: the PnP record rule under P_c (p2 >= 2^-537, F < inf,
+ *                F <= threshold p2^2), value F / p2^2 in px^2.
+ *   per track    1. every pair (i < j) of its observations, in lexicographic order, triangulated by the two-view DLT;
+ *                   a candidate iff both pass under its point; the winner has the most passing observations, then the
+ *                   smaller sum of their values (in observation order), then the lower pair index.  No candidate:
+ *                   SFM_TRACK_NO_PAIR; fewer than 2 observations: SFM_TRACK_SHORT (X NaN for both, and only these).
+ *                2. the N-view DLT over the winner's passing observations (a streaming Givens QR of the two-view rows;
+ *                   the pair's point itself when only its two pass).
+ *                3. refine_iterations > 0: Levenberg-Marquardt on X over the observations passing under the linear
+ *                   point (fixed), residuals p0 / p2 - u and p1 / p2 - v, the control of sfm_refine_pnp (lambda 1e-3,
+ *                   x / 10, Ftol 1e-12, Xtol 1e-9, lambda cap 1e16, refine_iterations evaluated proposals, cost floor
+ *                   1e-24 sum(u^2 + v^2)); a proposal with a list observation at p2 < 2^-537 or a non-finite residual
+ *                   costs +inf.
+ *                4. under the reported X: mask / err of every observation, num_inliers, angle = the largest angle
+ *                   (radians) between the lines of sight from two passing observations' camera centres -R^T t to X,
+ *                   atan2(|a x b|, |a . b|) in [0, pi/2] (opposite rays, a point between two centres, count as
+ *                   parallel), 0 with fewer than two; status OK iff num_inliers >= min_views and
+ *                   angle >= min_angle_deg * (pi / 180), else FEW_INLIERS (num_inliers short) or SMALL_ANGLE.
+ *   frame        the call runs in one frame in which every P's fourth column (K t) is scaled by 2^-s, s the binary
+ *                exponent of the largest |t| entry over all views, and reports X 2^s.  The DLT's minimum depends on
+ *                the frame; this one makes a world scaled by 2^k (t with it) give bit-identical reports after exact
+ *                rescaling, and pixels with K's first two rows scaled by 2^k (threshold by 4^k) the same decisions.
+ * A track's bits depend only on its observations and the cameras: not on the other tracks, their order or the split of
+ * a batch over calls.  Outputs may be NULL: X double[T][3], status int32[T] (enum sfm_track_status), num_inliers
+ * int32[T], angle double[T], mask uint8[M], err double[M], refine_report sfm_track_refinement[T] (written only when
+ * refine_iterations > 0; status SFM_REFINE_NO_MODEL for SHORT and NO_PAIR tracks).  SFM_ERR_ARG, before any launch, for
+ * a view index outside [0, V), malformed offsets, a track longer than SFM_TRACK_MAX_OBSERVATIONS, a non-finite Rt, a
+ * bad K, a non-finite threshold or min_angle_deg, min_views < 2 or refine_iterations < 0. */
+#define SFM_TRACK_MAX_OBSERVATIONS 64
+enum sfm_track_status {
+    SFM_TRACK_OK = 0,
+    SFM_TRACK_SHORT = 1,        /* fewer than 2 observations                                   */
+    SFM_TRACK_NO_PAIR = 2,      /* no pair whose own two observations pass under its point     */
+    SFM_TRACK_FEW_INLIERS = 3,  /* num_inliers < min_views under the reported X                */
+    SFM_TRACK_SMALL_ANGLE = 4   /* the largest ray angle between passing observations is below min_angle_deg */
+};
+typedef struct sfm_track_refinement {
+    double cost_start;             /* cost at the linear point                          */
+    double cost_final;             /* cost at the reported point, <= cost_start         */
+    int32_t num;                   /* observations in the list                          */
+    int32_t iterations, status, rejected;   /* status: enum sfm_refine_status          */
+} sfm_track_refinement;
+int sfm_triangulate_tracks(sfm_ctx *ctx, const double *K, const double *Rt, int32_t V, const int64_t *offsets, int64_t T,
+                           const int32_t *view, const double *x, double threshold, double min_angle_deg,
+                           int32_t min_views, int32_t refine_iterations, double *X, int32_t *status,
+                           int32_t *num_inliers, double *angle, uint8_t *mask, double *err,
+                           sfm_track_refinement *refine_report);
+
 /* Fused tail of the pipeline for the current winner (apps/sfm.py:110-186): inliers of the
  * winner -> decomposition -> cheirality vote -> triangulation of the passing inliers with
  * P1 = K[I|0], P2 = K[R|t], all on the device.  inlier_idx int64[cap] receives the indices

@@ -62,6 +62,13 @@ class PnpRefinement(C.Structure):
                 ("rejected", C.c_int32), ("reserved", C.c_int32)]
 
 
+class TrackRefinement(C.Structure):
+    _fields_ = [("cost_start", C.c_double), ("cost_final", C.c_double), ("num", C.c_int32), ("iterations", C.c_int32),
+                ("status", C.c_int32), ("rejected", C.c_int32)]
+
+
+TRACK_STATUS = {0: "ok", 1: "short", 2: "no_pair", 3: "few_inliers", 4: "small_angle"}
+
 REFINE_STATUS = {0: "converged", 1: "max_iterations", 2: "stalled", 3: "no_model", 4: "nonfinite"}
 
 _P = C.c_void_p
@@ -111,6 +118,8 @@ _SIGNATURES = {
     "sfm_recover_pose_pixels": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int64, C.c_int64, C.c_double,
                                           C.POINTER(Poses), _P]),
     "sfm_triangulate": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int64, C.c_int64, _P]),
+    "sfm_triangulate_tracks": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int64, _P, _P, C.c_double, C.c_double, C.c_int32,
+                                         C.c_int32, _P, _P, _P, _P, _P, _P, _P]),
     "sfm_pose_and_triangulate": (C.c_int, [_P, C.c_double, C.c_double, C.POINTER(Poses), C.c_int64,
                                            C.POINTER(C.c_int64), _P, _P, _P]),
     "sfm_two_view": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.c_double, C.POINTER(Best), C.POINTER(Poses),
@@ -605,6 +614,36 @@ class Engine:
         self._ck(self.lib.sfm_triangulate(self.h, _ptr(P1), _ptr(P2), _P(a), _P(a + 8), _P(b), _P(b + 8), 2, m,
                                           _ptr(X)), "sfm_triangulate")
         return X
+
+    def triangulate_tracks(self, K, Rt, offsets, view, x, threshold, min_angle_deg=1.5, min_views=2,
+                           refine_iterations=0):
+        """Multi-view triangulation of tracks (sfm_triangulate_tracks).  K float64[V,3,3], Rt float64[V,3,4], offsets
+        int64[T+1], view int32[M], x float64[M,2].  Returns (X [T,3], status int32[T], num_inliers int32[T], angle [T],
+        mask bool[M], err [M], TrackRefinement[T] array or None)."""
+        Rt = _f64(Rt).reshape(-1, 12)
+        V = Rt.shape[0]
+        K = _f64(K).reshape(V, 9)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64).reshape(-1)
+        view = np.ascontiguousarray(view, dtype=np.int32).reshape(-1)
+        x = _f64(x).reshape(-1, 2)
+        T = offsets.shape[0] - 1
+        M = view.shape[0]
+        if T < 0 or x.shape[0] != M:
+            raise ValueError(f"expected offsets [T+1], view [M] and x [M,2], got {offsets.shape}, {view.shape}, {x.shape}")
+        if T > 0 and offsets[-1] != M:
+            raise ValueError(f"offsets[T] = {offsets[-1]} but there are {M} observations")
+        X = np.empty((T, 3), dtype=np.float64)
+        status = np.empty(T, dtype=np.int32)
+        num = np.empty(T, dtype=np.int32)
+        angle = np.empty(T, dtype=np.float64)
+        mask = np.empty(M, dtype=np.uint8)
+        err = np.empty(M, dtype=np.float64)
+        rep = (TrackRefinement * T)() if refine_iterations > 0 and T > 0 else None
+        self._ck(self.lib.sfm_triangulate_tracks(
+            self.h, _ptr(K), _ptr(Rt), int(V), _ptr(offsets), int(T), _ptr(view), _ptr(x), float(threshold),
+            float(min_angle_deg), int(min_views), int(refine_iterations), _ptr(X), _ptr(status), _ptr(num), _ptr(angle),
+            _ptr(mask), _ptr(err), None if rep is None else C.cast(rep, _P)), "sfm_triangulate_tracks")
+        return X, status, num, angle, mask.astype(bool), err, rep
 
     def pose_and_triangulate(self, threshold, distance_threshold=50.0, cap=None, refine_iterations=0):
         self.set_refinement(refine_iterations)

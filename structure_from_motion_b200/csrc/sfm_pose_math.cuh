@@ -91,8 +91,8 @@ __device__ inline void decompose_essential(const double (&E)[9], PoseSet& out) {
 // right singular vector of the smallest singular value, dehomogenise.  P1, P2 are 3x4
 // row-major (only rows 0-2 of the reference's 4x4 Tmat are used, :24-31).
 // One copy per kernel (noinline): T2 calls it for the cheirality test and again for the short triangulation, and the
-// second use finds the code in the instruction cache.
-__device__ __noinline__ void dlt_triangulate(double xa, double ya, double xb, double yb,
+// second use finds the code in the instruction cache.  inline for the linkage only: two translation units include it.
+__device__ __noinline__ inline void dlt_triangulate(double xa, double ya, double xb, double yb,
                                              const double* __restrict__ P1,
                                              const double* __restrict__ P2, double (&X)[3]) {
     double g[16], v[16];
@@ -110,6 +110,38 @@ __device__ __noinline__ void dlt_triangulate(double xa, double ya, double xb, do
         X[2] = xf[2] / xf[3];
         return;
     }
+    jacobi_svd_onesided<4, 4>(g, v, 20);
+    double nrm[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+        nrm[j] = fma(g[12 + j], g[12 + j], fma(g[8 + j], g[8 + j], fma(g[4 + j], g[4 + j], g[j] * g[j])));
+    int m = 0;
+#pragma unroll
+    for (int j = 1; j < 4; ++j) {
+        const double cur = (m == 0) ? nrm[0] : ((m == 1) ? nrm[1] : ((m == 2) ? nrm[2] : nrm[3]));
+        if (nrm[j] < cur) m = j;
+    }
+    double x[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+        x[i] = (m == 0) ? v[i * 4] : ((m == 1) ? v[i * 4 + 1] : ((m == 2) ? v[i * 4 + 2] : v[i * 4 + 3]));
+    X[0] = x[0] / x[3];
+    X[1] = x[1] / x[3];
+    X[2] = x[2] / x[3];
+}
+
+// The point of a 4-column DLT system given as a row-major 4x4 g (sfm_tracks.cuh: the triangular factor of an N-view
+// system): the null vector of dlt_triangulate - null_vector4_fast, else the Jacobi SVD's column of the smallest singular
+// value - dehomogenised.  dlt_triangulate keeps its own inline copy: calling this from it changes the code of its kernels.
+__device__ __forceinline__ void dlt_null_point(double (&g)[16], double (&X)[3]) {
+    double xf[4];
+    if (null_vector4_fast(g, xf)) {  // QR + checked inverse iteration (sfm_fastsvd.cuh); inliers always take this route
+        X[0] = xf[0] / xf[3];
+        X[1] = xf[1] / xf[3];
+        X[2] = xf[2] / xf[3];
+        return;
+    }
+    double v[16];
     jacobi_svd_onesided<4, 4>(g, v, 20);
     double nrm[4];
 #pragma unroll

@@ -83,6 +83,7 @@ template <int KIND> struct RefineDims;
 template <> struct RefineDims<MODEL_E> { static constexpr int NP = 5; };
 template <> struct RefineDims<MODEL_H> { static constexpr int NP = 8; };
 template <> struct RefineDims<MODEL_P> { static constexpr int NP = 6; };
+template <> struct RefineDims<MODEL_X> { static constexpr int NP = 3; };  // X of a track (sfm_tracks.cuh)
 // partial sums: cost, cost of the RANSAC model (first evaluation only), sum of squared coordinates, J^T J upper triangle
 // (row-major), J^T r
 template <int KIND> __host__ __device__ constexpr int refine_nv() { return 3 + RefineDims<KIND>::NP * (RefineDims<KIND>::NP + 1) / 2 + RefineDims<KIND>::NP; }
@@ -635,9 +636,11 @@ __device__ __noinline__ void refine_control(RefineState& s, const double* tot, i
         for (int k = 0; k < 3; ++k) s.px[9 + k] = t[k] * inv;
     } else if constexpr (KIND == MODEL_H) {
         for (int k = 0; k < 8; ++k) s.px[k] = s.x[k] + d[k];
-    } else {
+    } else if constexpr (KIND == MODEL_P) {
         refine_rotate(s.x, d, s.px);
         for (int k = 0; k < 3; ++k) s.px[9 + k] = s.x[9 + k] + d[3 + k];
+    } else {
+        for (int k = 0; k < 3; ++k) s.px[k] = s.x[k] + d[k];
     }
 }
 

@@ -11,7 +11,8 @@ namespace sfm {
 // (4-point samples of 2-D-3-D records, reprojection error in pixels; sfm_pnp.cuh).  The kind fixes the record type,
 // the model stride, the sample size and the exact scorer of the sample rule and of the rescore; the selection rule
 // itself is the same.
-enum { MODEL_E = 0, MODEL_H = 1, MODEL_P = 2 };
+enum { MODEL_E = 0, MODEL_H = 1, MODEL_P = 2,
+       MODEL_X = 3 };  // a 3-D point of a track (sfm_tracks.cuh): a refinement kind only, never a RANSAC model
 
 struct Best {
     double err;

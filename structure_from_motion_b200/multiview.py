@@ -1,0 +1,91 @@
+"""Multi-view triangulation of tracks on arrays: one 3-D point per track from its observations in registered views.
+
+A track is one 3-D point observed in some subset of the registered views: observations (view index, pixel) in CSR form,
+``offsets`` int64[T+1], ``view`` int32[M] and ``x`` float64[M,2].  Per track, every pair of observations is
+triangulated (two-view DLT) and scored by the PnP reprojection decision over the whole track; the best pair's passing
+observations give the N-view DLT point, optionally refined by Levenberg-Marquardt on the reprojection error.  A track
+is usable when its status is "ok": at least ``min_views`` inliers and rays that meet at ``min_angle_deg`` or more.
+The semantics are pinned in include/sfm_b200.h (sfm_triangulate_tracks) and csrc/sfm_tracks.cuh.  Everything numeric
+runs in libsfm_b200.so; there is no CPU fallback.
+"""
+from __future__ import annotations
+
+import dataclasses
+from typing import Optional
+
+import numpy as np
+
+from . import _native
+
+
+@dataclasses.dataclass
+class TrackRefinement:
+    cost_start: np.ndarray        # float64[T] summed squared reprojection error (px^2) at the linear point, over the list
+    cost_final: np.ndarray        # float64[T] the same at the reported point, <= cost_start
+    num: np.ndarray               # int32[T] observations in the list (those passing under the linear point)
+    iterations: np.ndarray        # int32[T] proposals evaluated
+    status: np.ndarray            # str[T] converged, max_iterations, stalled, no_model (short / no_pair) or nonfinite
+    rejected: np.ndarray          # int32[T] of those, proposals rejected
+
+
+@dataclasses.dataclass
+class TracksResult:
+    points: np.ndarray            # float64[T,3] world points; NaN for "short" and "no_pair" tracks
+    status: np.ndarray            # str[T] ok, short, no_pair, few_inliers or small_angle
+    num_inliers: np.ndarray       # int32[T] passing observations under the reported point
+    angle: np.ndarray             # float64[T] largest angle (radians) between the rays of two passing observations
+    mask: np.ndarray              # bool[M] decision of every observation under its track's point
+    err: np.ndarray               # float64[M] squared reprojection error (px^2) under its track's point
+    refinement: Optional[TrackRefinement] = None  # refine_iterations > 0
+
+
+def tracks_from_dense(visible, pixels):
+    """CSR tracks for the layout "point i seen in the views where visible[i, c]": visible bool[N,V], pixels
+    float64[N,V,2] (read where visible).  Observations are in view order.  Returns (offsets int64[N+1], view int32[M],
+    x float64[M,2])."""
+    visible = np.asarray(visible, dtype=bool)
+    pixels = np.asarray(pixels, dtype=np.float64)
+    if visible.ndim != 2 or pixels.shape != visible.shape + (2,):
+        raise ValueError(f"expected visible [N,V] and pixels [N,V,2], got {visible.shape} and {pixels.shape}")
+    pt, view = np.nonzero(visible)  # row-major: by point, then by view
+    offsets = np.zeros(visible.shape[0] + 1, dtype=np.int64)
+    np.cumsum(visible.sum(axis=1), out=offsets[1:])
+    return offsets, view.astype(np.int32), np.ascontiguousarray(pixels[pt, view])
+
+
+def triangulate_tracks_arrays(K, R, t, offsets, view, x, threshold: float, min_angle_deg: float = 1.5,
+                              min_views: int = 2, refine_iterations: int = 0,
+                              engine: Optional[_native.Engine] = None) -> TracksResult:
+    """Triangulate T tracks seen in V registered views.
+
+    K: one (3,3) camera for every view or (V,3,3), upper triangular with K[2,2] = 1.  R (V,3,3), t (V,3): world to
+    camera, x_cam = R X + t (the ``ransac_pnp_arrays`` convention).  offsets int64[T+1], view int32[M], x float64[M,2]
+    pixels.  threshold: on the squared reprojection error in px^2, finite.  A track has at most 64 observations.
+    refine_iterations > 0 refines each point over the observations passing under its linear point.
+    """
+    R = np.asarray(R, dtype=np.float64)
+    t = np.asarray(t, dtype=np.float64)
+    if R.ndim != 3 or R.shape[1:] != (3, 3) or t.shape != (R.shape[0], 3):
+        raise ValueError(f"expected R (V,3,3) and t (V,3), got {R.shape} and {t.shape}")
+    V = R.shape[0]
+    K = np.asarray(K, dtype=np.float64)
+    if K.shape == (3, 3):
+        K = np.broadcast_to(K, (V, 3, 3))
+    if K.shape != (V, 3, 3):
+        raise ValueError(f"expected K (3,3) or ({V},3,3), got {K.shape}")
+    refine_iterations = int(refine_iterations)
+    if refine_iterations < 0:
+        raise ValueError(f"refine_iterations must be >= 0, got {refine_iterations}")
+    Rt = np.concatenate([R, t[:, :, None]], axis=2)
+    eng = engine or _native.get_engine()
+    X, status, num, angle, mask, err, rep = eng.triangulate_tracks(K, Rt, offsets, view, x, threshold, min_angle_deg,
+                                                                  min_views, refine_iterations)
+    names = np.array([_native.TRACK_STATUS[s] for s in range(len(_native.TRACK_STATUS))])
+    result = TracksResult(points=X, status=names[status], num_inliers=num, angle=angle, mask=mask, err=err)
+    if rep is not None:
+        r = np.ctypeslib.as_array(rep)
+        rnames = np.array([_native.REFINE_STATUS[s] for s in range(len(_native.REFINE_STATUS))])
+        result.refinement = TrackRefinement(
+            cost_start=r["cost_start"].copy(), cost_final=r["cost_final"].copy(), num=r["num"].copy(),
+            iterations=r["iterations"].copy(), status=rnames[r["status"]], rejected=r["rejected"].copy())
+    return result

@@ -237,3 +237,47 @@ def make_pnp_samples(m: int, seed: int, noise_px: float = 0.0, K=None, w: int = 
         x = p[:, :2] / p[:, 2:] + rng.normal(0, noise_px, (4, 2))
         out.append((Ki, np.ascontiguousarray(X), np.ascontiguousarray(x), R, t))
     return out
+
+
+def make_multi_view_scene(n_points: int, n_views: int, seed: int, noise_px: float = 0.5, outlier_frac: float = 0.0,
+                          f: float = 800.0, w: int = 1280, h: int = 960, K=None, arc_deg: float = 60.0,
+                          min_len: int = 2, max_len: int = 8):
+    """Return (K, R[V,3,3], t[V,3], X[N,3], offsets int64[N+1], view int32[M], x[M,2], outlier bool[M]): tracks of
+    the ``make_scene`` point cloud seen by V cameras on an arc.
+
+    The cameras lie on a horizontal circular arc of ``arc_deg`` degrees and radius 6 about the cloud's centre (0, 0, 6),
+    view 0 at one end, each looking at the centre; x_cam = R X + t.  Point i is seen in a contiguous window of views
+    whose length is uniform in [min_len, max_len] (at most V) and whose start is uniform among the windows that fit;
+    its observations are in view order.  x = the projection plus Gaussian noise of ``noise_px``; a fraction
+    ``outlier_frac`` of all observations is replaced by uniform pixels (``outlier`` marks them).  K as in
+    ``make_scene``."""
+    rng = np.random.default_rng(seed)
+    K = _camera(K, f, w, h)
+    N, V = int(n_points), int(n_views)
+    X = np.column_stack([rng.uniform(-2, 2, N), rng.uniform(-1.5, 1.5, N), rng.uniform(4, 8, N)])
+    centre = np.array([0.0, 0.0, 6.0])
+    R = np.empty((V, 3, 3))
+    t = np.empty((V, 3))
+    for c, th in enumerate(np.radians(np.linspace(-arc_deg / 2, arc_deg / 2, V))):
+        C = centre + 6.0 * np.array([np.sin(th), 0.0, -np.cos(th)])
+        z = (centre - C) / np.linalg.norm(centre - C)
+        xa = np.cross([0.0, 1.0, 0.0], z)
+        xa /= np.linalg.norm(xa)
+        R[c] = np.stack([xa, np.cross(z, xa), z])
+        t[c] = -R[c] @ C
+    hi = min(max_len, V)
+    length = rng.integers(min(min_len, hi), hi + 1, N)
+    start = (rng.uniform(0, 1, N) * (V - length + 1)).astype(np.int64)
+    offsets = np.zeros(N + 1, dtype=np.int64)
+    np.cumsum(length, out=offsets[1:])
+    M = int(offsets[-1])
+    pt = np.repeat(np.arange(N), length)
+    view = (start[pt] + np.arange(M) - offsets[pt]).astype(np.int32)
+    cam = np.einsum("mij,mj->mi", R[view], X[pt]) + t[view]
+    p = cam @ K.T
+    x = p[:, :2] / p[:, 2:] + rng.normal(0, noise_px, (M, 2))
+    outlier = np.zeros(M, dtype=bool)
+    outlier[rng.choice(M, int(round(outlier_frac * M)), replace=False)] = True
+    n_out = int(outlier.sum())
+    x[outlier] = np.column_stack([rng.uniform(0, w, n_out), rng.uniform(0, h, n_out)])
+    return K, R, t, X, offsets, view, np.ascontiguousarray(x), outlier
