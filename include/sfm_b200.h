@@ -341,6 +341,51 @@ int sfm_triangulate_tracks(sfm_ctx *ctx, const double *K, const double *Rt, int3
                            int32_t *num_inliers, double *angle, uint8_t *mask, double *err,
                            sfm_track_refinement *refine_report);
 
+/* ---- bundle adjustment of views and points (csrc/sfm_bundle.cuh) ---------------------------
+ * Joint Levenberg-Marquardt over every free pose and every parameter point, on the reprojection error.
+ *   cameras      K double[V][9] fixed, checked as in sfm_triangulate_tracks; Rt double[V][12] the finite start, world
+ *                to camera.  1 <= V <= SFM_BA_MAX_VIEWS.
+ *   tracks       the CSR of sfm_triangulate_tracks (at most SFM_TRACK_MAX_OBSERVATIONS per track) and X double[T][3],
+ *                the start point of every track.  A track whose start X has a non-finite entry is not a parameter
+ *                (so TracksResult points with non-ok tracks set to NaN can be passed as they are).
+ *   list         formed once under the start and fixed: the observations whose PnP record decision under
+ *                P_c = K_c [R_c | t_c] passes at threshold, of the tracks with at least 2 of them (the parameter
+ *                points).  Every other track is reported unchanged, bits included, and has no observation in the list.
+ *   gauge        fixed uint8[V] marks the poses held constant; at least one.  scale_view (-1 = none) is a free view
+ *                the component of whose start t with the largest |value| (lowest index on ties) is held constant.
+ *                Fixed views, that component and the non-parameter points come out bit-identical to the input.
+ *   parameters   per free view R <- R exp([w]x), t <- t + dt, from the rotation nearest its given R (as
+ *                sfm_refine_pnp); per parameter point X <- X + dX.  A free view with no list observation has a zero
+ *                Jacobian block: its step is 0 and it stays at its projected start.
+ *   cost         the sum over the list of (p0 / p2 - u)^2 + (p1 / p2 - v)^2; a proposal with a list observation at
+ *                p2 < 2^-537 or a non-finite residual costs +inf and is rejected; at the start that is
+ *                SFM_REFINE_NONFINITE and the input is reported.
+ *   control      that of sfm_refine_pnp: lambda 1e-3, / 10 on a strictly lower cost and x 10 otherwise, Ftol 1e-12,
+ *                Xtol 1e-9 on the Marquardt-scaled step, lambda cap 1e16 (stalled), cost floor 1e-24 sum(u^2 + v^2)
+ *                over the list, max_iterations evaluated proposals; a damped system that is not numerically positive
+ *                definite multiplies lambda by 10 and is solved again.  The step eliminates the points by a Schur
+ *                complement and factors the reduced camera system (6 x free views) by Cholesky on the device.
+ *   outputs      optional: Rt_out double[V][12], X_out double[T][3], report, mask uint8[M] / err double[M] (the PnP
+ *                record decision and value of every observation under the reported parameters).  An empty list is
+ *                converged at iteration 0 with cost 0 and the projected start.
+ * The results depend on the inputs alone: not on the grid, the run or the context.  SFM_ERR_ARG, before any launch,
+ * for V outside [1, SFM_BA_MAX_VIEWS], a bad K, a non-finite Rt, no fixed view, a scale_view that is fixed or out of
+ * range, malformed offsets, a view index out of range, a track longer than SFM_TRACK_MAX_OBSERVATIONS, a non-finite
+ * threshold or max_iterations < 1. */
+#define SFM_BA_MAX_VIEWS 256
+typedef struct sfm_bundle_report {
+    double cost_start;             /* cost at the (projected) start                     */
+    double cost_final;             /* cost at the reported parameters, <= cost_start    */
+    int64_t num_observations;      /* list length                                       */
+    int64_t num_points;            /* parameter points                                  */
+    int32_t num_free_views;
+    int32_t iterations, status, rejected;   /* status: enum sfm_refine_status          */
+} sfm_bundle_report;
+int sfm_bundle_adjust(sfm_ctx *ctx, const double *K, const double *Rt, int32_t V, const uint8_t *fixed,
+                      int32_t scale_view, const int64_t *offsets, int64_t T, const int32_t *view, const double *x,
+                      const double *X, double threshold, int32_t max_iterations, double *Rt_out, double *X_out,
+                      sfm_bundle_report *report, uint8_t *mask, double *err);
+
 /* Fused tail of the pipeline for the current winner (apps/sfm.py:110-186): inliers of the
  * winner -> decomposition -> cheirality vote -> triangulation of the passing inliers with
  * P1 = K[I|0], P2 = K[R|t], all on the device.  inlier_idx int64[cap] receives the indices

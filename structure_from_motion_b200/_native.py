@@ -67,6 +67,12 @@ class TrackRefinement(C.Structure):
                 ("status", C.c_int32), ("rejected", C.c_int32)]
 
 
+class BundleReport(C.Structure):
+    _fields_ = [("cost_start", C.c_double), ("cost_final", C.c_double), ("num_observations", C.c_int64),
+                ("num_points", C.c_int64), ("num_free_views", C.c_int32), ("iterations", C.c_int32),
+                ("status", C.c_int32), ("rejected", C.c_int32)]
+
+
 TRACK_STATUS = {0: "ok", 1: "short", 2: "no_pair", 3: "few_inliers", 4: "small_angle"}
 
 REFINE_STATUS = {0: "converged", 1: "max_iterations", 2: "stalled", 3: "no_model", 4: "nonfinite"}
@@ -120,6 +126,8 @@ _SIGNATURES = {
     "sfm_triangulate": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, C.c_int64, C.c_int64, _P]),
     "sfm_triangulate_tracks": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int64, _P, _P, C.c_double, C.c_double, C.c_int32,
                                          C.c_int32, _P, _P, _P, _P, _P, _P, _P]),
+    "sfm_bundle_adjust": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, C.c_int64, _P, _P, _P, C.c_double, C.c_int32,
+                                    _P, _P, C.POINTER(BundleReport), _P, _P]),
     "sfm_pose_and_triangulate": (C.c_int, [_P, C.c_double, C.c_double, C.POINTER(Poses), C.c_int64,
                                            C.POINTER(C.c_int64), _P, _P, _P]),
     "sfm_two_view": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.c_double, C.POINTER(Best), C.POINTER(Poses),
@@ -644,6 +652,38 @@ class Engine:
             float(min_angle_deg), int(min_views), int(refine_iterations), _ptr(X), _ptr(status), _ptr(num), _ptr(angle),
             _ptr(mask), _ptr(err), None if rep is None else C.cast(rep, _P)), "sfm_triangulate_tracks")
         return X, status, num, angle, mask.astype(bool), err, rep
+
+    def bundle_adjust(self, K, Rt, fixed, scale_view, offsets, view, x, X, threshold, max_iterations=50):
+        """Bundle adjustment of views and points (sfm_bundle_adjust).  K float64[V,3,3], Rt float64[V,3,4], fixed
+        bool[V], scale_view int (-1 = none), offsets int64[T+1], view int32[M], x float64[M,2], X float64[T,3].
+        Returns (Rt [V,3,4], X [T,3], BundleReport, mask bool[M], err [M])."""
+        Rt = _f64(Rt).reshape(-1, 12)
+        V = Rt.shape[0]
+        K = _f64(K).reshape(V, 9)
+        fixed = np.ascontiguousarray(fixed, dtype=np.uint8).reshape(-1)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64).reshape(-1)
+        view = np.ascontiguousarray(view, dtype=np.int32).reshape(-1)
+        x = _f64(x).reshape(-1, 2)
+        X = _f64(X).reshape(-1, 3)
+        T = offsets.shape[0] - 1
+        M = view.shape[0]
+        if fixed.shape[0] != V:
+            raise ValueError(f"expected fixed [{V}], got {fixed.shape}")
+        if T < 0 or x.shape[0] != M or X.shape[0] != T:
+            raise ValueError(f"expected offsets [T+1], view [M], x [M,2] and X [T,3], got {offsets.shape}, {view.shape}, "
+                             f"{x.shape} and {X.shape}")
+        if offsets[-1] != M:
+            raise ValueError(f"offsets[T] = {offsets[-1]} but there are {M} observations")
+        Rt_out = np.empty((V, 12), dtype=np.float64)
+        X_out = np.empty((T, 3), dtype=np.float64)
+        mask = np.empty(M, dtype=np.uint8)
+        err = np.empty(M, dtype=np.float64)
+        rep = BundleReport()
+        self._ck(self.lib.sfm_bundle_adjust(
+            self.h, _ptr(K), _ptr(Rt), int(V), _ptr(fixed), int(scale_view), _ptr(offsets), int(T), _ptr(view), _ptr(x),
+            _ptr(X), float(threshold), int(max_iterations), _ptr(Rt_out), _ptr(X_out), C.byref(rep), _ptr(mask),
+            _ptr(err)), "sfm_bundle_adjust")
+        return Rt_out.reshape(V, 3, 4), X_out, rep, mask.astype(bool), err
 
     def pose_and_triangulate(self, threshold, distance_threshold=50.0, cap=None, refine_iterations=0):
         self.set_refinement(refine_iterations)

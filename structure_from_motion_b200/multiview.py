@@ -5,7 +5,9 @@ A track is one 3-D point observed in some subset of the registered views: observ
 triangulated (two-view DLT) and scored by the PnP reprojection decision over the whole track; the best pair's passing
 observations give the N-view DLT point, optionally refined by Levenberg-Marquardt on the reprojection error.  A track
 is usable when its status is "ok": at least ``min_views`` inliers and rays that meet at ``min_angle_deg`` or more.
-The semantics are pinned in include/sfm_b200.h (sfm_triangulate_tracks) and csrc/sfm_tracks.cuh.  Everything numeric
+``bundle_adjust_arrays`` then refines the free poses and the points jointly (Levenberg-Marquardt on the reprojection
+error, the points eliminated by a Schur complement).  The semantics are pinned in include/sfm_b200.h
+(sfm_triangulate_tracks, sfm_bundle_adjust), csrc/sfm_tracks.cuh and csrc/sfm_bundle.cuh.  Everything numeric
 runs in libsfm_b200.so; there is no CPU fallback.
 """
 from __future__ import annotations
@@ -89,3 +91,65 @@ def triangulate_tracks_arrays(K, R, t, offsets, view, x, threshold: float, min_a
             cost_start=r["cost_start"].copy(), cost_final=r["cost_final"].copy(), num=r["num"].copy(),
             iterations=r["iterations"].copy(), status=rnames[r["status"]], rejected=r["rejected"].copy())
     return result
+
+
+@dataclasses.dataclass
+class BundleReport:
+    cost_start: float             # summed squared reprojection error (px^2) over the list at the (projected) start
+    cost_final: float             # the same at the reported parameters, <= cost_start
+    num_observations: int         # observations in the list
+    num_points: int               # parameter points (finite start, at least 2 list observations)
+    num_free_views: int
+    iterations: int               # proposals evaluated
+    status: str                   # converged, max_iterations, stalled or nonfinite
+    rejected: int                 # of those, proposals rejected
+
+
+@dataclasses.dataclass
+class BundleResult:
+    R: np.ndarray                 # float64[V,3,3] world to camera
+    t: np.ndarray                 # float64[V,3]
+    points: np.ndarray            # float64[T,3]; non-parameter tracks exactly as given
+    mask: np.ndarray              # bool[M] decision of every observation under the reported parameters
+    err: np.ndarray               # float64[M] squared reprojection error (px^2) under them
+    report: BundleReport
+
+
+def bundle_adjust_arrays(K, R, t, X, offsets, view, x, threshold: float, fixed=(0,), scale_view=None,
+                         max_iterations: int = 50, engine: Optional[_native.Engine] = None) -> BundleResult:
+    """Refine V registered views and the points of T tracks jointly.
+
+    K: one (3,3) camera or (V,3,3), upper triangular with K[2,2] = 1.  R (V,3,3), t (V,3): the start, x_cam = R X + t.
+    X (T,3): the start points; a track with a non-finite X (a non-ok track of ``triangulate_tracks_arrays`` set to
+    NaN) is left as it is.  offsets, view, x: the tracks as for ``triangulate_tracks_arrays``.  The observations
+    passing the reprojection rule at ``threshold`` (px^2) under the start form the fixed list.  ``fixed``: the indices
+    of the views held constant (at least one).  ``scale_view``: a free view whose largest translation component is
+    held constant; None picks the lowest-index free view when exactly one view is fixed, and none otherwise.
+    """
+    R = np.asarray(R, dtype=np.float64)
+    t = np.asarray(t, dtype=np.float64)
+    if R.ndim != 3 or R.shape[1:] != (3, 3) or t.shape != (R.shape[0], 3):
+        raise ValueError(f"expected R (V,3,3) and t (V,3), got {R.shape} and {t.shape}")
+    V = R.shape[0]
+    K = np.asarray(K, dtype=np.float64)
+    if K.shape == (3, 3):
+        K = np.broadcast_to(K, (V, 3, 3))
+    if K.shape != (V, 3, 3):
+        raise ValueError(f"expected K (3,3) or ({V},3,3), got {K.shape}")
+    fixed_mask = np.zeros(V, dtype=bool)
+    idx = np.asarray(fixed, dtype=np.int64).reshape(-1)
+    if idx.size and (idx.min() < 0 or idx.max() >= V):
+        raise ValueError(f"fixed view index outside [0, {V})")
+    fixed_mask[idx] = True
+    if scale_view is None:
+        free = np.flatnonzero(~fixed_mask)
+        scale_view = int(free[0]) if fixed_mask.sum() == 1 and free.size else -1
+    Rt = np.concatenate([R, t[:, :, None]], axis=2)
+    eng = engine or _native.get_engine()
+    Rt_out, X_out, rep, mask, err = eng.bundle_adjust(K, Rt, fixed_mask, int(scale_view), offsets, view, x, X,
+                                                      threshold, int(max_iterations))
+    report = BundleReport(cost_start=rep.cost_start, cost_final=rep.cost_final, num_observations=rep.num_observations,
+                          num_points=rep.num_points, num_free_views=rep.num_free_views, iterations=rep.iterations,
+                          status=_native.REFINE_STATUS[rep.status], rejected=rep.rejected)
+    return BundleResult(R=np.ascontiguousarray(Rt_out[:, :, :3]), t=np.ascontiguousarray(Rt_out[:, :, 3]), points=X_out,
+                        mask=mask, err=err, report=report)
