@@ -341,6 +341,36 @@ int sfm_triangulate_tracks(sfm_ctx *ctx, const double *K, const double *Rt, int3
                            int32_t *num_inliers, double *angle, uint8_t *mask, double *err,
                            sfm_track_refinement *refine_report);
 
+/* ---- tracks from pairwise matches (csrc/sfm_track_build.cuh) ------------------------------
+ * The tracks that sfm_triangulate_tracks and sfm_bundle_adjust take, built from the matches of image pairs.  Indices
+ * only: no pixels are read.
+ *   features     V >= 1 views; feature_offsets int64[V+1] (first entry 0, non-decreasing) gives view v the features
+ *                [off[v], off[v+1]); local feature i of view v has the global id off[v] + i.  N = off[V] <= INT32_MAX.
+ *   matches      P >= 0 pair entries pair_views int32[P][2] = (a, b), a != b, both in [0, V); match_offsets int64[P+1]
+ *                (first entry 0, non-decreasing) gives entry p the matches [mo[p], mo[p+1]) of matches int32[E][2] =
+ *                (i, j), local indices in a and in b.  Each match is the undirected edge {off[a] + i, off[b] + j}.  A pair
+ *                may appear more than once, in either direction, and matches may repeat: only the edge set counts.
+ *   tracks       the connected components of that graph with at least 2 features, ordered by their smallest global
+ *                id; a track's observations in ascending global id (by view, then by local index).
+ *   status       SFM_BUILT_TRACK_CONFLICT when a view holds two or more of the track's features (the track is reported
+ *                whole, not split); else SFM_BUILT_TRACK_LONG with more than SFM_TRACK_MAX_OBSERVATIONS observations
+ *                (which sfm_triangulate_tracks refuses); else SFM_BUILT_TRACK_OK.
+ *   outputs      each may be NULL, all sized from N: *T tracks and *M observations; offsets int64[N/2+1] (T + 1
+ *                written), status int32[N/2] (T written), view int32[N] and feature int32[N] (global id; M written),
+ *                track int32[N] the track of every feature, -1 for a feature in no track (N written).
+ * The outputs depend on the edge set alone: not on edge order, multiplicity or direction, the grouping of matches into
+ * pair entries, scheduling or the context.  SFM_ERR_ARG, before any launch, for V < 1, P < 0, malformed feature or
+ * match offsets, N > INT32_MAX, a == b or a view outside [0, V), a local index outside its view, or a NULL input that
+ * is needed (feature_offsets always; pair_views and match_offsets when P > 0; matches when E > 0). */
+enum sfm_built_track_status {
+    SFM_BUILT_TRACK_OK = 0,
+    SFM_BUILT_TRACK_CONFLICT = 1,  /* some view holds two or more of its features */
+    SFM_BUILT_TRACK_LONG = 2       /* more than SFM_TRACK_MAX_OBSERVATIONS observations */
+};
+int sfm_build_tracks(sfm_ctx *ctx, int32_t V, const int64_t *feature_offsets, int64_t P, const int32_t *pair_views,
+                     const int64_t *match_offsets, const int32_t *matches, int64_t *T, int64_t *M, int64_t *offsets,
+                     int32_t *status, int32_t *view, int32_t *feature, int32_t *track);
+
 /* ---- bundle adjustment of views and points (csrc/sfm_bundle.cuh) ---------------------------
  * Joint Levenberg-Marquardt over every free pose and every parameter point, on the reprojection error.
  *   cameras      K double[V][9] fixed, checked as in sfm_triangulate_tracks; Rt double[V][12] the finite start, world

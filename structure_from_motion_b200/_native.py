@@ -77,6 +77,8 @@ TRACK_STATUS = {0: "ok", 1: "short", 2: "no_pair", 3: "few_inliers", 4: "small_a
 
 REFINE_STATUS = {0: "converged", 1: "max_iterations", 2: "stalled", 3: "no_model", 4: "nonfinite"}
 
+BUILT_TRACK_STATUS = {0: "ok", 1: "conflict", 2: "long"}
+
 _P = C.c_void_p
 _SIGNATURES = {
     "sfm_version": (C.c_int, []),
@@ -128,6 +130,8 @@ _SIGNATURES = {
                                          C.c_int32, _P, _P, _P, _P, _P, _P, _P]),
     "sfm_bundle_adjust": (C.c_int, [_P, _P, _P, C.c_int32, _P, C.c_int32, _P, C.c_int64, _P, _P, _P, C.c_double, C.c_int32,
                                     _P, _P, C.POINTER(BundleReport), _P, _P]),
+    "sfm_build_tracks": (C.c_int, [_P, C.c_int32, _P, C.c_int64, _P, _P, _P, C.POINTER(C.c_int64), C.POINTER(C.c_int64),
+                                   _P, _P, _P, _P, _P]),
     "sfm_pose_and_triangulate": (C.c_int, [_P, C.c_double, C.c_double, C.POINTER(Poses), C.c_int64,
                                            C.POINTER(C.c_int64), _P, _P, _P]),
     "sfm_two_view": (C.c_int, [_P, C.c_double, C.c_double, C.c_int, C.c_int, C.c_double, C.POINTER(Best), C.POINTER(Poses),
@@ -684,6 +688,33 @@ class Engine:
             _ptr(X), float(threshold), int(max_iterations), _ptr(Rt_out), _ptr(X_out), C.byref(rep), _ptr(mask),
             _ptr(err)), "sfm_bundle_adjust")
         return Rt_out.reshape(V, 3, 4), X_out, rep, mask.astype(bool), err
+
+    def build_tracks(self, feature_offsets, pair_views, match_offsets, matches):
+        """Tracks from pairwise matches (sfm_build_tracks).  feature_offsets int64[V+1], pair_views int32[P,2],
+        match_offsets int64[P+1], matches int32[E,2] local indices.  Returns (offsets int64[T+1], status int32[T],
+        view int32[M], feature int32[M] global ids, track int32[N])."""
+        fo = np.ascontiguousarray(feature_offsets, dtype=np.int64).reshape(-1)
+        pv = np.ascontiguousarray(pair_views, dtype=np.int32).reshape(-1, 2)
+        mo = np.ascontiguousarray(match_offsets, dtype=np.int64).reshape(-1)
+        m = np.ascontiguousarray(matches, dtype=np.int32).reshape(-1, 2)
+        V, P = fo.shape[0] - 1, pv.shape[0]
+        if V < 1 or mo.shape[0] != P + 1:
+            raise ValueError(f"expected feature_offsets [V+1] (V >= 1) and match_offsets [P+1], got {fo.shape} and "
+                             f"{mo.shape} for {P} pairs")
+        if mo[-1] != m.shape[0]:
+            raise ValueError(f"match_offsets[P] = {mo[-1]} but there are {m.shape[0]} matches")
+        N = max(int(fo[-1]), 0)
+        offsets = np.empty(N // 2 + 1, dtype=np.int64)
+        status = np.empty(N // 2, dtype=np.int32)
+        view = np.empty(N, dtype=np.int32)
+        feature = np.empty(N, dtype=np.int32)
+        track = np.empty(N, dtype=np.int32)
+        T, M = C.c_int64(), C.c_int64()
+        self._ck(self.lib.sfm_build_tracks(self.h, int(V), _ptr(fo), int(P), _ptr(pv), _ptr(mo), _ptr(m), C.byref(T),
+                                           C.byref(M), _ptr(offsets), _ptr(status), _ptr(view), _ptr(feature),
+                                           _ptr(track)), "sfm_build_tracks")
+        T, M = T.value, M.value
+        return offsets[:T + 1].copy(), status[:T].copy(), view[:M].copy(), feature[:M].copy(), track
 
     def pose_and_triangulate(self, threshold, distance_threshold=50.0, cap=None, refine_iterations=0):
         self.set_refinement(refine_iterations)

@@ -10,7 +10,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 # one translation unit per stage (csrc/sfm_host.h); the .cpp files are host only and go straight to the host compiler
 TUS = ["sfm_api.cu", "sfm_ransac.cu", "sfm_two_view.cu", "sfm_model_select.cu", "sfm_front_end.cu", "sfm_tracks.cu",
-       "sfm_bundle.cu", "sfm_nccl.cpp", "sfm_sampler.cpp"]
+       "sfm_bundle.cu", "sfm_track_build.cu", "sfm_nccl.cpp", "sfm_sampler.cpp"]
 OBJ_DIR = os.path.join(HERE, "..", "build", "sfm_b200")
 SO = os.path.join(HERE, "libsfm_b200.so")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]

@@ -79,7 +79,7 @@ int sfm_destroy(sfm_ctx* c) {
                    &c->invalid, &c->winnerE, &c->record, &c->merged, &c->rows, &c->blockinv, &c->mask, &c->sed, &c->poses, &c->pass, &c->X, &c->idx,
                    &c->planes, &c->hK, &c->selstate, &c->selio, &c->selpp, &c->refstate, &c->refpart, &c->reftick, &c->refrec, &c->refrep, &c->k2pts, &c->k2box, &c->k2sort,
                    &c->ppts, &c->pK, &c->pmodels, &c->pwin, &c->trkin, &c->trkpairs, &c->trkout,
-                   &c->bain, &c->bawork, &c->batick,
+                   &c->bain, &c->bawork, &c->batick, &c->tbin, &c->tbwork, &c->tbsort,
                    &c->scan, &c->tmp, &c->gathered, &c->tailstate, &c->num, &c->winrec, &c->bout, &c->spts, &c->bounds, &c->fitflag,
                    &c->m_img, &c->m_feat, &c->m_W, &c->m_ss, &c->m_ok, &c->m_S, &c->m_out,
                    &c->h_img, &c->h_gx, &c->h_gy, &c->h_corner, &c->h_alive, &c->h_key, &c->h_idx, &c->h_small, &c->h_xy};

@@ -9,6 +9,7 @@
 //   sfm_front_end.cu    matcher, cross-correlation, Harris                      sfm_match.cuh, sfm_harris.cuh
 //   sfm_tracks.cu       multi-view triangulation of tracks                      sfm_tracks.cuh
 //   sfm_bundle.cu       bundle adjustment of views and points                   sfm_bundle.cuh
+//   sfm_track_build.cu  tracks from pairwise matches (union-find)               sfm_track_build.cuh
 //   sfm_nccl.cpp, sfm_sampler.cpp: host only, compiled by the host compiler
 // include/sfm_b200.h declares every sfm_* entry point extern "C"; their definitions in the stage files take that linkage.
 #pragma once
@@ -86,6 +87,7 @@ struct sfm_ctx {
                                                           // self-cleaning tickets, pose / forced indices / report
     sfm_host::Buf trkin, trkpairs, trkout;  // tracks: cameras, frame and observations; pair-search items; results
     sfm_host::Buf bain, bawork, batick;  // bundle adjustment: inputs and structure; state, equations and outputs; tickets
+    sfm_host::Buf tbin, tbwork, tbsort;  // track building: offsets, pairs, matches; union-find and select; sort and outputs
     long long n = 0, h = 0, npairs = 1;
     long long first_len = 0;  // batched: correspondences of the first pair (what the AUTO pilot samples)
     long long batch_max_len = 0;  // batched: correspondences of the longest pair

@@ -6,9 +6,10 @@ triangulated (two-view DLT) and scored by the PnP reprojection decision over the
 observations give the N-view DLT point, optionally refined by Levenberg-Marquardt on the reprojection error.  A track
 is usable when its status is "ok": at least ``min_views`` inliers and rays that meet at ``min_angle_deg`` or more.
 ``bundle_adjust_arrays`` then refines the free poses and the points jointly (Levenberg-Marquardt on the reprojection
-error, the points eliminated by a Schur complement).  The semantics are pinned in include/sfm_b200.h
-(sfm_triangulate_tracks, sfm_bundle_adjust), csrc/sfm_tracks.cuh and csrc/sfm_bundle.cuh.  Everything numeric
-runs in libsfm_b200.so; there is no CPU fallback.
+error, the points eliminated by a Schur complement).  ``build_tracks_arrays`` makes the tracks from pairwise feature
+matches (the connected components of the match graph).  The semantics are pinned in include/sfm_b200.h
+(sfm_build_tracks, sfm_triangulate_tracks, sfm_bundle_adjust), csrc/sfm_track_build.cuh, csrc/sfm_tracks.cuh and
+csrc/sfm_bundle.cuh.  Everything numeric runs in libsfm_b200.so; there is no CPU fallback.
 """
 from __future__ import annotations
 
@@ -53,6 +54,71 @@ def tracks_from_dense(visible, pixels):
     offsets = np.zeros(visible.shape[0] + 1, dtype=np.int64)
     np.cumsum(visible.sum(axis=1), out=offsets[1:])
     return offsets, view.astype(np.int32), np.ascontiguousarray(pixels[pt, view])
+
+
+@dataclasses.dataclass
+class TrackSet:
+    feature_offsets: np.ndarray   # int64[V+1]: view v owns the global feature ids [feature_offsets[v], feature_offsets[v+1])
+    offsets: np.ndarray           # int64[T+1] track CSR
+    view: np.ndarray              # int32[M] view of every observation
+    feature: np.ndarray           # int32[M] its global feature id; the local index is feature - feature_offsets[view]
+    x: np.ndarray                 # float64[M,2] its pixel
+    status: np.ndarray            # str[T] ok, conflict (a view holds two of its features) or long (more than 64)
+    track: np.ndarray             # int32[N] the track of every feature, -1 for a feature in no track
+
+    def ok(self) -> "TrackSet":
+        """The "ok" tracks only, renumbered in order; ``track`` maps the features of every other track to -1."""
+        keep = self.status == "ok"
+        n = np.diff(self.offsets)
+        obs = np.repeat(keep, n)
+        offsets = np.zeros(int(keep.sum()) + 1, dtype=np.int64)
+        np.cumsum(n[keep], out=offsets[1:])
+        renum = (np.cumsum(keep) - 1).astype(np.int32)
+        tr = self.track
+        inside = tr >= 0
+        track = np.full_like(tr, -1)
+        track[inside] = np.where(keep[tr[inside]], renum[tr[inside]], -1)
+        return TrackSet(feature_offsets=self.feature_offsets, offsets=offsets, view=self.view[obs],
+                        feature=self.feature[obs], x=self.x[obs], status=self.status[keep], track=track)
+
+
+def build_tracks_arrays(features, pairs, matches, engine: Optional[_native.Engine] = None) -> TrackSet:
+    """Tracks from pairwise feature matches: the connected components of the match graph with two or more features.
+
+    features: a list of V float64[n_v,2] pixel arrays (only their lengths and, for ``x``, their pixels are used).
+    pairs: int[P,2] view pairs (a, b), a != b.  matches: a list of P int[E_p,2] arrays of local indices (i in a, j in b).
+    A pair may repeat, in either order, and so may matches.  For one pair matched by ``sfm_match_brute_force``
+    (``Engine.match_brute_force``), optionally filtered by a RANSAC inlier mask ``inl`` over the kept matches::
+
+        i = np.flatnonzero(keep)
+        m = np.column_stack([i, best_b[keep]])      # or m[inl]
+
+    Tracks are ordered by their smallest global feature id, and observations run by view, then by local index.  A
+    track whose features include two of one view is "conflict" (reported whole); otherwise one of more than 64
+    observations is "long"; the rest are "ok".  ``TrackSet.ok()`` keeps the ok tracks, ready for
+    ``triangulate_tracks_arrays`` and ``bundle_adjust_arrays``.
+    """
+    feats = [np.asarray(f, dtype=np.float64).reshape(-1, 2) for f in features]
+    if not feats:
+        raise ValueError("at least one view is needed")
+    fo = np.zeros(len(feats) + 1, dtype=np.int64)
+    np.cumsum([len(f) for f in feats], out=fo[1:])
+    pv = np.asarray(pairs, dtype=np.int64).reshape(-1, 2)
+    if len(matches) != len(pv):
+        raise ValueError(f"{len(pv)} pairs but {len(matches)} match arrays")
+    ms = [np.asarray(m, dtype=np.int64).reshape(-1, 2) for m in matches]
+    mo = np.zeros(len(ms) + 1, dtype=np.int64)
+    np.cumsum([len(m) for m in ms], out=mo[1:])
+    for name, a in (("pairs", pv), ("matches", np.concatenate(ms) if ms else pv)):
+        if a.size and (a.min() < np.iinfo(np.int32).min or a.max() > np.iinfo(np.int32).max):
+            raise ValueError(f"{name} do not fit int32")
+    m = np.concatenate(ms).astype(np.int32) if ms else np.zeros((0, 2), dtype=np.int32)
+    eng = engine or _native.get_engine()
+    offsets, status, view, feature, track = eng.build_tracks(fo, pv.astype(np.int32), mo, m)
+    allx = np.concatenate(feats) if fo[-1] else np.zeros((0, 2))
+    names = np.array([_native.BUILT_TRACK_STATUS[s] for s in range(len(_native.BUILT_TRACK_STATUS))])
+    return TrackSet(feature_offsets=fo, offsets=offsets, view=view, feature=feature,
+                    x=np.ascontiguousarray(allx[feature]), status=names[status], track=track)
 
 
 def triangulate_tracks_arrays(K, R, t, offsets, view, x, threshold: float, min_angle_deg: float = 1.5,

@@ -5,6 +5,8 @@ fraction of outliers (image-2 coordinates replaced by uniform pixels).  numpy on
 """
 from __future__ import annotations
 
+import dataclasses
+
 import numpy as np
 
 
@@ -281,3 +283,72 @@ def make_multi_view_scene(n_points: int, n_views: int, seed: int, noise_px: floa
     n_out = int(outlier.sum())
     x[outlier] = np.column_stack([rng.uniform(0, w, n_out), rng.uniform(0, h, n_out)])
     return K, R, t, X, offsets, view, np.ascontiguousarray(x), outlier
+
+
+@dataclasses.dataclass
+class MatchGraph:
+    K: np.ndarray                 # (3,3)
+    R: np.ndarray                 # float64[V,3,3] world to camera, x_cam = R X + t
+    t: np.ndarray                 # float64[V,3]
+    X: np.ndarray                 # float64[n_points,3]
+    features: list                # V arrays float64[n_v,2]: the pixels of view v's features, in shuffled order
+    point: list                   # V arrays int64[n_v]: the point of each feature, -1 for a distractor
+    pairs: np.ndarray             # int32[P,2] (a, b), a < b, b - a <= span
+    matches: list                 # P arrays int32[E_p,2]: (local index in a, local index in b)
+    wrong: list                   # P arrays bool[E_p]: the match was redirected to a random feature of b
+
+
+def make_match_graph(n_points: int, n_views: int, seed: int, span: int = 2, wrong_frac: float = 0.0,
+                     distractor_frac: float = 0.0, **scene_kw) -> MatchGraph:
+    """Per-view features and pairwise matches over the tracks of ``make_multi_view_scene(n_points, n_views, seed,
+    **scene_kw)``.
+
+    View v's features are its observations plus round(distractor_frac x their number) uniform pixels, in a random
+    order.  For every two views a < b with b - a <= span, the pair holds one match per point observed in both (in
+    point order), and a fraction ``wrong_frac`` of all matches has its b index replaced by a uniform random feature of
+    b.  A point's observations lie in a contiguous window of views, so with span >= 1 the true matches connect all of
+    them, and no view holds two of them."""
+    K, R, t, X, off, view, x, _ = make_multi_view_scene(n_points, n_views, seed, **scene_kw)
+    rng = np.random.default_rng([seed, 1])
+    V = int(n_views)
+    w, h = float(2 * K[0, 2]), float(2 * K[1, 2])
+    pt = np.repeat(np.arange(len(off) - 1), np.diff(off))
+    local = np.empty(len(view), dtype=np.int64)
+    features, point = [], []
+    for v in range(V):
+        obs = np.flatnonzero(view == v)
+        nd = int(round(distractor_frac * len(obs)))
+        n = len(obs) + nd
+        perm = rng.permutation(n)  # feature perm[k] of the view is entry k of (observations, distractors)
+        local[obs] = perm[:len(obs)]
+        f = np.empty((n, 2))
+        f[perm[:len(obs)]] = x[obs]
+        f[perm[len(obs):]] = np.column_stack([rng.uniform(0, w, nd), rng.uniform(0, h, nd)])
+        p = np.full(n, -1, dtype=np.int64)
+        p[perm[:len(obs)]] = pt[obs]
+        features.append(f)
+        point.append(p)
+    # observation m and m + d belong to one point when the point's window holds both; their views are then d apart
+    ia, ib = [], []
+    for d in range(1, int(span) + 1):
+        m = np.arange(len(view) - d)
+        same = pt[m] == pt[m + d] if len(m) else np.zeros(0, dtype=bool)
+        ia.append(m[same])
+        ib.append(m[same] + d)
+    ia = np.concatenate(ia) if ia else np.zeros(0, dtype=np.int64)
+    ib = np.concatenate(ib) if ib else np.zeros(0, dtype=np.int64)
+    key = view[ia].astype(np.int64) * V + view[ib]
+    order = np.lexsort((pt[ia], key))
+    ia, ib, key = ia[order], ib[order], key[order]
+    mj = local[ib].copy()
+    wrong = np.zeros(len(mj), dtype=bool)
+    wrong[rng.choice(len(mj), int(round(wrong_frac * len(mj))), replace=False)] = True
+    nb = np.array([len(f) for f in features])[view[ib[wrong]]]
+    mj[wrong] = (rng.uniform(0, 1, int(wrong.sum())) * nb).astype(np.int64)
+    pairs = [(a, b) for a in range(V) for b in range(a + 1, min(a + int(span), V - 1) + 1)]
+    lo = np.searchsorted(key, [a * V + b for a, b in pairs])
+    hi = np.searchsorted(key, [a * V + b for a, b in pairs], side="right")
+    matches = [np.column_stack([local[ia[s:e]], mj[s:e]]).astype(np.int32) for s, e in zip(lo, hi)]
+    return MatchGraph(K=K, R=R, t=t, X=X, features=features, point=point,
+                      pairs=np.array(pairs, dtype=np.int32).reshape(-1, 2), matches=matches,
+                      wrong=[wrong[s:e] for s, e in zip(lo, hi)])
